@@ -7,16 +7,20 @@ independent Anymal fly-trot / Block-terrain problem instances
 own 4096 instances, no data-path collective).
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          # CUDA arm
+  python bench.py --dump-outputs DIR [...]                      # + the outputs of the last timed step as DIR/*.npy
   python bench.py --impl reference [...]                        # CPU restatement arm (oracle, all host cores)
   torchrun --nproc-per-node N bench.py --gpus N ...             # N > 1
 
 Prints ONE JSON line (rank 0).  See DESIGN.md §6 for how every field is measured.
+Writes nothing into the tree: the build lock lives in the temporary directory.
 """
 import argparse
+import hashlib
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -35,6 +39,7 @@ DESCR = {
 }
 METRIC = "nlp_evals_per_sec"
 UNIT = "evals/s"
+DUMP_BYTES = 48 << 20      # --dump-outputs: at most this many bytes of instances (g + jac + status, as float64)
 
 
 def read_peak():
@@ -306,6 +311,20 @@ def run_config5(args, tb, dev, world, rank, local):
                            "backend": "nccl" if world > 1 else "none (one rank: local copy)", "gathered_instances": gathered, "flagged": flagged}}
 
 
+def dump_outputs(out_dir, g, jac, status):
+    """Writes what the caller of twb_batch_eval_device received: g[k][m], jac[k][nnz] (CSR values) and status[k] (as float64)
+    of k instances.  k is the whole batch when it fits DUMP_BYTES, else a fixed, seeded sample of instances in ascending
+    order, so that two builds run with the same arguments can be compared output for output."""
+    import numpy as np
+    import torch
+    B = g.shape[0]
+    k = min(B, DUMP_BYTES // (8 * (g.shape[1] + jac.shape[1] + 1)))
+    idx = torch.from_numpy(np.sort(np.random.default_rng(0).choice(B, k, replace=False))).to(g.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("g", g), ("jac", jac), ("status", status)):
+        np.save(os.path.join(out_dir, f"{name}.npy"), t[idx].to(torch.float64).cpu().numpy())
+
+
 def run_cuda(args):
     import numpy as np
     import torch
@@ -368,6 +387,8 @@ def run_cuda(args):
     sync_all()
     total_ms = ev[0].elapsed_time(ev[-1])
     per_step = sorted(ev[i].elapsed_time(ev[i + 1]) for i in range(args.steps))
+    if args.dump_outputs and rank == 0:    # before the clock-sampling steps below overwrite g / jac
+        dump_outputs(args.dump_outputs, g, jac, status)
     if sampler:
         # the timed region lasts a few milliseconds; keep the same loop running ~1 s more so that nvidia-smi (one
         # sample per ~60 ms) sees the clocks under this load; these steps are not part of any reported number
@@ -506,15 +527,24 @@ def main():
     ap.add_argument("--quick", action="store_true", help="kernel timing only (tuning sweeps): skip e2e and the CPU arm")
     ap.add_argument("--workload", default=None, help="recipe name of towr_b200.configs (default: BASELINE configs[1])")
     ap.add_argument("--batch", type=int, default=0, help="instances per GPU (default 4096)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write g, jac and status of the last timed step as DIR/<name>.npy (float64; rank 0's "
+                         f"instances, a fixed seeded sample of them when the batch exceeds {DUMP_BYTES >> 20} MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs needs --impl cuda (the reference arm sizes its sample by time)")
     global WORKLOAD
     if args.workload:
         WORKLOAD = args.workload
     import fcntl
     import __graft_entry__ as ge
     # every rank builds under one file lock: the first one runs make, the others find everything up to date — nobody
-    # imports a half-written library (torchrun starts all ranks at once)
-    with open(os.path.join(ROOT, ".build.lock"), "w") as lock:
+    # imports a half-written library (torchrun starts all ranks at once).  The lock is per user and per tree, outside it.
+    lock_path = os.path.join(tempfile.gettempdir(),
+                             f"towr_b200-build-{os.getuid()}-{hashlib.sha1(ROOT.encode()).hexdigest()[:16]}.lock")
+    with open(lock_path, "w") as lock:
         fcntl.flock(lock, fcntl.LOCK_EX)
         ge.build(quiet=True, import_package=(args.impl != "reference"))
         fcntl.flock(lock, fcntl.LOCK_UN)
