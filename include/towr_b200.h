@@ -249,7 +249,8 @@ int twb_batch_initial_guess_host(twb_batch* b, const double* x, const double* ti
 /* fpowr::ExtractFootstepPlan (fpowr/include/fpowr/footstep_plan_extractor.h:55-133) for every instance, without the
  * nearest-plane lookup (boost::geometry over a ROS PlanarTerrain message: stays with the caller, who gets the contact
  * positions): the trajectory sampled every 0.01 s is scanned for changes of the contact set; the first state and every
- * change are footstep states.  Per footstep state n_values = 2 + 4 n_ee doubles: t_global | duration (to the next
+ * change are footstep states.  (One fused kernel: only the contact flags are walked and the feet's positions evaluated at
+ * the changes — bit-identical to sampling the trajectory and scanning it, without the sampled trajectory in memory.)  Per footstep state n_values = 2 + 4 n_ee doubles: t_global | duration (to the next
  * footstep state; the last one up to time_horizon) | per foot: contact flag 0/1, ee position (3).
  * max_states = 1 + sum over feet of (phases - 1) bounds the number of footstep states. */
 int twb_problem_footstep_plan_dims(const twb_problem* p, int* max_states, int* n_values);
@@ -266,6 +267,29 @@ int twb_batch_footstep_plan_host(twb_batch* b, const double* x, double time_hori
  * plan: host [B][max_states][2 + 4 n_ee]; n_states: host [B]; contact_set: host [B][max_states][n_ee]. */
 int twb_batch_nearest_planes_host(twb_batch* b, const double* plan, const int* n_states, const int* poly_offsets, int n_polys,
                                   const double* vertices, int* contact_set);
+
+/* Device-pointer variants of the four post-processing calls above: the same outputs in the same layouts, computed by the
+ * same kernels, for arrays that live on the batch's device (e.g. the iterates of a device-resident solver loop), so that
+ * only the results the caller asks for cross PCIe.  `stream` is a cudaStream_t (NULL = default stream).
+ *   x [B][n]; out as for the _host twin; n_states [B]; plan [B][max_states][2 + 4 n_ee]; contact_set [B][max_states][n_ee];
+ *   poly_offsets [n_polys + 1] and vertices [poly_offsets[n_polys]][2] are device arrays too; `times` stays a HOST array
+ *   [n_times] (it selects the sample tables).
+ * The footstep plan's rows past n_states[b] are written as 0 by the call (no memset needed).  The offsets cannot be checked
+ * on the host here: a polygon with a negative vertex count (poly_offsets[k + 1] < poly_offsets[k]) counts as empty and is
+ * never the nearest.  Errors: null required pointers, dt <= 0, n_times <= 0, n_polys < 0: TWB_ERR_INVALID; n_ee > 4 for
+ * initial guesses: TWB_ERR_UNSUPPORTED; a failed launch: TWB_ERR_CUDA.  Nothing is enqueued when a call fails its checks.
+ * A call only enqueues on `stream` (no host synchronisation, no device allocation) — except the FIRST call with a given
+ * table key (trajectory dt; footstep plan; the contents of `times`): it builds the sample tables on the host and uploads
+ * them with a blocking copy into a per-batch cache (8 keys, least recently used replaced, freed by twb_batch_destroy).
+ * After that first call the same call can be captured into a CUDA graph; the graph stays valid while its key is cached.
+ * Like twb_batch_eval_device these calls stage the iterates in the batch's shared transposed matrix: a batch serves ONE
+ * evaluation / post-processing call at a time, so a second call on another stream must be ordered after the first by the
+ * caller. */
+int twb_batch_sample_trajectory_device(twb_batch* b, const double* x, double dt, double* out, void* stream);
+int twb_batch_initial_guess_device(twb_batch* b, const double* x, const double* times, int n_times, double* out, void* stream);
+int twb_batch_footstep_plan_device(twb_batch* b, const double* x, double time_horizon, int* n_states, double* out, void* stream);
+int twb_batch_nearest_planes_device(twb_batch* b, const double* plan, const int* n_states, const int* poly_offsets, int n_polys,
+                                    const double* vertices, int* contact_set, void* stream);
 
 /* ---- the two ifopt components of towr that no Parameters::ConstraintName / CostName reaches ---------------------------
  * towr::LinearEqualityConstraint (towr/src/linear_constraint.cc:35-73) on variable set `var_set` (index of

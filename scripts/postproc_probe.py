@@ -1,5 +1,5 @@
 """Runs every kernel outside the per-iterate path once at B = 4096 (config 2 / config 4 recipes) so that an ncu launch list
-(--metrics gpu__time_duration.sum) shows their durations: TrajectoryKernel, InitialGuessKernel, FootstepKernel, NearestPlaneKernel,
+(--metrics gpu__time_duration.sum) shows their durations: TrajectoryKernel, InitialGuessKernel, FootstepPlanKernel, NearestPlaneKernel,
 GoalInstanceKernel, CostKernel, LinearEqualityKernel, SoftConstraintKernel, LmStepKernel.
     ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file out.csv python scripts/postproc_probe.py"""
 import os, sys
@@ -22,7 +22,7 @@ for name in ("anymal_trot_block", "hyq_gallop_gap"):
     bt.eval_host(X, flags=capi.EVAL_ALL)                       # CostKernel
     bt.sample_trajectory(X, 0.01)                              # TrajectoryKernel (201 samples)
     bt.initial_guesses(X, np.linspace(0.0, 2.0, 41))           # InitialGuessKernel
-    plan = bt.footstep_plans(X, 2.0)                           # TrajectoryKernel + FootstepKernel
+    plan = bt.footstep_plans(X, 2.0)                           # FootstepPlanKernel
     polys = [np.array([[-1.0, -1.0], [4.0, -1.0], [4.0, 1.0], [-1.0, 1.0], [-1.0, -1.0]]), np.array([[0.5, -0.5], [1.5, -0.5], [1.5, 0.5], [0.5, 0.5], [0.5, -0.5]])]
     bt.footstep_contact_sets(X, 2.0, polys)                    # NearestPlaneKernel
     goals = np.column_stack([np.full(B, 1.5), np.zeros(B), np.full(B, 0.5), np.zeros(B), np.zeros(B), np.zeros(B)])

@@ -56,6 +56,10 @@ def _load():
         "twb_problem_footstep_plan_dims": (C.c_int, [P, I, I]),
         "twb_batch_footstep_plan_host": (C.c_int, [P, P, C.c_double, P, P]),
         "twb_batch_nearest_planes_host": (C.c_int, [P, P, P, P, C.c_int, P, P]),
+        "twb_batch_sample_trajectory_device": (C.c_int, [P, P, C.c_double, P, P]),
+        "twb_batch_initial_guess_device": (C.c_int, [P, P, P, C.c_int, P, P]),
+        "twb_batch_footstep_plan_device": (C.c_int, [P, P, C.c_double, P, P, P]),
+        "twb_batch_nearest_planes_device": (C.c_int, [P, P, P, P, C.c_int, P, P, P]),
         "twb_batch_linear_equality_host": (C.c_int, [P, P, C.c_int, P, C.c_int, P]),
         "twb_batch_soft_constraint_host": (C.c_int, [P, C.c_int, P, P, P]),
         "twb_batch_launches_per_eval": (C.c_int, [P, C.c_uint]),

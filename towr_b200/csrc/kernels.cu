@@ -1767,34 +1767,83 @@ __global__ void __launch_bounds__(128) InitialGuessKernel(const Plan P, const do
 
 // fpowr::ExtractFootstepPlan (footstep_plan_extractor.h:68-133) without the nearest-plane lookup: the trajectory of
 // fpowr::GetTrajectory(dt) is scanned for changes of the contact set (HasEndEffectorContactChanged, :55-66); every change
-// (and the first state) is a footstep state.  Per footstep state 2 + 4 n_ee doubles: t_global | duration (time to the next
-// footstep state, the last one up to time_horizon) | per foot: contact flag, ee position.  One thread per instance.
-__global__ void __launch_bounds__(128) FootstepKernel(const double* __restrict__ traj, int n_steps, int n_ee, double dt, double time_horizon,
-                                                      int max_states, int* __restrict__ n_states, double* __restrict__ out, int nb) {
-  const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b >= nb) return;
-  const int K = 19 + 13 * n_ee, V = 2 + 4 * n_ee;
-  const double* tr = traj + (size_t)b * n_steps * K;
-  double* o = out + (size_t)b * max_states * V;
-  int count = 0; double t = 0.0;
-  for (int k = 0; k < n_steps; ++k, t += dt) {   // t accumulates like the reference's loop (t += dt)
-    const double* cur = tr + (size_t)k * K;
-    bool changed = (k == 0);
-    for (int e = 0; e < n_ee && !changed; ++e) changed = cur[19 + 13 * e] != cur[19 + 13 * e - K];
-    if (!changed) continue;
-    if (count > 0 && count <= max_states) o[(size_t)(count - 1) * V + 1] = t - o[(size_t)(count - 1) * V];
-    if (count < max_states) {
-      double* s = o + (size_t)count * V;
-      s[0] = t; s[1] = 0.0;
-      for (int e = 0; e < n_ee; ++e) {
-        s[2 + 4 * e] = cur[19 + 13 * e];
-        for (int d = 0; d < 3; ++d) s[3 + 4 * e + d] = cur[20 + 13 * e + d];
+// (and the first state) is a footstep state.  Per footstep state V = 2 + 4 n_ee doubles: t_global | duration (time to the
+// next footstep state, the last one up to time_horizon) | per foot: contact flag, ee position.
+// Fused: the trajectory is never materialised.  Only the contact flags are walked, step by step, and the feet's ee-motion
+// positions are evaluated at the change steps alone — from the same SplineSample entries, by the same EvalSpline position
+// term (independent of kWant), at the same times (times[k] = the table's t += dt), so every value is bit-identical to
+// sampling the trajectory and scanning it.  A change is coded (step << 4) | contact mask (bit e: foot e in contact).
+// Fixed durations: the flags are structure-class data, and the host's table holds the change codes (`codes`, n_codes of
+// them), the same for every instance.  Optimised durations: each lane walks the steps with its instance's durations and
+// the phase search of TrajectoryKernel (acc >= t - 1e-10 over the phases, last phase = T - sum), resumed from the previous
+// step's phase (the first phase that qualifies never moves back as t grows, so the result is the full search's), and
+// keeps its codes in shared memory.  Warp = tile of 32 instances, lane = instance; each state row goes out through
+// StoreRowsCoalesced; rows past the instance's count are written as 0.
+template <int kNEE, bool kPhase>
+__global__ void __launch_bounds__(128) FootstepPlanKernel(const Plan P, const double* __restrict__ XT, const SplineSample* __restrict__ samples,
+                                                          const double* __restrict__ times, const int* __restrict__ contact, const int* __restrict__ codes,
+                                                          int n_codes, int n_steps, double time_horizon, int max_states, int tiles, int* __restrict__ n_states,
+                                                          double* __restrict__ out, int nb) {
+  constexpr int V = 2 + 4 * kNEE;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, tile = blockIdx.x * 4 + warp, nc = P.nc_jac;
+  if (tile >= tiles || TileCount(nc, tile, nb) == 0) return;   // whole warps
+  const ConstCol xs = TileCol(XT, tile, lane, P.n + 1);
+  extern __shared__ __align__(16) double fp_smem[];
+  double* stage = fp_smem + (size_t)warp * V * 33;
+  int* my_codes = reinterpret_cast<int*>(fp_smem + 4 * V * 33) + (size_t)warp * (max_states + 1) * 32 + lane;   // [max_states + 1][32]
+  int count = n_codes;
+  if (kPhase) {
+    int ph[kNEE], n_ph[kNEE], s0[kNEE]; double acc[kNEE], last[kNEE]; bool first[kNEE];
+#pragma unroll
+    for (int e = 0; e < kNEE; ++e) {
+      const PhaseSplineDef def = P.phase_defs[2 * e];
+      n_ph[e] = def.n_phases; s0[e] = def.sched0;
+      double sum = 0.0;
+      for (int i = 0; i + 1 < def.n_phases; ++i) sum += xs[def.sched0 + i];
+      last[e] = def.t_total - sum;
+      ph[e] = 0; acc[e] = 0.0 + (def.n_phases == 1 ? last[e] : xs[def.sched0]);   // acc = 0, acc += first duration
+      first[e] = __ldg(contact + e) != 0;
+    }
+    count = 0;
+    unsigned prev = 0;
+    for (int k = 0; k < n_steps; ++k) {
+      const double thr = __ldg(times + k) - 1e-10;
+      unsigned mask = 0;
+#pragma unroll
+      for (int e = 0; e < kNEE; ++e) {
+        while (ph[e] < n_ph[e] - 1 && !(acc[e] >= thr)) { ++ph[e]; acc[e] += (ph[e] == n_ph[e] - 1) ? last[e] : xs[s0[e] + ph[e]]; }
+        if ((ph[e] % 2 == 0) ? first[e] : !first[e]) mask |= 1u << e;
+      }
+      if (k == 0 || mask != prev) {
+        if (count <= max_states) my_codes[(size_t)count * 32] = (k << 4) | (int)mask;
+        ++count;
+      }
+      prev = mask;
+    }
+  }
+  const int b = TileInstance(nc, tile, lane);
+  if (b < nb) n_states[b] = count;
+  for (int i = 0; i < max_states; ++i) {
+    double o[V];
+#pragma unroll
+    for (int v = 0; v < V; ++v) o[v] = 0.0;
+    if (i < count) {
+      const int code = kPhase ? my_codes[(size_t)i * 32] : __ldg(codes + i), k = code >> 4;
+      const double t = __ldg(times + k);
+      o[0] = t;
+      if (i + 1 < count) o[1] = __ldg(times + ((kPhase ? my_codes[(size_t)(i + 1) * 32] : __ldg(codes + i + 1)) >> 4)) - t;
+      else o[1] = time_horizon - t;
+      const SplineSample* sp = samples + (size_t)k * (2 + 2 * kNEE);
+#pragma unroll
+      for (int e = 0; e < kNEE; ++e) {
+        double unused[3];
+        o[2 + 4 * e] = ((code >> e) & 1) ? 1.0 : 0.0;
+        EvalSpline<0, kPhase>(P, sp + 2 + e, xs, o + 3 + 4 * e, unused, unused);
       }
     }
-    ++count;
+    StoreRowsCoalesced<V>(o, stage, out, (size_t)max_states * V, (size_t)i * V, nc, tile, nb, lane);
+    __syncwarp();   // the stage is rewritten by the next state
   }
-  if (count > 0 && count <= max_states) o[(size_t)(count - 1) * V + 1] = time_horizon - o[(size_t)(count - 1) * V];
-  n_states[b] = count;
 }
 
 // ---- fpowr::NearestPlaneLookup::GetNearestPlaneIndex (fpowr/include/fpowr/nearest_plane_lookup.h:62-84) ----------------
@@ -1830,7 +1879,7 @@ __device__ __forceinline__ double PolygonDistance(const double* __restrict__ v, 
   if (touches || winding != 0) return 0.0;
   return sqrt(best);
 }
-// thread = (instance, footstep state, foot) of a footstep plan (FootstepKernel's layout): index of the nearest polygon for a
+// thread = (instance, footstep state, foot) of a footstep plan ([b][state][2 + 4 n_ee]): index of the nearest polygon for a
 // foot in contact, -1 for a foot in the air (footstep_plan_extractor.h:106-116) and for unused states
 __global__ void __launch_bounds__(128) NearestPlaneKernel(const double* __restrict__ plan, const int* __restrict__ n_states, int max_states, int n_ee,
                                                           const int* __restrict__ poly_offset, int n_polys, const double* __restrict__ verts,
@@ -2106,10 +2155,28 @@ int LaunchInitialGuess(const Plan& P, const double* x, double* XT, const SplineS
   return (int)cudaGetLastError();
 }
 
-int LaunchFootstepScan(const double* traj, int n_steps, int n_ee, double dt, double time_horizon, int max_states, int* n_states,
-                       double* out, int nb, cudaStream_t s) {
-  if (nb <= 0) return 0;
-  FootstepKernel<<<(nb + 127) / 128, 128, 0, s>>>(traj, n_steps, n_ee, dt, time_horizon, max_states, n_states, out, nb);
+int LaunchFootstepPlan(const Plan& P, const double* x, double* XT, const SplineSample* samples, const double* times, const int* contact,
+                       const int* codes, int n_codes, int n_steps, double time_horizon, int max_states, int* n_states, double* out, int nb,
+                       cudaStream_t s) {
+  if (nb <= 0 || max_states <= 0) return 0;
+  const int tiles = TileTotal(P.nc_jac, nb);
+  TransposeIn<<<dim3((P.n + 32 * kTinTiles - 1) / (32 * kTinTiles), tiles), dim3(32, 8), 0, s>>>(x, XT, nullptr, P.n, nb, P.nc_jac);
+  const bool phase = P.n_phase_defs > 0;
+  // dynamic shared memory per warp: the staging tile [V][33] of the coalesced stores; optimised durations: the change codes [max_states + 1][32]
+#define TWB_FSP(NEE) { const size_t sm = 4 * ((size_t)(2 + 4 * NEE) * 33 * sizeof(double) + (phase ? (size_t)(max_states + 1) * 32 * sizeof(int) : 0)); \
+    if (phase) { cudaFuncSetAttribute(FootstepPlanKernel<NEE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);                           \
+                 FootstepPlanKernel<NEE, true><<<(tiles + 3) / 4, 128, sm, s>>>(P, XT, samples, times, contact, codes, n_codes, n_steps,            \
+                                                                                 time_horizon, max_states, tiles, n_states, out, nb); }             \
+    else { cudaFuncSetAttribute(FootstepPlanKernel<NEE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);                                \
+           FootstepPlanKernel<NEE, false><<<(tiles + 3) / 4, 128, sm, s>>>(P, XT, samples, times, contact, codes, n_codes, n_steps,                  \
+                                                                            time_horizon, max_states, tiles, n_states, out, nb); } }
+  switch (P.n_ee) {
+    case 1: TWB_FSP(1); break;
+    case 2: TWB_FSP(2); break;
+    case 4: TWB_FSP(4); break;
+    default: return (int)cudaErrorInvalidValue;
+  }
+#undef TWB_FSP
   return (int)cudaGetLastError();
 }
 

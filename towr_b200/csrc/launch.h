@@ -25,10 +25,13 @@ int LaunchTrajectory(const Plan& P, const double* x, double* XT, const SplineSam
 // fpowr::ExtractInitialGuess at `n_times` caller-given times: x -> XT, then out[b][time][49]; `samples` as for the trajectory
 int LaunchInitialGuess(const Plan& P, const double* x, double* XT, const SplineSample* samples, const double* times, int n_times,
                        double* out, int nb, cudaStream_t s);
-// contact-change scan of a sampled trajectory (fpowr::ExtractFootstepPlan): traj[b][n_steps][19 + 13 n_ee] ->
-// out[b][max_states][2 + 4 n_ee], n_states[b]
-int LaunchFootstepScan(const double* traj, int n_steps, int n_ee, double dt, double time_horizon, int max_states, int* n_states,
-                       double* out, int nb, cudaStream_t s);
+// fpowr::ExtractFootstepPlan without the nearest-plane lookup, fused (no sampled trajectory): x -> XT, then
+// out[b][max_states][2 + 4 n_ee] (rows past n_states[b] written as 0) and n_states[b].  samples / times: the tables of
+// Formulation::TrajectoryTables(0.01); fixed durations: codes[n_codes] = (step << 4) | contact mask of the first step and of
+// every change of the contact set, contact unused; optimised durations: contact = in_contact_at_start per foot, codes unused
+int LaunchFootstepPlan(const Plan& P, const double* x, double* XT, const SplineSample* samples, const double* times, const int* contact,
+                       const int* codes, int n_codes, int n_steps, double time_horizon, int max_states, int* n_states, double* out, int nb,
+                       cudaStream_t s);
 // fpowr::NearestPlaneLookup for every (instance, footstep state, foot) of a footstep plan: out[b][state][foot] = index of
 // the nearest polygon (polygon k = vertices poly_offset[k] .. poly_offset[k+1]-1 of verts[][2]) or -1 (foot in the air)
 int LaunchNearestPlanes(const double* plan, const int* n_states, int max_states, int n_ee, const int* poly_offset, int n_polys,

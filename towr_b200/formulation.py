@@ -253,6 +253,25 @@ class Problem:
         return Batch(self, batch_size, device)
 
 
+def pack_polygons(polygons):
+    """A list of (k_i, 2) vertex arrays (world x, y of the planar regions' boundaries) as the C ABI takes them:
+    (poly_offsets int32 (n_polys + 1,), vertices float64 (total, 2)); polygon k owns vertices[offs[k]:offs[k + 1]]."""
+    offs = np.zeros(len(polygons) + 1, np.int32)
+    offs[1:] = np.cumsum([len(q) for q in polygons])
+    verts = np.ascontiguousarray(np.concatenate([np.asarray(q, np.float64).reshape(-1, 2) for q in polygons]) if polygons else np.zeros((0, 2)))
+    return offs, verts
+
+
+def _stream_ptr(stream, tensor):
+    import torch
+    return C.c_void_p((torch.cuda.current_stream(tensor.device) if stream is None else stream).cuda_stream)
+
+
+def _check_tensor(t, dtype, shape, what):
+    assert t.is_cuda and t.dtype == dtype and t.is_contiguous() and tuple(t.shape) == tuple(shape), \
+        f"{what}: expected a contiguous CUDA {dtype} tensor of shape {tuple(shape)}"
+
+
 class Batch:
     """B instances of one Problem resident on one GPU."""
 
@@ -318,14 +337,85 @@ class Batch:
         count = np.empty(self.B, np.int32)
         check(lib.twb_batch_footstep_plan_host(self._h, x.ctypes.data_as(C.c_void_p), float(time_horizon),
                                                count.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p)))
-        offs = np.zeros(len(polygons) + 1, np.int32)
-        offs[1:] = np.cumsum([len(q) for q in polygons])
-        verts = np.ascontiguousarray(np.concatenate([np.asarray(q, np.float64).reshape(-1, 2) for q in polygons]) if polygons else np.zeros((0, 2)))
+        offs, verts = pack_polygons(polygons)
         cs = np.empty((self.B, ms.value, n_ee), np.int32)
         check(lib.twb_batch_nearest_planes_host(self._h, out.ctypes.data_as(C.c_void_p), count.ctypes.data_as(C.c_void_p),
                                                 offs.ctypes.data_as(C.c_void_p), len(polygons), verts.ctypes.data_as(C.c_void_p),
                                                 cs.ctypes.data_as(C.c_void_p)))
         return [out[b, :count[b]] for b in range(self.B)], [cs[b, :count[b]] for b in range(self.B)]
+
+    # ---- device-pointer variants: torch CUDA tensors in and out, only enqueued on `stream` (default: the current one) ----
+    # The first call with a given dt / sample-time list builds and uploads the sample tables (blocking); the later ones can
+    # be captured in a CUDA graph.
+
+    def sample_trajectory_device(self, x, dt, out=None, stream=None):
+        """sample_trajectory on the device: x (B, n) CUDA float64 -> (B, n_samples, 19 + 13 n_ee) CUDA float64."""
+        import torch
+        p = self.problem
+        _check_tensor(x, torch.float64, (self.B, p.n), "x")
+        ns, nv = C.c_int(), C.c_int()
+        check(lib.twb_problem_trajectory_dims(p._h, float(dt), C.byref(ns), C.byref(nv)))
+        if out is None:
+            out = torch.empty((self.B, ns.value, nv.value), dtype=torch.float64, device=x.device)
+        _check_tensor(out, torch.float64, (self.B, ns.value, nv.value), "out")
+        check(lib.twb_batch_sample_trajectory_device(self._h, C.c_void_p(x.data_ptr()), float(dt), C.c_void_p(out.data_ptr()),
+                                                     _stream_ptr(stream, x)))
+        return out
+
+    def initial_guesses_device(self, x, times, out=None, stream=None):
+        """initial_guesses on the device: x (B, n) CUDA float64, times a host sequence -> (B, n_times, 49) CUDA float64."""
+        import torch
+        p = self.problem
+        _check_tensor(x, torch.float64, (self.B, p.n), "x")
+        times = np.ascontiguousarray(times, np.float64)
+        if out is None:
+            out = torch.empty((self.B, times.size, 49), dtype=torch.float64, device=x.device)
+        _check_tensor(out, torch.float64, (self.B, times.size, 49), "out")
+        check(lib.twb_batch_initial_guess_device(self._h, C.c_void_p(x.data_ptr()), times.ctypes.data_as(C.c_void_p), int(times.size),
+                                                 C.c_void_p(out.data_ptr()), _stream_ptr(stream, x)))
+        return out
+
+    def footstep_plan_dims(self):
+        ms, nv = C.c_int(), C.c_int()
+        check(lib.twb_problem_footstep_plan_dims(self.problem._h, C.byref(ms), C.byref(nv)))
+        return ms.value, nv.value
+
+    def footstep_plans_device(self, x, time_horizon, out=None, stream=None):
+        """footstep_plans on the device: x (B, n) CUDA float64 -> (plans (B, max_states, 2 + 4 n_ee) CUDA float64, rows past
+        n_states[b] are 0; n_states (B,) CUDA int32).  `out`: an optional (plans, n_states) pair to write into."""
+        import torch
+        p = self.problem
+        _check_tensor(x, torch.float64, (self.B, p.n), "x")
+        ms, nv = self.footstep_plan_dims()
+        if out is None:
+            out = (torch.empty((self.B, ms, nv), dtype=torch.float64, device=x.device), torch.empty(self.B, dtype=torch.int32, device=x.device))
+        plans, count = out
+        _check_tensor(plans, torch.float64, (self.B, ms, nv), "plans")
+        _check_tensor(count, torch.int32, (self.B,), "n_states")
+        check(lib.twb_batch_footstep_plan_device(self._h, C.c_void_p(x.data_ptr()), float(time_horizon), C.c_void_p(count.data_ptr()),
+                                                 C.c_void_p(plans.data_ptr()), _stream_ptr(stream, x)))
+        return plans, count
+
+    def nearest_planes_device(self, plans, n_states, poly_offsets, vertices, out=None, stream=None):
+        """The nearest-plane lookup of footstep_contact_sets on the device: plans / n_states as footstep_plans_device returns
+        them, poly_offsets (n_polys + 1,) CUDA int32 and vertices (total, 2) CUDA float64 (pack_polygons, then moved to the
+        device) -> contact sets (B, max_states, n_ee) CUDA int32: polygon index under every foot in contact, -1 in the air
+        and for unused states.  Offsets must ascend: a polygon with a negative vertex count is treated as empty."""
+        import torch
+        ms, nv = self.footstep_plan_dims()
+        n_ee = (nv - 2) // 4
+        _check_tensor(plans, torch.float64, (self.B, ms, nv), "plans")
+        _check_tensor(n_states, torch.int32, (self.B,), "n_states")
+        assert poly_offsets.ndim == 1 and poly_offsets.numel() >= 1, "poly_offsets: (n_polys + 1,)"
+        _check_tensor(poly_offsets, torch.int32, (poly_offsets.numel(),), "poly_offsets")
+        _check_tensor(vertices, torch.float64, (vertices.shape[0], 2), "vertices")
+        if out is None:
+            out = torch.empty((self.B, ms, n_ee), dtype=torch.int32, device=plans.device)
+        _check_tensor(out, torch.int32, (self.B, ms, n_ee), "out")
+        check(lib.twb_batch_nearest_planes_device(self._h, C.c_void_p(plans.data_ptr()), C.c_void_p(n_states.data_ptr()),
+                                                  C.c_void_p(poly_offsets.data_ptr()), poly_offsets.numel() - 1,
+                                                  C.c_void_p(vertices.data_ptr()), C.c_void_p(out.data_ptr()), _stream_ptr(stream, plans)))
+        return out
 
     def linear_equality(self, x, var_set, M):
         """towr::LinearEqualityConstraint::GetValues for every instance: (B, rows) = M x_set; var_set is a set name."""
