@@ -158,6 +158,24 @@ int twb_problem_x0(const twb_problem* p, double* x0);
 int twb_problem_goal_instances(const twb_problem* p, int n_goals, const double* goals, double* x0, double* x_lower,
                                double* x_upper);
 
+/* Per-instance start AND goal states: one fixed-stride record per instance that mirrors NlpFormulation's three state fields
+ * (towr/include/towr/nlp_formulation.h:100-105), with the meaning they have in twb_spec. */
+#define TWB_STATE_DOUBLES 36
+/* per instance, in this order:
+ *   initial_base_: lin p[3], lin v[3], ang p[3] (Euler, as twb_spec), ang v[3]      doubles  0..11
+ *   final_base_:   lin p[3], lin v[3], ang p[3], ang v[3]                            doubles 12..23
+ *   initial_ee_W_: [TWB_MAX_EE][3]; feet beyond n_ee are ignored                     doubles 24..35
+ * The final base z only enters the final-position bound (bounds_final_lin_pos); the initial guess ends at the terrain height
+ * minus the nominal z, as for the spec.  The final velocities only enter the bounds bounds_final_*_vel selects.  The initial
+ * feet are taken as given (not projected onto the terrain). */
+/* Initial guess, variable bounds AND constraint bounds of n_states such instances of one structure class.  states: host
+ * [n_states][TWB_STATE_DOUBLES]; x0 / x_lower / x_upper: [n_states][n]; g_lower / g_upper: [n_states][m]; any output may be
+ * NULL.  The constraint bounds are twb_problem_bounds' except the BaseMotionConstraint (TWB_C_BASE_ROM) LZ rows, which are
+ * [z_init - 0.02, z_init + 0.1] around the instance's initial base z (base_motion_constraint.cc:51-54); without
+ * TWB_C_BASE_ROM every instance has the problem's constraint bounds.  Errors: NULL states, n_states <= 0: TWB_ERR_INVALID. */
+int twb_problem_state_instances(const twb_problem* p, int n_states, const double* states, double* x0, double* x_lower,
+                                double* x_upper, double* g_lower, double* g_upper);
+
 /* Component layout: variable sets (column ranges) and constraint sets (row
  * ranges) in ifopt's Add*Set order; names are the reference's
  * ("base-lin", "ee-motion_0", "dynamic", "rangeofmotion-1", ...). */
@@ -193,6 +211,17 @@ int twb_batch_set_grid_map(twb_batch* b, const float* heights, int size_x, int s
  * [B][6]; x0 / x_lower / x_upper: device [B][n] (any may be NULL).  The terrain under each goal is the INSTANCE's terrain
  * (twb_batch_set_terrains, height grids included; else twb_spec.terrain).  The call only enqueues on `stream`. */
 int twb_batch_goal_instances_device(twb_batch* b, const double* goals, double* x0, double* x_lower, double* x_upper, void* stream);
+
+/* Batched setup on the device: twb_problem_state_instances for the B instances of the batch, so that a device-resident
+ * pipeline can start every instance from its own measured state.  states: device [B][TWB_STATE_DOUBLES]; x0 / x_lower /
+ * x_upper: device [B][n]; g_lower / g_upper: device [B][m]; any output may be NULL, but not all of them.  The terrain under
+ * each goal is the instance's own, as for twb_batch_goal_instances_device.  The call only enqueues on `stream` (no host
+ * synchronisation, no allocation), so it can be captured in a CUDA graph.  Errors: NULL states, every output NULL:
+ * TWB_ERR_INVALID, nothing enqueued.
+ * twb_batch_lm_step_device keeps using the problem's own constraint bounds: only the BaseMotionConstraint LZ rows differ per
+ * instance, and only when TWB_C_BASE_ROM is among the constraints (the default list has no such rows). */
+int twb_batch_state_instances_device(twb_batch* b, const double* states, double* x0, double* x_lower, double* x_upper,
+                                     double* g_lower, double* g_upper, void* stream);
 
 #define TWB_EVAL_G 1u     /* constraint values        (Problem::EvaluateConstraints)       */
 #define TWB_EVAL_JAC 2u   /* Jacobian values          (Problem::EvalNonzerosOfJacobian)    */

@@ -47,6 +47,8 @@ def _load():
         "twb_batch_set_grid_terrain": (C.c_int, [P, D, C.c_int, C.c_int]),
         "twb_batch_set_grid_map": (C.c_int, [P, C.POINTER(C.c_float), C.c_int, C.c_int, C.c_double, C.c_double, C.c_double]),
         "twb_batch_goal_instances_device": (C.c_int, [P, P, P, P, P, P]),
+        "twb_problem_state_instances": (C.c_int, [P, C.c_int, D, D, D, D, D, D]),
+        "twb_batch_state_instances_device": (C.c_int, [P, P, P, P, P, P, P, P]),
         "twb_batch_eval_device": (C.c_int, [P, P, P, P, P, P, P, C.c_uint, P]),
         "twb_batch_eval_host": (C.c_int, [P, P, P, P, P, P, P, C.c_uint]),
         "twb_batch_lm_step_device": (C.c_int, [P, P, P, P, P, P, C.c_double, C.c_double, C.c_int, P, P]),

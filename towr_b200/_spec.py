@@ -3,6 +3,7 @@ load libtowr_b200.so (bench.py's reference arm and the fixture scripts load it b
 import ctypes as C
 
 MAX_EE, MAX_PHASES, MAX_CONSTRAINTS, MAX_COSTS = 4, 32, 16, 8
+STATE_DOUBLES = 36   # TWB_STATE_DOUBLES: per-instance state record (formulation.pack_states)
 
 OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_NO_DEVICE = 0, 1, 2, 3, 4
 EVAL_G, EVAL_JAC, EVAL_COST, EVAL_ALL = 1, 2, 4, 7

@@ -59,6 +59,8 @@ cudaError_t Upload(const std::vector<T>& h, const T** d, std::vector<void*>* own
 }
 }  // namespace
 
+static_assert(TWB_STATE_DOUBLES == twb::kStateDoubles && twb::kStInitEE + 3 * TWB_MAX_EE == TWB_STATE_DOUBLES, "state record layout");
+
 struct twb_problem {
   twb::Formulation f;
 };
@@ -296,6 +298,17 @@ int twb_problem_goal_instances(const twb_problem* p, int n_goals, const double* 
   }
   return TWB_OK;
 }
+int twb_problem_state_instances(const twb_problem* p, int n_states, const double* states, double* x0, double* xl, double* xu, double* gl,
+                                double* gu) {
+  if (!p || !states || n_states <= 0) return Fail(TWB_ERR_INVALID, "bad argument");
+  const size_t n = (size_t)p->f.n, m = (size_t)p->f.m;
+  for (int i = 0; i < n_states; ++i) {
+    int rc = p->f.StateInstance(states + (size_t)TWB_STATE_DOUBLES * i, x0 ? x0 + i * n : nullptr, xl ? xl + i * n : nullptr,
+                                xu ? xu + i * n : nullptr, gl ? gl + i * m : nullptr, gu ? gu + i * m : nullptr);
+    if (rc != TWB_OK) return Fail(rc, "state instance");
+  }
+  return TWB_OK;
+}
 int twb_layout_num_variable_sets(const twb_problem* p) { return p ? (int)p->f.var_sets.size() : 0; }
 int twb_layout_num_constraint_sets(const twb_problem* p) { return p ? (int)p->f.con_sets.size() : 0; }
 static int CopyComponent(const std::vector<twb::Component>& v, int i, char* name, int cap, int* start, int* count) {
@@ -336,7 +349,12 @@ int twb_batch_create(const twb_problem* p, int batch_size, int device, twb_batch
   TWB_UP(samples) TWB_UP(dyn) TWB_UP(rom) TWB_UP(groups) TWB_UP(terr) TWB_UP(force) TWB_UP(swing) TWB_UP(acc)
   TWB_UP(base_motion) TWB_UP(cost) TWB_UP(pairs) TWB_UP(coefs) TWB_UP(cta_lists) TWB_UP(dyn_ang_basis)
   TWB_UP(phase_defs) TWB_UP(phase_polys) TWB_UP(phase_units) TWB_UP(exts) TWB_UP(goal_vars) TWB_UP(const_runs) TWB_UP(const_vals)
+  TWB_UP(state_vars) TWB_UP(base_z_rows)
 #undef TWB_UP
+  if ((e = Upload(p->f.g_lower, &b->plan.g_lower, &b->owned)) != cudaSuccess || (e = Upload(p->f.g_upper, &b->plan.g_upper, &b->owned)) != cudaSuccess) {
+    twb_batch_destroy(b);
+    return CudaFail(e, "table upload");
+  }
   if (std::getenv("TWB_PROFILE") && !g_prof_on) { g_prof_on = true; twb::g_after_launch = ProfHook; std::atexit(ProfReport); }
   if (g_prof_on) std::fprintf(stderr, "[twb profile] n=%d m=%d nnz=%d\n", b->plan.n, b->plan.m, b->plan.nnz);
   if (const char* v = std::getenv("TWB_E2E_CHUNK")) b->e2e_chunk = std::max(32, std::atoi(v));
@@ -471,6 +489,19 @@ int twb_batch_goal_instances_device(twb_batch* b, const double* goals, double* x
   const twb::Formulation& f = b->prob->f;
   int rc = twb::LaunchGoalInstances(b->plan, f.tables.goal_setup, goals, b->d_terrain, f.spec.terrain, x0, x_lower, x_upper, b->B, static_cast<cudaStream_t>(stream));
   if (rc != 0) return CudaFail(static_cast<cudaError_t>(rc), "goal-instance kernel launch");
+  return TWB_OK;
+}
+
+int twb_batch_state_instances_device(twb_batch* b, const double* states, double* x0, double* x_lower, double* x_upper, double* g_lower,
+                                     double* g_upper, void* stream) {
+  if (!b || !states) return Fail(TWB_ERR_INVALID, "null argument");
+  if (!x0 && !x_lower && !x_upper && !g_lower && !g_upper) return Fail(TWB_ERR_INVALID, "no output requested");
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  const twb::Formulation& f = b->prob->f;
+  int rc = twb::LaunchStateInstances(b->plan, f.tables.goal_setup, states, b->d_terrain, f.spec.terrain, x0, x_lower, x_upper, g_lower, g_upper, b->B,
+                                     static_cast<cudaStream_t>(stream));
+  if (rc != 0) return CudaFail(static_cast<cudaError_t>(rc), "state-instance kernel launch");
   return TWB_OK;
 }
 

@@ -224,11 +224,14 @@ struct CostEntry {
 // with (a, b) = (initial, final) of the variable's set: base-lin (final z = terrain height - nominal z), base-ang, ee-motion_e
 // (final = goal base + yaw-rotated nominal stance, z on the terrain), ee-force_e (a = b = (0, 0, m g / n_ee)); ee-schedule
 // variables are constants.  Bounds: free, a constant on both sides, the goal's own base position / angle, or a constant pair.
-enum GoalBound : int8_t { kBoundFree = 0, kBoundConst = 1, kBoundGoalLin = 2, kBoundGoalAng = 3, kBoundPair = 4 };
+// The start-state recipe (Plan::state_vars, StateInstanceKernel) is the same recipe with the endpoints taken from a per-instance
+// state record (TWB_STATE_DOUBLES, layout below) and every bound that copies a spec field turned into kBoundState: both sides
+// = record[src].  Only the state recipe holds kBoundState; goal_vars keeps the four goal-recipe modes.
+enum GoalBound : int8_t { kBoundFree = 0, kBoundConst = 1, kBoundGoalLin = 2, kBoundGoalAng = 3, kBoundPair = 4, kBoundState = 5 };
 enum GoalKind : int8_t { kGoalLin = 0, kGoalAng = 1, kGoalMotion = 2, kGoalForce = 3, kGoalConst = 4 };
 struct GoalVar {
   int8_t kind, ee, deriv, dim;   // GoalKind, foot (motion / force), 0 position / 1 velocity, dimension
-  int8_t bound, pad[3];          // GoalBound
+  int8_t bound, src, pad[2];     // GoalBound; kBoundState: index into the state record
   double frac;                   // node fraction (positions); constant x0 (kGoalConst)
   double c0, c1;                 // bound constants
 };
@@ -236,6 +239,10 @@ struct GoalSetup {                // goal-independent inputs of the recipe (twb_
   double initial_lin[3], initial_ang[3], initial_ee[kMaxEE][3], nominal[kMaxEE][3];
   double t_total, f_stance_z;
 };
+// per-instance state record (include/towr_b200.h: TWB_STATE_DOUBLES): offsets of NlpFormulation's three state fields
+constexpr int kStateDoubles = 36;
+enum StateField : int8_t { kStInitLinPos = 0, kStInitLinVel = 3, kStInitAngPos = 6, kStInitAngVel = 9, kStFinalLinPos = 12, kStFinalLinVel = 15,
+                           kStFinalAngPos = 18, kStFinalAngVel = 21, kStInitEE = 24 };
 
 struct Plan {
   int n, m, nnz, n_ee;
@@ -274,6 +281,11 @@ struct Plan {
   int gmap_sx, gmap_sy;
   double gmap_res, gmap_px, gmap_py;
   const GoalVar* goal_vars;             // [n] recipe of x0 / bounds per variable
+  const GoalVar* state_vars;            // [n] the same recipe for per-instance start states (bounds from the state record)
+  const double* g_lower;                // [m] the problem's constraint bounds (per-instance setup copies them)
+  const double* g_upper;
+  const int32_t* base_z_rows;           // BaseMotionConstraint LZ rows, bounds [z_init - 0.02, z_init + 0.1] (none without TWB_C_BASE_ROM)
+  int n_base_z_rows;
   int n_const_runs;                     // constant runs (TMA-written; fixed durations, row length a multiple of 4)
   const ConstRun* const_runs;
   const double* const_vals;

@@ -319,6 +319,31 @@ int Formulation::GoalInstance(const double final_lin_pos[3], const double final_
   return TWB_OK;
 }
 
+// x0, variable bounds and constraint bounds of an instance whose NlpFormulation::initial_base_, final_base_ and initial_ee_W_
+// are the state record `st` (TWB_STATE_DOUBLES): the constraint bounds are the problem's except the BaseMotionConstraint LZ
+// rows, whose z_init is the instance's own initial guess of base-lin node 0 (base_motion_constraint.cc:51-54)
+int Formulation::StateInstance(const double* st, double* x0_out, double* lo_out, double* up_out, double* gl_out, double* gu_out) const {
+  if (!holder || !st) return TWB_ERR_INVALID;
+  twb_spec sp = spec;
+  for (int k = 0; k < 3; ++k) {
+    sp.initial_base_lin_pos[k] = st[kStInitLinPos + k]; sp.initial_base_lin_vel[k] = st[kStInitLinVel + k];
+    sp.initial_base_ang_pos[k] = st[kStInitAngPos + k]; sp.initial_base_ang_vel[k] = st[kStInitAngVel + k];
+    sp.final_base_lin_pos[k] = st[kStFinalLinPos + k]; sp.final_base_lin_vel[k] = st[kStFinalLinVel + k];
+    sp.final_base_ang_pos[k] = st[kStFinalAngPos + k]; sp.final_base_ang_vel[k] = st[kStFinalAngVel + k];
+  }
+  for (int e = 0; e < spec.n_ee; ++e) for (int k = 0; k < 3; ++k) sp.initial_ee_W[e][k] = st[kStInitEE + 3 * e + k];
+  std::vector<NodeSet> sets = holder->sets;
+  std::vector<double> a, b, c;
+  InitialGuessAndBounds(sp, holder->robot, holder->T, optimize_timings, &sets, &a, &b, &c);
+  if (x0_out) std::copy(a.begin(), a.end(), x0_out);
+  if (lo_out) std::copy(b.begin(), b.end(), lo_out);
+  if (up_out) std::copy(c.begin(), c.end(), up_out);
+  const double z_init = sets[0].x0[sets[0].Var(0, kPos, Z)];
+  if (gl_out) { std::copy(g_lower.begin(), g_lower.end(), gl_out); for (int r : tables.base_z_rows) gl_out[r] = z_init - 0.02; }
+  if (gu_out) { std::copy(g_upper.begin(), g_upper.end(), gu_out); for (int r : tables.base_z_rows) gu_out[r] = z_init + 0.1; }
+  return TWB_OK;
+}
+
 int Formulation::Build(const twb_spec& sp, std::string* err) {
   auto fail = [&](int code, const char* why) { if (err) *err = why; return code; };
   spec = sp;
@@ -427,6 +452,22 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
           GoalVar& g = gv[sched0[e] + i];
           g.kind = kGoalConst; g.frac = sp.phase_durations[e][i]; g.bound = kBoundPair; g.c0 = sp.bound_phase_duration_min; g.c1 = sp.bound_phase_duration_max;
         }
+    // the start-state recipe: every bound above that copies a twb_spec state field reads the instance's state record instead
+    // (the same Fix calls in the same order, so that a later Fix of the same variable still wins)
+    std::vector<GoalVar>& sv = tables.state_vars; sv = gv;
+    auto fix_state = [&](const NodeSet& ns, int node, int deriv, int dim, int src) {
+      const int v = ns.Var(node, deriv, dim);
+      if (v >= 0) { GoalVar& g = sv[ns.offset + v]; g.bound = kBoundState; g.src = (int8_t)src; g.c0 = g.c1 = 0.0; }
+    };
+    for (int d = 0; d < 3; ++d) {
+      fix_state(lin, 0, kPos, d, kStInitLinPos + d); fix_state(lin, 0, kVel, d, kStInitLinVel + d);
+      fix_state(ang, 0, kPos, d, kStInitAngPos + d); fix_state(ang, 0, kVel, d, kStInitAngVel + d);
+      if (sp.bounds_final_lin_pos[d]) fix_state(lin, last, kPos, d, kStFinalLinPos + d);
+      if (sp.bounds_final_lin_vel[d]) fix_state(lin, last, kVel, d, kStFinalLinVel + d);
+      if (sp.bounds_final_ang_pos[d]) fix_state(ang, last, kPos, d, kStFinalAngPos + d);
+      if (sp.bounds_final_ang_vel[d]) fix_state(ang, last, kVel, d, kStFinalAngVel + d);
+      for (int e = 0; e < n_ee; ++e) fix_state(motion(e), 0, kPos, d, kStInitEE + 3 * e + d);
+    }
     GoalSetup& gs = tables.goal_setup; gs = GoalSetup{};
     for (int d = 0; d < 3; ++d) { gs.initial_lin[d] = sp.initial_base_lin_pos[d]; gs.initial_ang[d] = sp.initial_base_ang_pos[d]; }
     for (int e = 0; e < n_ee; ++e) for (int d = 0; d < 3; ++d) { gs.initial_ee[e][d] = sp.initial_ee_W[e][d]; gs.nominal[e][d] = rb.nominal[e][d]; }
@@ -668,6 +709,7 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
           add_node_unit(kGroupBaseMotion, (int)tb.base_motion.size() - 1, 0, 6, row);
           bound(row + 0, -dev_rad, dev_rad); bound(row + 1, -dev_rad, dev_rad); bound(row + 2, -kInf, +kInf);
           bound(row + 3, -kInf, +kInf); bound(row + 4, -kInf, +kInf); bound(row + 5, z_init - 0.02, z_init + 0.1);
+          tb.base_z_rows.push_back(row + 5);   // the only constraint bounds that depend on the start state (StateInstance)
           int p; double tl;
           Locate(sp_ang, ts[k], &p, &tl);
           for (auto& b : Basis(sp_ang, p, tl, kPos)) emit1(row + b.dim, ang.offset + b.var, S_ONE, b.val);
@@ -996,6 +1038,7 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
   // ---- plan scalars
   pl.n = n; pl.m = m; pl.nnz = nnz; pl.n_ee = n_ee;
   pl.n_groups = (int)tb.groups.size(); pl.n_cost = (int)tb.cost.size();
+  pl.n_base_z_rows = (int)tb.base_z_rows.size();
   pl.mass = rb.mass; pl.gravity = 9.80665;  // dynamic_model.cc:37
   const double* I = rb.inertia;             // single_rigid_body_dynamics.cc:36-44
   double Ib[9] = {I[0], -I[3], -I[4], -I[3], I[1], -I[5], -I[4], -I[5], I[2]};

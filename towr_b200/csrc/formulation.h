@@ -54,6 +54,8 @@ struct HostTables {
   std::vector<PhaseUnit> phase_units;
   std::vector<PhaseExt> exts;
   std::vector<GoalVar> goal_vars;
+  std::vector<GoalVar> state_vars;    // goal_vars with the bounds of the start / goal state read from a state record
+  std::vector<int32_t> base_z_rows;   // BaseMotionConstraint LZ rows (their bounds follow the instance's initial base z)
   std::vector<ConstRun> const_runs;
   std::vector<double> const_vals;
   GoalSetup goal_setup{};
@@ -70,6 +72,9 @@ class Formulation {
   // the same tables at caller-given times (fpowr::ExtractInitialGuess)
   int SampleTables(const std::vector<double>& times, std::vector<SplineSample>* samples, std::vector<int>* contact) const;
   int GoalInstance(const double final_lin_pos[3], const double final_ang_pos[3], double* x0, double* x_lower, double* x_upper) const;
+  // the same with the whole state record (TWB_STATE_DOUBLES: initial_base_, final_base_, initial_ee_W_), plus the m
+  // constraint bounds of that instance; any output may be null
+  int StateInstance(const double* state, double* x0, double* x_lower, double* x_upper, double* g_lower, double* g_upper) const;
 
   int n = 0, m = 0, nnz = 0;
   std::vector<int> row_ptr, col_idx;

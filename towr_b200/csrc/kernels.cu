@@ -2291,6 +2291,83 @@ int LaunchGoalInstances(const Plan& P, const GoalSetup& S, const double* goals, 
   return (int)cudaGetLastError();
 }
 
+// Per-instance start states (Formulation::StateInstance), block = instance: the goal kernel's recipe walk with every endpoint
+// and every state bound read from the instance's record (Plan::state_vars), then the instance's constraint-bound rows = the
+// problem's with the BaseMotionConstraint LZ rows around the instance's z_init.  The initial feet are taken as given.
+__global__ void __launch_bounds__(128) StateInstanceKernel(const Plan P, const GoalSetup S, const double* __restrict__ states, const int* __restrict__ terrain_ids,
+                                                           int default_terrain, double* __restrict__ x0, double* __restrict__ lo, double* __restrict__ up,
+                                                           double* __restrict__ gl, double* __restrict__ gu, int nb) {
+  __shared__ double a_[2 + 2 * kMaxEE][3], b_[2 + 2 * kMaxEE][3];   // (initial, final) per set: lin, ang, motion_e.., force_e..
+  __shared__ double st[kStateDoubles];
+  __shared__ double z_init;
+  const int b = blockIdx.x;
+  if (b >= nb) return;
+  if (threadIdx.x < kStateDoubles) st[threadIdx.x] = states[(size_t)b * kStateDoubles + threadIdx.x];
+  __syncthreads();
+  const int terrain = terrain_ids ? __ldg(terrain_ids + b) : default_terrain;
+  if (threadIdx.x == 0) {
+    const double fx = st[kStFinalLinPos], fy = st[kStFinalLinPos + 1];
+    const double fz = EvalTerrain(P, terrain, fx, fy).h - S.nominal[0][2];
+    const double fin[3] = {fx, fy, fz};
+    for (int d = 0; d < 3; ++d) {
+      a_[0][d] = st[kStInitLinPos + d]; b_[0][d] = fin[d]; a_[1][d] = st[kStInitAngPos + d]; b_[1][d] = st[kStFinalAngPos + d];
+    }
+    z_init = a_[0][2] + 0.0 * (b_[0][2] - a_[0][2]);   // x0 of base-lin node 0, z: the interpolation at node fraction 0
+  } else if ((int)threadIdx.x <= P.n_ee) {
+    const int e = threadIdx.x - 1;
+    double sz, cz; sincos(st[kStFinalAngPos + 2], &sz, &cz);   // yaw-only rotation of the nominal stance, as in GoalInstanceKernel
+    const double* nom = S.nominal[e];
+    const double R[3][3] = {{cz, -sz, 0.0}, {sz, cz, 0.0}, {-0.0, 0.0, 1.0}};
+    double w[3];
+    for (int i = 0; i < 3; ++i) w[i] = st[kStFinalLinPos + i] + (R[i][0] * nom[0] + R[i][1] * nom[1] + R[i][2] * nom[2]);
+    const double goal[3] = {w[0], w[1], EvalTerrain(P, terrain, w[0], w[1]).h};
+    for (int d = 0; d < 3; ++d) {
+      a_[2 + e][d] = st[kStInitEE + 3 * e + d]; b_[2 + e][d] = goal[d];
+      a_[2 + kMaxEE + e][d] = b_[2 + kMaxEE + e][d] = (d == 2) ? S.f_stance_z : 0.0;
+    }
+  }
+  __syncthreads();
+  const double inf = 1e20;
+  if (x0 || lo || up)
+    for (int i = threadIdx.x; i < P.n; i += blockDim.x) {
+      const GoalVar v = P.state_vars[i];
+      double x, l = -inf, u = inf;
+      if (v.kind == kGoalConst) x = v.frac;
+      else {
+        const int set = v.kind == kGoalLin ? 0 : v.kind == kGoalAng ? 1 : v.kind == kGoalMotion ? 2 + v.ee : 2 + kMaxEE + v.ee;
+        const double a = a_[set][v.dim], dp = b_[set][v.dim] - a;
+        x = v.deriv == 0 ? a + v.frac * dp : dp / S.t_total;
+      }
+      if (v.bound == kBoundState) l = u = st[v.src];
+      else if (v.bound == kBoundConst) l = u = v.c0;
+      else if (v.bound == kBoundPair) { l = v.c0; u = v.c1; }
+      const size_t o = (size_t)b * P.n + i;
+      if (x0) x0[o] = x;
+      if (lo) lo[o] = l;
+      if (up) up[o] = u;
+    }
+  if (!gl && !gu) return;
+  double* gl_b = gl ? gl + (size_t)b * P.m : nullptr;
+  double* gu_b = gu ? gu + (size_t)b * P.m : nullptr;
+  for (int r = threadIdx.x; r < P.m; r += blockDim.x) {
+    if (gl_b) gl_b[r] = P.g_lower[r];
+    if (gu_b) gu_b[r] = P.g_upper[r];
+  }
+  if (P.n_base_z_rows == 0) return;
+  __syncthreads();   // the LZ rows were written with the problem's bounds above: overwrite them after every thread's copy
+  for (int k = threadIdx.x; k < P.n_base_z_rows; k += blockDim.x) {
+    const int r = P.base_z_rows[k];
+    if (gl_b) gl_b[r] = z_init - 0.02;
+    if (gu_b) gu_b[r] = z_init + 0.1;
+  }
+}
+int LaunchStateInstances(const Plan& P, const GoalSetup& S, const double* states, const int* terrain_ids, int default_terrain, double* x0, double* lo,
+                         double* up, double* gl, double* gu, int nb, cudaStream_t s) {
+  if (nb <= 0) return 0;
+  StateInstanceKernel<<<nb, 128, 0, s>>>(P, S, states, terrain_ids, default_terrain, x0, lo, up, gl, gu, nb);
+  return (int)cudaGetLastError();
+}
+
 // 1 when the constraint values go through GT and the TransposeOut kernel (optimised durations, experimental variants), else 0
 int TransposeOutPerEval(const Plan& P) { return (TWB_GDIRECT && TWB_ROMNODE && !TWB_FUSED && (TWB_GDIRECT_PHASE || P.n_phase_defs == 0)) ? 0 : 1; }
 int OutKernelsPerEval(const Plan& P, unsigned flags) {

@@ -44,6 +44,10 @@ int LaunchSoftConstraint(const Plan& P, const double* g, const double* jac, cons
 // x0 / variable bounds of `nb` goal-randomised instances (goals[b][6] = final base position, final base Euler angles)
 int LaunchGoalInstances(const Plan& P, const GoalSetup& S, const double* goals, const int* terrain_ids, int default_terrain, double* x0, double* lo,
                         double* up, int nb, cudaStream_t s);
+// x0 / variable bounds [nb][n] and constraint bounds [nb][m] of `nb` instances with their own start / goal states
+// (states[b][kStateDoubles]); any output may be null
+int LaunchStateInstances(const Plan& P, const GoalSetup& S, const double* states, const int* terrain_ids, int default_terrain, double* x0, double* lo,
+                         double* up, double* gl, double* gu, int nb, cudaStream_t s);
 // ---- device-resident solver step (lm_kernel.cu): the shared sparsity pattern and its transpose, constraint bounds (device pointers)
 struct LmPattern {
   const int* row_ptr;   // [m + 1]

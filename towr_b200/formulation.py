@@ -171,6 +171,28 @@ class NlpFormulation:
             s.cost_weights[i] = float(w)
         return s
 
+    def state_record(self):
+        """initial_base_, final_base_ and initial_ee_W_ of this formulation as one (STATE_DOUBLES,) state record."""
+        return pack_states([self.initial_base_], [self.final_base_], [self.initial_ee_W_])[0]
+
+
+def pack_states(initial_bases, final_bases, initial_ee_W):
+    """Per-instance start / goal states as the C ABI takes them (TWB_STATE_DOUBLES): a (B, 36) float64 array from B
+    initial BaseStates, B final BaseStates and B lists of foot positions (initial_ee_W_, at most MAX_EE feet of 3 values):
+    initial lin p, v, ang p, v | final lin p, v, ang p, v | feet [MAX_EE][3] (feet beyond the list stay 0)."""
+    B = len(initial_bases)
+    if len(final_bases) != B or len(initial_ee_W) != B:
+        raise ValueError("initial_bases, final_bases and initial_ee_W must have one entry per instance")
+    out = np.zeros((B, capi.STATE_DOUBLES))
+    for b in range(B):
+        i, f = initial_bases[b], final_bases[b]
+        out[b, :24] = np.concatenate([i.lin.p, i.lin.v, i.ang.p, i.ang.v, f.lin.p, f.lin.v, f.ang.p, f.ang.v])
+        feet = np.asarray(initial_ee_W[b], np.float64).reshape(-1, 3)
+        if len(feet) > capi.MAX_EE:
+            raise ValueError("more than MAX_EE feet")
+        out[b, 24:24 + 3 * len(feet)] = feet.ravel()
+    return out
+
 
 class Problem:
     """One structure class: what ifopt::Problem exposes besides evaluation."""
@@ -233,6 +255,20 @@ class Problem:
         check(lib.twb_problem_goal_instances(self._h, G, goals.ctypes.data_as(dp), x0.ctypes.data_as(dp),
                                              xl.ctypes.data_as(dp), xu.ctypes.data_as(dp)))
         return x0, xl, xu
+
+    def state_instances(self, states):
+        """x0, x_lower, x_upper (each (S, n)) and g_lower, g_upper (each (S, m)) of instances with their own start and goal
+        states; states: (S, 36) state records (pack_states).  Only the BaseMotionConstraint LZ rows of the constraint bounds
+        differ between instances."""
+        states = np.ascontiguousarray(states, np.float64)
+        assert states.ndim == 2 and states.shape[1] == capi.STATE_DOUBLES
+        S = states.shape[0]
+        x0, xl, xu = np.empty((S, self.n)), np.empty((S, self.n)), np.empty((S, self.n))
+        gl, gu = np.empty((S, self.m)), np.empty((S, self.m))
+        dp = C.POINTER(C.c_double)
+        check(lib.twb_problem_state_instances(self._h, S, states.ctypes.data_as(dp), x0.ctypes.data_as(dp), xl.ctypes.data_as(dp),
+                                              xu.ctypes.data_as(dp), gl.ctypes.data_as(dp), gu.ctypes.data_as(dp)))
+        return x0, xl, xu, gl, gu
 
     def _components(self, count_fn, get_fn):
         out = []
@@ -505,6 +541,25 @@ class Batch:
         ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
         check(lib.twb_batch_goal_instances_device(self._h, ptr(goals), ptr(x0), ptr(lo), ptr(up), C.c_void_p(stream.cuda_stream)))
         return x0, lo, up
+
+    def state_instances_device(self, states, want_bounds=True, want_g_bounds=False, stream=None):
+        """Batched setup on the device from per-instance start and goal states: states (B, 36) torch CUDA float64 state
+        records (pack_states).  Returns (x0, x_lower, x_upper) of shape (B, n) and (g_lower, g_upper) of shape (B, m) as CUDA
+        tensors (None where not wanted).  The terrain under each goal is the instance's own (set_terrains / grids)."""
+        import torch
+        p = self.problem
+        assert states.is_cuda and states.dtype == torch.float64 and states.is_contiguous() and tuple(states.shape) == (self.B, capi.STATE_DOUBLES)
+        if stream is None:
+            stream = torch.cuda.current_stream(states.device)
+        x0 = torch.empty((self.B, p.n), dtype=torch.float64, device=states.device)
+        lo = torch.empty_like(x0) if want_bounds else None
+        up = torch.empty_like(x0) if want_bounds else None
+        gl = torch.empty((self.B, p.m), dtype=torch.float64, device=states.device) if want_g_bounds else None
+        gu = torch.empty_like(gl) if want_g_bounds else None
+        ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        check(lib.twb_batch_state_instances_device(self._h, ptr(states), ptr(x0), ptr(lo), ptr(up), ptr(gl), ptr(gu),
+                                                   C.c_void_p(stream.cuda_stream)))
+        return x0, lo, up, gl, gu
 
     def lm_step_device(self, x, g, jac, x_lower=None, x_upper=None, mu=1e-2, cap=0.1, cg_iters=25, violation=None, stream=None):
         """twb_batch_lm_step_device: one Levenberg-Marquardt feasibility step for every instance on the outputs of
