@@ -55,7 +55,8 @@ enum { TWB_FLAT = 0, TWB_BLOCK = 1, TWB_STAIRS = 2, TWB_GAP = 3, TWB_SLOPE = 4,
        TWB_GRID_CSV = 7,
        /* towr `Grid` (towr/include/towr/terrain/grid_height_map.h:16-59, what fpowr's footstep_plan_server.cc:155 plans on):
         * a grid_map elevation layer, bilinear height in float, FLT_MAX outside the map, central-difference slopes with
-        * eps = resolution / 6; per-batch data (twb_batch_set_grid_map), per-instance terrain id like TWB_GRID_CSV */
+        * eps = resolution / 6; per-batch data (twb_batch_set_grid_map, or one map per instance with
+        * twb_batch_set_grid_maps), per-instance terrain id like TWB_GRID_CSV */
        TWB_GRID_MAP = 8 };
 
 /* towr::Parameters::ConstraintName, towr/include/towr/parameters.h:139-147 */
@@ -203,9 +204,23 @@ int twb_batch_set_grid_terrain(twb_batch* b, const double* heights, int rows, in
 
 /* The elevation layer of TWB_GRID_MAP for this batch: heights[ix * size_y + iy] (float, metres) = layer(ix, iy) of a
  * grid_map::GridMap with `resolution` metres per cell centred at (pos_x, pos_y); index 0 is the cell with the LARGEST
- * coordinate (grid_map convention), buffer start index (0, 0).  NULL removes it. */
+ * coordinate (grid_map convention), buffer start index (0, 0).  NULL removes it (and every map of twb_batch_set_grid_maps).
+ * The same as twb_batch_set_grid_maps(b, 1, heights, {size_x, size_y}, {resolution, pos_x, pos_y}, NULL). */
 int twb_batch_set_grid_map(twb_batch* b, const float* heights, int size_x, int size_y, double resolution,
                            double pos_x, double pos_y);
+
+/* n_maps grid_map elevation layers for this batch, so that instances standing on different maps (e.g. the requests of a plan
+ * server, each with its own perception) share one batch; instance b uses map map_of_instance[b] wherever its terrain id is
+ * TWB_GRID_MAP.  heights: the layers back to back, layer k = [sizes[k][0]][sizes[k][1]] floats, laid out as for
+ * twb_batch_set_grid_map; sizes: [n_maps][2] (size_x, size_y); geometry: [n_maps][3] (resolution, pos_x, pos_y);
+ * map_of_instance: host [B], each in [0, n_maps), or NULL = every instance uses map 0.  heights NULL or n_maps == 0
+ * removes every map (TWB_GRID_MAP instances are then outside the map everywhere: heights FLT_MAX).  The last call of this
+ * and twb_batch_set_grid_map wins; the terrain ids of twb_batch_set_terrains are kept, in either call order.
+ * Errors: n_maps < 0 or > 2^27, a map with a bad size (at most 2^28 cells) or a resolution / position that is not finite
+ * (resolution > 0), an index out of range: TWB_ERR_INVALID, and the previous maps and indices stay in place.
+ * Like the other terrain setters, the call drops the batch's cached evaluation graphs. */
+int twb_batch_set_grid_maps(twb_batch* b, int n_maps, const float* heights, const int* sizes, const double* geometry,
+                            const int* map_of_instance);
 
 /* Batched setup on the device (no host loop): twb_problem_goal_instances for the B instances of the batch.  goals: device
  * [B][6]; x0 / x_lower / x_upper: device [B][n] (any may be NULL).  The terrain under each goal is the INSTANCE's terrain
@@ -319,6 +334,20 @@ int twb_batch_initial_guess_device(twb_batch* b, const double* x, const double* 
 int twb_batch_footstep_plan_device(twb_batch* b, const double* x, double time_horizon, int* n_states, double* out, void* stream);
 int twb_batch_nearest_planes_device(twb_batch* b, const double* plan, const int* n_states, const int* poly_offsets, int n_polys,
                                     const double* vertices, int* contact_set, void* stream);
+
+/* twb_batch_nearest_planes_* where instance b looks only at polygons poly_ranges[b][0] .. poly_ranges[b][0] + poly_ranges[b][1] - 1
+ * of the shared list, and contact_set holds the index RELATIVE to that first polygon (what NearestPlaneLookup built from
+ * that request's own PlanarTerrain returns), -1 in the air / for unused states / for an empty range.  So one call serves a
+ * batch whose instances each have their own planar regions: pack every instance's polygons into one list.
+ * poly_ranges: [B][2] (first polygon, count), a host array for _ranges_host, a device array for _ranges_device.
+ * _ranges_host rejects a range outside [0, n_polys) (first < 0, count < 0, first + count > n_polys) with TWB_ERR_INVALID.
+ * _ranges_device cannot check the ranges: it clamps each to [0, n_polys) (it never reads outside the list) and counts the
+ * index from the first polygon of the clamped range.  Otherwise as the calls above. */
+int twb_batch_nearest_planes_ranges_host(twb_batch* b, const double* plan, const int* n_states, const int* poly_ranges,
+                                         const int* poly_offsets, int n_polys, const double* vertices, int* contact_set);
+int twb_batch_nearest_planes_ranges_device(twb_batch* b, const double* plan, const int* n_states, const int* poly_ranges,
+                                           const int* poly_offsets, int n_polys, const double* vertices, int* contact_set,
+                                           void* stream);
 
 /* ---- the two ifopt components of towr that no Parameters::ConstraintName / CostName reaches ---------------------------
  * towr::LinearEqualityConstraint (towr/src/linear_constraint.cc:35-73) on variable set `var_set` (index of

@@ -46,6 +46,7 @@ def _load():
         "twb_batch_set_terrains": (C.c_int, [P, I]),
         "twb_batch_set_grid_terrain": (C.c_int, [P, D, C.c_int, C.c_int]),
         "twb_batch_set_grid_map": (C.c_int, [P, C.POINTER(C.c_float), C.c_int, C.c_int, C.c_double, C.c_double, C.c_double]),
+        "twb_batch_set_grid_maps": (C.c_int, [P, C.c_int, C.POINTER(C.c_float), I, D, I]),
         "twb_batch_goal_instances_device": (C.c_int, [P, P, P, P, P, P]),
         "twb_problem_state_instances": (C.c_int, [P, C.c_int, D, D, D, D, D, D]),
         "twb_batch_state_instances_device": (C.c_int, [P, P, P, P, P, P, P, P]),
@@ -62,6 +63,8 @@ def _load():
         "twb_batch_initial_guess_device": (C.c_int, [P, P, P, C.c_int, P, P]),
         "twb_batch_footstep_plan_device": (C.c_int, [P, P, C.c_double, P, P, P]),
         "twb_batch_nearest_planes_device": (C.c_int, [P, P, P, P, C.c_int, P, P, P]),
+        "twb_batch_nearest_planes_ranges_host": (C.c_int, [P, P, P, P, P, C.c_int, P, P]),
+        "twb_batch_nearest_planes_ranges_device": (C.c_int, [P, P, P, P, P, C.c_int, P, P, P]),
         "twb_batch_linear_equality_host": (C.c_int, [P, P, C.c_int, P, C.c_int, P]),
         "twb_batch_soft_constraint_host": (C.c_int, [P, C.c_int, P, P, P]),
         "twb_batch_launches_per_eval": (C.c_int, [P, C.c_uint]),

@@ -13,7 +13,7 @@ MONOPED, BIPED, HYQ, ANYMAL, GO1 = range(5)
 # towr::HeightMap::TerrainID (height_map.h:79-86)
 FLAT, BLOCK, STAIRS, GAP, SLOPE, CHIMNEY, CHIMNEY_LR = range(7)
 GRID_CSV = 7   # towr::HeightMapFromCSV; grid data per batch (Batch.set_grid_terrain)
-GRID_MAP = 8   # towr Grid (grid_height_map.h): grid_map elevation layer per batch (Batch.set_grid_map)
+GRID_MAP = 8   # towr Grid (grid_height_map.h): grid_map elevation layer per batch (Batch.set_grid_map) or per instance (Batch.set_grid_maps)
 # towr::Parameters::ConstraintName (parameters.h:139-147)
 C_DYNAMIC, C_EE_ROM, C_TOTAL_TIME, C_TERRAIN, C_FORCE, C_SWING, C_BASE_ROM, C_BASE_ACC = range(8)
 # towr::Parameters::CostName

@@ -71,9 +71,12 @@ struct twb_batch {
   size_t ld = 0;                  // instances padded to a multiple of 32 (whole tiles of XT)
   twb::Plan plan{};
   std::vector<void*> owned;       // device allocations of the tables
-  int* d_terrain = nullptr;       // per-instance terrain ids (optional)
+  int* d_terrain = nullptr;       // per-instance terrain words (device_tables.h: TerrainWord; optional)
+  std::vector<int> h_terrain;     // host copies of the terrain ids (empty: twb_spec.terrain) and of the grid_map indices
+  std::vector<int> h_map_of;      // (empty: map 0) that d_terrain is packed from
   double* d_grid = nullptr;       // height grid of TWB_GRID_CSV (optional)
-  float* d_gmap = nullptr;        // elevation layer of TWB_GRID_MAP (optional)
+  float* d_gmap_pool = nullptr;   // elevation layers of TWB_GRID_MAP, back to back (optional)
+  twb::GridMapDesc* d_gmaps = nullptr;   // one descriptor per layer
   double* d_XT = nullptr;         // [ld/32][n+1][32] instance-tiled iterates; row n == 0
   double* d_GT = nullptr;         // [ld/32][m][32] instance-tiled constraint values (staging of g)
   int* d_TD = nullptr;            // [ld/32] per-tile completion counters of the output kernels (zero between evaluations)
@@ -227,12 +230,68 @@ int FootstepCore(twb_batch* b, const double* x, double time_horizon, int* n_stat
                                max_states, n_states, out, b->B, s);
   return rc != 0 ? CudaFail(static_cast<cudaError_t>(rc), "footstep-plan kernel launch") : TWB_OK;
 }
-int NearestPlanesCore(twb_batch* b, const double* plan, const int* n_states, const int* poly_offsets, int n_polys, const double* vertices,
-                      int* contact_set, cudaStream_t s) {
+int NearestPlanesCore(twb_batch* b, const double* plan, const int* n_states, const int* poly_ranges, const int* poly_offsets, int n_polys,
+                      const double* vertices, int* contact_set, cudaStream_t s) {
   int max_states = 0;
   twb_problem_footstep_plan_dims(b->prob, &max_states, nullptr);
-  const int rc = twb::LaunchNearestPlanes(plan, n_states, max_states, b->prob->f.spec.n_ee, poly_offsets, n_polys, vertices, contact_set, b->B, s);
+  const int rc = twb::LaunchNearestPlanes(plan, n_states, max_states, b->prob->f.spec.n_ee, poly_offsets, n_polys, poly_ranges, vertices,
+                                          contact_set, b->B, s);
   return rc != 0 ? CudaFail(static_cast<cudaError_t>(rc), "nearest-plane kernel launch") : TWB_OK;
+}
+// host arrays in, host contact sets out; poly_ranges may be null (every instance looks at all polygons)
+int NearestPlanesHost(twb_batch* b, const double* plan, const int* n_states, const int* poly_ranges, const int* poly_offsets, int n_polys,
+                      const double* vertices, int* contact_set) {
+  if (!b || !plan || !n_states || !poly_offsets || !contact_set || n_polys < 0 || (n_polys > 0 && !vertices)) return Fail(TWB_ERR_INVALID, "null argument");
+  for (int k = 0; k < n_polys; ++k) if (poly_offsets[k + 1] < poly_offsets[k] || poly_offsets[k] < 0) return Fail(TWB_ERR_INVALID, "polygon offsets must ascend");
+  if (poly_ranges)
+    for (int i = 0; i < b->B; ++i)
+      if (poly_ranges[2 * i] < 0 || poly_ranges[2 * i + 1] < 0 || (long long)poly_ranges[2 * i] + poly_ranges[2 * i + 1] > n_polys)
+        return Fail(TWB_ERR_INVALID, "polygon range outside the polygon list");
+  int max_states = 0, V = 0;
+  twb_problem_footstep_plan_dims(b->prob, &max_states, &V);
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  const size_t B = b->B, n_ee = b->prob->f.spec.n_ee, n_vert = n_polys > 0 ? (size_t)poly_offsets[n_polys] : 0;
+  double* d_plan = nullptr; int* d_count = nullptr; int* d_off = nullptr; double* d_vert = nullptr; int* d_out = nullptr; int* d_ranges = nullptr;
+  // scratch buffers stay with the batch (twb_batch::scratch) and are reused by the next call
+  if ((e = ScratchAlloc(b, 0, reinterpret_cast<void**>(&d_plan), sizeof(double) * B * max_states * V)) != cudaSuccess ||
+      (e = ScratchAlloc(b, 1, reinterpret_cast<void**>(&d_count), sizeof(int) * B)) != cudaSuccess ||
+      (e = ScratchAlloc(b, 2, reinterpret_cast<void**>(&d_off), sizeof(int) * (n_polys + 1))) != cudaSuccess ||
+      (e = ScratchAlloc(b, 3, reinterpret_cast<void**>(&d_vert), sizeof(double) * 2 * std::max<size_t>(n_vert, 1))) != cudaSuccess ||
+      (e = ScratchAlloc(b, 4, reinterpret_cast<void**>(&d_out), sizeof(int) * B * max_states * n_ee)) != cudaSuccess ||
+      (poly_ranges && (e = ScratchAlloc(b, 5, reinterpret_cast<void**>(&d_ranges), sizeof(int) * 2 * B)) != cudaSuccess)) return CudaFail(e, "cudaMalloc");
+  cudaStream_t s = b->stream;
+  cudaMemcpyAsync(d_plan, plan, sizeof(double) * B * max_states * V, cudaMemcpyHostToDevice, s);
+  cudaMemcpyAsync(d_count, n_states, sizeof(int) * B, cudaMemcpyHostToDevice, s);
+  cudaMemcpyAsync(d_off, poly_offsets, sizeof(int) * (n_polys + 1), cudaMemcpyHostToDevice, s);
+  if (n_vert) cudaMemcpyAsync(d_vert, vertices, sizeof(double) * 2 * n_vert, cudaMemcpyHostToDevice, s);
+  if (poly_ranges) cudaMemcpyAsync(d_ranges, poly_ranges, sizeof(int) * 2 * B, cudaMemcpyHostToDevice, s);
+  int rc = NearestPlanesCore(b, d_plan, d_count, d_ranges, d_off, n_polys, d_vert, d_out, s);
+  if (rc == TWB_OK) cudaMemcpyAsync(contact_set, d_out, sizeof(int) * B * max_states * n_ee, cudaMemcpyDeviceToHost, s);
+  e = cudaStreamSynchronize(s);
+  if (rc != TWB_OK) return rc;
+  if (e != cudaSuccess) return CudaFail(e, "nearest-plane lookup");
+  return TWB_OK;
+}
+int NearestPlanesDevice(twb_batch* b, const double* plan, const int* n_states, const int* poly_ranges, const int* poly_offsets, int n_polys,
+                        const double* vertices, int* contact_set, void* stream) {
+  if (!b || !plan || !n_states || !poly_offsets || !contact_set || n_polys < 0 || (n_polys > 0 && !vertices)) return Fail(TWB_ERR_INVALID, "null argument");
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  return NearestPlanesCore(b, plan, n_states, poly_ranges, poly_offsets, n_polys, vertices, contact_set, static_cast<cudaStream_t>(stream));
+}
+
+// d_terrain from the host copies of the terrain ids and grid_map indices (device_tables.h: TerrainWord); none of either:
+// no per-instance words, every instance evaluates twb_spec.terrain
+int UploadTerrainWords(twb_batch* b) {
+  if (b->h_terrain.empty() && b->h_map_of.empty()) { cudaFree(b->d_terrain); b->d_terrain = nullptr; return TWB_OK; }
+  std::vector<int> words(b->B);
+  for (int i = 0; i < b->B; ++i)
+    words[i] = twb::TerrainWord(b->h_terrain.empty() ? b->prob->f.spec.terrain : b->h_terrain[i], b->h_map_of.empty() ? 0 : b->h_map_of[i]);
+  cudaError_t e;
+  if (!b->d_terrain && (e = cudaMalloc(&b->d_terrain, sizeof(int) * b->B)) != cudaSuccess) return CudaFail(e, "cudaMalloc");
+  if ((e = cudaMemcpy(b->d_terrain, words.data(), sizeof(int) * b->B, cudaMemcpyHostToDevice)) != cudaSuccess) return CudaFail(e, "cudaMemcpy");
+  return TWB_OK;
 }
 }  // namespace
 
@@ -422,7 +481,7 @@ void twb_batch_destroy(twb_batch* b) {
   for (void* p : b->owned) cudaFree(p);
   for (auto& sc : b->scratch) cudaFree(sc.first);
   for (auto& t : b->post_tables) cudaFree(t.mem);
-  cudaFree(b->d_terrain); cudaFree(b->d_grid); cudaFree(b->d_gmap); cudaFree(b->d_XT); cudaFree(b->d_FS); cudaFree(b->d_TD);   // (d_GT is part of d_XT's allocation)
+  cudaFree(b->d_terrain); cudaFree(b->d_grid); cudaFree(b->d_gmap_pool); cudaFree(b->d_gmaps); cudaFree(b->d_XT); cudaFree(b->d_FS); cudaFree(b->d_TD);   // (d_GT is part of d_XT's allocation)
   for (auto ev : b->ev) if (ev) cudaEventDestroy(ev);
   if (b->aux0) cudaStreamDestroy(b->aux0);
   if (b->aux1) cudaStreamDestroy(b->aux1);
@@ -438,14 +497,11 @@ int twb_batch_set_terrains(twb_batch* b, const int* terrain_ids) {
   if (!b) return Fail(TWB_ERR_INVALID, "null batch");
   cudaSetDevice(b->device);
   DropGraphs(b);
-  if (!terrain_ids) { cudaFree(b->d_terrain); b->d_terrain = nullptr; return TWB_OK; }
+  if (!terrain_ids) { b->h_terrain.clear(); return UploadTerrainWords(b); }
   for (int i = 0; i < b->B; ++i)
     if (terrain_ids[i] < 0 || terrain_ids[i] > TWB_GRID_MAP) return Fail(TWB_ERR_INVALID, "unknown terrain id");
-  cudaError_t e;
-  if (!b->d_terrain && (e = cudaMalloc(&b->d_terrain, sizeof(int) * b->B)) != cudaSuccess) return CudaFail(e, "cudaMalloc");
-  if ((e = cudaMemcpy(b->d_terrain, terrain_ids, sizeof(int) * b->B, cudaMemcpyHostToDevice)) != cudaSuccess)
-    return CudaFail(e, "cudaMemcpy");
-  return TWB_OK;
+  b->h_terrain.assign(terrain_ids, terrain_ids + b->B);
+  return UploadTerrainWords(b);
 }
 
 int twb_batch_set_grid_terrain(twb_batch* b, const double* heights, int rows, int cols) {
@@ -465,21 +521,51 @@ int twb_batch_set_grid_terrain(twb_batch* b, const double* heights, int rows, in
 }
 
 int twb_batch_set_grid_map(twb_batch* b, const float* heights, int size_x, int size_y, double resolution, double pos_x, double pos_y) {
+  const int sizes[2] = {size_x, size_y};
+  const double geometry[3] = {resolution, pos_x, pos_y};
+  return twb_batch_set_grid_maps(b, heights ? 1 : 0, heights, sizes, geometry, nullptr);
+}
+
+int twb_batch_set_grid_maps(twb_batch* b, int n_maps, const float* heights, const int* sizes, const double* geometry, const int* map_of_instance) {
   if (!b) return Fail(TWB_ERR_INVALID, "null batch");
-  cudaSetDevice(b->device);
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  float* pool = nullptr; twb::GridMapDesc* table = nullptr;
+  std::vector<int> map_of;
+  if (n_maps < 0 || n_maps > twb::kMaxGridMaps) return Fail(TWB_ERR_INVALID, "bad number of grid maps");
+  if (heights && n_maps > 0) {   // checked and uploaded before the previous maps are released: a failed call keeps them
+    if (!sizes || !geometry) return Fail(TWB_ERR_INVALID, "null argument");
+    std::vector<twb::GridMapDesc> desc(n_maps);
+    long long cells = 0;
+    for (int k = 0; k < n_maps; ++k) {
+      const int sx = sizes[2 * k], sy = sizes[2 * k + 1];
+      const double res = geometry[3 * k], px = geometry[3 * k + 1], py = geometry[3 * k + 2];
+      if (sx <= 0 || sy <= 0 || (long long)sx * sy > (1ll << 28) || !(res > 0.0) || !std::isfinite(res) || !std::isfinite(px) || !std::isfinite(py))
+        return Fail(TWB_ERR_INVALID, "bad grid map geometry");
+      desc[k] = twb::GridMapDesc{cells, sx, sy, res, px, py};
+      cells += (long long)sx * sy;
+    }
+    if (map_of_instance) {
+      for (int i = 0; i < b->B; ++i)
+        if (map_of_instance[i] < 0 || map_of_instance[i] >= n_maps) return Fail(TWB_ERR_INVALID, "grid map index out of range");
+      map_of.assign(map_of_instance, map_of_instance + b->B);
+    }
+    if ((e = cudaMalloc(reinterpret_cast<void**>(&pool), sizeof(float) * (size_t)cells)) != cudaSuccess ||
+        (e = cudaMalloc(reinterpret_cast<void**>(&table), sizeof(twb::GridMapDesc) * n_maps)) != cudaSuccess ||
+        (e = cudaMemcpy(pool, heights, sizeof(float) * (size_t)cells, cudaMemcpyHostToDevice)) != cudaSuccess ||
+        (e = cudaMemcpy(table, desc.data(), sizeof(twb::GridMapDesc) * n_maps, cudaMemcpyHostToDevice)) != cudaSuccess) {
+      cudaFree(pool); cudaFree(table);
+      return CudaFail(e, "grid map upload");
+    }
+  } else {
+    n_maps = 0;
+  }
   DropGraphs(b);
-  cudaFree(b->d_gmap); b->d_gmap = nullptr;
-  b->plan.gmap = nullptr; b->plan.gmap_sx = b->plan.gmap_sy = 0; b->plan.gmap_res = 1.0; b->plan.gmap_px = b->plan.gmap_py = 0.0;
-  if (!heights) return TWB_OK;
-  if (size_x <= 0 || size_y <= 0 || (long long)size_x * size_y > (1ll << 28) || !(resolution > 0.0) || !std::isfinite(resolution) ||
-      !std::isfinite(pos_x) || !std::isfinite(pos_y))
-    return Fail(TWB_ERR_INVALID, "bad grid map geometry");
-  cudaError_t e;
-  const size_t bytes = sizeof(float) * (size_t)size_x * size_y;
-  if ((e = cudaMalloc(reinterpret_cast<void**>(&b->d_gmap), bytes)) != cudaSuccess) return CudaFail(e, "cudaMalloc");
-  if ((e = cudaMemcpy(b->d_gmap, heights, bytes, cudaMemcpyHostToDevice)) != cudaSuccess) return CudaFail(e, "cudaMemcpy");
-  b->plan.gmap = b->d_gmap; b->plan.gmap_sx = size_x; b->plan.gmap_sy = size_y; b->plan.gmap_res = resolution; b->plan.gmap_px = pos_x; b->plan.gmap_py = pos_y;
-  return TWB_OK;
+  cudaFree(b->d_gmap_pool); cudaFree(b->d_gmaps);
+  b->d_gmap_pool = pool; b->d_gmaps = table;
+  b->plan.gmap_pool = pool; b->plan.gmaps = table; b->plan.n_gmaps = n_maps;
+  b->h_map_of.swap(map_of);
+  return UploadTerrainWords(b);
 }
 
 int twb_batch_goal_instances_device(twb_batch* b, const double* goals, double* x0, double* x_lower, double* x_upper, void* stream) {
@@ -617,39 +703,25 @@ int twb_batch_footstep_plan_device(twb_batch* b, const double* x, double time_ho
 
 int twb_batch_nearest_planes_host(twb_batch* b, const double* plan, const int* n_states, const int* poly_offsets, int n_polys,
                                   const double* vertices, int* contact_set) {
-  if (!b || !plan || !n_states || !poly_offsets || !contact_set || n_polys < 0 || (n_polys > 0 && !vertices)) return Fail(TWB_ERR_INVALID, "null argument");
-  for (int k = 0; k < n_polys; ++k) if (poly_offsets[k + 1] < poly_offsets[k] || poly_offsets[k] < 0) return Fail(TWB_ERR_INVALID, "polygon offsets must ascend");
-  int max_states = 0, V = 0;
-  twb_problem_footstep_plan_dims(b->prob, &max_states, &V);
-  cudaError_t e = cudaSetDevice(b->device);
-  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
-  const size_t B = b->B, n_ee = b->prob->f.spec.n_ee, n_vert = n_polys > 0 ? (size_t)poly_offsets[n_polys] : 0;
-  double* d_plan = nullptr; int* d_count = nullptr; int* d_off = nullptr; double* d_vert = nullptr; int* d_out = nullptr;
-  // scratch buffers stay with the batch (twb_batch::scratch) and are reused by the next call
-  if ((e = ScratchAlloc(b, 0, reinterpret_cast<void**>(&d_plan), sizeof(double) * B * max_states * V)) != cudaSuccess ||
-      (e = ScratchAlloc(b, 1, reinterpret_cast<void**>(&d_count), sizeof(int) * B)) != cudaSuccess ||
-      (e = ScratchAlloc(b, 2, reinterpret_cast<void**>(&d_off), sizeof(int) * (n_polys + 1))) != cudaSuccess ||
-      (e = ScratchAlloc(b, 3, reinterpret_cast<void**>(&d_vert), sizeof(double) * 2 * std::max<size_t>(n_vert, 1))) != cudaSuccess ||
-      (e = ScratchAlloc(b, 4, reinterpret_cast<void**>(&d_out), sizeof(int) * B * max_states * n_ee)) != cudaSuccess) return CudaFail(e, "cudaMalloc");
-  cudaStream_t s = b->stream;
-  cudaMemcpyAsync(d_plan, plan, sizeof(double) * B * max_states * V, cudaMemcpyHostToDevice, s);
-  cudaMemcpyAsync(d_count, n_states, sizeof(int) * B, cudaMemcpyHostToDevice, s);
-  cudaMemcpyAsync(d_off, poly_offsets, sizeof(int) * (n_polys + 1), cudaMemcpyHostToDevice, s);
-  if (n_vert) cudaMemcpyAsync(d_vert, vertices, sizeof(double) * 2 * n_vert, cudaMemcpyHostToDevice, s);
-  int rc = NearestPlanesCore(b, d_plan, d_count, d_off, n_polys, d_vert, d_out, s);
-  if (rc == TWB_OK) cudaMemcpyAsync(contact_set, d_out, sizeof(int) * B * max_states * n_ee, cudaMemcpyDeviceToHost, s);
-  e = cudaStreamSynchronize(s);
-  if (rc != TWB_OK) return rc;
-  if (e != cudaSuccess) return CudaFail(e, "nearest-plane lookup");
-  return TWB_OK;
+  return NearestPlanesHost(b, plan, n_states, nullptr, poly_offsets, n_polys, vertices, contact_set);
 }
 
 int twb_batch_nearest_planes_device(twb_batch* b, const double* plan, const int* n_states, const int* poly_offsets, int n_polys,
                                     const double* vertices, int* contact_set, void* stream) {
-  if (!b || !plan || !n_states || !poly_offsets || !contact_set || n_polys < 0 || (n_polys > 0 && !vertices)) return Fail(TWB_ERR_INVALID, "null argument");
-  cudaError_t e = cudaSetDevice(b->device);
-  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
-  return NearestPlanesCore(b, plan, n_states, poly_offsets, n_polys, vertices, contact_set, static_cast<cudaStream_t>(stream));
+  return NearestPlanesDevice(b, plan, n_states, nullptr, poly_offsets, n_polys, vertices, contact_set, stream);
+}
+
+int twb_batch_nearest_planes_ranges_host(twb_batch* b, const double* plan, const int* n_states, const int* poly_ranges,
+                                         const int* poly_offsets, int n_polys, const double* vertices, int* contact_set) {
+  if (!poly_ranges) return Fail(TWB_ERR_INVALID, "null argument");
+  return NearestPlanesHost(b, plan, n_states, poly_ranges, poly_offsets, n_polys, vertices, contact_set);
+}
+
+int twb_batch_nearest_planes_ranges_device(twb_batch* b, const double* plan, const int* n_states, const int* poly_ranges,
+                                           const int* poly_offsets, int n_polys, const double* vertices, int* contact_set,
+                                           void* stream) {
+  if (!poly_ranges) return Fail(TWB_ERR_INVALID, "null argument");
+  return NearestPlanesDevice(b, plan, n_states, poly_ranges, poly_offsets, n_polys, vertices, contact_set, stream);
 }
 
 int twb_batch_linear_equality_host(twb_batch* b, const double* x, int var_set, const double* M, int rows, double* g) {

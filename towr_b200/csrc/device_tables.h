@@ -244,6 +244,22 @@ constexpr int kStateDoubles = 36;
 enum StateField : int8_t { kStInitLinPos = 0, kStInitLinVel = 3, kStInitAngPos = 6, kStInitAngVel = 9, kStFinalLinPos = 12, kStFinalLinVel = 15,
                            kStFinalAngPos = 18, kStFinalAngVel = 21, kStInitEE = 24 };
 
+// ---- per-instance terrain word (twb_batch::d_terrain): the terrain id, and for TWB_GRID_MAP (8) instances the index of the
+// instance's map in Plan::gmaps above the low four bits.  Every other id is stored as it is, so the analytic terrains see
+// their raw id; words of 7 and above are decoded only in the out-of-line grid path (kernels.cu: EvalGridTerrain).
+#ifdef __CUDACC__
+#define TWB_HOST_DEVICE __host__ __device__
+#else
+#define TWB_HOST_DEVICE
+#endif
+constexpr int kTerrainGridMap = 8;
+constexpr int kMaxGridMaps = 1 << 27;   // map << 4 stays a positive int
+inline TWB_HOST_DEVICE int TerrainWord(int id, int map) { return id == kTerrainGridMap ? id | (map << 4) : id; }
+inline TWB_HOST_DEVICE int TerrainWordId(int word) { return word & 15; }
+inline TWB_HOST_DEVICE int TerrainWordMap(int word) { return word >> 4; }
+// one grid_map elevation layer of a batch: layer(ix, iy) = pool[offset + ix * sy + iy], `res` metres per cell, centred at (px, py)
+struct GridMapDesc { long long offset; int sx, sy; double res, px, py; };
+
 struct Plan {
   int n, m, nnz, n_ee;
   int n_dyn, n_rom, n_groups, n_cost;
@@ -276,10 +292,11 @@ struct Plan {
   // height grid of the TWB_GRID_CSV terrain (per batch; null: heights 0)
   const double* grid;
   int grid_rows, grid_cols;
-  // elevation layer of the TWB_GRID_MAP terrain (per batch; null: every position is outside the map)
-  const float* gmap;
-  int gmap_sx, gmap_sy;
-  double gmap_res, gmap_px, gmap_py;
+  // elevation layers of the TWB_GRID_MAP terrain (per batch): instance b reads gmaps[TerrainWordMap(word_b)]; an index
+  // >= n_gmaps (no maps) puts every position outside the map
+  const float* gmap_pool;
+  const GridMapDesc* gmaps;
+  int n_gmaps;
   const GoalVar* goal_vars;             // [n] recipe of x0 / bounds per variable
   const GoalVar* state_vars;            // [n] the same recipe for per-instance start states (bounds from the state record)
   const double* g_lower;                // [m] the problem's constraint bounds (per-instance setup copies them)

@@ -448,8 +448,15 @@ struct TerrainPoint { double h, hx, hy, hxx; };
 // (RomNodeOut shrank from 12 952 to 8 456 SASS instructions; the step time did not change)
 struct GridArgs {
   const double* grid; int grid_rows, grid_cols;
-  const float* gmap; int gmap_sx, gmap_sy; double gmap_res, gmap_px, gmap_py;
+  const float* gmap_pool; const GridMapDesc* gmaps; int n_gmaps;
 };
+// one instance's grid_map layer, read from the batch's map table (null heights: no such map, every position is outside)
+struct GridMap { const float* h; int sx, sy; double res, px, py; };
+__device__ __forceinline__ GridMap LoadGridMap(const GridArgs& P, int map) {
+  if (map >= P.n_gmaps) return GridMap{nullptr, 0, 0, 1.0, 0.0, 0.0};
+  const GridMapDesc* d = P.gmaps + map;
+  return GridMap{P.gmap_pool + __ldg(&d->offset), __ldg(&d->sx), __ldg(&d->sy), __ldg(&d->res), __ldg(&d->px), __ldg(&d->py)};
+}
 __device__ __forceinline__ bool GridCell(const GridArgs& P, double x, double y, long long* xc, long long* yc) {
   const double res = 0.17;
   const double fx = x / res, fy = y / res;
@@ -474,15 +481,15 @@ __device__ __forceinline__ double GridEdgeSlope(const GridArgs& P, long long c, 
 // towr `Grid` (grid_height_map.h:16-59) over grid_map::GridMap::atPosition(layer, p, INTER_LINEAR) (grid_map_core, restated;
 // un-vendored dependency): bilinear over the four cell centres around p with double weights stored to FLOAT, nearest cell
 // when one of the four is outside, FLT_MAX outside the map; cell (ix, iy) is centred at pos + L/2 - res/2 - res * (ix, iy).
-__device__ __forceinline__ void GridMapCentre(const GridArgs& P, int ix, int iy, double* x, double* y) {
-  *x = P.gmap_px + (0.5 * (P.gmap_sx * P.gmap_res) - 0.5 * P.gmap_res) + P.gmap_res * (double)(-ix);
-  *y = P.gmap_py + (0.5 * (P.gmap_sy * P.gmap_res) - 0.5 * P.gmap_res) + P.gmap_res * (double)(-iy);
+__device__ __forceinline__ void GridMapCentre(const GridMap& P, int ix, int iy, double* x, double* y) {
+  *x = P.px + (0.5 * (P.sx * P.res) - 0.5 * P.res) + P.res * (double)(-ix);
+  *y = P.py + (0.5 * (P.sy * P.res) - 0.5 * P.res) + P.res * (double)(-iy);
 }
-__device__ __noinline__ float GridMapHeight(const GridArgs& P, double x, double y) {
+__device__ __noinline__ float GridMapHeight(const GridMap& P, double x, double y) {
   const float outside = 3.402823466e+38f;   // std::numeric_limits<float>::max(), grid_height_map.h:43
-  if (!P.gmap) return outside;
-  const double Lx = P.gmap_sx * P.gmap_res, Ly = P.gmap_sy * P.gmap_res;
-  const int ix0 = (int)(-((x - 0.5 * Lx - P.gmap_px) / P.gmap_res)), iy0 = (int)(-((y - 0.5 * Ly - P.gmap_py) / P.gmap_res));
+  if (!P.h) return outside;
+  const double Lx = P.sx * P.res, Ly = P.sy * P.res;
+  const int ix0 = (int)(-((x - 0.5 * Lx - P.px) / P.res)), iy0 = (int)(-((y - 0.5 * Ly - P.py) / P.res));
   double cx, cy; GridMapCentre(P, ix0, iy0, &cx, &cy);
   const bool dir = x >= cx, up = y >= cy;
   const int ix1 = dir ? ix0 - 1 : ix0 + 1, iy2 = up ? iy0 - 1 : iy0 + 1;
@@ -491,32 +498,34 @@ __device__ __noinline__ float GridMapHeight(const GridArgs& P, double x, double 
   int sh[4];
   if (up) { if (dir) { sh[0] = 0; sh[1] = 1; sh[2] = 2; sh[3] = 3; } else { sh[0] = 1; sh[1] = 0; sh[2] = 3; sh[3] = 2; } }
   else    { if (dir) { sh[0] = 2; sh[1] = 3; sh[2] = 0; sh[3] = 1; } else { sh[0] = 3; sh[1] = 2; sh[2] = 1; sh[3] = 0; } }
-  const unsigned long long buffer = (unsigned long long)P.gmap_sx * P.gmap_sy;
+  const unsigned long long buffer = (unsigned long long)P.sx * P.sy;
   float f[4]; bool ok = true;
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
-    const unsigned long long lin = (unsigned long long)((long long)cys[sh[i]] * P.gmap_sx + cxs[sh[i]]);   // column-major linear index in size_t, as grid_map
+    const unsigned long long lin = (unsigned long long)((long long)cys[sh[i]] * P.sx + cxs[sh[i]]);   // column-major linear index in size_t, as grid_map
     if (lin >= buffer) { ok = false; f[i] = 0.0f; }
-    else f[i] = __ldg(P.gmap + (lin % (unsigned long long)P.gmap_sx) * P.gmap_sy + lin / (unsigned long long)P.gmap_sx);
+    else f[i] = __ldg(P.h + (lin % (unsigned long long)P.sx) * P.sy + lin / (unsigned long long)P.sx);
   }
   if (ok) {
     GridMapCentre(P, cxs[sh[0]], cys[sh[0]], &cx, &cy);
-    const double rx = (x - cx) / P.gmap_res, ry = (y - cy) / P.gmap_res, fx = 1.0 - rx, fy = 1.0 - ry;
+    const double rx = (x - cx) / P.res, ry = (y - cy) / P.res, fx = 1.0 - rx, fy = 1.0 - ry;
     return (float)(f[0] * fx * fy + f[1] * rx * fy + f[2] * fx * ry + f[3] * rx * ry);
   }
-  const double tx = -(x - P.gmap_px - 0.5 * Lx), ty = -(y - P.gmap_py - 0.5 * Ly);   // checkIfPositionWithinMap + checkIfIndexInRange
-  if (tx >= 0.0 && ty >= 0.0 && tx < Lx && ty < Ly && ix0 >= 0 && iy0 >= 0 && ix0 < P.gmap_sx && iy0 < P.gmap_sy)
-    return __ldg(P.gmap + (size_t)ix0 * P.gmap_sy + iy0);
+  const double tx = -(x - P.px - 0.5 * Lx), ty = -(y - P.py - 0.5 * Ly);   // checkIfPositionWithinMap + checkIfIndexInRange
+  if (tx >= 0.0 && ty >= 0.0 && tx < Lx && ty < Ly && ix0 >= 0 && iy0 >= 0 && ix0 < P.sx && iy0 < P.sy)
+    return __ldg(P.h + (size_t)ix0 * P.sy + iy0);
   return outside;
 }
-__device__ __noinline__ TerrainPoint EvalGridTerrain(const GridArgs P, int id, double x, double y) {
+// `word`: the instance's terrain word (device_tables.h: TerrainWord), 7 or above
+__device__ __noinline__ TerrainPoint EvalGridTerrain(const GridArgs P, int word, double x, double y) {
   TerrainPoint o{0.0, 0.0, 0.0, 0.0};
-  switch (id) {
+  switch (TerrainWordId(word)) {
     case 8: {  // Grid (grid_map elevation layer), grid_height_map.h:29-60: float heights, central differences with eps = res / 6
-      const double eps = P.gmap_res / 6.0;
-      o.h = (double)GridMapHeight(P, x, y);
-      o.hx = (double)(GridMapHeight(P, x + eps, y) - GridMapHeight(P, x - eps, y)) / (2 * eps);
-      o.hy = (double)(GridMapHeight(P, x, y + eps) - GridMapHeight(P, x, y - eps)) / (2 * eps);
+      const GridMap M = LoadGridMap(P, TerrainWordMap(word));
+      const double eps = M.res / 6.0;
+      o.h = (double)GridMapHeight(M, x, y);
+      o.hx = (double)(GridMapHeight(M, x + eps, y) - GridMapHeight(M, x - eps, y)) / (2 * eps);
+      o.hy = (double)(GridMapHeight(M, x, y + eps) - GridMapHeight(M, x, y - eps)) / (2 * eps);
       break; }
     case 7: {  // Grid (CSV)
       long long xc, yc;
@@ -531,7 +540,7 @@ __device__ __noinline__ TerrainPoint EvalGridTerrain(const GridArgs P, int id, d
   return o;
 }
 __device__ __forceinline__ TerrainPoint EvalTerrain(const Plan& P, int id, double x, double y) {
-  if (id >= 7) return EvalGridTerrain(GridArgs{P.grid, P.grid_rows, P.grid_cols, P.gmap, P.gmap_sx, P.gmap_sy, P.gmap_res, P.gmap_px, P.gmap_py}, id, x, y);
+  if (id >= 7) return EvalGridTerrain(GridArgs{P.grid, P.grid_rows, P.grid_cols, P.gmap_pool, P.gmaps, P.n_gmaps}, id, x, y);
   TerrainPoint o{0.0, 0.0, 0.0, 0.0};
   switch (id) {
     case 1: {  // Block
@@ -1880,22 +1889,30 @@ __device__ __forceinline__ double PolygonDistance(const double* __restrict__ v, 
   return sqrt(best);
 }
 // thread = (instance, footstep state, foot) of a footstep plan ([b][state][2 + 4 n_ee]): index of the nearest polygon for a
-// foot in contact, -1 for a foot in the air (footstep_plan_extractor.h:106-116) and for unused states
+// foot in contact, -1 for a foot in the air (footstep_plan_extractor.h:106-116) and for unused states.  ranges (optional,
+// [B][2] = first polygon, count): instance b looks only at its own polygons, clamped to [0, n_polys), and gets the index
+// relative to the first of them; null: every instance looks at all n_polys
 __global__ void __launch_bounds__(128) NearestPlaneKernel(const double* __restrict__ plan, const int* __restrict__ n_states, int max_states, int n_ee,
-                                                          const int* __restrict__ poly_offset, int n_polys, const double* __restrict__ verts,
-                                                          int* __restrict__ out, long long total) {
+                                                          const int* __restrict__ poly_offset, int n_polys, const int* __restrict__ ranges,
+                                                          const double* __restrict__ verts, int* __restrict__ out, long long total) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) return;
   const int e = (int)(i % n_ee); const long long bs = i / n_ee; const int st = (int)(bs % max_states); const long long b = bs / max_states;
   const int V = 2 + 4 * n_ee;
   const double* rec = plan + (size_t)bs * V + 2 + 4 * e;
+  int k0 = 0, k1 = n_polys;
+  if (ranges) {
+    const long long first = __ldg(ranges + 2 * b), last = first + __ldg(ranges + 2 * b + 1);
+    k0 = (int)min(max(first, 0ll), (long long)n_polys);
+    k1 = (int)min(max(last, (long long)k0), (long long)n_polys);
+  }
   int idx = -1;
   if (st < n_states[b] && rec[0] != 0.0) {
     double min_distance = 1.7976931348623157e308;   // std::numeric_limits<double>::max(), :70
-    for (int k = 0; k < n_polys; ++k) {
+    for (int k = k0; k < k1; ++k) {
       const int o = __ldg(poly_offset + k), cnt = __ldg(poly_offset + k + 1) - o;
       const double d = PolygonDistance(verts + 2 * (size_t)o, cnt, rec[1], rec[2]);
-      if (d < min_distance) { min_distance = d; idx = k; }
+      if (d < min_distance) { min_distance = d; idx = k - k0; }
     }
   }
   out[i] = idx;
@@ -2181,10 +2198,10 @@ int LaunchFootstepPlan(const Plan& P, const double* x, double* XT, const SplineS
 }
 
 int LaunchNearestPlanes(const double* plan, const int* n_states, int max_states, int n_ee, const int* poly_offset, int n_polys,
-                        const double* verts, int* out, int nb, cudaStream_t s) {
+                        const int* ranges, const double* verts, int* out, int nb, cudaStream_t s) {
   const long long total = (long long)nb * max_states * n_ee;
   if (total <= 0) return 0;
-  NearestPlaneKernel<<<(unsigned)((total + 127) / 128), 128, 0, s>>>(plan, n_states, max_states, n_ee, poly_offset, n_polys, verts, out, total);
+  NearestPlaneKernel<<<(unsigned)((total + 127) / 128), 128, 0, s>>>(plan, n_states, max_states, n_ee, poly_offset, n_polys, ranges, verts, out, total);
   return (int)cudaGetLastError();
 }
 

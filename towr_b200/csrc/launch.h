@@ -33,9 +33,10 @@ int LaunchFootstepPlan(const Plan& P, const double* x, double* XT, const SplineS
                        const int* codes, int n_codes, int n_steps, double time_horizon, int max_states, int* n_states, double* out, int nb,
                        cudaStream_t s);
 // fpowr::NearestPlaneLookup for every (instance, footstep state, foot) of a footstep plan: out[b][state][foot] = index of
-// the nearest polygon (polygon k = vertices poly_offset[k] .. poly_offset[k+1]-1 of verts[][2]) or -1 (foot in the air)
+// the nearest polygon (polygon k = vertices poly_offset[k] .. poly_offset[k+1]-1 of verts[][2]) or -1 (foot in the air);
+// ranges [nb][2] (first, count; may be null = all polygons): instance b's own polygons, index relative to the first of them
 int LaunchNearestPlanes(const double* plan, const int* n_states, int max_states, int n_ee, const int* poly_offset, int n_polys,
-                        const double* verts, int* out, int nb, cudaStream_t s);
+                        const int* ranges, const double* verts, int* out, int nb, cudaStream_t s);
 // towr::LinearEqualityConstraint values g[b][rows] = M x_set (x -> XT first); towr::SoftConstraint cost / gradient of one
 // constraint set from device-resident g / jac
 int LaunchLinearEquality(const Plan& P, const double* x, double* XT, int col0, int n_cols, const double* M, int rows, double* g, int nb, cudaStream_t s);

@@ -298,6 +298,17 @@ def pack_polygons(polygons):
     return offs, verts
 
 
+def pack_polygon_sets(polygon_sets):
+    """One list of polygons per instance (each as pack_polygons takes it) as one shared list: (poly_offsets, vertices,
+    poly_ranges int32 (n_sets, 2)); instance b's polygons are poly_ranges[b, 0] .. poly_ranges[b, 0] + poly_ranges[b, 1] - 1."""
+    counts = np.array([len(s) for s in polygon_sets], np.int64)
+    ranges = np.zeros((len(polygon_sets), 2), np.int32)
+    ranges[:, 1] = counts
+    ranges[1:, 0] = np.cumsum(counts)[:-1]
+    offs, verts = pack_polygons([q for s in polygon_sets for q in s])
+    return offs, verts, ranges
+
+
 def _stream_ptr(stream, tensor):
     import torch
     return C.c_void_p((torch.cuda.current_stream(tensor.device) if stream is None else stream).cuda_stream)
@@ -364,6 +375,17 @@ class Batch:
         """fpowr::ExtractFootstepPlan including the nearest-plane lookup: `polygons` is a list of (k_i, 2) vertex arrays
         (world x, y of the planar regions' boundaries).  Returns (plans, contact_sets): per instance the footstep states
         (see footstep_plans) and an (n_states_b, n_ee) int array — polygon index under every foot in contact, -1 in the air."""
+        offs, verts = pack_polygons(polygons)
+        return self._footstep_contact_sets(x, time_horizon, offs, verts, None)
+
+    def footstep_contact_sets_per_instance(self, x, time_horizon, polygon_sets):
+        """footstep_contact_sets where every instance has its own planar regions: polygon_sets[b] is instance b's list of
+        (k_i, 2) vertex arrays, and its contact sets index into that list."""
+        assert len(polygon_sets) == self.B, "one polygon list per instance"
+        offs, verts, ranges = pack_polygon_sets(polygon_sets)
+        return self._footstep_contact_sets(x, time_horizon, offs, verts, ranges)
+
+    def _footstep_contact_sets(self, x, time_horizon, offs, verts, ranges):
         p = self.problem
         x = np.ascontiguousarray(x, np.float64)
         ms, nv = C.c_int(), C.c_int()
@@ -373,11 +395,13 @@ class Batch:
         count = np.empty(self.B, np.int32)
         check(lib.twb_batch_footstep_plan_host(self._h, x.ctypes.data_as(C.c_void_p), float(time_horizon),
                                                count.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p)))
-        offs, verts = pack_polygons(polygons)
         cs = np.empty((self.B, ms.value, n_ee), np.int32)
-        check(lib.twb_batch_nearest_planes_host(self._h, out.ctypes.data_as(C.c_void_p), count.ctypes.data_as(C.c_void_p),
-                                                offs.ctypes.data_as(C.c_void_p), len(polygons), verts.ctypes.data_as(C.c_void_p),
-                                                cs.ctypes.data_as(C.c_void_p)))
+        ptr = lambda a: a.ctypes.data_as(C.c_void_p)
+        if ranges is None:
+            check(lib.twb_batch_nearest_planes_host(self._h, ptr(out), ptr(count), ptr(offs), len(offs) - 1, ptr(verts), ptr(cs)))
+        else:
+            check(lib.twb_batch_nearest_planes_ranges_host(self._h, ptr(out), ptr(count), ptr(ranges), ptr(offs), len(offs) - 1,
+                                                           ptr(verts), ptr(cs)))
         return [out[b, :count[b]] for b in range(self.B)], [cs[b, :count[b]] for b in range(self.B)]
 
     # ---- device-pointer variants: torch CUDA tensors in and out, only enqueued on `stream` (default: the current one) ----
@@ -453,6 +477,28 @@ class Batch:
                                                   C.c_void_p(vertices.data_ptr()), C.c_void_p(out.data_ptr()), _stream_ptr(stream, plans)))
         return out
 
+    def nearest_planes_ranges_device(self, plans, n_states, poly_ranges, poly_offsets, vertices, out=None, stream=None):
+        """nearest_planes_device where instance b looks only at its own polygons: poly_ranges (B, 2) CUDA int32 = (first
+        polygon, count) of instance b in the shared list (pack_polygon_sets, then moved to the device); the contact sets hold
+        the index relative to that first polygon.  Ranges outside the list are clamped to it (the device cannot check them)."""
+        import torch
+        ms, nv = self.footstep_plan_dims()
+        n_ee = (nv - 2) // 4
+        _check_tensor(plans, torch.float64, (self.B, ms, nv), "plans")
+        _check_tensor(n_states, torch.int32, (self.B,), "n_states")
+        _check_tensor(poly_ranges, torch.int32, (self.B, 2), "poly_ranges")
+        assert poly_offsets.ndim == 1 and poly_offsets.numel() >= 1, "poly_offsets: (n_polys + 1,)"
+        _check_tensor(poly_offsets, torch.int32, (poly_offsets.numel(),), "poly_offsets")
+        _check_tensor(vertices, torch.float64, (vertices.shape[0], 2), "vertices")
+        if out is None:
+            out = torch.empty((self.B, ms, n_ee), dtype=torch.int32, device=plans.device)
+        _check_tensor(out, torch.int32, (self.B, ms, n_ee), "out")
+        check(lib.twb_batch_nearest_planes_ranges_device(self._h, C.c_void_p(plans.data_ptr()), C.c_void_p(n_states.data_ptr()),
+                                                         C.c_void_p(poly_ranges.data_ptr()), C.c_void_p(poly_offsets.data_ptr()),
+                                                         poly_offsets.numel() - 1, C.c_void_p(vertices.data_ptr()),
+                                                         C.c_void_p(out.data_ptr()), _stream_ptr(stream, plans)))
+        return out
+
     def linear_equality(self, x, var_set, M):
         """towr::LinearEqualityConstraint::GetValues for every instance: (B, rows) = M x_set; var_set is a set name."""
         p = self.problem
@@ -501,6 +547,26 @@ class Batch:
         assert h.ndim == 2
         check(lib.twb_batch_set_grid_map(self._h, h.ctypes.data_as(C.POINTER(C.c_float)), h.shape[0], h.shape[1], float(resolution),
                                          float(position[0]), float(position[1])))
+
+    def set_grid_maps(self, maps, map_of_instance=None):
+        """Several GRID_MAP layers for this batch: maps is a list of (heights[ix, iy], resolution, position) tuples as
+        set_grid_map takes them; instance b uses maps[map_of_instance[b]] (None: every instance uses maps[0]).  An empty
+        list removes every map."""
+        if not maps:
+            check(lib.twb_batch_set_grid_maps(self._h, 0, None, None, None, None))
+            return
+        layers = [np.ascontiguousarray(h, np.float32) for h, _, _ in maps]
+        assert all(h.ndim == 2 for h in layers), "heights: 2-D arrays"
+        heights = np.ascontiguousarray(np.concatenate([h.ravel() for h in layers]))
+        sizes = np.array([h.shape for h in layers], np.int32)
+        geometry = np.array([(float(res), float(pos[0]), float(pos[1])) for _, res, pos in maps], np.float64)
+        idx = None
+        if map_of_instance is not None:
+            idx = np.ascontiguousarray(map_of_instance, np.int32)
+            assert idx.shape == (self.B,), "map_of_instance: one map index per instance"
+        check(lib.twb_batch_set_grid_maps(self._h, len(layers), heights.ctypes.data_as(C.POINTER(C.c_float)),
+                                          sizes.ctypes.data_as(C.POINTER(C.c_int)), geometry.ctypes.data_as(C.POINTER(C.c_double)),
+                                          None if idx is None else idx.ctypes.data_as(C.POINTER(C.c_int))))
 
     def launches_per_eval(self, flags=capi.EVAL_ALL):
         return lib.twb_batch_launches_per_eval(self._h, flags)
