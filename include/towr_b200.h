@@ -266,7 +266,14 @@ int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac,
  *   (Js^T Js + mu I) dx = -Js^T (s r) by `cg_iters` conjugate-gradient iterations, x <- clip(x + dx min(1, cap / max|dx|)).
  * x [B][n] in / out, g [B][m] and jac [B][nnz] as written by twb_batch_eval_device, x_lower / x_upper [B][n] per-instance
  * variable bounds (both NULL: the problem's own), violation [B] out = max |s r| before the step (may be NULL).  All device
- * pointers; the call only enqueues on `stream`.  Deterministic (fixed summation orders, no atomics). */
+ * pointers.  Deterministic (fixed summation orders, no atomics).
+ * An instance whose x, g or jac holds a non-finite entry (NaN or +-Inf, e.g. status bit0 of the evaluation) is not stepped:
+ * its x is left exactly as it was and violation[b] is NaN.  The other instances of the batch are not affected.
+ * The call only enqueues on `stream` (no host synchronisation) — except the FIRST call on a batch: it builds the pattern's
+ * transpose on the host and uploads it with cudaMalloc and blocking copies.  After that first call the step can be captured
+ * into a CUDA graph.  Errors: NULL b / x / g / jac, only one of x_lower / x_upper NULL, mu < 0, cap <= 0 (or NaN), cg_iters
+ * outside [0, 10000]: TWB_ERR_INVALID; solver vectors over 200 KiB of shared memory (8 (2 m + 4 n + 32) bytes):
+ * TWB_ERR_UNSUPPORTED.  Nothing is enqueued when a call fails its checks. */
 int twb_batch_lm_step_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower,
                              const double* x_upper, double mu, double cap, int cg_iters, double* violation, void* stream);
 

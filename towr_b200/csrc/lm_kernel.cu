@@ -13,7 +13,11 @@
 // CTAs per SM).  All solver vectors live in shared memory.  Both products walk the ONE sparsity pattern of the structure class:
 // Js p row by row (thread = row), Js^T u column by column through the pattern's transpose (thread = column) — fixed
 // summation orders, no atomics, bit-reproducible.
+// An instance with a non-finite x, g or J entry keeps its x and reports violation NaN.  Left to the step, such an entry would
+// be dropped by fmax (row scale, violation) and a NaN step turned into a bound by the projection: the instance would jump to
+// its bounds and report a finite violation.
 #include <cuda_runtime.h>
+#include <math_constants.h>
 
 #include <cstdint>
 
@@ -68,21 +72,24 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
   const double* __restrict__ g = G + (size_t)b * m;
   // row scales, the scaled values and the scaled violation
   double vmax = 0.0;
+  double chk = 0.0;                           // fma(v, 0, chk): NaN once a v that is not finite has been seen
   for (int q = tid; q < m; q += nt) {
     const int i = __ldg(pat.row_order + q);   // rows in descending length: the lanes of a warp walk rows of similar length
     const int k0 = __ldg(pat.row_ptr + i), k1 = __ldg(pat.row_ptr + i + 1);
     double big = 0.0;
-    for (int k = k0; k < k1; ++k) big = fmax(big, fabs(J[k]));
+    for (int k = k0; k < k1; ++k) { const double v = J[k]; big = fmax(big, fabs(v)); chk = fma(v, 0.0, chk); }
     const double si = 1.0 / fmax(big, 1.0);
     if (kSmemJ) for (int k = k0; k < k1; ++k) Js[k] = J[k] * si;
     const double gi = g[i], lo = __ldg(pat.g_lower + i), up = __ldg(pat.g_upper + i);
     const double r = gi < lo ? gi - lo : gi > up ? gi - up : 0.0;
+    chk = fma(gi, 0.0, chk);
     s[i] = si;
     const double rs = si * r;
     u[i] = rs;
     vmax = fmax(vmax, fabs(rs));
   }
   vmax = BlockMax(vmax, scratch);        // (also orders the writes of s, u, Js)
+  const bool finite_gj = BlockMax(chk != chk ? 1.0 : 0.0, scratch) == 0.0;
   auto row_dot = [&](int i) {            // (Js p)_i
     double acc = 0.0;
     const int k0 = __ldg(pat.row_ptr + i), k1 = __ldg(pat.row_ptr + i + 1);
@@ -133,15 +140,17 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
     rr = rr_new;
     __syncthreads();
   }
-  double big = 0.0;
-  for (int j = tid; j < n; j += nt) big = fmax(big, fabs(dx[j]));
+  double big = 0.0, chk_x = 0.0;
+  for (int j = tid; j < n; j += nt) { big = fmax(big, fabs(dx[j])); chk_x = fma(X[(size_t)b * n + j], 0.0, chk_x); }
   big = BlockMax(big, scratch);
+  const bool finite = BlockMax(chk_x != chk_x ? 1.0 : 0.0, scratch) == 0.0 && finite_gj;
   const double scale = big > cap ? cap / big : 1.0;
   double* x = X + (size_t)b * n;
   const double* lo = x_lower + (size_t)b * bound_stride;
   const double* up = x_upper + (size_t)b * bound_stride;
-  for (int j = tid; j < n; j += nt) x[j] = fmin(fmax(x[j] + dx[j] * scale, lo[j]), up[j]);
-  if (tid == 0 && violation) violation[b] = vmax;
+  if (finite)
+    for (int j = tid; j < n; j += nt) x[j] = fmin(fmax(x[j] + dx[j] * scale, lo[j]), up[j]);
+  if (tid == 0 && violation) violation[b] = finite ? vmax : CUDART_NAN;
 }
 
 template <bool kSmemJ, class Idx>
@@ -169,8 +178,8 @@ int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const d
     return smem_j ? LaunchLm<true>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s)
                   : LaunchLm<false>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s);
   }
-  return smem_j ? LaunchLm<true>(pat, pat.col_idx, pat.slot_t, pat.row_t, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s)
-                : LaunchLm<false>(pat, pat.col_idx, pat.slot_t, pat.row_t, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s);
+  // 32-bit indices mean n, m or nnz >= 65 536, so with_j >= 8 * 65 536 bytes > 220 KiB: never the shared-memory Js path
+  return LaunchLm<false>(pat, pat.col_idx, pat.slot_t, pat.row_t, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s);
 }
 
 }  // namespace twb

@@ -12,8 +12,11 @@ restoration phase minimises — for every instance of a batch in lock step:
 The iterates, g, the Jacobian values and all solver vectors stay on the GPU.  An iteration is two library calls:
 `twb_batch_eval_device` (g and the CSR Jacobian values of all instances) and `twb_batch_lm_step_device`
 (towr_b200/csrc/lm_kernel.cu: CTA = instance, the conjugate gradients run in shared memory on the problem's ONE shared
-CSR pattern and its transpose, fixed summation orders, no atomics).  `native=False` keeps the first implementation of the
-same step in PyTorch tensor algebra (padded ELL gathers) — 30 x slower, used by the tests as a second opinion.
+CSR pattern and its transpose, fixed summation orders, no atomics).  An instance whose x, g or Jacobian values hold a
+non-finite entry (the evaluation flags it in `status` bit 0) is not stepped by the native step: its x stays exactly as it
+was and its violation is NaN, so the caller can tell it apart instead of finding it clipped to its bounds.
+`native=False` keeps the first implementation of the same step in PyTorch tensor algebra (padded ELL gathers) — 30 x
+slower, used by the tests as a second opinion.
 tests/test_solver_loop.py holds the same algorithm in numpy, driven one instance at a time like ifopt by the CPU
 restatement of the reference; all three must walk the same iterates.
 """
