@@ -13,5 +13,5 @@ fi
 timeout 900 python bench.py --steps 50 --warmup 5 > $OUT/bench.json 2> $OUT/bench.err; echo "bench rc=$?"
 cat $OUT/bench.json
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 200 --csv --log-file $OUT/launches.csv python bench.py --quick --steps 3 --warmup 3 > $OUT/ncu_launches.log 2>&1; echo "ncu launches rc=$?"
-timeout 900 ncu --set full --clock-control none --import-source on -k regex:'DynOut|RomNodeOut|TransposeIn|TransposeOut' --launch-skip 12 --launch-count 4 -o $OUT/full python bench.py --quick --steps 3 --warmup 3 > $OUT/ncu_full.log 2>&1; echo "ncu full rc=$?"
+timeout 900 ncu --set full --clock-control none --import-source on -k regex:'DynOut|RomNodeOut|TransposeIn' --launch-skip 12 --launch-count 4 -o $OUT/full python bench.py --quick --steps 3 --warmup 3 > $OUT/ncu_full.log 2>&1; echo "ncu full rc=$?"
 ls -la $OUT

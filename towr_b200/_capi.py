@@ -11,7 +11,7 @@ from ._spec import *   # noqa: F401,F403  (Spec, the enums and size limits)
 from ._spec import Spec
 
 
-# TWB_LIB: developer knob for tuning sweeps (scripts/build_variants.sh) — another build of the same library
+# TWB_LIB: path of another build of the same library (for example the parent commit's), to compare outputs and timings
 LIB_PATH = os.environ.get("TWB_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "libtowr_b200.so")
 
 

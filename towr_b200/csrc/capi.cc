@@ -78,8 +78,6 @@ struct twb_batch {
   float* d_gmap_pool = nullptr;   // elevation layers of TWB_GRID_MAP, back to back (optional)
   twb::GridMapDesc* d_gmaps = nullptr;   // one descriptor per layer
   double* d_XT = nullptr;         // [ld/32][n+1][32] instance-tiled iterates; row n == 0
-  double* d_GT = nullptr;         // [ld/32][m][32] instance-tiled constraint values (staging of g)
-  int* d_TD = nullptr;            // [ld/32] per-tile completion counters of the output kernels (zero between evaluations)
   double* d_FS = nullptr;         // [ld/32][n_dyn][6 n_ee][32] feet positions / forces per dynamic sample (optimised durations only)
   // staging for the host-pointer variant
   double *d_x = nullptr, *d_g = nullptr, *d_jac = nullptr, *d_cost = nullptr, *d_grad = nullptr;
@@ -90,8 +88,6 @@ struct twb_batch {
   int e2e_chunk = 512;                            // instances per chunk of twb_batch_eval_host (TWB_E2E_CHUNK)
   std::vector<cudaEvent_t> ev;    // fork/join events of the two-stream pipeline
   int launches_last = 0;
-  cudaAccessPolicyWindow l2_window{};            // XT + GT persisting in the L2 (experiment, TWB_L2_PERSIST=1)
-  bool use_l2_window = false;
   std::vector<std::pair<void*, size_t>> scratch;   // device scratch of the post-processing calls, grown on demand, freed with the batch
   // CUDA graphs of twb_batch_eval_device: one evaluation is 4 - 6 kernels on three streams joined by events; replayed as a
   // graph, the dependencies are resolved on the device instead of through cross-stream event waits.  One instantiated graph
@@ -423,17 +419,8 @@ int twb_batch_create(const twb_problem* p, int batch_size, int device, twb_batch
   const size_t group = 32 * (size_t)std::max(b->plan.nc_jac, 1);
   b->ld = ((size_t)batch_size + group - 1) / group * group;
   const size_t xt_bytes = (size_t)(b->plan.n + 1) * b->ld * sizeof(double);
-  // XT and GT live in ONE allocation, so that one L2 access-policy window can cover both staging matrices (TWB_L2_PERSIST=1;
-  // measured, profiles/README.md experiment 39: marking them persisting makes the step SLOWER, 175 instead of 139 us — off)
-  const size_t xt_padded = (xt_bytes + 255) & ~(size_t)255, gt_bytes = (size_t)std::max(b->plan.m, 1) * b->ld * sizeof(double);
-  if ((e = cudaMalloc(reinterpret_cast<void**>(&b->d_XT), xt_padded + gt_bytes)) != cudaSuccess ||
+  if ((e = cudaMalloc(reinterpret_cast<void**>(&b->d_XT), xt_bytes)) != cudaSuccess ||
       (e = cudaMemset(b->d_XT, 0, xt_bytes)) != cudaSuccess) {
-    twb_batch_destroy(b);
-    return CudaFail(e, "state allocation");
-  }
-  b->d_GT = reinterpret_cast<double*>(reinterpret_cast<char*>(b->d_XT) + xt_padded);
-  if ((e = cudaMalloc(reinterpret_cast<void**>(&b->d_TD), sizeof(int) * (b->ld / 32))) != cudaSuccess ||
-      (e = cudaMemset(b->d_TD, 0, sizeof(int) * (b->ld / 32))) != cudaSuccess) {
     twb_batch_destroy(b);
     return CudaFail(e, "state allocation");
   }
@@ -441,21 +428,6 @@ int twb_batch_create(const twb_problem* p, int batch_size, int device, twb_batch
       (e = cudaMalloc(reinterpret_cast<void**>(&b->d_FS), (size_t)b->plan.n_dyn * 6 * b->plan.n_ee * b->ld * sizeof(double))) != cudaSuccess) {
     twb_batch_destroy(b);
     return CudaFail(e, "state allocation");
-  }
-  {
-    const char* v = std::getenv("TWB_L2_PERSIST");
-    cudaDeviceProp prop{};
-    if (v && std::atoi(v) != 0 && cudaGetDeviceProperties(&prop, device) == cudaSuccess && prop.persistingL2CacheMaxSize > 0) {
-      const size_t want = xt_padded + gt_bytes, cap = (size_t)prop.persistingL2CacheMaxSize;
-      size_t cur = 0; cudaDeviceGetLimit(&cur, cudaLimitPersistingL2CacheSize);
-      if (cur < std::min(want, cap)) cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, std::min(want, cap));
-      b->l2_window.base_ptr = b->d_XT;
-      b->l2_window.num_bytes = std::min(want, (size_t)prop.accessPolicyMaxWindowSize);
-      b->l2_window.hitRatio = want <= cap ? 1.0f : (float)((double)cap / (double)want);
-      b->l2_window.hitProp = cudaAccessPropertyPersisting;
-      b->l2_window.missProp = cudaAccessPropertyNormal;
-      b->use_l2_window = true;
-    }
   }
   if ((e = cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking)) != cudaSuccess ||
       (e = cudaStreamCreateWithFlags(&b->aux0, cudaStreamNonBlocking)) != cudaSuccess ||
@@ -477,11 +449,10 @@ void twb_batch_destroy(twb_batch* b) {
   if (!b) return;
   cudaSetDevice(b->device);
   DropGraphs(b);
-  if (b->use_l2_window) cudaCtxResetPersistingL2Cache();   // lines of XT / GT must not stay pinned in the L2 after the batch is gone
   for (void* p : b->owned) cudaFree(p);
   for (auto& sc : b->scratch) cudaFree(sc.first);
   for (auto& t : b->post_tables) cudaFree(t.mem);
-  cudaFree(b->d_terrain); cudaFree(b->d_grid); cudaFree(b->d_gmap_pool); cudaFree(b->d_gmaps); cudaFree(b->d_XT); cudaFree(b->d_FS); cudaFree(b->d_TD);   // (d_GT is part of d_XT's allocation)
+  cudaFree(b->d_terrain); cudaFree(b->d_grid); cudaFree(b->d_gmap_pool); cudaFree(b->d_gmaps); cudaFree(b->d_XT); cudaFree(b->d_FS);
   for (auto ev : b->ev) if (ev) cudaEventDestroy(ev);
   if (b->aux0) cudaStreamDestroy(b->aux0);
   if (b->aux1) cudaStreamDestroy(b->aux1);
@@ -791,9 +762,8 @@ int twb_batch_launches_per_eval(const twb_batch* b, unsigned flags) {
   const twb::Plan& p = b->plan;
   const bool want_cost = b->prob->f.has_cost && (flags & TWB_EVAL_COST);
   int n = 1;   // TransposeIn
-  if (flags & (TWB_EVAL_G | TWB_EVAL_JAC)) n += twb::OutKernelsPerEval(p, flags);   // DynOut [+ DynTailOut] + RomNodeOut (or RomOut, NodeOut)
+  if (flags & (TWB_EVAL_G | TWB_EVAL_JAC)) n += twb::OutKernelsPerEval(p, flags);   // DynOut [+ DynTailOut] + RomNodeOut
   if ((flags & (TWB_EVAL_G | TWB_EVAL_JAC)) && p.n_phase_units > 0) n += 1;   // PhaseJac
-  if (flags & TWB_EVAL_G) n += twb::TransposeOutPerEval(p);   // TransposeOut (not with fixed durations: the values are written directly)
   if (want_cost) n += 1;
   {   // large batches are evaluated chunk after chunk (twb_batch::eval_chunk)
     const size_t B = (size_t)b->B, chunk = EvalChunk(b);
@@ -815,7 +785,6 @@ int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac,
   unsigned kflags = flags & (TWB_EVAL_G | TWB_EVAL_JAC);
   if (f.has_cost && (flags & TWB_EVAL_COST)) kflags |= TWB_EVAL_COST;
   int launches = 0;
-  twb::SetL2Window(b->use_l2_window ? &b->l2_window : nullptr);
   // the whole batch, or chunk after chunk (twb_batch::eval_chunk), enqueued on s0 and the batch's two auxiliary streams
   auto enqueue = [&](cudaStream_t s0) -> int {
     const size_t B = (size_t)b->B;
@@ -823,8 +792,8 @@ int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac,
     const size_t n = f.n, m = f.m;
     for (size_t off = 0; off < B; off += chunk) {
       const size_t nb = std::min(chunk, B - off), t0 = off / 32;
-      const int rc = twb::LaunchEval(b->plan, x + off * n, b->d_XT + t0 * (n + 1) * 32, b->d_GT + t0 * (size_t)std::max(f.m, 1) * 32,
-                                     b->d_FS ? b->d_FS + t0 * (size_t)b->plan.n_dyn * 6 * b->plan.n_ee * 32 : nullptr, b->d_TD + t0,
+      const int rc = twb::LaunchEval(b->plan, x + off * n, b->d_XT + t0 * (n + 1) * 32,
+                                     b->d_FS ? b->d_FS + t0 * (size_t)b->plan.n_dyn * 6 * b->plan.n_ee * 32 : nullptr,
                                      g ? g + off * m : nullptr, jac ? jac + off * (size_t)f.nnz : nullptr, cost ? cost + off : nullptr,
                                      grad ? grad + off * n : nullptr, status ? status + off : nullptr,
                                      b->d_terrain ? b->d_terrain + off : nullptr, f.spec.terrain, (int)nb, kflags, s0, b->aux0, b->aux1, b->ev.data(), &launches);
@@ -950,15 +919,14 @@ int twb_batch_eval_host(twb_batch* b, const double* x, double* g, double* jac, d
   unsigned kflags = flags & (TWB_EVAL_G | TWB_EVAL_JAC);
   if (has_cost) kflags |= TWB_EVAL_COST;
   int launches = 0;
-  twb::SetL2Window(b->use_l2_window ? &b->l2_window : nullptr);
   for (size_t c = 0; c < n_chunks; ++c) {
     const size_t off = c * chunk, nb = std::min(chunk, B - off), tile0 = off / 32;
     if ((e = cudaMemcpyAsync(b->d_x + off * f.n, x + off * f.n, sizeof(double) * nb * f.n, cudaMemcpyHostToDevice, b->s_in)) != cudaSuccess)
       return CudaFail(e, "H2D copy");
     cudaEventRecord(b->ev_chunk[2 * c], b->s_in);
     cudaStreamWaitEvent(s, b->ev_chunk[2 * c], 0);
-    int rc = twb::LaunchEval(b->plan, b->d_x + off * f.n, b->d_XT + tile0 * (size_t)(f.n + 1) * 32, b->d_GT + tile0 * (size_t)std::max(f.m, 1) * 32,
-                             b->d_FS ? b->d_FS + tile0 * (size_t)b->plan.n_dyn * 6 * b->plan.n_ee * 32 : nullptr, b->d_TD + tile0,
+    int rc = twb::LaunchEval(b->plan, b->d_x + off * f.n, b->d_XT + tile0 * (size_t)(f.n + 1) * 32,
+                             b->d_FS ? b->d_FS + tile0 * (size_t)b->plan.n_dyn * 6 * b->plan.n_ee * 32 : nullptr,
                              (flags & TWB_EVAL_G) ? b->d_g + off * f.m : nullptr, (flags & TWB_EVAL_JAC) ? b->d_jac + off * f.nnz : nullptr,
                              has_cost ? b->d_cost + off : nullptr, has_cost ? b->d_grad + off * f.n : nullptr, b->d_status + off,
                              b->d_terrain ? b->d_terrain + off : nullptr, f.spec.terrain, (int)nb, kflags, s, b->aux0, b->aux1, b->ev.data(), &launches);

@@ -64,8 +64,7 @@ struct PhaseUnit {
 // by the CTA that owns its last element; only sectors shared with another CTA fall back to 8-byte single-element
 // stores.  The alignment of an instance's row inside its sectors depends on (instance * row length) mod 4, so a
 // list exists per alignment class q = instance mod n_classes (n_classes = 1 when the row length is a multiple of 4).
-// The constraint values are written by the CTAs as well (kernels.cu: StoreValuesDirect); the instance-tiled staging matrix GT
-// of round 1 survives in the -DTWB_GDIRECT=0 variants.
+// The constraint values are written by the CTAs as well (kernels.cu: StoreValuesDirect).
 constexpr int kMaxClasses = 4;
 // ---- phase elements (optimised phase durations) ----------------------------------------------------------------------
 // With PhaseSplines a constraint sample's row is structurally dense in ALL node variables of the foot's set
@@ -92,13 +91,7 @@ constexpr int kMaxClasses = 4;
 enum PhaseElemKind : uint32_t { kElemPlain = 0, kElemNode = 1, kElemDuration = 2 };
 struct PhaseExt { uint32_t e0, e1; };
 constexpr int kInfoRows = 12;
-#ifndef TWB_DYN_DURWIN
-#define TWB_DYN_DURWIN 2
-#endif
-#ifndef TWB_ROM_DURWIN
-#define TWB_ROM_DURWIN 2
-#endif
-constexpr int kDynDurWin = TWB_DYN_DURWIN, kRomDurWin = TWB_ROM_DURWIN;   // duration columns finished per instance (window form) in DynTailOut / RomBody
+constexpr int kDynDurWin = 2, kRomDurWin = 2;   // duration columns finished per instance (window form) in DynTailOut / RomBody
 // state rows of one foot in the DynTailOut kernel: 0: 1 | 1..3: f_e | 4..6: c - p_e | 7..18: info block of ee-motion_e |
 // 19..30: info block of ee-force_e | 31..36: U | 37..54: X   (duration columns of the sample's 6 rows)
 constexpr int kTailRows = 7 + 2 * kInfoRows + 6 + 6 * kDynDurWin;
@@ -115,65 +108,24 @@ struct OutList {                        // per alignment class
   OutRange pairs[kMaxClasses];          // whole sectors, two pairs each
   OutRange singles[kMaxClasses];        // single elements (lane = instance)
   OutRange phase[kMaxClasses];          // whole sectors that hold at least one phase element (same layout as `pairs`, with Plan::exts)
-  // TMA store path: when the pairs of a class form ONE contiguous run of the row (pair i covers elements run_off + 2i,
-  // run_off + 2i + 1 — the normal case: a CTA owns adjacent CSR rows), the CTA assembles the run in shared memory in
-  // output order and writes it with one cp.async.bulk per instance; -1: not contiguous, 16-byte st.global path
-  int32_t run_off[kMaxClasses];
 };
-// Range-of-motion state block: [0]=1 | R^T (9) | buffers of { D_e (9) | g_e (3) }.  TWB_ROM_ALLFEET = 0: two buffers
-// used by the feet in turn (one CTA barrier and one list per foot); 1: one buffer per foot (one barrier, one list).
-#ifndef TWB_ROM_ALLFEET
-#define TWB_ROM_ALLFEET 0
-#endif
-// With optimised phase durations a foot's buffer is D_e (9) | info block of its PhaseSpline (kInfoRows) | U (3) | X (3 kRomDurWin).
+// Range-of-motion state block: [0]=1 | R^T (9) | two buffers of { D_e (9) | g_e (3) } used by the feet in turn (one CTA
+// barrier and one list per foot).  With optimised phase durations a foot's buffer is D_e (9) | info block of its PhaseSpline
+// (kInfoRows) | U (3) | X (3 kRomDurWin).
 #define RomBufRows(phase) ((phase) ? 9 + kInfoRows + 3 + 3 * kRomDurWin : 12)
-#define RomBufferP(e, phase) (TWB_ROM_ALLFEET ? RomBufRows(phase) * (e) : RomBufRows(phase) * ((e) & 1))   /* first row of foot e's buffer, relative to row 10 */
-#define RomBlockRowsP(n_ee, phase) (10 + RomBufRows(phase) * (TWB_ROM_ALLFEET ? (n_ee) : 2))
-#define RomBuffer(e) RomBufferP(e, false)
-#define RomBlockRows(n_ee) RomBlockRowsP(n_ee, false)
-#define RomListsPerCta(n_ee) (TWB_ROM_ALLFEET ? 1 : (n_ee))
+#define RomBufferP(e, phase) (RomBufRows(phase) * ((e) & 1))   /* first row of foot e's buffer, relative to row 10 */
+#define RomBlockRowsP(n_ee, phase) (10 + RomBufRows(phase) * 2)
 
-// TWB_GDIRECT = 1 (fixed durations): the constraint values leave the output kernels straight into g[B][m] — after the CTA
-// barrier all threads write the CTA's consecutive rows (24 per dynamic CTA, 12 per range-of-motion CTA and foot) with
-// consecutive threads = consecutive rows of one instance; no GT staging matrix, no TransposeOut kernel.  The dynamic unit then
-// keeps its 6 values in 6 more state rows.  0: values staged instance-tiled in GT, transposed by TransposeOut.
-#ifndef TWB_GDIRECT
-#define TWB_GDIRECT 1
-#endif
-#define DynBlockRows(n_ee) (40 + 6 * (n_ee) + (TWB_GDIRECT ? 6 : 0))   /* 1 | 3 | 36 | 6 per foot [| 6 values] */
+// The constraint values leave the output kernels straight into g[B][m]: after the CTA barrier all threads write the CTA's
+// consecutive rows (24 per dynamic CTA, 12 per range-of-motion CTA and foot) with consecutive threads = consecutive rows of
+// one instance.  The dynamic unit keeps its 6 values in 6 more state rows.
+#define DynBlockRows(n_ee) (46 + 6 * (n_ee))   /* 1 | 3 | 36 | 6 per foot | 6 values */
 
-// warps per CTA of the output kernels = consecutive units whose output ranges are chained through carry rows.
-// TWB_FUSED = 1: one kernel (EvalOut) serves all three unit kinds with CTAs of TWB_WARPS warps.
-#ifndef TWB_FUSED
-#define TWB_FUSED 0
-#endif
-#if TWB_FUSED
-#ifndef TWB_WARPS
-#define TWB_WARPS 5
-#endif
-#define TWB_ROMNODE 0
-constexpr int kWarps = TWB_WARPS;
-constexpr int kDynWarps = kWarps, kRomWarps = kWarps, kNodeWarps = kWarps;
-#else
-#ifndef TWB_DYN_WARPS
-#define TWB_DYN_WARPS 4
-#endif
-// TWB_ROMNODE = 1 (default): the range-of-motion and node CTAs of a tile run in ONE kernel (RomNodeOut, equal CTA sizes),
-// so that the CTAs resident at any moment fill long contiguous stretches of the tile's rows; the dynamic samples
-// (different register budget) keep their own kernel on a second stream.
-#ifndef TWB_ROMNODE
-#define TWB_ROMNODE 1
-#endif
-#ifndef TWB_ROM_WARPS
-#define TWB_ROM_WARPS 4
-#endif
-#ifndef TWB_NODE_WARPS
-#define TWB_NODE_WARPS (TWB_ROMNODE ? TWB_ROM_WARPS : 8)
-#endif
-constexpr int kDynWarps = TWB_DYN_WARPS;     // consecutive dynamic samples per CTA (one instance tile)
-constexpr int kRomWarps = TWB_ROM_WARPS;     // consecutive range-of-motion samples per CTA
-constexpr int kNodeWarps = TWB_NODE_WARPS;   // consecutive node groups per CTA
-#endif
+// warps per CTA of the output kernels = consecutive units whose output ranges are chained through carry rows.  The
+// range-of-motion and node CTAs of a tile run in ONE kernel (RomNodeOut) and need equal CTA sizes.
+constexpr int kDynWarps = 4;    // consecutive dynamic samples per CTA (one instance tile)
+constexpr int kRomWarps = 4;    // consecutive range-of-motion samples per CTA
+constexpr int kNodeWarps = 4;   // consecutive node groups per CTA
 
 // TerrainConstraint row (terrain_constraint.cc:59-108): one ee-motion node.
 // local state: [base + 0] = -dh/dx, [base + 1] = -dh/dy, g at [g_base]
@@ -194,10 +146,10 @@ struct BaseMotionUnit { int32_t sample_lin, sample_ang; };
 
 // A dynamic sample (6 rows): 2 + 2 n_ee spline samples starting at `sample0`
 // (base-lin, base-ang, ee-motion.., ee-force..) and its output lists.
-struct DynUnit { int32_t sample0; int32_t g_row0; OutRange values; };   // g_row0: first of the sample's 6 constraint rows
+struct DynUnit { int32_t sample0; int32_t g_row0; };   // g_row0: first of the sample's 6 constraint rows
 // A range-of-motion sample (3 rows for every foot): 2 + n_ee spline samples (base-lin, base-ang, ee-motion..);
-// the feet are evaluated and written one after the other (values[foot]: the foot's constraint values).
-struct RomUnit { int32_t sample0; int32_t pad; OutRange values[kMaxEE]; };
+// the feet are evaluated and written one after the other.
+struct RomUnit { int32_t sample0; };
 
 // Node-wise work of one warp: `count` consecutive units of one kind evaluated into one state block,
 // then one pass over the group's output lists.
@@ -264,10 +216,9 @@ struct Plan {
   int n, m, nnz, n_ee;
   int n_dyn, n_rom, n_groups, n_cost;
   int node_rows, dyn_rows, rom_rows;   // state rows of one unit's block: node groups (largest), dynamic samples, range-of-motion samples
-  int nc_jac, nc_g;   // alignment classes of the Jacobian-value rows (length nnz); nc_g = 1 (unused)
+  int nc_jac;         // alignment classes of the Jacobian-value rows (length nnz)
   int dyn_list0, rom_list0, node_list0;   // first entry of cta_lists of the dynamic CTAs, (rom CTA, foot) pairs, node CTAs
   int tail_list0;                         // optimised durations: list of dynamic sample k's PhaseSpline columns (DynTailOut) = tail_list0 + k
-  int stage_dyn, stage_rom, stage_node;   // longest contiguous run (in doubles, even) of a dynamic / range-of-motion / node list: staging row of the TMA store path
   int rom_row0[kMaxEE];                   // first constraint row of foot e's range-of-motion set (sample k owns rows rom_row0[e] + 3k ..+2)
   // robot
   double mass, gravity;

@@ -18,7 +18,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstdlib>
 #include <map>
 #include <numeric>
 
@@ -174,13 +173,6 @@ std::vector<double> BasePolyDurations(double T, double dt) {  // parameters.cc:8
   return v;
 }
 
-// tuning knob read from the environment (clamped); the default is what ships
-int EnvInt(const char* name, int def, int lo, int hi) {
-  const char* v = std::getenv(name);
-  if (!v || !*v) return def;
-  return std::max(lo, std::min(hi, std::atoi(v)));
-}
-
 // a: local state row of the owning unit (0 = the constant 1); ext: phase-element word (device_tables.h: PhaseExt) with the
 // info row local to the unit as well; tail >= 0: element of dynamic sample `tail` written by the DynTailOut kernel (a and
 // the info row are then rows of that kernel's CTA)
@@ -191,8 +183,7 @@ uint32_t PackExt(uint32_t kind, int deriv, bool shared, int a_or_ph, uint32_t in
 
 // Who computes a constraint row: a dynamic sample, a range-of-motion sample (all feet) or a node unit.
 enum OwnerKind { kOwnDyn, kOwnRom, kOwnNode, kOwnPhase };   // kOwnPhase: rows written by the PhaseJac kernel (total duration)
-struct RowOwner { int kind = -1, index = -1; uint32_t g_local = 0; };   // g_local: state row of the row's value inside the unit
-constexpr uint32_t kDirectValue = 0xFFFFFFFFu;   // the unit writes this row's value straight into GT (no state row)
+struct RowOwner { int kind = -1, index = -1; uint32_t g_local = 0; };   // g_local: state row of a node unit's value inside the unit
 // node unit before grouping: kind, index into its table, rows of local state / values it needs
 struct NodeUnitRef { int kind, index, n_state, n_g, set_id; };
 
@@ -568,14 +559,14 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
         std::vector<double> ts = SampleTimes(T, sp.dt_constraint_dynamic);
         int r0 = add_set("dynamic", (int)ts.size() * 6);
         pl.n_dyn = (int)ts.size();
-        // local state: [0]=1 | sum f (3) | base-ang block (36) | f_e, c-p_e (6 per foot); the 6 constraint values go straight to GT
+        // local state: [0]=1 | sum f (3) | base-ang block (36) | f_e, c-p_e (6 per foot) | the 6 constraint values
         for (int k = 0; k < pl.n_dyn; ++k) {
           const double t = ts[k];
           const int row = r0 + 6 * k;
           const uint32_t sb = 1;
           DynUnit du{}; du.sample0 = (int32_t)tb.samples.size(); du.g_row0 = row;
           tb.dyn.push_back(du);
-          for (int r = 0; r < 6; ++r) { bound(row + r, 0.0, 0.0); own(row + r, kOwnDyn, k, kDirectValue); }
+          for (int r = 0; r < 6; ++r) { bound(row + r, 0.0, 0.0); own(row + r, kOwnDyn, k, 0); }
           // spline samples: base-lin, base-ang, ee-motion.., ee-force..
           tb.samples.push_back(MakeSample(sp_lin, t, zero_slot));
           tb.samples.push_back(MakeSample(sp_ang, t, zero_slot));
@@ -664,11 +655,10 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
           pl.rom_row0[e] = r0;
           for (int k = 0; k < pl.n_rom; ++k) {
             const double t = ts[k]; const int row = r0 + 3 * k;
-            // (with optimised durations the foot's values exist in registers only: G0 is a placeholder)
-            const uint32_t sb = 1, sd = 10 + RomBufferP(e, optimize_timings), G0 = optimize_timings ? sd : 19 + RomBufferP(e, optimize_timings);
+            const uint32_t sb = 1, sd = 10 + RomBufferP(e, optimize_timings);
             for (int d = 0; d < 3; ++d) {
               bound(row + d, (0.0 + rb.nominal[e][d]) - rb.max_dev[d], (0.0 + rb.nominal[e][d]) + rb.max_dev[d]);
-              own(row + d, kOwnRom, k * n_ee + e, G0 + d);
+              own(row + d, kOwnRom, k * n_ee + e, 0);
             }
             int p; double tl;
             Locate(sp_lin, t, &p, &tl);   // -R^T dc
@@ -851,8 +841,7 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
   std::vector<GroupBuild> groups;
   std::vector<int> unit_group(node_units.size(), -1), unit_state0(node_units.size(), 0), unit_g0(node_units.size(), 0);
   {
-    const int force_cap = EnvInt("TWB_FORCE_CAP", 1, 1, 2);
-    auto cap = [&](int kind) { return kind == kGroupForce ? force_cap : kind == kGroupTerrain ? 10 : kind == kGroupSwing ? 7 : kind == kGroupAcc ? 10 : 5; };
+    auto cap = [&](int kind) { return kind == kGroupForce ? 1 : kind == kGroupTerrain ? 10 : kind == kGroupSwing ? 7 : kind == kGroupAcc ? 10 : 5; };
     for (size_t u = 0; u < node_units.size(); ++u) {
       const NodeUnitRef& nu = node_units[u];
       bool open = !groups.empty() && groups.back().kind == nu.kind && groups.back().count < cap(nu.kind) &&
@@ -876,7 +865,8 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
   // combined list of 16-byte pairs (`d` = row in the CTA's shared memory = warp * block_rows + local row).  Every
   // 32-byte sector is written whole by the list that owns its last element; only sectors shared with another CTA (or a
   // row of the PhaseJac kernel, or the ends of the row) fall back to single-element stores.  The constraint values
-  // are per unit (lane = instance, into GT).
+  // are written from the units' state rows (kernels.cu: StoreValuesDirect); only a node group's rows that are not
+  // consecutive state rows need a table (NodeGroup::values).
   const int n_rom_blocks = pl.n_rom * n_ee, n_blocks = pl.n_dyn + n_rom_blocks + (int)groups.size();
   auto block_id = [&](const RowOwner& o) {   // global block number: dynamic samples | (rom sample, foot) | node groups; -1: not an output-kernel row
     if (o.kind == kOwnPhase) return -1;
@@ -886,32 +876,33 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
   };
   const int n_dyn_ctas = (pl.n_dyn + kDynWarps - 1) / kDynWarps, n_rom_ctas = (pl.n_rom + kRomWarps - 1) / kRomWarps;
   const int n_node_ctas = ((int)groups.size() + kNodeWarps - 1) / kNodeWarps;
-  const int rom_lists = RomListsPerCta(n_ee);
-  const int tail_list0 = n_dyn_ctas + n_rom_ctas * rom_lists + n_node_ctas;
-  const int n_lists = tail_list0 + (optimize_timings ? pl.n_dyn : 0);   // dynamic CTAs | (rom CTA[, foot]) | node CTAs | PhaseSpline columns of dynamic sample k
+  const int tail_list0 = n_dyn_ctas + n_rom_ctas * n_ee + n_node_ctas;
+  const int n_lists = tail_list0 + (optimize_timings ? pl.n_dyn : 0);   // dynamic CTAs | (rom CTA, foot) | node CTAs | PhaseSpline columns of dynamic sample k
   pl.tail_list0 = tail_list0;
   pl.dyn_rows = DynBlockRows(n_ee); pl.rom_rows = RomBlockRowsP(n_ee, optimize_timings);
   std::vector<int> list_of(n_blocks, -1), row_base(n_blocks, 0);   // list a block's elements belong to; first row of the block inside its CTA
   for (int k = 0; k < pl.n_dyn; ++k) { list_of[k] = k / kDynWarps; row_base[k] = (k % kDynWarps) * pl.dyn_rows; }
   for (int k = 0; k < pl.n_rom; ++k) for (int e = 0; e < n_ee; ++e) {
     const int b = pl.n_dyn + k * n_ee + e;
-    list_of[b] = n_dyn_ctas + (k / kRomWarps) * rom_lists + (rom_lists > 1 ? e : 0); row_base[b] = (k % kRomWarps) * pl.rom_rows;
+    list_of[b] = n_dyn_ctas + (k / kRomWarps) * n_ee + e; row_base[b] = (k % kRomWarps) * pl.rom_rows;
   }
   for (int gi = 0; gi < (int)groups.size(); ++gi) {
     const int b = pl.n_dyn + n_rom_blocks + gi;
-    list_of[b] = n_dyn_ctas + n_rom_ctas * rom_lists + gi / kNodeWarps; row_base[b] = (gi % kNodeWarps) * pl.node_rows;
+    list_of[b] = n_dyn_ctas + n_rom_ctas * n_ee + gi / kNodeWarps; row_base[b] = (gi % kNodeWarps) * pl.node_rows;
   }
   struct Elem { int list; uint16_t d; double c; uint32_t ext; };
   std::vector<Elem> elems(nnz);
   struct Entry { OutPair p; OutCoef c; PhaseExt x{0, 0}; };
-  std::vector<std::vector<Entry>> values(n_blocks);   // constraint values of a block: (g row, local state row, 1)
+  std::vector<std::vector<Entry>> values(groups.size());   // constraint values of a node group: (g row, local state row, 1)
   for (int r = 0; r < m; ++r) {
     const RowOwner& o = owner[r];
     if (o.kind < 0) return fail(TWB_ERR_UNSUPPORTED, "constraint row without an owner");
-    uint32_t g_row = o.g_local, state0 = 1;
-    if (o.kind == kOwnNode) { g_row = unit_g0[o.index] + o.g_local; state0 = unit_state0[o.index]; }
+    uint32_t state0 = 1;
+    if (o.kind == kOwnNode) {
+      state0 = unit_state0[o.index];
+      values[unit_group[o.index]].push_back({OutPair{r, (uint16_t)(unit_g0[o.index] + o.g_local), 0}, OutCoef{1.0, 0.0}});
+    }
     const int blk = block_id(o);
-    if (blk >= 0 && o.g_local != kDirectValue) values[blk].push_back({OutPair{r, (uint16_t)g_row, 0}, OutCoef{1.0, 0.0}});
     for (int s = row_ptr[r]; s < row_ptr[r + 1]; ++s) {
       uint32_t a = em[s].a;
       if (em[s].tail >= 0) { elems[s] = Elem{tail_list0 + em[s].tail, (uint16_t)a, em[s].c0, em[s].ext}; continue; }   // rows of the tail kernel's CTA
@@ -924,14 +915,14 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
   // lists[list][class][0: pairs, 1: singles, 2: pairs of sectors with a phase element]
   std::vector<std::array<std::array<std::vector<Entry>, 3>, kMaxClasses>> lists(n_lists);
   const int NC = (nnz % 4 == 0) ? 1 : (nnz % 2 == 0) ? 2 : 4;
-  pl.nc_jac = NC; pl.nc_g = 1;
+  pl.nc_jac = NC;
   // ---- constant runs (device_tables.h: ConstRun): whole sectors whose elements all multiply the constant-1 state row.
   // Only with one alignment class (every instance's row starts on a sector) and without PhaseJac overwrites.
   std::vector<char> is_const_run(nnz, 0);
-  if (NC == 1 && !optimize_timings && TWB_ROMNODE && !TWB_FUSED && EnvInt("TWB_CONST_TMA", 1, 0, 1)) {   // (the constant CTAs live in RomNodeOut's grid)
+  if (NC == 1 && !optimize_timings) {   // (the constant CTAs live in RomNodeOut's grid)
     auto constant = [&](int i) {
       if (elems[i].list < 0) return false;
-      const int kind_rows = elems[i].list < n_dyn_ctas ? pl.dyn_rows : elems[i].list < n_dyn_ctas + n_rom_ctas * rom_lists ? pl.rom_rows : pl.node_rows;
+      const int kind_rows = elems[i].list < n_dyn_ctas ? pl.dyn_rows : elems[i].list < n_dyn_ctas + n_rom_ctas * n_ee ? pl.rom_rows : pl.node_rows;
       return elems[i].d % kind_rows == 0;   // row 0 of a warp's state block
     };
     int i = 0;
@@ -972,21 +963,9 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
     for (int i = 0; i < L; ++i) if (hits[i] != (elems[i].list >= 0 ? 1 : 0)) return fail(TWB_ERR_UNSUPPORTED, "output lists do not cover every element exactly once");
     for (int i = 0; i < L; ++i) if (is_const_run[i] && hits[i] != 0) return fail(TWB_ERR_UNSUPPORTED, "constant run also written by a list");
   }
-  pl.stage_dyn = pl.stage_rom = pl.stage_node = 0;
   auto flush_list = [&](int list) {
     OutList out{};
-    for (int q = 0; q < kMaxClasses; ++q) out.run_off[q] = -1;
     for (int q = 0; q < NC; ++q) {
-      {   // contiguous run of pairs? (sectors are pushed in ascending order)
-        const auto& v = lists[list][q][0];
-        bool run = !v.empty();
-        for (size_t i = 1; i < v.size() && run; ++i) run = v[i].p.off == v[0].p.off + 2 * (int)i;
-        if (run) {
-          out.run_off[q] = v[0].p.off;
-          int& cap = list < n_dyn_ctas ? pl.stage_dyn : list < n_dyn_ctas + n_rom_ctas * rom_lists ? pl.stage_rom : pl.stage_node;
-          cap = std::max(cap, 2 * (int)v.size());
-        }
-      }
       OutRange* dst[3] = {&out.pairs[q], &out.singles[q], &out.phase[q]};
       for (int w = 0; w < 3; ++w) {
         const auto& v = lists[list][q][w];
@@ -996,25 +975,19 @@ int Formulation::Build(const twb_spec& sp, std::string* err) {
     }
     return out;
   };
-  auto flush_values = [&](int block) {
-    OutRange r{(int32_t)tb.pairs.size(), (int32_t)values[block].size()};
-    for (const Entry& en : values[block]) { tb.pairs.push_back(en.p); tb.coefs.push_back(en.c); if (optimize_timings) tb.exts.push_back(en.x); }
-    return r;
-  };
   for (int i = 0; i < n_lists; ++i) tb.cta_lists.push_back(flush_list(i));
-  for (int k = 0; k < pl.n_dyn; ++k) tb.dyn[k].values = flush_values(k);
-  for (int k = 0; k < pl.n_rom; ++k) for (int e = 0; e < n_ee; ++e) tb.rom[k].values[e] = flush_values(pl.n_dyn + k * n_ee + e);
   for (size_t gi = 0; gi < groups.size(); ++gi) {
     NodeGroup ng{}; ng.kind = groups[gi].kind; ng.first = groups[gi].first; ng.count = groups[gi].count;
-    const auto& vals = values[pl.n_dyn + n_rom_blocks + (int)gi];
+    const auto& vals = values[gi];
     bool consecutive = !vals.empty();
     for (size_t i = 1; i < vals.size() && consecutive; ++i)
       consecutive = vals[i].p.off == vals[0].p.off + (int)i && vals[i].p.d0 == vals[0].p.d0 + (int)i;
     ng.g_row0 = consecutive ? vals[0].p.off : -1; ng.g_d0 = consecutive ? vals[0].p.d0 : 0; ng.g_n = consecutive ? (int32_t)vals.size() : 0;
-    ng.values = flush_values(pl.n_dyn + n_rom_blocks + (int)gi);
+    ng.values = OutRange{(int32_t)tb.pairs.size(), (int32_t)vals.size()};
+    for (const Entry& en : vals) { tb.pairs.push_back(en.p); tb.coefs.push_back(en.c); if (optimize_timings) tb.exts.push_back(en.x); }
     tb.groups.push_back(ng);
   }
-  pl.dyn_list0 = 0; pl.rom_list0 = n_dyn_ctas; pl.node_list0 = n_dyn_ctas + n_rom_ctas * rom_lists;
+  pl.dyn_list0 = 0; pl.rom_list0 = n_dyn_ctas; pl.node_list0 = n_dyn_ctas + n_rom_ctas * n_ee;
 
   // ---- costs (nlp_formulation.cc:333-376, node_cost.cc:53-76)
   has_cost = false;

@@ -13,7 +13,7 @@
 //   DynTailOut    (optimised phase durations only) the PhaseSpline columns of the dynamic rows (warp = foot)
 //   PhaseJac      (optimised phase durations only) the TotalDurationConstraint rows
 //   CostKernel    XT        -> cost + gradient (only when the formulation has cost terms)
-//   (TransposeOut GT[tile][m][32] -> g[B][m]: only in the -DTWB_GDIRECT=0 variants; the output CTAs write g themselves)
+// The output CTAs write the constraint values straight into g[B][m] as well.
 //
 // In the output kernels a warp owns one unit of 32 instances: each lane evaluates the splines its unit needs
 // (reference operation order) and computes its instance's unit state into a padded shared-memory block (row =
@@ -40,81 +40,17 @@
 namespace twb {
 void (*g_after_launch)(const char* label, cudaStream_t stream) = nullptr;   // profiling hook (capi.cc, TWB_PROFILE=1)
 #define TWB_MARK(label, stream) do { if (g_after_launch) g_after_launch(label, stream); } while (0)
-// L2 access-policy window of the evaluation kernels (capi.cc sets it per call): the two staging matrices XT / GT are marked
-// persisting, so that the 524 MB of streaming output per step cannot push them out of the L2 before their readers run
-// (ncu, round 2: 38 MB of XT were re-fetched from HBM by the output kernels and all 29 MB of GT by TransposeOut).
-thread_local const cudaAccessPolicyWindow* t_l2_window = nullptr;
-void SetL2Window(const cudaAccessPolicyWindow* w) { t_l2_window = w; }
 namespace {
 
-#ifndef TWB_TOUT_LD
-#define TWB_TOUT_LD 0    // cache operator of TransposeOut's loads of GT: 0 .cs, 1 .cg, 2 default, 3 .lu
-#endif
-#ifndef TWB_DISCARD
-#define TWB_DISCARD 1    // TransposeOut drops the dead L2 lines of GT and XT (discard.global.L2) instead of letting them be written back
-#endif
-#ifndef TWB_PDL
-#define TWB_PDL 1        // 1: RomNodeOut is launched with programmatic stream serialization behind TransposeIn (138.9 vs 144.6 us per step on config 2)
-#endif
-#if TWB_FUSED
-#ifndef TWB_CTAS
-#define TWB_CTAS 2   // CTAs per SM the fused output kernel is compiled for (bounds its registers)
-#endif
-#else
-#ifndef TWB_DYN_CTAS
-#define TWB_DYN_CTAS 2
-#endif
-#ifndef TWB_ROM_CTAS
-#define TWB_ROM_CTAS 4
-#endif
-#ifndef TWB_NODE_CTAS
-#define TWB_NODE_CTAS 3
-#endif
-#endif
-#ifndef TWB_TMA
-#define TWB_TMA 0        // 1: the Jacobian values of a CTA list leave the SM as cp.async.bulk.global.shared::cta copies of contiguous row segments assembled in shared memory; 0 (ships): 16-byte st.global.cs from the pair loop.  Measured (profiles/README.md, round 2): parity green, but 192 us per step instead of 139 us on config 2 — the extra pass through shared memory costs more than the better DRAM pattern gains
-#endif
-#ifndef TWB_CONST_WAIT_ALL
-#define TWB_CONST_WAIT_ALL 0
-#endif
-#ifndef TWB_ST_HINT
-#define TWB_ST_HINT 0    // cache operator of the Jacobian-value stores: 0 .cs (evict-first), 1 default (.wb), 2 .wt
-#endif
-#ifndef TWB_XT_EVICT_LAST
-#define TWB_XT_EVICT_LAST 0   // 1: TransposeIn writes XT with an L2 evict_last policy (experiment)
-#endif
-#ifndef TWB_ST256
-#define TWB_ST256 0     // 1: thread = whole sector (two consecutive pairs of the list), 256-bit stores, items of 8 instances
-#endif
-#ifndef TWB_TMA_DYN
-#define TWB_TMA_DYN TWB_TMA   // per-kernel switches of the TMA store path (tuning)
-#endif
-#ifndef TWB_TMA_ROM
-#define TWB_TMA_ROM TWB_TMA
-#endif
-#ifndef TWB_TMA_G
-#define TWB_TMA_G 2      // instances assembled per staging step (2: 16-byte reads of the state rows)
-#endif
-#ifndef TWB_TMA_BUF
-#define TWB_TMA_BUF 1    // staging buffers per warp (ring)
-#endif
 constexpr int kLD = 34;                      // leading dimension of a state block: 32 instances, padded; even keeps rows 16-byte aligned
+// resident CTAs per SM the output kernels are compiled for (__launch_bounds__: bounds their registers)
+constexpr int kDynCtas = 2, kRomCtas = 4;
+constexpr int kTailCtas = 4;   // DynTailOut: 128 registers; 49 state rows per foot = 53 KB per CTA
 
 // output stores: streaming (evict-first) — the values are consumed by the host / a solver, not by these kernels
 __device__ __forceinline__ void StoreOut(double* p, double v) { __stcs(p, v); }
 __device__ __forceinline__ void StoreOut2(double* p, double a, double b) {
-#if TWB_ST_HINT == 1
-  asm volatile("st.global.v2.f64 [%0], {%1, %2};" ::"l"(p), "d"(a), "d"(b) : "memory");
-#elif TWB_ST_HINT == 2
-  asm volatile("st.global.wt.v2.f64 [%0], {%1, %2};" ::"l"(p), "d"(a), "d"(b) : "memory");
-#else
   asm volatile("st.global.cs.v2.f64 [%0], {%1, %2};" ::"l"(p), "d"(a), "d"(b) : "memory");
-#endif
-}
-
-// 256-bit store (sm_100: SASS STG.E.256): a thread writes a whole 32-byte sector
-__device__ __forceinline__ void StoreOut4(double* p, double a, double b, double c, double d) {
-  asm volatile("st.global.cs.v4.f64 [%0], {%1, %2, %3, %4};" ::"l"(p), "d"(a), "d"(b), "d"(c), "d"(d) : "memory");
 }
 // column `b` of a row-major [rows][ld] matrix: element r lives at p[r * ld]
 struct Col {
@@ -791,7 +727,7 @@ __device__ __forceinline__ void CrossMatrix(const double v[3], double C[3][3]) {
 // alignment classes, instance b belongs to class b mod nc.  The tiles are then INTERLEAVED: tile nc G + q holds the
 // instances 32 nc G + nc lane + q, i.e. 32 instances of ONE class, so that a whole tile is written from one pair list
 // (one sector layout) with the same store loop as an aligned problem — the instance stride is nc rows.  nc = 1: tile t =
-// instances 32 t .. 32 t + 31.  XT, GT and the scratch matrices are indexed by (tile, lane).
+// instances 32 t .. 32 t + 31.  XT and the scratch matrices are indexed by (tile, lane).
 __device__ __forceinline__ int TileInstance(int nc, int tile, int lane) {
   return nc == 1 ? tile * 32 + lane : (tile / nc) * (32 * nc) + lane * nc + tile % nc;
 }
@@ -810,63 +746,15 @@ __device__ __forceinline__ ConstCol TiledCol(const double* base, int b, int rows
   return TileCol(base, grp * nc + rem % nc, rem / nc, rows);
 }
 
-// x[b][i] -> XT[tile][i][lane]: 32x32 tiles through shared memory, coalesced on both sides; clears status.  A CTA moves
-// kTinTiles consecutive column tiles: all their loads are issued before the barrier (more bytes in flight per thread, fewer
-// waves of CTAs for this short, latency-bound kernel that everything else waits for).
-#ifndef TWB_TIN_TILES
-#define TWB_TIN_TILES 1
-#endif
-constexpr int kTinTiles = TWB_TIN_TILES;
-__global__ void __launch_bounds__(256) TransposeIn(const double* __restrict__ x, double* __restrict__ XT,
-                                                   int* __restrict__ status, int n, int nb, int nc) {
-  __shared__ double tile[kTinTiles][32][33];
-#if TWB_PDL
-  asm volatile("griddepcontrol.launch_dependents;");   // the dependent output kernel may become resident while this grid drains
-#endif
-  if (status && blockIdx.x == 0 && threadIdx.y == 0 && TileInstance(nc, blockIdx.y, threadIdx.x) < nb) status[TileInstance(nc, blockIdx.y, threadIdx.x)] = 0;
-#pragma unroll
-  for (int c = 0; c < kTinTiles; ++c) {
-    const int i0 = (blockIdx.x * kTinTiles + c) * 32;
-#pragma unroll
-    for (int r = threadIdx.y; r < 32; r += 8) {
-      const int b = TileInstance(nc, blockIdx.y, r), i = i0 + threadIdx.x;
-      if (b < nb && i < n) tile[c][r][threadIdx.x] = __ldcs(x + (size_t)b * n + i);
-    }
-  }
-  __syncthreads();
-  double* dst = XT + ((size_t)blockIdx.y * (n + 1)) * 32;
-  const int b = TileInstance(nc, blockIdx.y, threadIdx.x);
-#pragma unroll
-  for (int c = 0; c < kTinTiles; ++c) {
-    const int i0 = (blockIdx.x * kTinTiles + c) * 32;
-#pragma unroll
-    for (int r = threadIdx.y; r < 32; r += 8) {
-      const int i = i0 + r;
-#if TWB_XT_EVICT_LAST
-      if (b < nb && i < n) {
-        unsigned long long pol;
-        asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-        asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(dst + (size_t)i * 32 + threadIdx.x), "d"(tile[c][threadIdx.x][r]), "l"(pol) : "memory");
-      }
-#else
-      if (b < nb && i < n) dst[(size_t)i * 32 + threadIdx.x] = tile[c][threadIdx.x][r];
-#endif
-    }
-  }
-}
-
-// Persistent variant (TWB_TIN_PERSIST = CTAs per SM, 0 = the kernel above): a fixed grid of 148 x 8 CTAs walks the 32 x 32 tiles; the
-// loads of a CTA's next tile are issued before the stores of the current one, and no CTA launch sits between the two.  Measured
-// (config 2, one box): 8.2 us instead of 12.3 us for the kernel, 127.1 instead of 131.5 us per step (6 / 4 CTAs per SM: 127.7 / 128.8 us).
-#ifndef TWB_TIN_PERSIST
-#define TWB_TIN_PERSIST 8
-#endif
+// x[b][i] -> XT[tile][i][lane]: 32x32 tiles through shared memory, coalesced on both sides; clears status.  Persistent: a fixed
+// grid of 148 x kTinPersist CTAs walks the 32 x 32 tiles; the loads of a CTA's next tile are issued before the stores of the
+// current one, and no CTA launch sits between the two.  Measured (config 2, one box): 8.2 us instead of 12.3 us for a kernel
+// with one CTA per tile, 127.1 instead of 131.5 us per step (6 / 4 CTAs per SM: 127.7 / 128.8 us).
+constexpr int kTinPersist = 8;   // CTAs per SM
 __global__ void __launch_bounds__(256) TransposeInP(const double* __restrict__ x, double* __restrict__ XT, int* __restrict__ status, int n, int nb,
                                                     int nc, int n_ctiles, int total) {
   __shared__ double tile[32][33];
-#if TWB_PDL
-  asm volatile("griddepcontrol.launch_dependents;");
-#endif
+  asm volatile("griddepcontrol.launch_dependents;");   // the dependent output kernel may become resident while this grid drains
   const int tx = threadIdx.x, ty = threadIdx.y;
   double v[4];
   auto load = [&](int t) {
@@ -897,71 +785,6 @@ __global__ void __launch_bounds__(256) TransposeInP(const double* __restrict__ x
   }
 }
 
-// GT[b/32][r][b%32] -> g[b][r]: 32x32 tiles through shared memory, coalesced on both sides
-// TWB_DISCARD: GT is dead once it has been read, and so is XT (rows 0 .. n-1; row n is the permanent zero row) — both
-// are still dirty in the L2; `discard.global.L2` drops the lines instead of writing them back to HBM (50 MB per step
-// on config 2, 9 % of the step's DRAM writes).  Both matrices are rewritten by the next evaluation before they are read.
-__device__ __forceinline__ void DiscardLine(const void* p) { asm volatile("discard.global.L2 [%0], 128;" ::"l"(p) : "memory"); }
-// Experiment (TWB_XT_DROP=1): without TransposeOut (direct constraint values) the LAST output CTA of a tile drops the tile's XT lines: every output CTA
-// counts itself on the tile's counter when it is done; the one that completes the count discards rows 0 .. n-1 (row n is the
-// permanent zero row; a ragged tile keeps its lines: its padded lanes are never rewritten) and resets the counter.
-// Measured (config 2, one box): 137.3 us per step with the counters against 132.1 us without — the atomics and the extra CTA
-// barriers cost more than the 21 MB of XT write-back they save.  Off.
-#ifndef TWB_XT_DROP
-#define TWB_XT_DROP 0
-#endif
-__device__ __forceinline__ void TileDone(int* __restrict__ tile_done, int total, const double* __restrict__ XT, int n, int nc, int tile, int nb) {
-#if TWB_XT_DROP
-  if (!tile_done) return;
-  __shared__ int last;
-  __syncthreads();   // every thread of the CTA is past its reads of XT
-  if (threadIdx.x == 0) last = (atomicAdd(tile_done + tile, 1) == total - 1);
-  __syncthreads();
-  if (!last) return;
-  if (threadIdx.x == 0) tile_done[tile] = 0;
-  if (TileCount(nc, tile, nb) != 32) return;
-  const double* xt = XT + ((size_t)tile * (n + 1)) * 32;
-  for (int l = threadIdx.x; l < 2 * n; l += blockDim.x) DiscardLine(xt + (size_t)l * 16);
-#endif
-}
-__global__ void __launch_bounds__(256) TransposeOut(const double* __restrict__ GT, double* __restrict__ g, int m, int nb,
-                                                    const double* __restrict__ XT, int n, int nc) {
-  __shared__ double tile[32][33];
-  const int r0 = blockIdx.x * 32;
-  const double* src = GT + ((size_t)blockIdx.y * m) * 32;
-#pragma unroll
-  for (int q = threadIdx.y; q < 32; q += 8) {
-    const int r = r0 + q;
-#if TWB_TOUT_LD == 1
-    if (r < m) tile[q][threadIdx.x] = __ldcg(src + (size_t)r * 32 + threadIdx.x);
-#elif TWB_TOUT_LD == 2
-    if (r < m) tile[q][threadIdx.x] = src[(size_t)r * 32 + threadIdx.x];
-#elif TWB_TOUT_LD == 3
-    if (r < m) tile[q][threadIdx.x] = __ldlu(src + (size_t)r * 32 + threadIdx.x);
-#else
-    if (r < m) tile[q][threadIdx.x] = __ldcs(src + (size_t)r * 32 + threadIdx.x);
-#endif
-  }
-  __syncthreads();
-#if TWB_DISCARD
-  {
-    const int tid = threadIdx.y * 32 + threadIdx.x;
-    if (tid < 64) {                       // the 32 GT rows of this CTA: two 128-byte lines each
-      const int r = r0 + (tid >> 1);
-      if (r < m) DiscardLine(src + (size_t)r * 32 + (tid & 1) * 16);
-    } else if (XT && tid < 128 && TileCount(nc, blockIdx.y, nb) == 32) {   // XT rows of this tile, 32 per CTA of the tile (CTAs wrap around when m < n); a ragged last tile keeps its lines: its padded lanes are never rewritten
-      const double* xt = XT + ((size_t)blockIdx.y * (n + 1)) * 32;
-      for (int r = r0 + ((tid - 64) >> 1); r < n; r += gridDim.x * 32) DiscardLine(xt + (size_t)r * 32 + (tid & 1) * 16);
-    }
-  }
-#endif
-#pragma unroll
-  for (int q = threadIdx.y; q < 32; q += 8) {
-    const int b = TileInstance(nc, blockIdx.y, q), r = r0 + threadIdx.x;
-    if (b < nb && r < m) StoreOut(g + (size_t)b * m + r, tile[threadIdx.x][q]);
-  }
-}
-
 // ---- CTA-collective output: threads switch from "instance" to "pair of output elements" ----------------------
 // out[j][off + h] = t[d_h][j] * c_h for the lanes j < n_inst of the tile; `t` is the CTA's shared memory (all state
 // blocks), `out` points at element 0 of the tile's first instance, `stride` is the distance between the rows of consecutive
@@ -978,31 +801,6 @@ __device__ __forceinline__ void LoadPair(const OutPair* __restrict__ pairs, cons
 __device__ __forceinline__ void StorePairs(const double* t, const OutPair* __restrict__ pairs, const OutCoef* __restrict__ coefs,
                                            int n_pairs, double* __restrict__ out, size_t stride, int n_inst,
                                            int tid, int n_threads) {
-#if TWB_ST256
-  if (n_inst == 32 && (reinterpret_cast<uintptr_t>(out) & 31) == 0 && (stride & 3) == 0) {
-    // thread = whole 32-byte sector (the list holds two consecutive pairs per sector), item = (sector, quarter of the tile's
-    // instances): one 256-bit store per instance, a warp instruction covers 1 KB of the instance's row
-    const int n_sec = n_pairs >> 1, n_items = 4 * n_sec;
-    for (int i = tid; i < n_items; i += n_threads) {
-      const int qd = i / n_sec, k = i - qd * n_sec;
-      int off = 0, d0 = 0, d1 = 0, off2 = 0, d2 = 0, d3 = 0; double c0 = 0.0, c1 = 0.0, c2 = 0.0, c3 = 0.0;
-      LoadPair(pairs, coefs, 2 * k, n_pairs, &off, &d0, &d1, &c0, &c1);
-      LoadPair(pairs, coefs, 2 * k + 1, n_pairs, &off2, &d2, &d3, &c2, &c3);
-      const int jb = 8 * qd;
-      double* o = out + off + (size_t)jb * stride;
-      const double* r0 = t + d0 * kLD + jb; const double* r1 = t + d1 * kLD + jb;
-      const double* r2 = t + d2 * kLD + jb; const double* r3 = t + d3 * kLD + jb;
-#pragma unroll
-      for (int j = 0; j < 8; j += 2) {
-        const double2 a = *reinterpret_cast<const double2*>(r0 + j), b = *reinterpret_cast<const double2*>(r1 + j);
-        const double2 c = *reinterpret_cast<const double2*>(r2 + j), d = *reinterpret_cast<const double2*>(r3 + j);
-        StoreOut4(o, a.x * c0, b.x * c1, c.x * c2, d.x * c3); o += stride;
-        StoreOut4(o, a.y * c0, b.y * c1, c.y * c2, d.y * c3); o += stride;
-      }
-    }
-    return;
-  }
-#endif
   if (n_inst == 32) {
     // Work items are (pair, half of the tile's instances): twice as many items as pairs keep the threads of a CTA
     // evenly busy when a list is only 1 - 2 pairs per thread long.  Items 0 .. n_pairs-1 are the first 16 instances,
@@ -1043,69 +841,10 @@ __device__ __forceinline__ void StorePairs(const double* t, const OutPair* __res
   }
 }
 
-// ---- TMA store path ---------------------------------------------------------------------------------------------
-// A CTA list whose pairs form one contiguous run of the CSR value row (OutList::run_off) is written per instance as ONE
-// bulk copy shared -> global (SASS UBLKCP): every warp owns 32 / W instances of the tile, assembles the run of kG of them
-// in its staging rows in OUTPUT ORDER (thread = pair: 16-byte shared stores, conflict-free), makes the writes visible to
-// the async proxy and lets lane 0 issue the copies.  The TMA engine drains the staging rows while the warp goes on
-// (next instances, then the evaluation of the next unit); a row is only refilled after its copy has finished reading.
+// bulk copies of the constant runs (ConstRunBody)
 __device__ __forceinline__ unsigned SmemAddr(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void BulkStore(void* gdst, const void* ssrc, unsigned bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst), "r"(SmemAddr(ssrc)), "r"(bytes) : "memory");
-}
 __device__ __forceinline__ void BulkCommit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void BulkWaitRead() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
-__device__ __forceinline__ void BulkWaitAll() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
-__device__ __forceinline__ void FenceProxyAsync() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-struct Stage { double* base; int cap; };   // staging rows of the CTA (after the state blocks): W x kBuf x kG rows of `cap` doubles (cap even)
-
-__device__ __forceinline__ void StorePairsTma(const double* t, const OutPair* __restrict__ pairs, const OutCoef* __restrict__ coefs, int n_pairs,
-                                              int run_off, double* __restrict__ out, size_t stride, int q, int nc, int n_inst, const Stage st) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, W = blockDim.x >> 5, per = 32 / W;
-  const int j_end = min(n_inst, (warp + 1) * per);
-  double* rows = st.base + (size_t)warp * (TWB_TMA_BUF * TWB_TMA_G) * st.cap;
-  const unsigned bytes = (unsigned)n_pairs * 16u;
-  if (lane == 0) BulkWaitRead<0>();   // copies of the previous list (issued before the evaluation of this unit) have long finished reading
-  __syncwarp();
-  int it = 0;
-  if (TWB_TMA_G == 2 && nc == 1) {
-    for (int j = warp * per; j < j_end; j += 2, ++it) {
-      double* b0 = rows + (size_t)(it % TWB_TMA_BUF) * 2 * st.cap; double* b1 = b0 + st.cap;
-      if (it >= TWB_TMA_BUF) { if (lane == 0) BulkWaitRead<TWB_TMA_BUF - 1>(); __syncwarp(); }
-      for (int i = lane; i < n_pairs; i += 32) {
-        int off = 0, d0 = 0, d1 = 0; double c0 = 0.0, c1 = 0.0;
-        LoadPair(pairs, coefs, i, n_pairs, &off, &d0, &d1, &c0, &c1);
-        const double2 a = *reinterpret_cast<const double2*>(t + d0 * kLD + j), b = *reinterpret_cast<const double2*>(t + d1 * kLD + j);
-        const int o = off - run_off;
-        *reinterpret_cast<double2*>(b0 + o) = make_double2(a.x * c0, b.x * c1);
-        *reinterpret_cast<double2*>(b1 + o) = make_double2(a.y * c0, b.y * c1);
-      }
-      FenceProxyAsync();
-      __syncwarp();
-      if (lane == 0) {
-        BulkStore(out + (size_t)j * stride + run_off, b0, bytes);
-        if (j + 1 < j_end) BulkStore(out + (size_t)(j + 1) * stride + run_off, b1, bytes);
-        BulkCommit();
-      }
-    }
-    return;
-  }
-  constexpr int kSlots = TWB_TMA_BUF * TWB_TMA_G;
-  for (int j = warp * per; j < j_end; ++j) {
-    if (j % nc != q) continue;
-    double* b0 = rows + (size_t)(it % kSlots) * st.cap;
-    if (it >= kSlots) { if (lane == 0) BulkWaitRead<kSlots - 1>(); __syncwarp(); }
-    ++it;
-    for (int i = lane; i < n_pairs; i += 32) {
-      int off = 0, d0 = 0, d1 = 0; double c0 = 0.0, c1 = 0.0;
-      LoadPair(pairs, coefs, i, n_pairs, &off, &d0, &d1, &c0, &c1);
-      *reinterpret_cast<double2*>(b0 + (off - run_off)) = make_double2(t[d0 * kLD + j] * c0, t[d1 * kLD + j] * c1);
-    }
-    FenceProxyAsync();
-    __syncwarp();
-    if (lane == 0) { BulkStore(out + (size_t)j * stride + run_off, b0, bytes); BulkCommit(); }
-  }
-}
 // ---- phase elements (device_tables.h: PhaseExt) --------------------------------------------------------------------
 // per-instance value of one element whose info block is in TABLE form / whose duration columns are not finished:
 // `x` is the element's PhaseExt word, d / c its state row and coefficient
@@ -1234,93 +973,61 @@ __device__ __forceinline__ void ForEachEntry(const OutPair* __restrict__ pairs, 
 __device__ __forceinline__ OutRange LoadRange(const OutRange* r) {
   const int2 v = __ldg(reinterpret_cast<const int2*>(r)); return OutRange{v.x, v.y};
 }
-// constraint values of one unit: lane = instance writes GT[row][lane] (instance-tiled, 256 contiguous bytes per row and
-// warp); TransposeOut turns the tiles into g[B][m] afterwards.  One unit owns only 3 - 10 constraint values per
-// instance — written straight into g[B][m] they would be 8-byte pieces of sectors shared with other units.
-__device__ __forceinline__ void StoreValuesTiled(const Plan& P, const double* t, const OutRange* values, double* __restrict__ gt_tile, int lane) {
-  const OutRange r = LoadRange(values);
-  ForEachEntry(P.pairs + r.first, P.coefs + r.first, r.count, lane,
-               [&](int g_row, int d, double c) { gt_tile[(size_t)g_row * 32 + lane] = t[d * kLD + lane] * c; });
-}
 // Jacobian values of a whole CTA (after its barrier): every thread takes pairs of the CTA's list; warp 0 writes the
 // single elements (sectors shared with a neighbouring CTA) with lane = instance.
 template <bool kPhase = false>
-__device__ __forceinline__ void StoreCta(const Plan& P, const double* cta_smem, const OutList* list, double* __restrict__ jac, int tile, int nb, const Stage st,
+__device__ __forceinline__ void StoreCta(const Plan& P, const double* cta_smem, const OutList* list, double* __restrict__ jac, int tile, int nb,
                                          int v_off = 0, int dwin = 0, int zrow = 0) {
-#ifdef TWB_EXP_NOSTORE   // timing experiment: compute phase only
-  return;
-#endif
   const int nc = P.nc_jac, lane = threadIdx.x & 31;
   // all instances of the tile belong to alignment class q (interleaved tiles); consecutive lanes are nc rows apart
   const int q = tile % nc, n_inst = TileCount(nc, tile, nb);
   const size_t stride = (size_t)nc * P.nnz;
   double* __restrict__ jac_tile = jac + (size_t)TileInstance(nc, tile, 0) * P.nnz;
-  {
-    const OutRange rp = LoadRange(&list->pairs[q]);
-    // warp 0 also owns the single elements: their range (and, below, their first 32 entries) is fetched BEFORE the pair
-    // loop, so that the two dependent loads are in flight under the warp's pair stores instead of after them
-    OutRange rs{0, 0};
-    if (threadIdx.x < 32) rs = LoadRange(&list->singles[q]);
-    uint2 raw = make_uint2(0u, 0u); double cs = 0.0; unsigned xs = 0u;
-    if (lane < rs.count) {
-      raw = __ldg(reinterpret_cast<const uint2*>(P.pairs + rs.first) + lane); cs = __ldg(reinterpret_cast<const double*>(P.coefs + rs.first + lane));
-      if (kPhase) xs = __ldg(reinterpret_cast<const unsigned*>(P.exts + rs.first + lane));
+  const OutRange rp = LoadRange(&list->pairs[q]);
+  // warp 0 also owns the single elements: their range (and, below, their first 32 entries) is fetched BEFORE the pair
+  // loop, so that the two dependent loads are in flight under the warp's pair stores instead of after them
+  OutRange rs{0, 0};
+  if (threadIdx.x < 32) rs = LoadRange(&list->singles[q]);
+  uint2 raw = make_uint2(0u, 0u); double cs = 0.0; unsigned xs = 0u;
+  if (lane < rs.count) {
+    raw = __ldg(reinterpret_cast<const uint2*>(P.pairs + rs.first) + lane); cs = __ldg(reinterpret_cast<const double*>(P.coefs + rs.first + lane));
+    if (kPhase) xs = __ldg(reinterpret_cast<const unsigned*>(P.exts + rs.first + lane));
+  }
+  StorePairs(cta_smem, P.pairs + rp.first, P.coefs + rp.first, rp.count, jac_tile, stride, n_inst, threadIdx.x, blockDim.x);
+  if (kPhase) {
+    const OutRange rq = LoadRange(&list->phase[q]);
+    StorePhasePairs(cta_smem, P.pairs + rq.first, P.coefs + rq.first, P.exts + rq.first, rq.count, jac_tile, stride, n_inst, v_off, dwin, zrow,
+                    threadIdx.x, blockDim.x);
+  }
+  if (threadIdx.x < 32 && rs.count > 0) {
+    const bool active = lane < n_inst;
+    double* o = jac_tile + (size_t)lane * stride;
+    const int cnt = min(32, rs.count);
+    for (int sidx = 0; sidx < cnt; ++sidx) {
+      const int off = __shfl_sync(0xffffffffu, (int)raw.x, sidx), d = __shfl_sync(0xffffffffu, (int)(raw.y & 0xFFFFu), sidx);
+      const double c = __shfl_sync(0xffffffffu, cs, sidx);
+      const unsigned x = kPhase ? __shfl_sync(0xffffffffu, xs, sidx) : 0u;
+      if (active) StoreOut(o + off, kPhase ? FormVal(cta_smem, lane, Classify(cta_smem, x, d, c, v_off, dwin, zrow), x, d, c, v_off) : cta_smem[d * kLD + lane] * c);
     }
-#if TWB_TMA
-    const int run_off = __ldg(&list->run_off[q]);
-    if (run_off >= 0 && 2 * rp.count <= st.cap && (32 % (blockDim.x >> 5)) == 0)
-      StorePairsTma(cta_smem, P.pairs + rp.first, P.coefs + rp.first, rp.count, run_off, jac_tile, stride, 0, 1, n_inst, st);
-    else
-#endif
-    StorePairs(cta_smem, P.pairs + rp.first, P.coefs + rp.first, rp.count, jac_tile, stride, n_inst, threadIdx.x, blockDim.x);
-    if (kPhase) {
-      const OutRange rq = LoadRange(&list->phase[q]);
-      StorePhasePairs(cta_smem, P.pairs + rq.first, P.coefs + rq.first, P.exts + rq.first, rq.count, jac_tile, stride, n_inst, v_off, dwin, zrow,
-                      threadIdx.x, blockDim.x);
-    }
-#ifndef TWB_EXP_NOSINGLES   // (timing experiment, profiles/README.md round 2: what the single-element stores cost)
-    if (threadIdx.x < 32 && rs.count > 0) {
-      const bool active = lane < n_inst;
-      double* o = jac_tile + (size_t)lane * stride;
-      const int cnt = min(32, rs.count);
-      for (int sidx = 0; sidx < cnt; ++sidx) {
+    for (int base = 32; base < rs.count; base += 32) {   // (rare) more than 32 single elements
+      raw = make_uint2(0u, 0u); cs = 0.0; xs = 0u;
+      if (base + lane < rs.count) {
+        raw = __ldg(reinterpret_cast<const uint2*>(P.pairs + rs.first + base) + lane); cs = __ldg(reinterpret_cast<const double*>(P.coefs + rs.first + base + lane));
+        if (kPhase) xs = __ldg(reinterpret_cast<const unsigned*>(P.exts + rs.first + base + lane));
+      }
+      const int more = min(32, rs.count - base);
+      for (int sidx = 0; sidx < more; ++sidx) {
         const int off = __shfl_sync(0xffffffffu, (int)raw.x, sidx), d = __shfl_sync(0xffffffffu, (int)(raw.y & 0xFFFFu), sidx);
         const double c = __shfl_sync(0xffffffffu, cs, sidx);
         const unsigned x = kPhase ? __shfl_sync(0xffffffffu, xs, sidx) : 0u;
         if (active) StoreOut(o + off, kPhase ? FormVal(cta_smem, lane, Classify(cta_smem, x, d, c, v_off, dwin, zrow), x, d, c, v_off) : cta_smem[d * kLD + lane] * c);
       }
-      for (int base = 32; base < rs.count; base += 32) {   // (rare) more than 32 single elements
-        raw = make_uint2(0u, 0u); cs = 0.0; xs = 0u;
-        if (base + lane < rs.count) {
-          raw = __ldg(reinterpret_cast<const uint2*>(P.pairs + rs.first + base) + lane); cs = __ldg(reinterpret_cast<const double*>(P.coefs + rs.first + base + lane));
-          if (kPhase) xs = __ldg(reinterpret_cast<const unsigned*>(P.exts + rs.first + base + lane));
-        }
-        const int more = min(32, rs.count - base);
-        for (int sidx = 0; sidx < more; ++sidx) {
-          const int off = __shfl_sync(0xffffffffu, (int)raw.x, sidx), d = __shfl_sync(0xffffffffu, (int)(raw.y & 0xFFFFu), sidx);
-          const double c = __shfl_sync(0xffffffffu, cs, sidx);
-          const unsigned x = kPhase ? __shfl_sync(0xffffffffu, xs, sidx) : 0u;
-          if (active) StoreOut(o + off, kPhase ? FormVal(cta_smem, lane, Classify(cta_smem, x, d, c, v_off, dwin, zrow), x, d, c, v_off) : cta_smem[d * kLD + lane] * c);
-        }
-      }
     }
-#endif
   }
 }
-// ---- constraint values straight into g[B][m] (TWB_GDIRECT) ----------------------------------------------------------------
-#ifndef TWB_GDIRECT_PHASE
-#define TWB_GDIRECT_PHASE 1   // 1: problems with optimised durations write g directly as well (their range-of-motion values lane = instance)
-#endif
-#ifndef TWB_G_ST
-#define TWB_G_ST 1   // cache operator of the direct constraint-value stores: 0 .cs (evict-first), 1 default (ships: 132.0 vs 134.5 us per step on config 2 — rows shared by two CTAs merge in the L2)
-#endif
-__device__ __forceinline__ void StoreG(double* p, double v) {
-#if TWB_G_ST == 1
-  *p = v;
-#else
-  __stcs(p, v);
-#endif
-}
+// ---- constraint values straight into g[B][m] ----------------------------------------------------------------------------
+// default cache operator, not .cs: rows shared by two CTAs merge in the L2 (132.0 vs 134.5 us per step on config 2)
+__device__ __forceinline__ void StoreG(double* p, double v) { *p = v; }
 // The `n_units` consecutive units of a CTA own kPer consecutive constraint rows each, starting at row `row0`; unit w keeps its
 // values in the state rows w * block_rows + d0 .. of the CTA's shared memory `t`.  All threads: consecutive threads write
 // consecutive rows of one instance (kPer * n_units * 8 contiguous bytes per instance), after the CTA barrier.
@@ -1348,29 +1055,24 @@ __device__ __forceinline__ void FlagNonFinite(const double* t, int n_rows, int l
 // DynamicConstraint: blockIdx.y = instance tile, warp = one of kDynWarps CONSECUTIVE samples, so a CTA writes
 // several KB of contiguous CSR values per instance (the samples' rows are adjacent).
 template <int kNEE, bool kPhase>
-__device__ __forceinline__ void DynBody(const Plan& P, const double* __restrict__ XT, double* __restrict__ GT, double* __restrict__ jac,
-                                        int* __restrict__ status, int nb, unsigned flags, double* out_smem, int cta, int tile, const Stage st,
-                                        const double* __restrict__ FS = nullptr, double* __restrict__ g = nullptr) {
+__device__ __forceinline__ void DynBody(const Plan& P, const double* __restrict__ XT, double* __restrict__ jac, int* __restrict__ status, int nb,
+                                        unsigned flags, double* out_smem, int cta, int tile, const double* __restrict__ FS, double* __restrict__ g) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int k = cta * kDynWarps + warp, b = TileInstance(P.nc_jac, tile, lane);
-  // local rows: 1 | 3 | 36 | 6 per foot [| the 6 constraint values (TWB_GDIRECT); else they go straight into GT, coalesced]
+  // local rows: 1 | 3 | 36 | 6 per foot | the 6 constraint values
   constexpr int n_rows = DynBlockRows(kNEE), g_d0 = n_rows - 6;
-  const bool g_direct = TWB_GDIRECT && g != nullptr;
   double* t = out_smem + (size_t)warp * n_rows * kLD;
   if (k < P.n_dyn) {
     const DynUnit* u = P.dyn + k;
     t[lane] = 1.0;
-#ifndef TWB_EXP_NOCOMPUTE   // (timing experiment: store phase only)
     DynamicUnit<kNEE, kPhase>(P, k, P.samples + __ldg(&u->sample0), TileCol(XT, tile, lane, P.n + 1), Col{t + kLD + lane, kLD},
-                              g_direct ? Col{t + g_d0 * kLD + lane, kLD} : Col{GT + (((size_t)tile * P.m + (size_t)__ldg(&u->g_row0)) * 32) + lane, 32},
-                              FS ? FS + (((size_t)tile * P.n_dyn + k) * (6 * kNEE)) * 32 + lane : nullptr);
+                              Col{t + g_d0 * kLD + lane, kLD}, FS ? FS + (((size_t)tile * P.n_dyn + k) * (6 * kNEE)) * 32 + lane : nullptr);
     FlagNonFinite(t, n_rows, lane, status, b, nb);
-#endif
   }
   __syncthreads();
-  if (g_direct && (flags & 1u) && cta * kDynWarps < P.n_dyn)
+  if ((flags & 1u) && cta * kDynWarps < P.n_dyn)
     StoreValuesDirect<6>(P, out_smem, g, tile, nb, __ldg(&P.dyn[cta * kDynWarps].g_row0), min(kDynWarps, P.n_dyn - cta * kDynWarps), n_rows, g_d0);
-  if (flags & 2u) StoreCta(P, out_smem, P.cta_lists + P.dyn_list0 + cta, jac, tile, nb, st);
+  if (flags & 2u) StoreCta(P, out_smem, P.cta_lists + P.dyn_list0 + cta, jac, tile, nb);
 }
 
 // RangeOfMotionConstraint (range_of_motion_constraint.cc:58-109): g_e = R^T (p_e - c); Jacobian state R^T and
@@ -1380,10 +1082,8 @@ __device__ __forceinline__ void DynBody(const Plan& P, const double* __restrict_
 // Jacobian values of foot e (one list per foot: the foot's rows of the CTA's samples are adjacent), every warp
 // already evaluates foot e + 1 — one CTA barrier per foot.
 template <int kNEE, bool kPhase>
-__device__ __forceinline__ void RomBody(const Plan& P, const double* __restrict__ XT, double* __restrict__ GT, double* __restrict__ jac,
-                                        int* __restrict__ status, int nb, unsigned flags, double* out_smem, int cta, int tile, const Stage st,
-                                        double* __restrict__ g = nullptr) {
-  const bool g_direct = TWB_GDIRECT && !kPhase && g != nullptr;
+__device__ __forceinline__ void RomBody(const Plan& P, const double* __restrict__ XT, double* __restrict__ jac, int* __restrict__ status, int nb,
+                                        unsigned flags, double* out_smem, int cta, int tile, double* __restrict__ g) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int k = cta * kRomWarps + warp, b = TileInstance(P.nc_jac, tile, lane);
   const bool valid = k < P.n_rom;
@@ -1396,7 +1096,6 @@ __device__ __forceinline__ void RomBody(const Plan& P, const double* __restrict_
   // buffer is D_e (9) | the PhaseSpline's info block (kInfoRows) | U (3) | X (3 kRomDurWin)   (g_e lives in registers only)
   const Col Sk{t + kLD + lane, kLD};
   t[lane] = 1.0;
-#ifndef TWB_EXP_NOCOMPUTE
   double c[3], th[3], unused[3];
   EvalSpline<0>(P, sp + 0, xs, c, unused, unused);
   EvalSpline<0>(P, sp + 1, xs, th, unused, unused);
@@ -1407,11 +1106,9 @@ __device__ __forceinline__ void RomBody(const Plan& P, const double* __restrict_
   for (int i = 0; i < 3; ++i)
 #pragma unroll
     for (int d = 0; d < 3; ++d) Sk[i * 3 + d] = R[d][i];
-#endif
 #pragma unroll 1
   for (int e = 0; e < kNEE; ++e) {
     const int buf = RomBufferP(e, kPhase);
-#ifndef TWB_EXP_NOCOMPUTE
     double pe[3];
     if (kPhase) {   // range_of_motion_constraint.cc:83-109 with the PhaseSpline of foot e: value, active polynomial, duration columns
       const PhaseFull mo = EvalPhaseFull(P, 2 * e, __ldg(&sp[2 + e].T), xs);
@@ -1453,44 +1150,23 @@ __device__ __forceinline__ void RomBody(const Plan& P, const double* __restrict_
       }
       if (status && chk != chk && b < nb) atomicOr(status + b, 1);
     }
-#endif
-    if (kPhase && TWB_GDIRECT && g != nullptr) {   // optimised durations: g_e exists in registers only; lane = instance straight into g
-#ifndef TWB_EXP_NOCOMPUTE
-      if (valid && (flags & 1u) && b < nb) {
-        double* gp = g + (size_t)b * P.m + P.rom_row0[e] + 3 * k;
+    if (kPhase && valid && (flags & 1u) && b < nb) {   // optimised durations: g_e exists in registers only; lane = instance straight into g
+      double* gp = g + (size_t)b * P.m + P.rom_row0[e] + 3 * k;
 #pragma unroll
-        for (int i = 0; i < 3; ++i) StoreG(gp + i, ge[i]);
-      }
-#endif
-    } else
-    if (valid && (flags & 1u) && !g_direct) {   // rows rom_row0[e] + 3k .. + 2 (range_of_motion_constraint.cc:58-66), lane = instance into GT
-      double* gt = GT + (((size_t)tile * P.m + (size_t)(P.rom_row0[e] + 3 * k)) * 32) + lane;
-#ifndef TWB_EXP_NOCOMPUTE
-#pragma unroll
-      for (int i = 0; i < 3; ++i) gt[i * 32] = ge[i];
-#else
-      for (int i = 0; i < 3; ++i) gt[i * 32] = t[(19 + buf + i) * kLD + lane];
-#endif
+      for (int i = 0; i < 3; ++i) StoreG(gp + i, ge[i]);
     }
-#if !TWB_ROM_ALLFEET
     __syncthreads();   // foot e complete in every block; everybody is done reading buffer (e + 1) & 1 (the list of foot e - 1)
-    if (g_direct && (flags & 1u))   // the foot's rows of the CTA's samples are adjacent: 3 kRomWarps consecutive values per instance
+    if (!kPhase && (flags & 1u))   // the foot's rows of the CTA's samples are adjacent: 3 kRomWarps consecutive values per instance
       StoreValuesDirect<3>(P, out_smem, g, tile, nb, P.rom_row0[e] + 3 * cta * kRomWarps, min(kRomWarps, P.n_rom - cta * kRomWarps), block_rows, 19 + buf);
-    if (flags & 2u) StoreCta<kPhase>(P, out_smem, P.cta_lists + P.rom_list0 + cta * kNEE + e, jac, tile, nb, st, 3, kRomDurWin, 20 + buf);
-#endif
+    if (flags & 2u) StoreCta<kPhase>(P, out_smem, P.cta_lists + P.rom_list0 + cta * kNEE + e, jac, tile, nb, 3, kRomDurWin, 20 + buf);
   }
-#if TWB_ROM_ALLFEET
-  __syncthreads();
-  if (flags & 2u) StoreCta<kPhase>(P, out_smem, P.cta_lists + P.rom_list0 + cta, jac, tile, nb, st, 3, kRomDurWin, 20);
-#endif
 }
 
 // node groups: blockIdx.y = instance tile, warp = one of kNodeWarps consecutive groups
-__device__ __forceinline__ void NodeBody(const Plan& P, const double* __restrict__ XT, double* __restrict__ GT, double* __restrict__ jac,
-                                         int* __restrict__ status, const int* __restrict__ terrain_ids, int default_terrain, int nb,
-                                         unsigned flags, double* node_smem, int cta, int tile, const Stage st, double* __restrict__ g = nullptr) {
+__device__ __forceinline__ void NodeBody(const Plan& P, const double* __restrict__ XT, double* __restrict__ jac, int* __restrict__ status,
+                                         const int* __restrict__ terrain_ids, int default_terrain, int nb, unsigned flags, double* node_smem,
+                                         int cta, int tile, double* __restrict__ g) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const bool g_direct = TWB_GDIRECT && g != nullptr;
   const int gi = cta * kNodeWarps + warp, b = TileInstance(P.nc_jac, tile, lane);
   double* t = node_smem + (size_t)warp * P.node_rows * kLD;
   if (gi < P.n_groups) {
@@ -1499,7 +1175,6 @@ __device__ __forceinline__ void NodeBody(const Plan& P, const double* __restrict
     const int kind = __ldg(&grp->kind), first = __ldg(&grp->first), count = __ldg(&grp->count);
     t[lane] = 1.0;
     int n_rows = 1;
-#ifndef TWB_EXP_NOCOMPUTE
     if (kind == kGroupForce) {
       const int terrain = (terrain_ids && b < nb) ? __ldg(terrain_ids + b) : default_terrain;
       for (int q = 0; q < count; ++q)
@@ -1521,8 +1196,7 @@ __device__ __forceinline__ void NodeBody(const Plan& P, const double* __restrict
       n_rows = (flags & 1u) ? 1 + 6 * count : 1;
     }
     FlagNonFinite(t, n_rows, lane, status, b, nb);
-#endif
-    if ((flags & 1u) && g_direct) {   // the group's consecutive rows, this warp's own state: lanes = (instance, row) pairs
+    if (flags & 1u) {   // the group's consecutive rows, this warp's own state: lanes = (instance, row) pairs
       const int g_row0 = __ldg(&grp->g_row0), nc = P.nc_jac, n_inst = TileCount(nc, tile, nb);
       __syncwarp();
       if (g_row0 >= 0) {
@@ -1544,19 +1218,10 @@ __device__ __forceinline__ void NodeBody(const Plan& P, const double* __restrict
         ForEachEntry(P.pairs + r.first, P.coefs + r.first, r.count, lane,
                      [&](int g_row, int d, double c) { if (b < nb) StoreG(g + (size_t)b * P.m + g_row, t[d * kLD + lane] * c); });
       }
-    } else if (flags & 1u) {
-      const int g_row0 = __ldg(&grp->g_row0);
-      if (g_row0 >= 0) {
-        const int d0 = __ldg(&grp->g_d0), gn = __ldg(&grp->g_n);
-        double* gt = GT + (((size_t)tile * P.m + (size_t)g_row0) * 32) + lane;
-        for (int i = 0; i < gn; ++i) gt[(size_t)i * 32] = t[(d0 + i) * kLD + lane];
-      } else {
-        StoreValuesTiled(P, t, &grp->values, GT + (size_t)tile * P.m * 32, lane);
-      }
     }
   }
   __syncthreads();
-  if (flags & 2u) StoreCta(P, node_smem, P.cta_lists + P.node_list0 + cta, jac, tile, nb, st);
+  if (flags & 2u) StoreCta(P, node_smem, P.cta_lists + P.node_list0 + cta, jac, tile, nb);
 }
 
 // NodeCost::GetCost summed over terms (node_cost.cc:53-63; Composite::GetValues for costs) and the dense gradient row
@@ -1588,18 +1253,14 @@ __global__ void __launch_bounds__(128) CostKernel(const Plan P, const double* __
 // into the foot's state block (device_tables.h: kTailRows); then all threads of the CTA walk the sample's list of phase
 // elements — the same coalesced whole-sector pair loop as every other Jacobian value.  (Until round 2 these entries were
 // scattered by lane = instance 8-byte stores over rows of zeros: 1.0 of config 4's 1.26 ms.)
-#ifndef TWB_TAIL_CTAS
-#define TWB_TAIL_CTAS 4   // resident CTAs per SM the DynTailOut kernel is compiled for (128 registers; 49 state rows per foot = 53 KB per CTA)
-#endif
 template <int kNEE>
-__global__ void __launch_bounds__(kNEE * 32, TWB_TAIL_CTAS) DynTailOut(const Plan P, const double* __restrict__ XT, double* __restrict__ jac, int nb,
+__global__ void __launch_bounds__(kNEE * 32, kTailCtas) DynTailOut(const Plan P, const double* __restrict__ XT, double* __restrict__ jac, int nb,
                                                         double* __restrict__ FS) {
   extern __shared__ __align__(16) double out_smem[];
   const int lane = threadIdx.x & 31, e = threadIdx.x >> 5, k = blockIdx.x;
   double* t = out_smem + (size_t)e * kTailRows * kLD;
   const SplineSample* __restrict__ sp = P.samples + __ldg(&P.dyn[k].sample0);
   const ConstCol xs = TileCol(XT, blockIdx.y, lane, P.n + 1);
-#ifndef TWB_EXP_NOCOMPUTE
   double c[3], unused[3];
   EvalSpline<0>(P, sp, xs, c, unused, unused);
   const double tg = __ldg(&sp[2 + e].T);   // phase samples carry the global time
@@ -1629,16 +1290,15 @@ __global__ void __launch_bounds__(kNEE * 32, TWB_TAIL_CTAS) DynTailOut(const Pla
     V[3 + i] = -jfV[i];
   }
   StorePhaseDurations<6, kDynDurWin>(mo.cur, U, V, t, 7, 7 + 2 * kInfoRows, lane);
-#endif
   __syncthreads();
-  StoreCta<true>(P, out_smem, P.cta_lists + P.tail_list0 + k, jac, blockIdx.y, nb, Stage{nullptr, 0}, 6, kDynDurWin, 8);
+  StoreCta<true>(P, out_smem, P.cta_lists + P.tail_list0 + k, jac, blockIdx.y, nb, 6, kDynDurWin, 8);
 }
 
 // TotalDurationConstraint (total_duration_constraint.cc:36-72; the only rows no output kernel owns): value = sum of the foot's
 // optimised durations, Jacobian = 1 in each of their columns, status bit 1 when the sum leaves nothing for the last phase
 // (phase_durations.cc:92).  warp = tile of 32 instances, lane = instance; 8 entries per foot at the very end of the CSR row.
 template <int kNEE>
-__global__ void __launch_bounds__(32) PhaseJac(const Plan P, const double* __restrict__ XT, double* __restrict__ GT, double* __restrict__ g, double* __restrict__ jac,
+__global__ void __launch_bounds__(32) PhaseJac(const Plan P, const double* __restrict__ XT, double* __restrict__ g, double* __restrict__ jac,
                                                int* __restrict__ status, int nb, unsigned flags) {
   const int lane = threadIdx.x, b = TileInstance(P.nc_jac, blockIdx.x, lane);
   const bool live = b < nb;
@@ -1653,10 +1313,7 @@ __global__ void __launch_bounds__(32) PhaseJac(const Plan P, const double* __res
         sum += xs[def.sched0 + i];
         if (live && (flags & 2u)) StoreOut(jac + (size_t)b * P.nnz + slot0 + i, 1.0);
       }
-      if (flags & 1u) {
-        if (g) { if (live) StoreG(g + (size_t)b * P.m + row, sum); }
-        else GT[((size_t)blockIdx.x * P.m + row) * 32 + lane] = sum;
-      }
+      if (live && (flags & 1u)) StoreG(g + (size_t)b * P.m + row, sum);
       if (live && status && !(def.t_total - sum > 0.0)) atomicOr(status + b, 2);
     }
   }
@@ -1940,186 +1597,94 @@ __device__ __noinline__ void ConstRunBody(const ConstRun* __restrict__ runs, con
   __syncthreads();   // the values are in shared memory (written by the async proxy, observed through the mbarrier by thread 0)
   if (threadIdx.x < 32 && b0 + (int)threadIdx.x < nb) {
     // evict-first like the st.global.cs of the pair loop: the values are consumed by the host / a solver, they must not push
-    // XT, GT and the lists out of the L2
+    // XT and the lists out of the L2
     unsigned long long pol;
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol));
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group.L2::cache_hint [%0], [%1], %2, %3;"
                  ::"l"(jac + (size_t)(b0 + threadIdx.x) * nnz + r.off), "r"(SmemAddr(smem)), "r"(bytes), "l"(pol) : "memory");
     BulkCommit();
-#if TWB_CONST_WAIT_ALL
-    BulkWaitAll();
-#else
     BulkWaitRead<0>();   // the CTA may retire once the engine has read the staging row (the writes complete before the grid does)
-#endif
   }
 }
 
-#if TWB_FUSED
-// One kernel writes a whole tile of rows: blockIdx.y = instance tile, blockIdx.x walks the tile's CTAs in row
-// order — dynamic samples, range-of-motion samples, node groups.
 template <int kNEE, bool kPhase>
-__global__ void __launch_bounds__(kWarps * 32, TWB_CTAS) EvalOut(const Plan P, const double* __restrict__ XT, double* __restrict__ GT,
-                                                              double* __restrict__ jac, int* __restrict__ status,
-                                                              const int* __restrict__ terrain_ids, int default_terrain, int nb, unsigned flags) {
+__global__ void __launch_bounds__(kDynWarps * 32, kDynCtas) DynOut(const Plan P, const double* __restrict__ XT, double* __restrict__ jac,
+                                                                   int* __restrict__ status, int nb, unsigned flags, const double* __restrict__ FS,
+                                                                   double* __restrict__ g) {
   extern __shared__ __align__(16) double out_smem[];
-  const int n_dyn_ctas = (P.n_dyn + kWarps - 1) / kWarps, n_rom_ctas = (P.n_rom + kWarps - 1) / kWarps;
-  int cta = blockIdx.x;
-  if (cta < n_dyn_ctas) { DynBody<kNEE, kPhase>(P, XT, GT, jac, status, nb, flags, out_smem, cta, blockIdx.y, Stage{nullptr, 0}); return; }
-  cta -= n_dyn_ctas;
-  if (cta < n_rom_ctas) { RomBody<kNEE, kPhase>(P, XT, GT, jac, status, nb, flags, out_smem, cta, blockIdx.y, Stage{nullptr, 0}); return; }
-  cta -= n_rom_ctas;
-  NodeBody(P, XT, GT, jac, status, terrain_ids, default_terrain, nb, flags, out_smem, cta, blockIdx.y, Stage{nullptr, 0});
+  DynBody<kNEE, kPhase>(P, XT, jac, status, nb, flags, out_smem, blockIdx.x, blockIdx.y, FS, g);
 }
-#else
+// The range-of-motion and node CTAs of a tile in one kernel (equal CTA sizes), in row order, so that the CTAs resident at any
+// moment fill long contiguous stretches of the tile's rows; then the constant-run CTAs (ConstRunBody).
 template <int kNEE, bool kPhase>
-__global__ void __launch_bounds__(kDynWarps * 32, TWB_DYN_CTAS) DynOut(const Plan P, const double* __restrict__ XT, double* __restrict__ GT,
-                                                           double* __restrict__ jac, int* __restrict__ status, int nb, unsigned flags,
-                                                           int stage_off, int stage_cap, const double* __restrict__ FS, double* __restrict__ g,
-                                                           int* __restrict__ tile_done, int done_total) {
+__global__ void __launch_bounds__(kRomWarps * 32, kRomCtas) RomNodeOut(const Plan P, const double* __restrict__ XT, double* __restrict__ jac,
+                                                                       int* __restrict__ status, const int* __restrict__ terrain_ids,
+                                                                       int default_terrain, int nb, unsigned flags, double* __restrict__ g) {
   extern __shared__ __align__(16) double out_smem[];
-  DynBody<kNEE, kPhase>(P, XT, GT, jac, status, nb, flags, out_smem, blockIdx.x, blockIdx.y, Stage{out_smem + stage_off, stage_cap}, FS, g);
-  TileDone(tile_done, done_total, XT, P.n, P.nc_jac, blockIdx.y, nb);
-#if TWB_TMA
-  if ((threadIdx.x & 31) == 0) BulkWaitAll();   // the staging rows stay allocated until the last copy has left
-#endif
-}
-template <int kNEE, bool kPhase>
-__global__ void __launch_bounds__(kRomWarps * 32, TWB_ROM_CTAS) RomOut(const Plan P, const double* __restrict__ XT, double* __restrict__ GT,
-                                                           double* __restrict__ jac, int* __restrict__ status, int nb, unsigned flags) {
-  extern __shared__ __align__(16) double out_smem[];
-  RomBody<kNEE, kPhase>(P, XT, GT, jac, status, nb, flags, out_smem, blockIdx.x, blockIdx.y, Stage{nullptr, 0});
-}
-__global__ void __launch_bounds__(kNodeWarps * 32, TWB_NODE_CTAS) NodeOut(const Plan P, const double* __restrict__ XT, double* __restrict__ GT,
-                                                           double* __restrict__ jac, int* __restrict__ status,
-                                                           const int* __restrict__ terrain_ids, int default_terrain, int nb, unsigned flags) {
-  extern __shared__ __align__(16) double out_smem[];
-  NodeBody(P, XT, GT, jac, status, terrain_ids, default_terrain, nb, flags, out_smem, blockIdx.x, blockIdx.y, Stage{nullptr, 0});
-}
-#if TWB_ROMNODE   // range-of-motion and node CTAs of a tile in one kernel (kRomWarps == kNodeWarps), in row order
-template <int kNEE, bool kPhase>
-__global__ void __launch_bounds__(kRomWarps * 32, TWB_ROM_CTAS) RomNodeOut(const Plan P, const double* __restrict__ XT, double* __restrict__ GT,
-                                                               double* __restrict__ jac, int* __restrict__ status,
-                                                               const int* __restrict__ terrain_ids, int default_terrain, int nb, unsigned flags,
-                                                               int stage_off, int stage_cap, double* __restrict__ g,
-                                                               int* __restrict__ tile_done, int done_total) {
-  extern __shared__ __align__(16) double out_smem[];
-  static_assert(kRomWarps == kNodeWarps, "TWB_ROMNODE needs equal CTA sizes");
-  const Stage st{out_smem + stage_off, stage_cap};
-#if TWB_PDL
-  asm volatile("griddepcontrol.wait;" ::: "memory");   // XT complete and visible (programmatic dependency on TransposeIn)
-#endif
+  static_assert(kRomWarps == kNodeWarps, "RomNodeOut needs equal CTA sizes");
+  asm volatile("griddepcontrol.wait;" ::: "memory");   // XT complete and visible (programmatic dependency on TransposeInP)
   const int n_rom_ctas = (P.n_rom + kRomWarps - 1) / kRomWarps;
   const int n_node_ctas = (P.n_groups + kNodeWarps - 1) / kNodeWarps;
   if ((int)blockIdx.x >= n_rom_ctas + n_node_ctas) {   // constant runs: TMA only
     if (flags & 2u) ConstRunBody(P.const_runs, P.const_vals, P.nnz, jac, nb, out_smem, blockIdx.x - n_rom_ctas - n_node_ctas, blockIdx.y);
-    TileDone(tile_done, done_total, XT, P.n, P.nc_jac, blockIdx.y, nb);
     return;
   }
-  if ((int)blockIdx.x < n_rom_ctas) RomBody<kNEE, kPhase>(P, XT, GT, jac, status, nb, flags, out_smem, blockIdx.x, blockIdx.y, st, g);
-#ifndef TWB_EXP_NONODE   // (timing experiment: node CTAs return at once)
-  else NodeBody(P, XT, GT, jac, status, terrain_ids, default_terrain, nb, flags, out_smem, blockIdx.x - n_rom_ctas, blockIdx.y, st, g);
-#endif
-#if TWB_TMA
-  if ((threadIdx.x & 31) == 0) BulkWaitAll();
-#endif
-  TileDone(tile_done, done_total, XT, P.n, P.nc_jac, blockIdx.y, nb);
+  if ((int)blockIdx.x < n_rom_ctas) RomBody<kNEE, kPhase>(P, XT, jac, status, nb, flags, out_smem, blockIdx.x, blockIdx.y, g);
+  else NodeBody(P, XT, jac, status, terrain_ids, default_terrain, nb, flags, out_smem, blockIdx.x - n_rom_ctas, blockIdx.y, g);
 }
-#endif
-#endif
 
 // number of tiles that cover nb instances (whole groups of nc interleaved tiles)
 inline int TileTotal(int nc, int nb) { return nc * ((nb + 32 * nc - 1) / (32 * nc)); }
 
-// kernel launch with the optional attributes of this pipeline: programmatic dependent launch, L2 access-policy window
+// kernel launch, optionally with programmatic dependent launch
 template <class... KArgs, class... Args>
 cudaError_t LaunchK(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool pdl, Args... args) {
   cudaLaunchConfig_t cfg{}; cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute attr[2]; unsigned na = 0;
-  if (pdl) { attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[na].val.programmaticStreamSerializationAllowed = 1; ++na; }
-  if (t_l2_window) { attr[na].id = cudaLaunchAttributeAccessPolicyWindow; attr[na].val.accessPolicyWindow = *t_l2_window; ++na; }
-  cfg.attrs = attr; cfg.numAttrs = na;
+  cudaLaunchAttribute attr{};
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization; attr.val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = &attr; cfg.numAttrs = pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
 }
 
-// s: caller's stream (after TransposeIn); a0, a1: auxiliary streams already waiting on the transposition
+// x -> XT (TransposeInP) for nb instances in `tiles` tiles; clears status when it is given
+cudaError_t LaunchTransposeIn(const Plan& P, const double* x, double* XT, int* status, int nb, int tiles, cudaStream_t s) {
+  const int n_ctiles = (P.n + 31) / 32, total = n_ctiles * tiles;
+  return LaunchK(TransposeInP, dim3(std::min(total, 148 * kTinPersist)), dim3(32, 8), 0, s, false, x, XT, status, P.n, nb, P.nc_jac, n_ctiles, total);
+}
+
+// s: caller's stream (after TransposeInP); a0: auxiliary stream already waiting on the transposition.  RomNodeOut on s, launched
+// with programmatic stream serialization behind TransposeInP (138.9 vs 144.6 us per step on config 2); the dynamic rows on a0:
+// with optimised durations and a Jacobian evaluation first DynTailOut (the PhaseSpline columns; it leaves the feet's positions
+// and forces in FS), then DynOut (base columns and the constraint values)
 template <int kNEE, bool kPhase>
-cudaError_t LaunchOut(const Plan& P, const double* XT, double* GT, double* FS, double* g_direct, int* tile_done_in, double* jac, int* status, const int* terrain_ids, int default_terrain,
-                      int nb, unsigned flags, int tiles, cudaStream_t s, cudaStream_t a0, cudaStream_t a1, int* count) {
+cudaError_t LaunchOut(const Plan& P, const double* XT, double* FS, double* g, double* jac, int* status, const int* terrain_ids, int default_terrain,
+                      int nb, unsigned flags, int tiles, cudaStream_t s, cudaStream_t a0, int* count) {
   const size_t row_bytes = (size_t)kLD * sizeof(double);
-  const int dyn_rows = DynBlockRows(kNEE), rom_rows = RomBlockRowsP(kNEE, kPhase), node_rows = P.node_rows;
-  cudaError_t e = cudaSuccess;
-  // CTAs per tile of the two output kernels (the count that completes a tile's counter, TileDone)
-  const int done_total = (P.n_dyn > 0 ? (P.n_dyn + kDynWarps - 1) / kDynWarps : 0) +
-                         (P.n_rom + kRomWarps - 1) / kRomWarps + (P.n_groups + kNodeWarps - 1) / kNodeWarps + P.n_const_runs;
-  int* tile_done = (TWB_ROMNODE && !TWB_FUSED) ? tile_done_in : nullptr;
-#if !TWB_FUSED
-  // the dynamic rows on stream a0: with optimised durations and a Jacobian evaluation first DynTailOut (the PhaseSpline columns; it
-  // leaves the feet's positions and forces in FS), then DynOut (base columns and the constraint values)
-  auto launch_dyn = [&]() -> cudaError_t {
-    if (P.n_dyn <= 0) return cudaSuccess;
-    cudaError_t err;
-    const bool tail = kPhase && (flags & 2u);
-    if (tail) {
-      const size_t tail_smem = (size_t)kNEE * kTailRows * row_bytes;
-      if ((err = cudaFuncSetAttribute(DynTailOut<kNEE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tail_smem)) != cudaSuccess) return err;
-      DynTailOut<kNEE><<<dim3(P.n_dyn, tiles), kNEE * 32, tail_smem, a0>>>(P, XT, jac, nb, FS);
-      ++*count; TWB_MARK("DynTailOut", a0);
-    }
-    const size_t state_bytes = (size_t)kDynWarps * dyn_rows * row_bytes;
-    const int stage_off = (int)(state_bytes / sizeof(double));
-    int stage_cap = TWB_TMA_DYN ? P.stage_dyn : 0;
-    if (state_bytes + (size_t)kDynWarps * (TWB_TMA_BUF * TWB_TMA_G) * stage_cap * sizeof(double) > 200 * 1024) stage_cap = 0;
-    const size_t smem = state_bytes + (size_t)kDynWarps * (TWB_TMA_BUF * TWB_TMA_G) * stage_cap * sizeof(double);
-    if ((err = cudaFuncSetAttribute(DynOut<kNEE, kPhase>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return err;
-    if ((err = LaunchK(DynOut<kNEE, kPhase>, dim3((P.n_dyn + kDynWarps - 1) / kDynWarps, tiles), dim3(kDynWarps * 32), smem, a0, false, P, XT, GT, jac, status, nb, flags,
-                       stage_off, stage_cap, (const double*)(tail ? FS : nullptr), g_direct, tile_done, done_total)) != cudaSuccess) return err;
-    ++*count; TWB_MARK("DynOut", a0);
-    return cudaSuccess;
-  };
-#endif
-#if TWB_FUSED
-  const int n_ctas = (P.n_dyn + kWarps - 1) / kWarps + (P.n_rom + kWarps - 1) / kWarps + (P.n_groups + kWarps - 1) / kWarps;
-  if (n_ctas == 0) return cudaSuccess;
-  if (kPhase) return cudaErrorNotSupported;   // the fused experiment does not carry the PhaseSpline columns
-  const int rows = std::max(std::max(P.n_dyn > 0 ? dyn_rows : 0, P.n_rom > 0 ? rom_rows : 0), P.n_groups > 0 ? node_rows : 0);
-  const size_t smem = (size_t)kWarps * rows * row_bytes;
-  if ((e = cudaFuncSetAttribute(EvalOut<kNEE, kPhase>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-  EvalOut<kNEE, kPhase><<<dim3(n_ctas, tiles), kWarps * 32, smem, s>>>(P, XT, GT, jac, status, terrain_ids, default_terrain, nb, flags);
-  ++*count; TWB_MARK("EvalOut", s);
-#else
-#if TWB_ROMNODE
+  cudaError_t e;
   {
-    const size_t state_bytes = (size_t)kRomWarps * std::max(rom_rows, node_rows) * row_bytes;
-    const int stage_off = (int)(state_bytes / sizeof(double));
-    int stage_cap = TWB_TMA_ROM ? std::max(P.stage_rom, P.stage_node) : 0;
-    if (state_bytes + (size_t)kRomWarps * (TWB_TMA_BUF * TWB_TMA_G) * stage_cap * sizeof(double) > 100 * 1024) stage_cap = 0;   // dense rows (optimised durations): st.global path
-    const size_t smem = std::max(state_bytes + (size_t)kRomWarps * (TWB_TMA_BUF * TWB_TMA_G) * stage_cap * sizeof(double),
-                                 P.n_const_runs > 0 ? (size_t)kConstRunMax * sizeof(double) : (size_t)0);
+    const size_t state_bytes = (size_t)kRomWarps * std::max(RomBlockRowsP(kNEE, kPhase), P.node_rows) * row_bytes;
+    const size_t smem = std::max(state_bytes, P.n_const_runs > 0 ? (size_t)kConstRunMax * sizeof(double) : (size_t)0);
     if ((e = cudaFuncSetAttribute(RomNodeOut<kNEE, kPhase>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
     const int n_ctas = (P.n_rom + kRomWarps - 1) / kRomWarps + (P.n_groups + kNodeWarps - 1) / kNodeWarps + P.n_const_runs;
     if (n_ctas > 0) {
-      if ((e = LaunchK(RomNodeOut<kNEE, kPhase>, dim3(n_ctas, tiles), dim3(kRomWarps * 32), smem, s, TWB_PDL != 0, P, XT, GT, jac, status, terrain_ids,
-                       default_terrain, nb, flags, stage_off, stage_cap, g_direct, tile_done, done_total)) != cudaSuccess) return e;
+      if ((e = LaunchK(RomNodeOut<kNEE, kPhase>, dim3(n_ctas, tiles), dim3(kRomWarps * 32), smem, s, true, P, XT, jac, status, terrain_ids,
+                       default_terrain, nb, flags, g)) != cudaSuccess) return e;
       ++*count; TWB_MARK("RomNodeOut", s);
     }
   }
-  if ((e = launch_dyn()) != cudaSuccess) return e;
-  return cudaSuccess;
-#endif
-  if (P.n_rom > 0) {
-    const size_t smem = (size_t)kRomWarps * rom_rows * row_bytes;
-    if ((e = cudaFuncSetAttribute(RomOut<kNEE, kPhase>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-    RomOut<kNEE, kPhase><<<dim3((P.n_rom + kRomWarps - 1) / kRomWarps, tiles), kRomWarps * 32, smem, s>>>(P, XT, GT, jac, status, nb, flags);
-    ++*count; TWB_MARK("RomOut", s);
+  if (P.n_dyn <= 0) return cudaSuccess;
+  const bool tail = kPhase && (flags & 2u);
+  if (tail) {
+    const size_t tail_smem = (size_t)kNEE * kTailRows * row_bytes;
+    if ((e = cudaFuncSetAttribute(DynTailOut<kNEE>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tail_smem)) != cudaSuccess) return e;
+    DynTailOut<kNEE><<<dim3(P.n_dyn, tiles), kNEE * 32, tail_smem, a0>>>(P, XT, jac, nb, FS);
+    ++*count; TWB_MARK("DynTailOut", a0);
   }
-  if ((e = launch_dyn()) != cudaSuccess) return e;
-  if (P.n_groups > 0) {
-    const size_t smem = (size_t)kNodeWarps * node_rows * row_bytes;
-    if ((e = cudaFuncSetAttribute(NodeOut, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-    NodeOut<<<dim3((P.n_groups + kNodeWarps - 1) / kNodeWarps, tiles), kNodeWarps * 32, smem, a1>>>(P, XT, GT, jac, status, terrain_ids, default_terrain, nb, flags);
-    ++*count; TWB_MARK("NodeOut", a1);
-  }
-#endif
+  const size_t smem = (size_t)kDynWarps * DynBlockRows(kNEE) * row_bytes;
+  if ((e = cudaFuncSetAttribute(DynOut<kNEE, kPhase>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+  if ((e = LaunchK(DynOut<kNEE, kPhase>, dim3((P.n_dyn + kDynWarps - 1) / kDynWarps, tiles), dim3(kDynWarps * 32), smem, a0, false, P, XT, jac, status, nb,
+                   flags, (const double*)(tail ? FS : nullptr), g)) != cudaSuccess) return e;
+  ++*count; TWB_MARK("DynOut", a0);
   return cudaSuccess;
 }
 
@@ -2131,7 +1696,7 @@ int LaunchTrajectory(const Plan& P, const double* x, double* XT, const SplineSam
                      double* out, int nb, cudaStream_t s) {
   if (nb <= 0 || n_steps <= 0) return 0;
   const int tiles = TileTotal(P.nc_jac, nb);
-  TransposeIn<<<dim3((P.n + 32 * kTinTiles - 1) / (32 * kTinTiles), tiles), dim3(32, 8), 0, s>>>(x, XT, nullptr, P.n, nb, P.nc_jac);
+  LaunchTransposeIn(P, x, XT, nullptr, nb, tiles, s);
   const dim3 grid((n_steps + 3) / 4, tiles);
   const bool phase = P.n_phase_defs > 0;
   // dynamic shared memory: the four warps' staging tiles [19 + 13 n_ee][33] of the coalesced stores
@@ -2154,7 +1719,7 @@ int LaunchInitialGuess(const Plan& P, const double* x, double* XT, const SplineS
                        double* out, int nb, cudaStream_t s) {
   if (nb <= 0 || n_times <= 0) return 0;
   const int tiles = TileTotal(P.nc_jac, nb);
-  TransposeIn<<<dim3((P.n + 32 * kTinTiles - 1) / (32 * kTinTiles), tiles), dim3(32, 8), 0, s>>>(x, XT, nullptr, P.n, nb, P.nc_jac);
+  LaunchTransposeIn(P, x, XT, nullptr, nb, tiles, s);
   const dim3 grid((n_times + 3) / 4, tiles);
   const bool phase = P.n_phase_defs > 0;
 #define TWB_IG(NEE) { const size_t sm = 4 * (size_t)49 * 33 * sizeof(double);                                                                    \
@@ -2177,7 +1742,7 @@ int LaunchFootstepPlan(const Plan& P, const double* x, double* XT, const SplineS
                        cudaStream_t s) {
   if (nb <= 0 || max_states <= 0) return 0;
   const int tiles = TileTotal(P.nc_jac, nb);
-  TransposeIn<<<dim3((P.n + 32 * kTinTiles - 1) / (32 * kTinTiles), tiles), dim3(32, 8), 0, s>>>(x, XT, nullptr, P.n, nb, P.nc_jac);
+  LaunchTransposeIn(P, x, XT, nullptr, nb, tiles, s);
   const bool phase = P.n_phase_defs > 0;
   // dynamic shared memory per warp: the staging tile [V][33] of the coalesced stores; optimised durations: the change codes [max_states + 1][32]
 #define TWB_FSP(NEE) { const size_t sm = 4 * ((size_t)(2 + 4 * NEE) * 33 * sizeof(double) + (phase ? (size_t)(max_states + 1) * 32 * sizeof(int) : 0)); \
@@ -2241,7 +1806,7 @@ __global__ void __launch_bounds__(128) SoftConstraintKernel(const double* __rest
 int LaunchLinearEquality(const Plan& P, const double* x, double* XT, int col0, int n_cols, const double* M, int rows, double* g, int nb, cudaStream_t s) {
   if (nb <= 0 || rows <= 0) return 0;
   const int tiles = TileTotal(P.nc_jac, nb);
-  TransposeIn<<<dim3((P.n + 32 * kTinTiles - 1) / (32 * kTinTiles), tiles), dim3(32, 8), 0, s>>>(x, XT, nullptr, P.n, nb, P.nc_jac);
+  LaunchTransposeIn(P, x, XT, nullptr, nb, tiles, s);
   LinearEqualityKernel<<<dim3((rows + 3) / 4, tiles), 128, 0, s>>>(XT, P.n, col0, n_cols, M, rows, g, nb, P.nc_jac);
   return (int)cudaGetLastError();
 }
@@ -2385,24 +1950,15 @@ int LaunchStateInstances(const Plan& P, const GoalSetup& S, const double* states
   return (int)cudaGetLastError();
 }
 
-// 1 when the constraint values go through GT and the TransposeOut kernel (optimised durations, experimental variants), else 0
-int TransposeOutPerEval(const Plan& P) { return (TWB_GDIRECT && TWB_ROMNODE && !TWB_FUSED && (TWB_GDIRECT_PHASE || P.n_phase_defs == 0)) ? 0 : 1; }
 int OutKernelsPerEval(const Plan& P, unsigned flags) {
   const int dyn = (P.n_dyn > 0) * ((P.n_phase_defs > 0 && (flags & 2u)) ? 2 : 1);   // DynOut [+ DynTailOut]
-#if TWB_FUSED
-  (void)dyn; return (P.n_dyn + P.n_rom + P.n_groups) > 0;
-#elif TWB_ROMNODE
-  return dyn + ((P.n_rom + P.n_groups) > 0);
-#else
-  return dyn + (P.n_rom > 0) + (P.n_groups > 0);
-#endif
+  return dyn + ((P.n_rom + P.n_groups) > 0);                                         // + RomNodeOut
 }
 
-// XT / GT are the instance-tiled iterate and constraint-value matrices of the whole batch (first tile = first
-// instance of x / g / jac).  Streams: `s` carries TransposeIn -> [out kernels] -> TransposeOut; with separate
-// out kernels DynOut / NodeOut (and the CostKernel) run beside RomOut on aux0 / aux1 after the transposition
-// (ev[0]) and are joined back into `s` (ev[1], ev[2]) before TransposeOut.
-int LaunchEval(const Plan& P, const double* x, double* XT, double* GT, double* FS, int* TD, double* g, double* jac, double* cost, double* grad,
+// XT is the instance-tiled iterate matrix of the whole batch (first tile = first instance of x / g / jac).  Streams: `s` carries
+// TransposeInP -> RomNodeOut; DynTailOut / DynOut run beside it on aux0, PhaseJac and the CostKernel on aux1, after the
+// transposition (ev[0]); both are joined back into `s` (ev[1], ev[2]).
+int LaunchEval(const Plan& P, const double* x, double* XT, double* FS, double* g, double* jac, double* cost, double* grad,
                int* status, const int* terrain_ids, int default_terrain, int nb, unsigned flags, cudaStream_t s,
                cudaStream_t aux0, cudaStream_t aux1, cudaEvent_t* ev, int* launches) {
   if (nb <= 0) return 0;
@@ -2413,38 +1969,28 @@ int LaunchEval(const Plan& P, const double* x, double* XT, double* GT, double* F
   const unsigned out_flags = flags & 3u;
   const bool want_cost = (flags & 4u) && P.n_cost > 0;
   TWB_MARK("begin", s);
-#if TWB_TIN_PERSIST
-  {
-    const int n_ctiles = (P.n + 31) / 32, total = n_ctiles * tiles;
-    LaunchK(TransposeInP, dim3(std::min(total, 148 * TWB_TIN_PERSIST)), dim3(32, 8), 0, s, false, x, XT, status, P.n, nb, P.nc_jac, n_ctiles, total); ++count; TWB_MARK("TransposeIn", s);
-  }
-#else
-  LaunchK(TransposeIn, dim3((P.n + 32 * kTinTiles - 1) / (32 * kTinTiles), tiles), dim3(32, 8), 0, s, false, x, XT, status, P.n, nb, P.nc_jac); ++count; TWB_MARK("TransposeIn", s);
-#endif
-  const bool fork = !serial && (want_cost || (!TWB_FUSED && out_flags));
+  LaunchTransposeIn(P, x, XT, status, nb, tiles, s); ++count; TWB_MARK("TransposeIn", s);
+  const bool fork = !serial && (want_cost || out_flags);
   if (fork) { cudaEventRecord(ev[0], s); cudaStreamWaitEvent(aux0, ev[0], 0); cudaStreamWaitEvent(aux1, ev[0], 0); }
   cudaError_t e = cudaSuccess;
-  // fixed durations: the output kernels write the constraint values straight into g (no GT, no TransposeOut)
-  const bool direct = TWB_GDIRECT && TWB_ROMNODE && !TWB_FUSED && (TWB_GDIRECT_PHASE || P.n_phase_defs == 0);
-  double* g_direct = (direct && (out_flags & 1u)) ? g : nullptr;
   if (out_flags) {
     const bool phase = P.n_phase_defs > 0;
     switch (P.n_ee) {
-      case 1: e = phase ? LaunchOut<1, true>(P, XT, GT, FS, g_direct, direct ? TD : nullptr, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, aux1, &count)
-                       : LaunchOut<1, false>(P, XT, GT, FS, g_direct, direct ? TD : nullptr, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, aux1, &count); break;
-      case 2: e = phase ? LaunchOut<2, true>(P, XT, GT, FS, g_direct, direct ? TD : nullptr, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, aux1, &count)
-                       : LaunchOut<2, false>(P, XT, GT, FS, g_direct, direct ? TD : nullptr, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, aux1, &count); break;
-      case 4: e = phase ? LaunchOut<4, true>(P, XT, GT, FS, g_direct, direct ? TD : nullptr, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, aux1, &count)
-                       : LaunchOut<4, false>(P, XT, GT, FS, g_direct, direct ? TD : nullptr, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, aux1, &count); break;
+      case 1: e = phase ? LaunchOut<1, true>(P, XT, FS, g, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, &count)
+                       : LaunchOut<1, false>(P, XT, FS, g, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, &count); break;
+      case 2: e = phase ? LaunchOut<2, true>(P, XT, FS, g, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, &count)
+                       : LaunchOut<2, false>(P, XT, FS, g, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, &count); break;
+      case 4: e = phase ? LaunchOut<4, true>(P, XT, FS, g, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, &count)
+                       : LaunchOut<4, false>(P, XT, FS, g, jac, status, terrain_ids, default_terrain, nb, out_flags, tiles, s, aux0, &count); break;
       default: return (int)cudaErrorInvalidValue;
     }
     if (e != cudaSuccess) return (int)e;
   }
   if (out_flags && P.n_phase_units > 0) {   // TotalDurationConstraint rows: needs XT only, beside the output kernels on the third stream
     switch (P.n_ee) {
-      case 1: PhaseJac<1><<<tiles, 32, 0, aux1>>>(P, XT, GT, g_direct, jac, status, nb, out_flags); break;
-      case 2: PhaseJac<2><<<tiles, 32, 0, aux1>>>(P, XT, GT, g_direct, jac, status, nb, out_flags); break;
-      default: PhaseJac<4><<<tiles, 32, 0, aux1>>>(P, XT, GT, g_direct, jac, status, nb, out_flags); break;
+      case 1: PhaseJac<1><<<tiles, 32, 0, aux1>>>(P, XT, g, jac, status, nb, out_flags); break;
+      case 2: PhaseJac<2><<<tiles, 32, 0, aux1>>>(P, XT, g, jac, status, nb, out_flags); break;
+      default: PhaseJac<4><<<tiles, 32, 0, aux1>>>(P, XT, g, jac, status, nb, out_flags); break;
     }
     ++count; TWB_MARK("PhaseJac", aux1);
   }
@@ -2456,7 +2002,6 @@ int LaunchEval(const Plan& P, const double* x, double* XT, double* GT, double* F
     cudaEventRecord(ev[1], aux0); cudaEventRecord(ev[2], aux1);
     cudaStreamWaitEvent(s, ev[1], 0); cudaStreamWaitEvent(s, ev[2], 0);
   }
-  if ((out_flags & 1u) && !direct) { LaunchK(TransposeOut, dim3((P.m + 31) / 32, tiles), dim3(32, 8), 0, s, false, (const double*)GT, g, P.m, nb, XT, P.n, P.nc_jac); ++count; TWB_MARK("TransposeOut", s); }
   if (launches) *launches += count;
   return (int)cudaGetLastError();
 }

@@ -14,10 +14,6 @@ namespace twb {
 // kernels are serialised on one stream
 extern void (*g_after_launch)(const char* label, cudaStream_t stream);
 
-// One batched evaluation of `nb` instances.  XT is [tiles][n+1][32] (zero-initialised once; row n stays 0;
-// tile = 32 consecutive instances), GT is [tiles][m][32] (staging of the constraint values).  x, g, jac, cost, grad, status and terrain_ids point at the first
-// instance.  `flags` are the TWB_EVAL_* bits.  Work is enqueued on `s` and on two auxiliary streams that
-// are forked from / joined back into `s` with ev[0..2].
 // fpowr::GetTrajectory for `nb` instances: x -> XT, then out[b][step][19 + 13 n_ee]; `samples` / `contact` are the device
 // copies of Formulation::TrajectoryTables (contact null when the durations are optimised)
 int LaunchTrajectory(const Plan& P, const double* x, double* XT, const SplineSample* samples, const int* contact, int n_steps,
@@ -67,14 +63,13 @@ size_t LmSharedBytes(int n, int m);
 // bounds x_lower / x_upper at b * bound_stride (0: the same bounds for every instance), violation[b] out (may be null)
 int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const double* g, const double* jac, const double* x_lower,
                  const double* x_upper, size_t bound_stride, double mu, double cap, int cg_iters, double* violation, int nb, cudaStream_t s);
-// L2 access-policy window applied to the evaluation kernels launched by this thread (null: none)
-void SetL2Window(const cudaAccessPolicyWindow* w);
 // number of output kernels one evaluation launches for this plan
 int OutKernelsPerEval(const Plan& P, unsigned flags);
-int TransposeOutPerEval(const Plan& P);
+// One batched evaluation of `nb` instances.  XT is [tiles][n+1][32] (zero-initialised once; row n stays 0; tile = 32
+// instances).  x, g, jac, cost, grad, status and terrain_ids point at the first instance.  `flags` are the TWB_EVAL_* bits.
+// Work is enqueued on `s` and on two auxiliary streams that are forked from / joined back into `s` with ev[0..2].
 // FS: scratch of the feet's positions / forces per dynamic sample, [tiles][n_dyn][6 n_ee][32] (optimised durations only, else null)
-// TD: one zero-initialised counter per tile (the output CTAs count themselves; the last one of a tile drops the tile's XT lines)
-int LaunchEval(const Plan& P, const double* x, double* XT, double* GT, double* FS, int* TD, double* g, double* jac, double* cost, double* grad,
+int LaunchEval(const Plan& P, const double* x, double* XT, double* FS, double* g, double* jac, double* cost, double* grad,
                int* status, const int* terrain_ids, int default_terrain, int nb, unsigned flags, cudaStream_t s,
                cudaStream_t aux0, cudaStream_t aux1, cudaEvent_t* ev, int* launches);
 
