@@ -233,8 +233,9 @@ int twb_batch_goal_instances_device(twb_batch* b, const double* goals, double* x
  * each goal is the instance's own, as for twb_batch_goal_instances_device.  The call only enqueues on `stream` (no host
  * synchronisation, no allocation), so it can be captured in a CUDA graph.  Errors: NULL states, every output NULL:
  * TWB_ERR_INVALID, nothing enqueued.
- * twb_batch_lm_step_device keeps using the problem's own constraint bounds: only the BaseMotionConstraint LZ rows differ per
- * instance, and only when TWB_C_BASE_ROM is among the constraints (the default list has no such rows). */
+ * Only the BaseMotionConstraint LZ rows of g_lower / g_upper differ per instance, and only when TWB_C_BASE_ROM is among the
+ * constraints (the default list has no such rows).  twb_batch_lm_step_bounds_device steps every instance against its own
+ * rows of these outputs; twb_batch_lm_step_device steps against the problem's own constraint bounds. */
 int twb_batch_state_instances_device(twb_batch* b, const double* states, double* x0, double* x_lower, double* x_upper,
                                      double* g_lower, double* g_upper, void* stream);
 
@@ -276,6 +277,18 @@ int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac,
  * TWB_ERR_UNSUPPORTED.  Nothing is enqueued when a call fails its checks. */
 int twb_batch_lm_step_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower,
                              const double* x_upper, double mu, double cap, int cg_iters, double* violation, void* stream);
+
+/* twb_batch_lm_step_device with per-instance CONSTRAINT bounds: instance b's violation r is measured against
+ * [g_lower[b][i], g_upper[b][i]] (device [B][m] each, e.g. the g_lower / g_upper of twb_batch_state_instances_device, whose
+ * BaseMotionConstraint rows follow each instance's initial base height).  Both NULL: the problem's own constraint bounds,
+ * exactly twb_batch_lm_step_device.  -Inf / +Inf (like +-1e20) mean unbounded; a NaN bound counts like a non-finite g entry
+ * (the instance is not stepped, violation[b] is NaN); with lower > upper the lower bound wins (g < lower is tested first).
+ * Everything else — the other arguments, the first call's upload, graph capture after it, determinism, the errors — as for
+ * twb_batch_lm_step_device; in addition only one of g_lower / g_upper NULL is TWB_ERR_INVALID.  Nothing is enqueued when a
+ * call fails its checks. */
+int twb_batch_lm_step_bounds_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower,
+                                    const double* x_upper, const double* g_lower, const double* g_upper, double mu, double cap,
+                                    int cg_iters, double* violation, void* stream);
 
 /* Host-pointer variant: copies x up, evaluates, copies the requested outputs
  * back and synchronises. Pinned host memory makes the copies asynchronous. */

@@ -247,6 +247,25 @@ class BatchedProblem {
 
   // ifopt::Problem::SetVariables(const double*) for instance b
   void SetVariables(int b, const double* x) { std::copy(x, x + n_, X.begin() + (size_t)b * n_); dirty_ = true; }
+  // Per-instance start and goal states (what the reference sets in NlpFormulation::initial_base_, final_base_ and
+  // initial_ee_W_ before building each request's ifopt::Problem): states[n_states][TWB_STATE_DOUBLES] for instances
+  // 0 .. n_states - 1.  Row b of X becomes that instance's initial guess, and from now on the views of instance b serve its
+  // own variable and constraint bounds (twb_problem_state_instances; host only, so it also works without a device batch).
+  // Instances past n_states keep their rows and bounds.
+  void SetStates(const double* states, int n_states = -1) {
+    if (n_states < 0) n_states = B_;
+    if (!states || n_states == 0 || n_states > B_) throw std::runtime_error("BatchedProblem::SetStates: bad argument");
+    if (ixl_.empty()) {   // first call: every instance starts from the problem's bounds
+      ixl_.resize((size_t)B_ * n_); ixu_.resize((size_t)B_ * n_); igl_.resize((size_t)B_ * m_); igu_.resize((size_t)B_ * m_);
+      for (int b = 0; b < B_; ++b) {
+        std::copy(xl_.begin(), xl_.end(), ixl_.begin() + (size_t)b * n_); std::copy(xu_.begin(), xu_.end(), ixu_.begin() + (size_t)b * n_);
+        std::copy(gl_.begin(), gl_.end(), igl_.begin() + (size_t)b * m_); std::copy(gu_.begin(), gu_.end(), igu_.begin() + (size_t)b * m_);
+      }
+    }
+    Check(twb_problem_state_instances(prob_, n_states, states, X.data(), ixl_.data(), ixu_.data(), igl_.data(), igu_.data()),
+          "twb_problem_state_instances");
+    dirty_ = true;
+  }
   // one batched evaluation: Problem::EvaluateConstraints + EvalNonzerosOfJacobian + EvaluateCostFunction[Gradient]
   void Evaluate(unsigned flags = TWB_EVAL_ALL) {
     if (!batch_) throw std::runtime_error("BatchedProblem: no device batch");
@@ -300,6 +319,11 @@ class BatchedProblem {
   const std::vector<double>& x_upper() const { return xu_; }
   const std::vector<double>& g_lower() const { return gl_; }
   const std::vector<double>& g_upper() const { return gu_; }
+  // instance b's bounds: the problem's (the accessors above) until SetStates gives the instance its own
+  const double* x_lower(int b) const { return ixl_.empty() ? xl_.data() : ixl_.data() + (size_t)b * n_; }
+  const double* x_upper(int b) const { return ixu_.empty() ? xu_.data() : ixu_.data() + (size_t)b * n_; }
+  const double* g_lower(int b) const { return igl_.empty() ? gl_.data() : igl_.data() + (size_t)b * m_; }
+  const double* g_upper(int b) const { return igu_.empty() ? gu_.data() : igu_.data() + (size_t)b * m_; }
   const twb_problem* handle() const { return prob_; }
 
   std::vector<double> X, G, JAC, COST, GRAD;   // [B][n], [B][m], [B][nnz], [B], [B][n]
@@ -312,12 +336,13 @@ class BatchedProblem {
   bool dirty_ = false;
   std::vector<int> row_ptr_, iRow_, jCol_;
   std::vector<double> xl_, xu_, gl_, gu_;
+  std::vector<double> ixl_, ixu_, igl_, igu_;   // [B][n], [B][n], [B][m], [B][m] after SetStates, else empty
 };
 
 namespace ifo = TWB_IFOPT_NS;
 
 // "base-lin", "ee-motion_0", "ee-schedule1", ... (NodesVariables / PhaseDurations, nodes_variables.cc:40-72,
-// phase_durations.cc:68-110) of instance b: a window of row b of X
+// phase_durations.cc:68-110) of instance b: a window of row b of X, bounded by instance b's variable bounds
 class GpuVariableSet : public ifo::VariableSet {
  public:
   GpuVariableSet(BatchedProblem* p, int b, const std::string& name, int col0, int n) : VariableSet(n, name), p_(p), b_(b), col0_(col0) {}
@@ -329,7 +354,8 @@ class GpuVariableSet : public ifo::VariableSet {
   }
   VecBound GetBounds() const override {
     VecBound v;
-    for (int i = 0; i < GetRows(); ++i) v.push_back(ifo::Bounds(p_->x_lower()[col0_ + i], p_->x_upper()[col0_ + i]));
+    const double *lo = p_->x_lower(b_), *up = p_->x_upper(b_);
+    for (int i = 0; i < GetRows(); ++i) v.push_back(ifo::Bounds(lo[col0_ + i], up[col0_ + i]));
     return v;
   }
   // NodesVariables::SetVariables (nodes_variables.cc:65-72): the values move into the batch's iterate; the next Get* of a
@@ -344,7 +370,8 @@ class GpuVariableSet : public ifo::VariableSet {
   BatchedProblem* p_; int b_, col0_;
 };
 
-// "dynamic", "rangeofmotion-0", "terrain-ee-motion_0", ... (towr::DynamicConstraint etc.) of instance b
+// "dynamic", "rangeofmotion-0", "terrain-ee-motion_0", ... (towr::DynamicConstraint etc.) of instance b, with instance b's
+// constraint bounds
 class GpuConstraintSet : public ifo::ConstraintSet {
  public:
   GpuConstraintSet(BatchedProblem* p, int b, const std::string& name, int row0, int rows,
@@ -359,7 +386,8 @@ class GpuConstraintSet : public ifo::ConstraintSet {
   }
   VecBound GetBounds() const override {
     VecBound v;
-    for (int i = 0; i < GetRows(); ++i) v.push_back(ifo::Bounds(p_->g_lower()[row0_ + i], p_->g_upper()[row0_ + i]));
+    const double *lo = p_->g_lower(b_), *up = p_->g_upper(b_);
+    for (int i = 0; i < GetRows(); ++i) v.push_back(ifo::Bounds(lo[row0_ + i], up[row0_ + i]));
     return v;
   }
   // the (rows x n_var_set) block of this set's Jacobian w.r.t. one variable set: a slice of the CSR value array

@@ -840,10 +840,12 @@ int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac,
   return TWB_OK;
 }
 
-int twb_batch_lm_step_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
-                             double mu, double cap, int cg_iters, double* violation, void* stream) {
+// twb_batch_lm_step_device and twb_batch_lm_step_bounds_device: g_lower / g_upper null = the problem's constraint bounds
+static int LmStepDevice(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
+                        const double* g_lower, const double* g_upper, double mu, double cap, int cg_iters, double* violation, void* stream) {
   if (!b || !x || !g || !jac) return Fail(TWB_ERR_INVALID, "null argument");
   if ((x_lower == nullptr) != (x_upper == nullptr)) return Fail(TWB_ERR_INVALID, "x_lower and x_upper: both or neither");
+  if ((g_lower == nullptr) != (g_upper == nullptr)) return Fail(TWB_ERR_INVALID, "g_lower and g_upper: both or neither");
   if (!(mu >= 0.0) || !(cap > 0.0) || cg_iters < 0 || cg_iters > 10000) return Fail(TWB_ERR_INVALID, "bad solver parameter");
   cudaError_t e = cudaSetDevice(b->device);
   if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
@@ -879,11 +881,23 @@ int twb_batch_lm_step_device(twb_batch* b, double* x, const double* g, const dou
     }
     b->lm_ready = true;
   }
-  const bool own = x_lower != nullptr;
-  int rc = twb::LaunchLmStep(b->lm_pat, f.n, f.m, f.nnz, x, g, jac, own ? x_lower : b->d_xl, own ? x_upper : b->d_xu, own ? (size_t)f.n : 0, mu, cap,
+  const bool own = x_lower != nullptr, own_g = g_lower != nullptr;
+  int rc = twb::LaunchLmStep(b->lm_pat, f.n, f.m, f.nnz, x, g, jac, own ? x_lower : b->d_xl, own ? x_upper : b->d_xu, own ? (size_t)f.n : 0,
+                             own_g ? g_lower : b->lm_pat.g_lower, own_g ? g_upper : b->lm_pat.g_upper, own_g ? (size_t)f.m : 0, mu, cap,
                              cg_iters, violation, b->B, static_cast<cudaStream_t>(stream));
   if (rc != 0) return CudaFail(static_cast<cudaError_t>(rc), "solver step launch");
   return TWB_OK;
+}
+
+int twb_batch_lm_step_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
+                             double mu, double cap, int cg_iters, double* violation, void* stream) {
+  return LmStepDevice(b, x, g, jac, x_lower, x_upper, nullptr, nullptr, mu, cap, cg_iters, violation, stream);
+}
+
+int twb_batch_lm_step_bounds_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
+                                    const double* g_lower, const double* g_upper, double mu, double cap, int cg_iters, double* violation,
+                                    void* stream) {
+  return LmStepDevice(b, x, g, jac, x_lower, x_upper, g_lower, g_upper, mu, cap, cg_iters, violation, stream);
 }
 
 int twb_batch_eval_host(twb_batch* b, const double* x, double* g, double* jac, double* cost, double* grad,

@@ -53,16 +53,18 @@ struct LmPattern {
   const int* slot_t;    // [nnz]    CSR slot of the transposed entry
   const int* row_t;     // [nnz]    its row
   const double* g_lower;
-  const double* g_upper;   // [m]
+  const double* g_upper;   // [m] the problem's constraint bounds (what twb_batch_lm_step_device steps against)
   const int* row_order;    // [m] rows in descending length (balanced warps in the row pass)
   const int* col_order;    // [n] columns in descending length
   const uint16_t *col_idx16, *slot_t16, *row_t16;   // the same index arrays in 16 bits when n, m, nnz < 65 536 (else null)
 };
 size_t LmSharedBytes(int n, int m);
 // one Levenberg-Marquardt feasibility step for nb instances (CTA = instance): x[b][n] in / out, g[b][m], jac[b][nnz] in,
-// bounds x_lower / x_upper at b * bound_stride (0: the same bounds for every instance), violation[b] out (may be null)
+// variable bounds x_lower / x_upper at b * bound_stride and constraint bounds g_lower / g_upper at b * g_bound_stride (0: the
+// same bounds for every instance), violation[b] out (may be null)
 int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const double* g, const double* jac, const double* x_lower,
-                 const double* x_upper, size_t bound_stride, double mu, double cap, int cg_iters, double* violation, int nb, cudaStream_t s);
+                 const double* x_upper, size_t bound_stride, const double* g_lower, const double* g_upper, size_t g_bound_stride, double mu,
+                 double cap, int cg_iters, double* violation, int nb, cudaStream_t s);
 // number of output kernels one evaluation launches for this plan
 int OutKernelsPerEval(const Plan& P, unsigned flags);
 // One batched evaluation of `nb` instances.  XT is [tiles][n+1][32] (zero-initialised once; row n stays 0; tile = 32

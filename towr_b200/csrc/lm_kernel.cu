@@ -3,7 +3,7 @@
 // The stand-in for the IPOPT solves BASELINE configs[0] / [4] name (hopper_example.cc:77-93, footstep_plan_server.cc:222-236;
 // neither IPOPT nor ifopt exists in this image): what towr_b200/solver.py documents and tests/test_solver_loop.py walks a
 // second time on the CPU —
-//     r  = violation of g(x) against [g_lower, g_upper]
+//     r  = violation of g(x) against [g_lower, g_upper]    (the problem's bounds, or one row of bounds per instance)
 //     Js = diag(s) J,  rs = s r,   s_i = 1 / max(1, max_k |J_ik|)
 //     (Js^T Js + mu I) dx = -Js^T rs          cg_iters conjugate-gradient iterations, matrix-free
 //     x <- clip(x + dx min(1, cap / max|dx|), x_lower, x_upper)
@@ -13,9 +13,11 @@
 // CTAs per SM).  All solver vectors live in shared memory.  Both products walk the ONE sparsity pattern of the structure class:
 // Js p row by row (thread = row), Js^T u column by column through the pattern's transpose (thread = column) — fixed
 // summation orders, no atomics, bit-reproducible.
-// An instance with a non-finite x, g or J entry keeps its x and reports violation NaN.  Left to the step, such an entry would
-// be dropped by fmax (row scale, violation) and a NaN step turned into a bound by the projection: the instance would jump to
-// its bounds and report a finite violation.
+// An instance with a non-finite x, g or J entry, or a NaN constraint bound, keeps its x and reports violation NaN.  Left to the
+// step, such an entry would be dropped by fmax (row scale, violation) and a NaN step turned into a bound by the projection:
+// the instance would jump to its bounds and report a finite violation (a NaN bound would silently mean "unbounded").
+// +-Inf constraint bounds mean unbounded, like the 1e20 convention.  With lower > upper the lower bound wins (g < lo is
+// tested first).
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
@@ -56,8 +58,9 @@ template <bool kSmemJ, class Idx>
 __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __restrict__ col_idx, const Idx* __restrict__ slot_t,
                                                     const Idx* __restrict__ row_t, int n, int m, int nnz, double* __restrict__ X,
                                                     const double* __restrict__ G, const double* __restrict__ JAC, const double* __restrict__ x_lower,
-                                                    const double* __restrict__ x_upper, size_t bound_stride, double mu, double cap, int cg_iters,
-                                                    double* __restrict__ violation) {
+                                                    const double* __restrict__ x_upper, size_t bound_stride,
+                                                    const double* __restrict__ g_lower, const double* __restrict__ g_upper, size_t g_bound_stride,
+                                                    double mu, double cap, int cg_iters, double* __restrict__ violation) {
   extern __shared__ __align__(16) double sm[];
   double* s = sm;             // [m] row scales
   double* u = s + m;          // [m] row vector (rs, then Js p)
@@ -70,6 +73,8 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
   const int b = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
   const double* __restrict__ J = JAC + (size_t)b * nnz;
   const double* __restrict__ g = G + (size_t)b * m;
+  const double* __restrict__ gl = g_lower + (size_t)b * g_bound_stride;
+  const double* __restrict__ gu = g_upper + (size_t)b * g_bound_stride;
   // row scales, the scaled values and the scaled violation
   double vmax = 0.0;
   double chk = 0.0;                           // fma(v, 0, chk): NaN once a v that is not finite has been seen
@@ -80,9 +85,10 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
     for (int k = k0; k < k1; ++k) { const double v = J[k]; big = fmax(big, fabs(v)); chk = fma(v, 0.0, chk); }
     const double si = 1.0 / fmax(big, 1.0);
     if (kSmemJ) for (int k = k0; k < k1; ++k) Js[k] = J[k] * si;
-    const double gi = g[i], lo = __ldg(pat.g_lower + i), up = __ldg(pat.g_upper + i);
+    const double gi = g[i], lo = __ldg(gl + i), up = __ldg(gu + i);
     const double r = gi < lo ? gi - lo : gi > up ? gi - up : 0.0;
     chk = fma(gi, 0.0, chk);
+    if (lo != lo || up != up) chk = CUDART_NAN;   // a NaN bound (an infinite one is a valid "unbounded")
     s[i] = si;
     const double rs = si * r;
     u[i] = rs;
@@ -155,11 +161,12 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
 
 template <bool kSmemJ, class Idx>
 int LaunchLm(const LmPattern& pat, const Idx* col_idx, const Idx* slot_t, const Idx* row_t, int threads, size_t smem, int n, int m, int nnz, double* x,
-             const double* g, const double* jac, const double* xl, const double* xu, size_t bound_stride, double mu, double cap, int cg_iters,
-             double* violation, int nb, cudaStream_t s) {
+             const double* g, const double* jac, const double* xl, const double* xu, size_t bound_stride, const double* gl, const double* gu,
+             size_t g_bound_stride, double mu, double cap, int cg_iters, double* violation, int nb, cudaStream_t s) {
   cudaError_t e = cudaFuncSetAttribute(LmStepKernel<kSmemJ, Idx>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  LmStepKernel<kSmemJ, Idx><<<nb, threads, smem, s>>>(pat, col_idx, slot_t, row_t, n, m, nnz, x, g, jac, xl, xu, bound_stride, mu, cap, cg_iters, violation);
+  LmStepKernel<kSmemJ, Idx><<<nb, threads, smem, s>>>(pat, col_idx, slot_t, row_t, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu, g_bound_stride, mu, cap,
+                                                     cg_iters, violation);
   return (int)cudaGetLastError();
 }
 
@@ -168,18 +175,19 @@ int LaunchLm(const LmPattern& pat, const Idx* col_idx, const Idx* slot_t, const 
 size_t LmSharedBytes(int n, int m) { return sizeof(double) * ((size_t)2 * m + 4 * (size_t)n + 32); }
 
 int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const double* g, const double* jac, const double* x_lower,
-                 const double* x_upper, size_t bound_stride, double mu, double cap, int cg_iters, double* violation, int nb, cudaStream_t s) {
+                 const double* x_upper, size_t bound_stride, const double* g_lower, const double* g_upper, size_t g_bound_stride, double mu,
+                 double cap, int cg_iters, double* violation, int nb, cudaStream_t s) {
   if (nb <= 0) return 0;
   const size_t vec = LmSharedBytes(n, m), with_j = vec + sizeof(double) * (size_t)nnz;
   const bool smem_j = with_j <= 220 * 1024;   // the scaled values fit beside the vectors: one CTA of 512 threads per SM
   const int threads = smem_j ? 512 : 256;
   const size_t smem = smem_j ? with_j : vec;
   if (pat.col_idx16) {
-    return smem_j ? LaunchLm<true>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s)
-                  : LaunchLm<false>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s);
+    return smem_j ? LaunchLm<true>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, nb, s)
+                  : LaunchLm<false>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, nb, s);
   }
   // 32-bit indices mean n, m or nnz >= 65 536, so with_j >= 8 * 65 536 bytes > 220 KiB: never the shared-memory Js path
-  return LaunchLm<false>(pat, pat.col_idx, pat.slot_t, pat.row_t, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, mu, cap, cg_iters, violation, nb, s);
+  return LaunchLm<false>(pat, pat.col_idx, pat.slot_t, pat.row_t, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, nb, s);
 }
 
 }  // namespace twb

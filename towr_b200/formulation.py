@@ -627,9 +627,12 @@ class Batch:
                                                    C.c_void_p(stream.cuda_stream)))
         return x0, lo, up, gl, gu
 
-    def lm_step_device(self, x, g, jac, x_lower=None, x_upper=None, mu=1e-2, cap=0.1, cg_iters=25, violation=None, stream=None):
+    def lm_step_device(self, x, g, jac, x_lower=None, x_upper=None, mu=1e-2, cap=0.1, cg_iters=25, violation=None, stream=None,
+                       g_lower=None, g_upper=None):
         """twb_batch_lm_step_device: one Levenberg-Marquardt feasibility step for every instance on the outputs of
-        eval_device; x (B, n) is updated in place.  All arguments are torch CUDA float64 tensors (bounds: (B, n) or None)."""
+        eval_device; x (B, n) is updated in place.  All arguments are torch CUDA float64 tensors (bounds: (B, n) or None).
+        g_lower / g_upper: per-instance constraint bounds, (B, m) each (e.g. from state_instances_device(...,
+        want_g_bounds=True)), stepped against with twb_batch_lm_step_bounds_device; None: the problem's own."""
         import torch
         if stream is None:
             stream = torch.cuda.current_stream(x.device)
@@ -637,9 +640,18 @@ class Batch:
         for t, count in ((x, self.B * p.n), (g, self.B * p.m), (jac, self.B * p.nnz), (x_lower, self.B * p.n), (x_upper, self.B * p.n),
                          (violation, self.B)):
             assert t is None or (t.is_cuda and t.dtype == torch.float64 and t.is_contiguous() and t.numel() == count), "bad tensor"
+        for t in (g_lower, g_upper):
+            assert t is None or (torch.is_tensor(t) and t.is_cuda and t.device == x.device and t.dtype == torch.float64 and t.is_contiguous()
+                                 and tuple(t.shape) == (self.B, p.m)), "bad constraint bounds: (B, m) contiguous CUDA float64"
+        assert (g_lower is None) == (g_upper is None), "g_lower and g_upper: both or neither"
         ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
-        check(lib.twb_batch_lm_step_device(self._h, ptr(x), ptr(g), ptr(jac), ptr(x_lower), ptr(x_upper), float(mu), float(cap), int(cg_iters),
-                                           ptr(violation), C.c_void_p(stream.cuda_stream)))
+        if g_lower is None:
+            check(lib.twb_batch_lm_step_device(self._h, ptr(x), ptr(g), ptr(jac), ptr(x_lower), ptr(x_upper), float(mu), float(cap),
+                                               int(cg_iters), ptr(violation), C.c_void_p(stream.cuda_stream)))
+        else:
+            check(lib.twb_batch_lm_step_bounds_device(self._h, ptr(x), ptr(g), ptr(jac), ptr(x_lower), ptr(x_upper), ptr(g_lower),
+                                                      ptr(g_upper), float(mu), float(cap), int(cg_iters), ptr(violation),
+                                                      C.c_void_p(stream.cuda_stream)))
 
     def eval_device(self, x, g=None, jac=None, cost=None, grad=None, status=None,
                     flags=capi.EVAL_G | capi.EVAL_JAC, stream=None):

@@ -4,15 +4,17 @@ neither IPOPT nor ifopt exists in this image, see DESIGN.md).
 The stand-in is a deterministic Levenberg-Marquardt FEASIBILITY iteration on the NLP's constraints — what IPOPT's
 restoration phase minimises — for every instance of a batch in lock step:
 
-    r  = violation of g(x) against [g_lower, g_upper]              (twb_batch_eval_device: g and the CSR Jacobian values)
+    r  = violation of g(x) against [g_lower, g_upper]              (twb_batch_eval_device: g and the CSR Jacobian values;
+                                                                    the problem's bounds or one row per instance)
     Js = diag(s) J,  rs = s r,   s_i = 1 / max(1, max_k |J_ik|)    (row scaling)
     (Js^T Js + mu I) dx = -Js^T rs                                 (`cg_iters` conjugate-gradient iterations, matrix-free)
     x <- clip(x + dx * min(1, cap / max|dx|), x_lower, x_upper)
 
 The iterates, g, the Jacobian values and all solver vectors stay on the GPU.  An iteration is two library calls:
-`twb_batch_eval_device` (g and the CSR Jacobian values of all instances) and `twb_batch_lm_step_device`
-(towr_b200/csrc/lm_kernel.cu: CTA = instance, the conjugate gradients run in shared memory on the problem's ONE shared
-CSR pattern and its transpose, fixed summation orders, no atomics).  An instance whose x, g or Jacobian values hold a
+`twb_batch_eval_device` (g and the CSR Jacobian values of all instances) and `twb_batch_lm_step_device`, or
+`twb_batch_lm_step_bounds_device` with per-instance constraint bounds (towr_b200/csrc/lm_kernel.cu: CTA = instance, the
+conjugate gradients run in shared memory on the problem's ONE shared CSR pattern and its transpose, fixed summation
+orders, no atomics).  An instance whose x, g or Jacobian values hold a
 non-finite entry (the evaluation flags it in `status` bit 0) is not stepped by the native step: its x stays exactly as it
 was and its violation is NaN, so the caller can tell it apart instead of finding it clipped to its bounds.
 `native=False` keeps the first implementation of the same step in PyTorch tensor algebra (padded ELL gathers) — 30 x
@@ -53,7 +55,10 @@ def ell_maps(row_ptr, col_idx, n):
 class BatchedLevenbergMarquardt:
     """All instances of a `Batch` in lock step, everything on the batch's GPU."""
 
-    def __init__(self, batch, x_lower=None, x_upper=None, mu=1e-2, cap=0.1, cg_iters=25, native=True):
+    def __init__(self, batch, x_lower=None, x_upper=None, g_lower=None, g_upper=None, mu=1e-2, cap=0.1, cg_iters=25, native=True):
+        """x_lower / x_upper: variable bounds, (n,) or per instance (B, n); g_lower / g_upper: constraint bounds, (m,) or per
+        instance (B, m) (e.g. the last two results of Batch.state_instances_device(..., want_g_bounds=True)); None: the
+        problem's own."""
         import torch
         self.torch = torch
         self.native = native
@@ -63,7 +68,12 @@ class BatchedLevenbergMarquardt:
         xl, xu, gl, gu = p.bounds()
         to = lambda a: a.to(self.dev, torch.float64) if torch.is_tensor(a) else torch.as_tensor(np.asarray(a, np.float64), device=self.dev)
         self.xl = to(xl if x_lower is None else x_lower); self.xu = to(xu if x_upper is None else x_upper)
-        self.gl, self.gu = to(gl), to(gu)
+        if (g_lower is None) != (g_upper is None):
+            raise ValueError("g_lower and g_upper: both or neither")
+        self.gl, self.gu = to(gl if g_lower is None else g_lower), to(gu if g_upper is None else g_upper)
+        # per-instance constraint bounds go to the native step as (B, m) rows; without them it uses the problem's own
+        self.gl_full = None if g_lower is None else self.gl.expand(self.B, p.m).contiguous()
+        self.gu_full = None if g_upper is None else self.gu.expand(self.B, p.m).contiguous()
         rows, cols_of, rowsT, rows_of = ell_maps(p.row_ptr(), p.structure()[1], p.n)
         ti = lambda a: torch.as_tensor(a, device=self.dev)
         self.rows, self.cols_of, self.rowsT, self.rows_of = ti(rows), ti(cols_of), ti(rowsT), ti(rows_of)
@@ -87,7 +97,8 @@ class BatchedLevenbergMarquardt:
         from . import capi
         self.batch.eval_device(X, g=self.g, jac=self.jac_vals, status=self.status, flags=capi.EVAL_G | capi.EVAL_JAC)
         if self.native:
-            self.batch.lm_step_device(X, self.g, self.jac_vals, self.xl_full, self.xu_full, self.mu, self.cap, self.cg_iters, self.viol)
+            self.batch.lm_step_device(X, self.g, self.jac_vals, self.xl_full, self.xu_full, self.mu, self.cap, self.cg_iters, self.viol,
+                                      g_lower=self.gl_full, g_upper=self.gu_full)
             return self.viol.clone()
         self.jac[:, :-1] = self.jac_vals; self.jac[:, -1] = 0.0
         A = self.jac[:, self.rows]                                   # (B, m, W) rows of J
