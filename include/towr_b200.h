@@ -290,6 +290,54 @@ int twb_batch_lm_step_bounds_device(twb_batch* b, double* x, const double* g, co
                                     const double* x_upper, const double* g_lower, const double* g_upper, double mu, double cap,
                                     int cg_iters, double* violation, void* stream);
 
+/* ---- solving to a tolerance: trial step, gain-ratio acceptance, damping per instance ----------------------------------
+ * One solve iteration for every instance of the batch in lock step is four calls, all of which only enqueue on `stream`:
+ *   twb_batch_eval_device(x -> g, jac, flags TWB_EVAL_G | TWB_EVAL_JAC)
+ *   twb_batch_lm_trial_device(x, g, jac -> x_trial, row_scale, merit, predicted, violation; sets converged / non-finite)
+ *   twb_batch_eval_device(x_trial -> g_trial, flags TWB_EVAL_G)
+ *   twb_batch_lm_accept_device(x_trial, g_trial -> x, mu, nu, solve_status, iterations)
+ * The host decides how many iterations run (nothing loops on the device) and may stop once no instance is RUNNING.  The
+ * caller initialises, per instance, mu [B] > 0 (e.g. 1e-2), nu [B] = 2, solve_status [B] = TWB_LM_RUNNING and
+ * iterations [B] = 0, all device arrays.  An instance that is still RUNNING when the host's budget ends has hit the iteration
+ * limit.  All other arrays are device pointers as for twb_batch_lm_step_device; x_trial must not overlap x. */
+#define TWB_LM_RUNNING 0     /* still being stepped                                                                      */
+#define TWB_LM_CONVERGED 1   /* max |s r| <= tol at x                                                                    */
+#define TWB_LM_STALLED 2     /* mu grew past mu_max on rejected trials                                                   */
+#define TWB_LM_NONFINITE 3   /* x, g, jac or a constraint bound holds a non-finite entry (a NaN bound); violation[b] NaN */
+
+/* Trial step: twb_batch_lm_step_bounds_device's arithmetic with mu[b] per instance, written to x_trial [B][n] instead of x
+ * (x is not changed).  For every instance whose solve_status is RUNNING when the call starts:
+ *   row_scale [B][m] = s at x;  merit [B] = phi0 = 1/2 ||s r(g)||^2;  violation [B] = max |s r(g)| (may be NULL);
+ *   predicted [B] = phi0 - 1/2 ||s r(g + J d)||^2, d = x_trial - x (the step after the cap and the projection): the decrease of
+ *   the linearised violation, with the rows' bounds taken into account.
+ * If max |s r| <= tol the status becomes TWB_LM_CONVERGED; if x, g, jac or a constraint bound is non-finite (as for
+ * twb_batch_lm_step_device) it becomes TWB_LM_NONFINITE with violation NaN and merit NaN.  In both cases x_trial = x and
+ * predicted = 0.  An instance that is not RUNNING when the call starts only gets x_trial = x; nothing else of it is written.
+ * With mu[b] = mu for every instance, x_trial and violation are bit for bit what twb_batch_lm_step_device (or _bounds_device)
+ * writes into x and violation, for every instance left RUNNING.  g_lower / g_upper: per-instance constraint bounds [B][m] (both
+ * NULL: the problem's own).  Errors: those of twb_batch_lm_step_bounds_device except the mu check, NULL mu / solve_status /
+ * x_trial / row_scale / merit / predicted, tol < 0 or NaN: TWB_ERR_INVALID; nothing is enqueued when a call fails its checks.
+ * The first call of the step family on a batch (this, the two step calls, twb_batch_lm_accept_device) uploads
+ * the pattern; after it, the calls can be captured into a CUDA graph. */
+int twb_batch_lm_trial_device(twb_batch* b, const double* x, const double* g, const double* jac, const double* x_lower,
+                              const double* x_upper, const double* g_lower, const double* g_upper, const double* mu, double cap,
+                              int cg_iters, double tol, int* solve_status, double* x_trial, double* row_scale, double* merit,
+                              double* predicted, double* violation, void* stream);
+
+/* Acceptance, for every instance whose solve_status is RUNNING (the others are not touched): g_trial [B][m] is g at x_trial
+ * (twb_batch_eval_device with TWB_EVAL_G), phi_t = 1/2 ||row_scale r(g_trial)||^2 with the row scales of x, and
+ * rho = (merit - phi_t) / predicted.
+ *   accept if predicted > 0, every g_trial entry and phi_t are finite and rho > eta:
+ *     x <- x_trial, mu <- max(mu_min, mu max(1/3, 1 - (2 rho - 1)^3)), nu <- 2
+ *   reject otherwise (a non-finite g_trial included; x keeps its bits): mu <- mu nu, nu <- 2 nu, and the status becomes
+ *     TWB_LM_STALLED if the new mu > mu_max
+ *   iterations[b] += 1 either way.
+ * g_lower / g_upper as for the trial call (they must be the same).  Errors: NULL b or a required pointer, only one of g_lower /
+ * g_upper NULL, eta outside [0, 1), not 0 < mu_min <= mu_max: TWB_ERR_INVALID, nothing enqueued. */
+int twb_batch_lm_accept_device(twb_batch* b, double* x, const double* x_trial, const double* g_trial, const double* g_lower,
+                               const double* g_upper, const double* row_scale, const double* merit, const double* predicted, double* mu,
+                               double* nu, int* solve_status, int* iterations, double eta, double mu_min, double mu_max, void* stream);
+
 /* Host-pointer variant: copies x up, evaluates, copies the requested outputs
  * back and synchronises. Pinned host memory makes the copies asynchronous. */
 int twb_batch_eval_host(twb_batch* b, const double* x, double* g, double* jac,

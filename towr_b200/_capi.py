@@ -54,6 +54,8 @@ def _load():
         "twb_batch_eval_host": (C.c_int, [P, P, P, P, P, P, P, C.c_uint]),
         "twb_batch_lm_step_device": (C.c_int, [P, P, P, P, P, P, C.c_double, C.c_double, C.c_int, P, P]),
         "twb_batch_lm_step_bounds_device": (C.c_int, [P, P, P, P, P, P, P, P, C.c_double, C.c_double, C.c_int, P, P]),
+        "twb_batch_lm_trial_device": (C.c_int, [P, P, P, P, P, P, P, P, P, C.c_double, C.c_int, C.c_double, P, P, P, P, P, P, P]),
+        "twb_batch_lm_accept_device": (C.c_int, [P, P, P, P, P, P, P, P, P, P, P, P, P, C.c_double, C.c_double, C.c_double, P]),
         "twb_problem_trajectory_dims": (C.c_int, [P, C.c_double, I, I]),
         "twb_batch_sample_trajectory_host": (C.c_int, [P, P, C.c_double, P]),
         "twb_batch_initial_guess_host": (C.c_int, [P, P, P, C.c_int, P]),

@@ -840,17 +840,12 @@ int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac,
   return TWB_OK;
 }
 
-// twb_batch_lm_step_device and twb_batch_lm_step_bounds_device: g_lower / g_upper null = the problem's constraint bounds
-static int LmStepDevice(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
-                        const double* g_lower, const double* g_upper, double mu, double cap, int cg_iters, double* violation, void* stream) {
-  if (!b || !x || !g || !jac) return Fail(TWB_ERR_INVALID, "null argument");
-  if ((x_lower == nullptr) != (x_upper == nullptr)) return Fail(TWB_ERR_INVALID, "x_lower and x_upper: both or neither");
-  if ((g_lower == nullptr) != (g_upper == nullptr)) return Fail(TWB_ERR_INVALID, "g_lower and g_upper: both or neither");
-  if (!(mu >= 0.0) || !(cap > 0.0) || cg_iters < 0 || cg_iters > 10000) return Fail(TWB_ERR_INVALID, "bad solver parameter");
-  cudaError_t e = cudaSetDevice(b->device);
-  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+// The first call of the step family on a batch uploads what the solver kernels read besides their arguments: the pattern, its
+// transpose (entries of column j in ascending row order: what a stable sort by column yields), the row / column orders, the
+// 16-bit index arrays when they fit, and the problem's variable and constraint bounds.  Later calls find it in place.
+static int LmPatternReady(twb_batch* b) {
+  cudaError_t e;
   const twb::Formulation& f = b->prob->f;
-  if (twb::LmSharedBytes(f.n, f.m) > 200 * 1024) return Fail(TWB_ERR_UNSUPPORTED, "problem too large for the shared-memory solver step");
   if (!b->lm_ready) {   // the pattern's transpose: entries of column j in ascending row order (what a stable sort by column yields)
     std::vector<int> col_ptr(f.n + 1, 0), slot_t(f.nnz), row_t(f.nnz);
     for (int k = 0; k < f.nnz; ++k) col_ptr[f.col_idx[k] + 1]++;
@@ -881,23 +876,75 @@ static int LmStepDevice(twb_batch* b, double* x, const double* g, const double* 
     }
     b->lm_ready = true;
   }
+  return TWB_OK;
+}
+
+// twb_batch_lm_step_device, twb_batch_lm_step_bounds_device and twb_batch_lm_trial_device (trial non-null: mu unused):
+// g_lower / g_upper null = the problem's constraint bounds
+static int LmStepDevice(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
+                        const double* g_lower, const double* g_upper, double mu, double cap, int cg_iters, double* violation,
+                        const twb::LmTrialArgs* trial, void* stream) {
+  if (!b || !x || !g || !jac) return Fail(TWB_ERR_INVALID, "null argument");
+  if ((x_lower == nullptr) != (x_upper == nullptr)) return Fail(TWB_ERR_INVALID, "x_lower and x_upper: both or neither");
+  if ((g_lower == nullptr) != (g_upper == nullptr)) return Fail(TWB_ERR_INVALID, "g_lower and g_upper: both or neither");
+  if (!(mu >= 0.0) || !(cap > 0.0) || cg_iters < 0 || cg_iters > 10000) return Fail(TWB_ERR_INVALID, "bad solver parameter");
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  const twb::Formulation& f = b->prob->f;
+  if (twb::LmSharedBytes(f.n, f.m) > 200 * 1024) return Fail(TWB_ERR_UNSUPPORTED, "problem too large for the shared-memory solver step");
+  int rc = LmPatternReady(b);
+  if (rc != TWB_OK) return rc;
   const bool own = x_lower != nullptr, own_g = g_lower != nullptr;
-  int rc = twb::LaunchLmStep(b->lm_pat, f.n, f.m, f.nnz, x, g, jac, own ? x_lower : b->d_xl, own ? x_upper : b->d_xu, own ? (size_t)f.n : 0,
-                             own_g ? g_lower : b->lm_pat.g_lower, own_g ? g_upper : b->lm_pat.g_upper, own_g ? (size_t)f.m : 0, mu, cap,
-                             cg_iters, violation, b->B, static_cast<cudaStream_t>(stream));
+  rc = twb::LaunchLmStep(b->lm_pat, f.n, f.m, f.nnz, x, g, jac, own ? x_lower : b->d_xl, own ? x_upper : b->d_xu, own ? (size_t)f.n : 0,
+                         own_g ? g_lower : b->lm_pat.g_lower, own_g ? g_upper : b->lm_pat.g_upper, own_g ? (size_t)f.m : 0, mu, cap,
+                         cg_iters, violation, trial, b->B, static_cast<cudaStream_t>(stream));
   if (rc != 0) return CudaFail(static_cast<cudaError_t>(rc), "solver step launch");
   return TWB_OK;
 }
 
 int twb_batch_lm_step_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
                              double mu, double cap, int cg_iters, double* violation, void* stream) {
-  return LmStepDevice(b, x, g, jac, x_lower, x_upper, nullptr, nullptr, mu, cap, cg_iters, violation, stream);
+  return LmStepDevice(b, x, g, jac, x_lower, x_upper, nullptr, nullptr, mu, cap, cg_iters, violation, nullptr, stream);
 }
 
 int twb_batch_lm_step_bounds_device(twb_batch* b, double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
                                     const double* g_lower, const double* g_upper, double mu, double cap, int cg_iters, double* violation,
                                     void* stream) {
-  return LmStepDevice(b, x, g, jac, x_lower, x_upper, g_lower, g_upper, mu, cap, cg_iters, violation, stream);
+  return LmStepDevice(b, x, g, jac, x_lower, x_upper, g_lower, g_upper, mu, cap, cg_iters, violation, nullptr, stream);
+}
+
+static_assert(TWB_LM_RUNNING == twb::kLmRunning && TWB_LM_CONVERGED == twb::kLmConverged && TWB_LM_STALLED == twb::kLmStalled &&
+              TWB_LM_NONFINITE == twb::kLmNonFinite, "solve status codes");
+
+int twb_batch_lm_trial_device(twb_batch* b, const double* x, const double* g, const double* jac, const double* x_lower, const double* x_upper,
+                              const double* g_lower, const double* g_upper, const double* mu, double cap, int cg_iters, double tol,
+                              int* solve_status, double* x_trial, double* row_scale, double* merit, double* predicted, double* violation,
+                              void* stream) {
+  if (!mu || !solve_status || !x_trial || !row_scale || !merit || !predicted) return Fail(TWB_ERR_INVALID, "null argument");
+  if (!(tol >= 0.0)) return Fail(TWB_ERR_INVALID, "bad tolerance");
+  const twb::LmTrialArgs trial{mu, tol, solve_status, x_trial, row_scale, merit, predicted};
+  // x is only read by the trial kernel
+  return LmStepDevice(b, const_cast<double*>(x), g, jac, x_lower, x_upper, g_lower, g_upper, 0.0, cap, cg_iters, violation, &trial, stream);
+}
+
+int twb_batch_lm_accept_device(twb_batch* b, double* x, const double* x_trial, const double* g_trial, const double* g_lower,
+                               const double* g_upper, const double* row_scale, const double* merit, const double* predicted, double* mu,
+                               double* nu, int* solve_status, int* iterations, double eta, double mu_min, double mu_max, void* stream) {
+  if (!b || !x || !x_trial || !g_trial || !row_scale || !merit || !predicted || !mu || !nu || !solve_status || !iterations)
+    return Fail(TWB_ERR_INVALID, "null argument");
+  if ((g_lower == nullptr) != (g_upper == nullptr)) return Fail(TWB_ERR_INVALID, "g_lower and g_upper: both or neither");
+  if (!(eta >= 0.0 && eta < 1.0) || !(mu_min > 0.0 && mu_min <= mu_max)) return Fail(TWB_ERR_INVALID, "bad solver parameter");
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  const twb::Formulation& f = b->prob->f;
+  int rc = LmPatternReady(b);
+  if (rc != TWB_OK) return rc;
+  const bool own_g = g_lower != nullptr;
+  rc = twb::LaunchLmAccept(f.n, f.m, x, x_trial, g_trial, own_g ? g_lower : b->lm_pat.g_lower, own_g ? g_upper : b->lm_pat.g_upper,
+                           own_g ? (size_t)f.m : 0, row_scale, merit, predicted, mu, nu, solve_status, iterations, eta, mu_min, mu_max, b->B,
+                           static_cast<cudaStream_t>(stream));
+  if (rc != 0) return CudaFail(static_cast<cudaError_t>(rc), "solver accept launch");
+  return TWB_OK;
 }
 
 int twb_batch_eval_host(twb_batch* b, const double* x, double* g, double* jac, double* cost, double* grad,

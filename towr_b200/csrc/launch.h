@@ -59,12 +59,30 @@ struct LmPattern {
   const uint16_t *col_idx16, *slot_t16, *row_t16;   // the same index arrays in 16 bits when n, m, nnz < 65 536 (else null)
 };
 size_t LmSharedBytes(int n, int m);
+// solve status of an instance (include/towr_b200.h: TWB_LM_*)
+enum LmStatus : int { kLmRunning = 0, kLmConverged = 1, kLmStalled = 2, kLmNonFinite = 3 };
+// the trial variant of the step (twb_batch_lm_trial_device): damping mu[b] per instance, x left unchanged and the step
+// written to x_trial; only instances whose status is kLmRunning are stepped
+struct LmTrialArgs {
+  const double* mu;     // [nb]
+  double tol;           // status kLmConverged when max |s r| <= tol
+  int* status;          // [nb] in / out
+  double* x_trial;      // [nb][n]
+  double* row_scale;    // [nb][m] s at x
+  double* merit;        // [nb] 1/2 ||s r(g)||^2
+  double* predicted;    // [nb] merit - 1/2 ||s r(g + J d)||^2, d = x_trial - x
+};
 // one Levenberg-Marquardt feasibility step for nb instances (CTA = instance): x[b][n] in / out, g[b][m], jac[b][nnz] in,
 // variable bounds x_lower / x_upper at b * bound_stride and constraint bounds g_lower / g_upper at b * g_bound_stride (0: the
-// same bounds for every instance), violation[b] out (may be null)
+// same bounds for every instance), violation[b] out (may be null).  trial non-null: the trial variant (x is only read, mu unused)
 int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const double* g, const double* jac, const double* x_lower,
                  const double* x_upper, size_t bound_stride, const double* g_lower, const double* g_upper, size_t g_bound_stride, double mu,
-                 double cap, int cg_iters, double* violation, int nb, cudaStream_t s);
+                 double cap, int cg_iters, double* violation, const LmTrialArgs* trial, int nb, cudaStream_t s);
+// the gain-ratio decision after a trial step for nb instances (CTA = instance, kLmRunning ones only): accept x <- x_trial and
+// lower mu, or keep x and raise mu (kLmStalled past mu_max); g_trial[b][m] is g at x_trial
+int LaunchLmAccept(int n, int m, double* x, const double* x_trial, const double* g_trial, const double* g_lower, const double* g_upper,
+                   size_t g_bound_stride, const double* row_scale, const double* merit, const double* predicted, double* mu, double* nu,
+                   int* status, int* iterations, double eta, double mu_min, double mu_max, int nb, cudaStream_t s);
 // number of output kernels one evaluation launches for this plan
 int OutKernelsPerEval(const Plan& P, unsigned flags);
 // One batched evaluation of `nb` instances.  XT is [tiles][n+1][32] (zero-initialised once; row n stays 0; tile = 32

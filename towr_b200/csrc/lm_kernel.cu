@@ -13,6 +13,11 @@
 // CTAs per SM).  All solver vectors live in shared memory.  Both products walk the ONE sparsity pattern of the structure class:
 // Js p row by row (thread = row), Js^T u column by column through the pattern's transpose (thread = column) — fixed
 // summation orders, no atomics, bit-reproducible.
+// The trial variant (kTrial, twb_batch_lm_trial_device) is the same step with mu[b] per instance; it writes the step to x_trial
+// and leaves x alone, sets the instance's solve status (converged: max |s r| <= tol, non-finite), and writes the row scales s,
+// the merit phi0 = 1/2 ||s r(g)||^2 and the decrease of the linear model, phi0 - 1/2 ||s r(g + J d)||^2 with d = x_trial - x
+// (one more row pass over Js, with d in pd and Js d in u).  LmAcceptKernel then decides on g at x_trial with the same row
+// scales: accept when rho = (phi0 - phi_t) / predicted > eta, else keep x and raise mu.
 // An instance with a non-finite x, g or J entry, or a NaN constraint bound, keeps its x and reports violation NaN.  Left to the
 // step, such an entry would be dropped by fmax (row scale, violation) and a NaN step turned into a bound by the projection:
 // the instance would jump to its bounds and report a finite violation (a NaN bound would silently mean "unbounded").
@@ -54,13 +59,13 @@ __device__ __forceinline__ double BlockMax(double v, double* scratch) {
 // Idx: the pattern's index arrays as 16-bit (n, m, nnz < 65 536: 90 KB instead of 180 KB, so that they stay in the L1 beside
 // one CTA's shared memory — with 32-bit indices every index load was an L2 round trip: 14.6 instead of 10.5 ms per step) or 32-bit.
 // thread = row (Js p) / thread = column (Js^T u): measured faster than 16 lanes per row with shuffle trees (25.4 vs 14.6 ms).
-template <bool kSmemJ, class Idx>
+template <bool kSmemJ, class Idx, bool kTrial>
 __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __restrict__ col_idx, const Idx* __restrict__ slot_t,
                                                     const Idx* __restrict__ row_t, int n, int m, int nnz, double* __restrict__ X,
                                                     const double* __restrict__ G, const double* __restrict__ JAC, const double* __restrict__ x_lower,
                                                     const double* __restrict__ x_upper, size_t bound_stride,
                                                     const double* __restrict__ g_lower, const double* __restrict__ g_upper, size_t g_bound_stride,
-                                                    double mu, double cap, int cg_iters, double* __restrict__ violation) {
+                                                    double mu, double cap, int cg_iters, double* __restrict__ violation, LmTrialArgs tr) {
   extern __shared__ __align__(16) double sm[];
   double* s = sm;             // [m] row scales
   double* u = s + m;          // [m] row vector (rs, then Js p)
@@ -75,8 +80,15 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
   const double* __restrict__ g = G + (size_t)b * m;
   const double* __restrict__ gl = g_lower + (size_t)b * g_bound_stride;
   const double* __restrict__ gu = g_upper + (size_t)b * g_bound_stride;
+  if constexpr (kTrial) {
+    if (tr.status[b] != kLmRunning) {    // finished before this call: x_trial = x and nothing else (uniform over the CTA)
+      for (int j = tid; j < n; j += nt) tr.x_trial[(size_t)b * n + j] = X[(size_t)b * n + j];
+      return;
+    }
+    mu = tr.mu[b];
+  }
   // row scales, the scaled values and the scaled violation
-  double vmax = 0.0;
+  double vmax = 0.0, phi = 0.0;               // phi: sum of (s r)^2 (kTrial)
   double chk = 0.0;                           // fma(v, 0, chk): NaN once a v that is not finite has been seen
   for (int q = tid; q < m; q += nt) {
     const int i = __ldg(pat.row_order + q);   // rows in descending length: the lanes of a warp walk rows of similar length
@@ -90,12 +102,30 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
     chk = fma(gi, 0.0, chk);
     if (lo != lo || up != up) chk = CUDART_NAN;   // a NaN bound (an infinite one is a valid "unbounded")
     s[i] = si;
+    if constexpr (kTrial) tr.row_scale[(size_t)b * m + i] = si;
     const double rs = si * r;
     u[i] = rs;
     vmax = fmax(vmax, fabs(rs));
+    if constexpr (kTrial) phi += rs * rs;
   }
   vmax = BlockMax(vmax, scratch);        // (also orders the writes of s, u, Js)
   const bool finite_gj = BlockMax(chk != chk ? 1.0 : 0.0, scratch) == 0.0;
+  if constexpr (kTrial) {                // converged or non-finite: no step (uniform over the CTA)
+    double chk_x = 0.0;
+    for (int j = tid; j < n; j += nt) chk_x = fma(X[(size_t)b * n + j], 0.0, chk_x);
+    const bool finite = BlockMax(chk_x != chk_x ? 1.0 : 0.0, scratch) == 0.0 && finite_gj;
+    phi = 0.5 * BlockSum(phi, scratch);
+    if (!finite || vmax <= tr.tol) {
+      for (int j = tid; j < n; j += nt) tr.x_trial[(size_t)b * n + j] = X[(size_t)b * n + j];
+      if (tid == 0) {
+        tr.status[b] = finite ? kLmConverged : kLmNonFinite;
+        tr.merit[b] = finite ? phi : CUDART_NAN;
+        tr.predicted[b] = 0.0;
+        if (violation) violation[b] = finite ? vmax : CUDART_NAN;
+      }
+      return;
+    }
+  }
   auto row_dot = [&](int i) {            // (Js p)_i
     double acc = 0.0;
     const int k0 = __ldg(pat.row_ptr + i), k1 = __ldg(pat.row_ptr + i + 1);
@@ -147,27 +177,109 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
     __syncthreads();
   }
   double big = 0.0, chk_x = 0.0;
-  for (int j = tid; j < n; j += nt) { big = fmax(big, fabs(dx[j])); chk_x = fma(X[(size_t)b * n + j], 0.0, chk_x); }
+  for (int j = tid; j < n; j += nt) { big = fmax(big, fabs(dx[j])); if (!kTrial) chk_x = fma(X[(size_t)b * n + j], 0.0, chk_x); }
   big = BlockMax(big, scratch);
-  const bool finite = BlockMax(chk_x != chk_x ? 1.0 : 0.0, scratch) == 0.0 && finite_gj;
+  const bool finite = kTrial || (BlockMax(chk_x != chk_x ? 1.0 : 0.0, scratch) == 0.0 && finite_gj);
   const double scale = big > cap ? cap / big : 1.0;
   double* x = X + (size_t)b * n;
   const double* lo = x_lower + (size_t)b * bound_stride;
   const double* up = x_upper + (size_t)b * bound_stride;
+  if constexpr (kTrial) {
+    double* xt = tr.x_trial + (size_t)b * n;
+    for (int j = tid; j < n; j += nt) {
+      const double xj = x[j], v = fmin(fmax(xj + dx[j] * scale, lo[j]), up[j]);
+      xt[j] = v;
+      pd[j] = v - xj;                    // d: the step after cap and projection
+    }
+    __syncthreads();
+    double phi_lin = 0.0;                // sum of (s r(g + J d))^2, J d = (Js d) / s
+    for (int q = tid; q < m; q += nt) {
+      const int i = __ldg(pat.row_order + q);
+      const double si = s[i];
+      const double gi = g[i] + row_dot(i) / si, lo_i = __ldg(gl + i), up_i = __ldg(gu + i);
+      const double rs = si * (gi < lo_i ? gi - lo_i : gi > up_i ? gi - up_i : 0.0);
+      phi_lin += rs * rs;
+    }
+    phi_lin = 0.5 * BlockSum(phi_lin, scratch);
+    if (tid == 0) {
+      tr.merit[b] = phi;
+      tr.predicted[b] = phi - phi_lin;
+      if (violation) violation[b] = vmax;
+    }
+    return;
+  }
   if (finite)
     for (int j = tid; j < n; j += nt) x[j] = fmin(fmax(x[j] + dx[j] * scale, lo[j]), up[j]);
   if (tid == 0 && violation) violation[b] = finite ? vmax : CUDART_NAN;
 }
 
+template <bool kSmemJ, class Idx, bool kTrial>
+int LaunchLmKernel(const LmPattern& pat, const Idx* col_idx, const Idx* slot_t, const Idx* row_t, int threads, size_t smem, int n, int m, int nnz,
+                   double* x, const double* g, const double* jac, const double* xl, const double* xu, size_t bound_stride, const double* gl,
+                   const double* gu, size_t g_bound_stride, double mu, double cap, int cg_iters, double* violation, const LmTrialArgs& tr, int nb,
+                   cudaStream_t s) {
+  cudaError_t e = cudaFuncSetAttribute(LmStepKernel<kSmemJ, Idx, kTrial>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return (int)e;
+  LmStepKernel<kSmemJ, Idx, kTrial><<<nb, threads, smem, s>>>(pat, col_idx, slot_t, row_t, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
+                                                              g_bound_stride, mu, cap, cg_iters, violation, tr);
+  return (int)cudaGetLastError();
+}
+
 template <bool kSmemJ, class Idx>
 int LaunchLm(const LmPattern& pat, const Idx* col_idx, const Idx* slot_t, const Idx* row_t, int threads, size_t smem, int n, int m, int nnz, double* x,
              const double* g, const double* jac, const double* xl, const double* xu, size_t bound_stride, const double* gl, const double* gu,
-             size_t g_bound_stride, double mu, double cap, int cg_iters, double* violation, int nb, cudaStream_t s) {
-  cudaError_t e = cudaFuncSetAttribute(LmStepKernel<kSmemJ, Idx>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return (int)e;
-  LmStepKernel<kSmemJ, Idx><<<nb, threads, smem, s>>>(pat, col_idx, slot_t, row_t, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu, g_bound_stride, mu, cap,
-                                                     cg_iters, violation);
-  return (int)cudaGetLastError();
+             size_t g_bound_stride, double mu, double cap, int cg_iters, double* violation, const LmTrialArgs* trial, int nb, cudaStream_t s) {
+  if (trial)
+    return LaunchLmKernel<kSmemJ, Idx, true>(pat, col_idx, slot_t, row_t, threads, smem, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
+                                             g_bound_stride, mu, cap, cg_iters, violation, *trial, nb, s);
+  return LaunchLmKernel<kSmemJ, Idx, false>(pat, col_idx, slot_t, row_t, threads, smem, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
+                                            g_bound_stride, mu, cap, cg_iters, violation, LmTrialArgs{}, nb, s);
+}
+
+// CTA = instance, RUNNING instances only.  phi_t = 1/2 ||row_scale r(g_trial)||^2 (fixed summation order), rho = (phi0 - phi_t) /
+// predicted; accept when predicted > 0, every g_trial entry is finite (an infinite g against an infinite bound would count as
+// no violation) and rho > eta.  Every thread takes the same decision from the broadcast sums; thread 0 updates the scalars.
+__global__ void __launch_bounds__(256) LmAcceptKernel(int n, int m, double* __restrict__ X, const double* __restrict__ x_trial,
+                                                      const double* __restrict__ g_trial, const double* __restrict__ g_lower,
+                                                      const double* __restrict__ g_upper, size_t g_bound_stride,
+                                                      const double* __restrict__ row_scale, const double* __restrict__ merit,
+                                                      const double* __restrict__ predicted, double* __restrict__ mu, double* __restrict__ nu,
+                                                      int* __restrict__ status, int* __restrict__ iterations, double eta, double mu_min,
+                                                      double mu_max) {
+  __shared__ double scratch[32];
+  const int b = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
+  if (status[b] != kLmRunning) return;
+  const double* __restrict__ g = g_trial + (size_t)b * m;
+  const double* __restrict__ s = row_scale + (size_t)b * m;
+  const double* __restrict__ gl = g_lower + (size_t)b * g_bound_stride;
+  const double* __restrict__ gu = g_upper + (size_t)b * g_bound_stride;
+  double phi = 0.0, chk = 0.0;
+  for (int i = tid; i < m; i += nt) {
+    const double gi = g[i], lo = __ldg(gl + i), up = __ldg(gu + i);
+    const double rs = s[i] * (gi < lo ? gi - lo : gi > up ? gi - up : 0.0);
+    phi += rs * rs;
+    chk = fma(gi, 0.0, chk);
+  }
+  phi = 0.5 * BlockSum(phi, scratch);
+  const bool finite = BlockMax(chk != chk ? 1.0 : 0.0, scratch) == 0.0 && isfinite(phi);
+  const double pred = predicted[b];
+  const double rho = (merit[b] - phi) / pred;
+  const bool accept = pred > 0.0 && finite && rho > eta;
+  if (accept)
+    for (int j = tid; j < n; j += nt) X[(size_t)b * n + j] = x_trial[(size_t)b * n + j];
+  if (tid == 0) {
+    if (accept) {                        // mu <- max(mu_min, mu max(1/3, 1 - (2 rho - 1)^3)), nu <- 2
+      const double t = 2.0 * rho - 1.0;
+      mu[b] = fmax(mu_min, mu[b] * fmax(1.0 / 3.0, 1.0 - t * t * t));
+      nu[b] = 2.0;
+    } else {                             // mu <- mu nu, nu <- 2 nu; past mu_max: stalled
+      const double mu_new = mu[b] * nu[b];
+      mu[b] = mu_new;
+      nu[b] = 2.0 * nu[b];
+      if (mu_new > mu_max) status[b] = kLmStalled;
+    }
+    iterations[b] += 1;
+  }
 }
 
 }  // namespace
@@ -176,18 +288,27 @@ size_t LmSharedBytes(int n, int m) { return sizeof(double) * ((size_t)2 * m + 4 
 
 int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const double* g, const double* jac, const double* x_lower,
                  const double* x_upper, size_t bound_stride, const double* g_lower, const double* g_upper, size_t g_bound_stride, double mu,
-                 double cap, int cg_iters, double* violation, int nb, cudaStream_t s) {
+                 double cap, int cg_iters, double* violation, const LmTrialArgs* trial, int nb, cudaStream_t s) {
   if (nb <= 0) return 0;
   const size_t vec = LmSharedBytes(n, m), with_j = vec + sizeof(double) * (size_t)nnz;
   const bool smem_j = with_j <= 220 * 1024;   // the scaled values fit beside the vectors: one CTA of 512 threads per SM
   const int threads = smem_j ? 512 : 256;
   const size_t smem = smem_j ? with_j : vec;
   if (pat.col_idx16) {
-    return smem_j ? LaunchLm<true>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, nb, s)
-                  : LaunchLm<false>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, nb, s);
+    return smem_j ? LaunchLm<true>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, trial, nb, s)
+                  : LaunchLm<false>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, trial, nb, s);
   }
   // 32-bit indices mean n, m or nnz >= 65 536, so with_j >= 8 * 65 536 bytes > 220 KiB: never the shared-memory Js path
-  return LaunchLm<false>(pat, pat.col_idx, pat.slot_t, pat.row_t, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, nb, s);
+  return LaunchLm<false>(pat, pat.col_idx, pat.slot_t, pat.row_t, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, trial, nb, s);
+}
+
+int LaunchLmAccept(int n, int m, double* x, const double* x_trial, const double* g_trial, const double* g_lower, const double* g_upper,
+                   size_t g_bound_stride, const double* row_scale, const double* merit, const double* predicted, double* mu, double* nu,
+                   int* status, int* iterations, double eta, double mu_min, double mu_max, int nb, cudaStream_t s) {
+  if (nb <= 0) return 0;
+  LmAcceptKernel<<<nb, 256, 0, s>>>(n, m, x, x_trial, g_trial, g_lower, g_upper, g_bound_stride, row_scale, merit, predicted, mu, nu, status,
+                                    iterations, eta, mu_min, mu_max);
+  return (int)cudaGetLastError();
 }
 
 }  // namespace twb

@@ -653,6 +653,52 @@ class Batch:
                                                       ptr(g_upper), float(mu), float(cap), int(cg_iters), ptr(violation),
                                                       C.c_void_p(stream.cuda_stream)))
 
+    def _check_lm_tensors(self, x, specs, g_lower, g_upper):
+        import torch
+        p = self.problem
+        sizes = {"n": p.n, "m": p.m, "nnz": p.nnz, "1": 1}
+        for t, dt, per in specs:
+            assert t is None or (torch.is_tensor(t) and t.is_cuda and t.device == x.device and t.dtype == dt and t.is_contiguous()
+                                 and t.numel() == self.B * sizes[per]), "bad tensor"
+        for t in (g_lower, g_upper):
+            assert t is None or (torch.is_tensor(t) and t.is_cuda and t.device == x.device and t.dtype == torch.float64 and t.is_contiguous()
+                                 and tuple(t.shape) == (self.B, p.m)), "bad constraint bounds: (B, m) contiguous CUDA float64"
+        assert (g_lower is None) == (g_upper is None), "g_lower and g_upper: both or neither"
+
+    def lm_trial_device(self, x, g, jac, mu, solve_status, x_trial, row_scale, merit, predicted, x_lower=None, x_upper=None,
+                        g_lower=None, g_upper=None, cap=0.1, cg_iters=25, tol=1e-6, violation=None, stream=None):
+        """twb_batch_lm_trial_device: the trial step of a solve iteration.  Reads x (B, n), g, jac, mu (B,) and solve_status
+        (B,) int32; writes x_trial (B, n), row_scale (B, m), merit, predicted and violation (B,) for the RUNNING instances and
+        sets their status to LM_CONVERGED or LM_NONFINITE where that applies.  torch CUDA tensors; only enqueues."""
+        import torch
+        f64, i32 = torch.float64, torch.int32
+        self._check_lm_tensors(x, ((x, f64, "n"), (g, f64, "m"), (jac, f64, "nnz"), (mu, f64, "1"), (solve_status, i32, "1"),
+                                   (x_trial, f64, "n"), (row_scale, f64, "m"), (merit, f64, "1"), (predicted, f64, "1"),
+                                   (x_lower, f64, "n"), (x_upper, f64, "n"), (violation, f64, "1")), g_lower, g_upper)
+        if stream is None:
+            stream = torch.cuda.current_stream(x.device)
+        ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        check(lib.twb_batch_lm_trial_device(self._h, ptr(x), ptr(g), ptr(jac), ptr(x_lower), ptr(x_upper), ptr(g_lower), ptr(g_upper),
+                                            ptr(mu), float(cap), int(cg_iters), float(tol), ptr(solve_status), ptr(x_trial),
+                                            ptr(row_scale), ptr(merit), ptr(predicted), ptr(violation), C.c_void_p(stream.cuda_stream)))
+
+    def lm_accept_device(self, x, x_trial, g_trial, row_scale, merit, predicted, mu, nu, solve_status, iterations, g_lower=None,
+                         g_upper=None, eta=1e-4, mu_min=1e-12, mu_max=1e10, stream=None):
+        """twb_batch_lm_accept_device: the gain-ratio decision of a solve iteration for the RUNNING instances, on g_trial (B, m)
+        evaluated at x_trial.  Updates x (accepted: x_trial), mu, nu, solve_status and iterations (B,) int32 in place.  torch
+        CUDA tensors; only enqueues."""
+        import torch
+        f64, i32 = torch.float64, torch.int32
+        self._check_lm_tensors(x, ((x, f64, "n"), (x_trial, f64, "n"), (g_trial, f64, "m"), (row_scale, f64, "m"), (merit, f64, "1"),
+                                   (predicted, f64, "1"), (mu, f64, "1"), (nu, f64, "1"), (solve_status, i32, "1"),
+                                   (iterations, i32, "1")), g_lower, g_upper)
+        if stream is None:
+            stream = torch.cuda.current_stream(x.device)
+        ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        check(lib.twb_batch_lm_accept_device(self._h, ptr(x), ptr(x_trial), ptr(g_trial), ptr(g_lower), ptr(g_upper), ptr(row_scale),
+                                             ptr(merit), ptr(predicted), ptr(mu), ptr(nu), ptr(solve_status), ptr(iterations),
+                                             float(eta), float(mu_min), float(mu_max), C.c_void_p(stream.cuda_stream)))
+
     def eval_device(self, x, g=None, jac=None, cost=None, grad=None, status=None,
                     flags=capi.EVAL_G | capi.EVAL_JAC, stream=None):
         """Device-pointer variant. Arguments are torch CUDA float64 tensors (or None);

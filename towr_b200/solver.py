@@ -17,6 +17,12 @@ conjugate gradients run in shared memory on the problem's ONE shared CSR pattern
 orders, no atomics).  An instance whose x, g or Jacobian values hold a
 non-finite entry (the evaluation flags it in `status` bit 0) is not stepped by the native step: its x stays exactly as it
 was and its violation is NaN, so the caller can tell it apart instead of finding it clipped to its bounds.
+`solve(X, max_iters, tol)` solves to a tolerance instead: per iteration `twb_batch_eval_device`, the trial step
+`twb_batch_lm_trial_device` (the same step with a damping mu per instance, written to x_trial; merit 1/2 ||s r||^2, the
+decrease the linear model predicts, status CONVERGED when max |s r| <= tol or NONFINITE), a g-only evaluation at x_trial and
+`twb_batch_lm_accept_device` (gain ratio rho > eta: x <- x_trial and mu lowered, else x kept and mu raised, STALLED past
+mu_max).  The host picks the budget and stops early once no instance is RUNNING; tests/test_lm_solve.py holds the
+acceptance rule in numpy (tests/lm_solve_reference.py) and compares decisions on identical inputs.
 `native=False` keeps the first implementation of the same step in PyTorch tensor algebra (padded ELL gathers) — 30 x
 slower, used by the tests as a second opinion.
 tests/test_solver_loop.py holds the same algorithm in numpy, driven one instance at a time like ifopt by the CPU
@@ -132,3 +138,64 @@ class BatchedLevenbergMarquardt:
         for it in range(iters):
             hist[it] = self.step(X)
         return hist
+
+    def solve_state(self):
+        """A fresh per-instance solve state for `iterate`: mu = the constructor's mu, nu = 2, status RUNNING, 0 iterations,
+        and the trial buffers."""
+        if not self.native:
+            raise ValueError("solve / iterate run on the native path only")
+        if not self.mu > 0:
+            raise ValueError("solve needs an initial mu > 0")
+        return SolveState(self)
+
+    def iterate(self, X, st, tol, eta=1e-4, mu_min=1e-12, mu_max=1e10, cg_iters=None):
+        """One solve iteration for every instance in lock step, four calls that only enqueue (graph-capturable after the
+        first): evaluate g and J at X, the trial step (sets CONVERGED / NONFINITE), evaluate g at the trial point, accept or
+        reject.  X (B, n) and the solve state `st` are updated in place."""
+        from . import capi
+        bt, f = self.batch, capi.EVAL_G | capi.EVAL_JAC
+        bt.eval_device(X, g=self.g, jac=self.jac_vals, status=self.status, flags=f)
+        bt.lm_trial_device(X, self.g, self.jac_vals, st.mu, st.status, st.x_trial, st.row_scale, st.merit, st.predicted,
+                           self.xl_full, self.xu_full, self.gl_full, self.gu_full, self.cap,
+                           self.cg_iters if cg_iters is None else cg_iters, tol, st.violation)
+        if cg_iters == 0:
+            return
+        bt.eval_device(st.x_trial, g=st.g_trial, flags=capi.EVAL_G)
+        bt.lm_accept_device(X, st.x_trial, st.g_trial, st.row_scale, st.merit, st.predicted, st.mu, st.nu, st.status, st.iterations,
+                            self.gl_full, self.gu_full, eta, mu_min, mu_max)
+
+    def solve(self, X, max_iters, tol, eta=1e-4, mu_min=1e-12, mu_max=1e10, check_every=4):
+        """Solve every instance to max |s r| <= tol, at most `max_iters` iterations (native path only).  X (B, n) is updated
+        in place.  The loop stops early once no instance is RUNNING (one host read of a flag every `check_every`
+        iterations); afterwards one more evaluation and a trial without conjugate gradients make the status and the
+        violation describe the returned X.  Returns (status, iterations, violation, mu), (B,) CUDA tensors: status LM_*
+        (an instance still RUNNING has used up max_iters), iterations the trials taken, violation max |s r| at X."""
+        import torch
+        from . import capi
+        st = self.solve_state()
+        for it in range(max_iters):
+            self.iterate(X, st, tol, eta, mu_min, mu_max)
+            if (it + 1) % check_every == 0 and not bool(torch.any(st.status == capi.LM_RUNNING)):
+                break
+        self.iterate(X, st, tol, cg_iters=0)
+        return st.status, st.iterations, st.violation, st.mu
+
+
+class SolveState:
+    """Per-instance state of BatchedLevenbergMarquardt.solve: damping mu and its growth factor nu, the solve status and the
+    trials taken, plus the buffers of the trial point (x_trial, g_trial, row_scale, merit, predicted, violation)."""
+
+    def __init__(self, lm):
+        import torch
+        from . import capi
+        B, p, dev, f64 = lm.B, lm.p, lm.dev, torch.float64
+        self.mu = torch.full((B,), float(lm.mu), dtype=f64, device=dev)
+        self.nu = torch.full((B,), 2.0, dtype=f64, device=dev)
+        self.status = torch.full((B,), capi.LM_RUNNING, dtype=torch.int32, device=dev)
+        self.iterations = torch.zeros(B, dtype=torch.int32, device=dev)
+        self.x_trial = torch.empty((B, p.n), dtype=f64, device=dev)
+        self.g_trial = torch.empty((B, p.m), dtype=f64, device=dev)
+        self.row_scale = torch.empty((B, p.m), dtype=f64, device=dev)
+        self.merit = torch.empty(B, dtype=f64, device=dev)
+        self.predicted = torch.empty(B, dtype=f64, device=dev)
+        self.violation = torch.full((B,), float("nan"), dtype=f64, device=dev)
