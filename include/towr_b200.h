@@ -338,6 +338,61 @@ int twb_batch_lm_accept_device(twb_batch* b, double* x, const double* x_trial, c
                                const double* g_upper, const double* row_scale, const double* merit, const double* predicted, double* mu,
                                double* nu, int* solve_status, int* iterations, double eta, double mu_min, double mu_max, void* stream);
 
+/* ---- a whole solve in one call: the loop of the four calls above runs on the device ------------------------------------
+ * The stand-in for ipopt.Solve(nlp) (towr/test/hopper_example.cc:93).  Enqueues on `stream` one CUDA graph:
+ *   start: mu = mu0, nu = 2, status RUNNING, iterations 0 per instance
+ *   WHILE (an instance is RUNNING and fewer than max_iters loop iterations ran) {
+ *     eval (g, jac at x); trial; eval (g at x_trial); accept; count the instances per status }
+ *   tail: eval (g, jac at x); trial with cg_iters = 0 (so that status and violation describe the returned x); count
+ * The loop's exit test is a kernel: the loop stops at the iteration after which no instance is RUNNING, with no host round
+ * trip.  The outputs equal, bit for bit, what BatchedLevenbergMarquardt.solve (towr_b200/solver.py) returns for the same
+ * inputs — the four-call loop with its host-side early exit — since a finished instance does not move in further iterations.
+ *   x [B][n] in / out; x_lower / x_upper [B][n] (both NULL: the problem's own variable bounds); g_lower / g_upper [B][m] (both
+ *   NULL: the problem's own constraint bounds; exactly one NULL is TWB_ERR_INVALID); solve_status [B], iterations [B] (trials
+ *   taken), violation [B] (max |s r| at the returned x; NaN for TWB_LM_NONFINITE), mu [B] (the final damping) out;
+ *   status_counts [4] (instances per TWB_LM_* status after the tail; may be NULL) and loop_count [1] (loop iterations run; may
+ *   be NULL) out.  All device pointers of the batch's device, in the layouts of the trial and accept calls.
+ * The batch owns the work arrays (g, jac, x_trial, g_trial, row scales, merit, predicted, nu): allocated by the first solve
+ * call, freed by twb_batch_destroy.  The first call with an argument set (the pointers and the options) also uploads the
+ * pattern (as the step family's first call does) and builds and instantiates the graph; it is cached per argument set (up to
+ * 16 per batch, least recently used replaced, dropped when terrains or grids change).  After that a call only launches the
+ * graph into `stream`: no host synchronisation, no allocation.
+ * A batch serves ONE evaluation or solve at a time (the work arrays and the staging matrix are shared): a second call on
+ * another stream must be ordered after the first by the caller.
+ * Errors, with nothing enqueued and no output touched: NULL b / x / opt / solve_status / iterations / violation / mu, one of
+ * x_lower / x_upper or of g_lower / g_upper NULL, max_iters < 0, tol < 0 or NaN, eta outside [0, 1), not
+ * 0 < mu_min <= mu_max, mu0 <= 0 or NaN, cap <= 0 or NaN, cg_iters outside [0, 10000]: TWB_ERR_INVALID; a stream that is
+ * being captured (a solve cannot be captured into the caller's graph), TWB_PROFILE set, or solver vectors over 200 KiB of
+ * shared memory (as for twb_batch_lm_step_device): TWB_ERR_UNSUPPORTED. */
+typedef struct twb_lm_solve_options {
+  double mu0;      /* initial damping (> 0)                                      */
+  double cap;      /* largest step entry, as for twb_batch_lm_step_device         */
+  double tol;      /* CONVERGED when max |s r| <= tol                             */
+  double eta;      /* accept when the gain ratio rho > eta, eta in [0, 1)         */
+  double mu_min;   /* damping floor after an accepted trial                       */
+  double mu_max;   /* STALLED once a rejected trial raises mu past mu_max         */
+  int cg_iters;    /* conjugate-gradient iterations per trial                     */
+  int max_iters;   /* iteration budget (>= 0)                                     */
+} twb_lm_solve_options;
+
+/* the defaults of BatchedLevenbergMarquardt.solve: mu0 1e-2, cap 0.1, tol 1e-6, eta 1e-4, mu_min 1e-12, mu_max 1e10,
+ * cg_iters 25, max_iters 60 */
+void twb_lm_solve_options_default(twb_lm_solve_options* o);
+
+int twb_batch_lm_solve_device(twb_batch* b, double* x, const double* x_lower, const double* x_upper, const double* g_lower,
+                              const double* g_upper, const twb_lm_solve_options* opt, int* solve_status, int* iterations,
+                              double* violation, double* mu, int* status_counts, int* loop_count, void* stream);
+
+/* Host-pointer twin of twb_batch_lm_solve_device, for callers without the CUDA runtime (BatchedProblem::Solve in
+ * towr_b200_ifopt.hpp): copies x and the bounds given into buffers of the batch, runs the same solve graph on the batch's
+ * stream, copies x and the outputs back and synchronises.  Arguments and errors as for the device call, all host arrays. */
+int twb_batch_lm_solve_host(twb_batch* b, double* x, const double* x_lower, const double* x_upper, const double* g_lower,
+                            const double* g_upper, const twb_lm_solve_options* opt, int* solve_status, int* iterations,
+                            double* violation, double* mu, int* status_counts, int* loop_count);
+
+/* For tests: the solve graphs this batch has instantiated so far (a call that reuses a cached graph adds none). */
+int twb_batch_lm_solve_graph_stats(const twb_batch* b, int* instantiations);
+
 /* Host-pointer variant: copies x up, evaluates, copies the requested outputs
  * back and synchronises. Pinned host memory makes the copies asynchronous. */
 int twb_batch_eval_host(twb_batch* b, const double* x, double* g, double* jac,

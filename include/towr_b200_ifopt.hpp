@@ -277,6 +277,25 @@ class BatchedProblem {
   // (structure-only use) the host arrays are served as they are.
   void MarkDirty() { dirty_ = true; }
   void EnsureEvaluated() { if (dirty_ && batch_) Evaluate(TWB_EVAL_ALL); }
+  // ipopt.Solve(nlp) for every instance at once (hopper_example.cc:93): the device-side solve loop of twb_batch_lm_solve_device
+  // from the current X, against each instance's own bounds after SetStates (else the problem's), through its host twin
+  // twb_batch_lm_solve_host (this header needs no CUDA runtime).  X receives the solutions, so GpuProblem(*this, b)
+  // .GetVariableValues() returns instance b's; the constraint and cost views re-evaluate at them on their next Get*.
+  // solve_status(b), solve_iterations(b) and solve_violation(b) report per instance.  Returns the call's TWB_* code
+  // (TWB_ERR_NO_DEVICE without a device batch; twb_last_error() says more).
+  int Solve(const twb_lm_solve_options& opt) {
+    if (!batch_) return TWB_ERR_NO_DEVICE;
+    SOLVE_STATUS.assign(B_, 0); SOLVE_ITERATIONS.assign(B_, 0); SOLVE_VIOLATION.assign(B_, 0.0); SOLVE_MU.assign(B_, 0.0);
+    const bool own = !ixl_.empty();
+    const int rc = twb_batch_lm_solve_host(batch_, X.data(), own ? ixl_.data() : nullptr, own ? ixu_.data() : nullptr, own ? igl_.data() : nullptr,
+                                           own ? igu_.data() : nullptr, &opt, SOLVE_STATUS.data(), SOLVE_ITERATIONS.data(), SOLVE_VIOLATION.data(),
+                                           SOLVE_MU.data(), nullptr, nullptr);
+    if (rc == TWB_OK) dirty_ = true;
+    return rc;
+  }
+  int solve_status(int b) const { return SOLVE_STATUS.at(b); }         // TWB_LM_* of the last Solve
+  int solve_iterations(int b) const { return SOLVE_ITERATIONS.at(b); } // trials taken
+  double solve_violation(int b) const { return SOLVE_VIOLATION.at(b); }   // max |s r| at the returned x
   // ---- solution post-processing of the current X (fpowr) ----
   // fpowr::GetTrajectory(solution, dt) for every instance: [B][n_samples][19 + 13 n_ee]
   std::vector<double> SampleTrajectory(double dt, int* n_samples = nullptr, int* n_values = nullptr) {
@@ -328,6 +347,8 @@ class BatchedProblem {
 
   std::vector<double> X, G, JAC, COST, GRAD;   // [B][n], [B][m], [B][nnz], [B], [B][n]
   std::vector<int> STATUS;
+  std::vector<int> SOLVE_STATUS, SOLVE_ITERATIONS;   // [B] each, from the last Solve
+  std::vector<double> SOLVE_VIOLATION, SOLVE_MU;     // [B] each, from the last Solve
 
  private:
   twb_problem* prob_ = nullptr;

@@ -118,6 +118,18 @@ struct twb_batch {
   };
   std::vector<PostTables> post_tables;
   unsigned long long post_clock = 0;
+  // twb_batch_lm_solve_device: the work arrays of the loop (one allocation, made by the first solve call) and the instantiated
+  // solve graphs, one per argument set, cached like the evaluation graphs (up to 16, least recently used replaced, dropped
+  // with them).  lm_stage: the host twin's device copies of its arguments (first host call).
+  struct LmWork { double *g, *jac, *x_trial, *g_trial, *row_scale, *merit, *predicted, *nu; int* loop; };
+  void* lm_work_mem = nullptr;
+  LmWork lm_work{};
+  struct LmStage { double *x, *xl, *xu, *gl, *gu, *violation, *mu; int *status, *iterations, *counts, *loop_count; };
+  void* lm_stage_mem = nullptr;
+  LmStage lm_stage{};
+  struct SolveGraph { const void* ptr[11]; twb_lm_solve_options opt; cudaGraphExec_t exec; unsigned long long used; };
+  std::vector<SolveGraph> solve_graphs;
+  int solve_instantiations = 0;   // graphs instantiated so far (twb_batch_lm_solve_graph_stats)
 };
 
 namespace {
@@ -132,6 +144,8 @@ size_t EvalChunk(const twb_batch* b) {
 void DropGraphs(twb_batch* b) {
   for (auto& gr : b->graphs) cudaGraphExecDestroy(gr.exec);
   b->graphs.clear();
+  for (auto& gr : b->solve_graphs) cudaGraphExecDestroy(gr.exec);
+  b->solve_graphs.clear();
 }
 // slot `slot` of the batch's scratch pool with at least `bytes` bytes (the post-processing entry points synchronise before
 // they return and a batch has one caller at a time, so the slots are free again at the next call)
@@ -452,6 +466,7 @@ void twb_batch_destroy(twb_batch* b) {
   for (void* p : b->owned) cudaFree(p);
   for (auto& sc : b->scratch) cudaFree(sc.first);
   for (auto& t : b->post_tables) cudaFree(t.mem);
+  cudaFree(b->lm_work_mem); cudaFree(b->lm_stage_mem);
   cudaFree(b->d_terrain); cudaFree(b->d_grid); cudaFree(b->d_gmap_pool); cudaFree(b->d_gmaps); cudaFree(b->d_XT); cudaFree(b->d_FS);
   for (auto ev : b->ev) if (ev) cudaEventDestroy(ev);
   if (b->aux0) cudaStreamDestroy(b->aux0);
@@ -772,6 +787,31 @@ int twb_batch_launches_per_eval(const twb_batch* b, unsigned flags) {
   return n;
 }
 
+}  // extern "C"
+
+// The kernels of one evaluation (what twb_batch_eval_device enqueues without its graph cache): the whole batch, or chunk after
+// chunk (twb_batch::eval_chunk), on s0 and the batch's two auxiliary streams
+static int EnqueueEval(twb_batch* b, const double* x, double* g, double* jac, double* cost, double* grad, int* status, unsigned kflags,
+                       cudaStream_t s0, int* launches) {
+  const twb::Formulation& f = b->prob->f;
+  const size_t B = (size_t)b->B;
+  const size_t chunk = EvalChunk(b);
+  const size_t n = f.n, m = f.m;
+  for (size_t off = 0; off < B; off += chunk) {
+    const size_t nb = std::min(chunk, B - off), t0 = off / 32;
+    const int rc = twb::LaunchEval(b->plan, x + off * n, b->d_XT + t0 * (n + 1) * 32,
+                                   b->d_FS ? b->d_FS + t0 * (size_t)b->plan.n_dyn * 6 * b->plan.n_ee * 32 : nullptr,
+                                   g ? g + off * m : nullptr, jac ? jac + off * (size_t)f.nnz : nullptr, cost ? cost + off : nullptr,
+                                   grad ? grad + off * n : nullptr, status ? status + off : nullptr,
+                                   b->d_terrain ? b->d_terrain + off : nullptr, f.spec.terrain, (int)nb, kflags, s0, b->aux0, b->aux1, b->ev.data(),
+                                   launches);
+    if (rc != 0) return rc;
+  }
+  return 0;
+}
+
+extern "C" {
+
 int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac, double* cost, double* grad,
                           int* status, unsigned flags, void* stream) {
   if (!b || !x) return Fail(TWB_ERR_INVALID, "null argument");
@@ -785,21 +825,8 @@ int twb_batch_eval_device(twb_batch* b, const double* x, double* g, double* jac,
   unsigned kflags = flags & (TWB_EVAL_G | TWB_EVAL_JAC);
   if (f.has_cost && (flags & TWB_EVAL_COST)) kflags |= TWB_EVAL_COST;
   int launches = 0;
-  // the whole batch, or chunk after chunk (twb_batch::eval_chunk), enqueued on s0 and the batch's two auxiliary streams
   auto enqueue = [&](cudaStream_t s0) -> int {
-    const size_t B = (size_t)b->B;
-    const size_t chunk = EvalChunk(b);
-    const size_t n = f.n, m = f.m;
-    for (size_t off = 0; off < B; off += chunk) {
-      const size_t nb = std::min(chunk, B - off), t0 = off / 32;
-      const int rc = twb::LaunchEval(b->plan, x + off * n, b->d_XT + t0 * (n + 1) * 32,
-                                     b->d_FS ? b->d_FS + t0 * (size_t)b->plan.n_dyn * 6 * b->plan.n_ee * 32 : nullptr,
-                                     g ? g + off * m : nullptr, jac ? jac + off * (size_t)f.nnz : nullptr, cost ? cost + off : nullptr,
-                                     grad ? grad + off * n : nullptr, status ? status + off : nullptr,
-                                     b->d_terrain ? b->d_terrain + off : nullptr, f.spec.terrain, (int)nb, kflags, s0, b->aux0, b->aux1, b->ev.data(), &launches);
-      if (rc != 0) return rc;
-    }
-    return 0;
+    return EnqueueEval(b, x, g, jac, cost, grad, status, kflags, s0, &launches);
   };
   if (b->use_graphs && !g_prof_on) {
     // replay (or first capture on the batch's own stream) the evaluation of this argument set as a CUDA graph
@@ -944,6 +971,236 @@ int twb_batch_lm_accept_device(twb_batch* b, double* x, const double* x_trial, c
                            own_g ? (size_t)f.m : 0, row_scale, merit, predicted, mu, nu, solve_status, iterations, eta, mu_min, mu_max, b->B,
                            static_cast<cudaStream_t>(stream));
   if (rc != 0) return CudaFail(static_cast<cudaError_t>(rc), "solver accept launch");
+  return TWB_OK;
+}
+
+void twb_lm_solve_options_default(twb_lm_solve_options* o) {
+  if (o) *o = twb_lm_solve_options{1e-2, 0.1, 1e-6, 1e-4, 1e-12, 1e10, 25, 60};
+}
+
+// ---- twb_batch_lm_solve_device: the solve loop as one CUDA graph with a WHILE node --------------------------------------
+// the arguments of one solve; together they are the key of the graph cache
+struct LmSolveCall {
+  double* x; const double *xl, *xu, *gl, *gu;
+  int *status, *iterations; double *violation, *mu; int *counts, *loop_count;
+  twb_lm_solve_options opt;
+  void Key(const void* (&k)[11]) const {
+    const void* v[11] = {x, xl, xu, gl, gu, status, iterations, violation, mu, counts, loop_count};
+    std::copy(v, v + 11, k);
+  }
+};
+
+// the checks of the device call and its host twin that need no device
+static int LmSolveArgs(const twb_batch* b, const LmSolveCall& c) {
+  if (!b || !c.x || !c.status || !c.iterations || !c.violation || !c.mu) return Fail(TWB_ERR_INVALID, "null argument");
+  if ((c.xl == nullptr) != (c.xu == nullptr)) return Fail(TWB_ERR_INVALID, "x_lower and x_upper: both or neither");
+  if ((c.gl == nullptr) != (c.gu == nullptr)) return Fail(TWB_ERR_INVALID, "g_lower and g_upper: both or neither");
+  const twb_lm_solve_options& o = c.opt;
+  if (o.max_iters < 0) return Fail(TWB_ERR_INVALID, "max_iters < 0");
+  if (!(o.tol >= 0.0)) return Fail(TWB_ERR_INVALID, "bad tolerance");
+  if (!(o.eta >= 0.0 && o.eta < 1.0) || !(o.mu_min > 0.0 && o.mu_min <= o.mu_max) || !(o.mu0 > 0.0) || !(o.cap > 0.0) || o.cg_iters < 0 ||
+      o.cg_iters > 10000)
+    return Fail(TWB_ERR_INVALID, "bad solver parameter");
+  if (g_prof_on) return Fail(TWB_ERR_UNSUPPORTED, "TWB_PROFILE records events around every kernel, which a device-side loop cannot hold");
+  const twb::Formulation& f = b->prob->f;
+  if (twb::LmSharedBytes(f.n, f.m) > 200 * 1024) return Fail(TWB_ERR_UNSUPPORTED, "problem too large for the shared-memory solver step");
+  return TWB_OK;
+}
+
+// the loop's work arrays, one allocation (every array at a 256-byte boundary), made on the first solve call
+static int LmWorkReady(twb_batch* b) {
+  if (b->lm_work_mem) return TWB_OK;
+  const twb::Formulation& f = b->prob->f;
+  const size_t B = b->B;
+  auto up = [](size_t bytes) { return (bytes + 255) & ~(size_t)255; };
+  const size_t counts[8] = {B * f.m, B * f.nnz, B * f.n, B * f.m, B * f.m, B, B, B};   // g, jac, x_trial, g_trial, row_scale, merit, predicted, nu
+  size_t off[9] = {0};
+  for (int k = 0; k < 8; ++k) off[k + 1] = off[k] + up(sizeof(double) * counts[k]);
+  void* mem = nullptr;
+  cudaError_t e = cudaMalloc(&mem, off[8] + up(sizeof(int) * twb::kLoopInts));
+  if (e != cudaSuccess) return CudaFail(e, "cudaMalloc");
+  char* p = static_cast<char*>(mem);
+  double* a[8];
+  for (int k = 0; k < 8; ++k) a[k] = reinterpret_cast<double*>(p + off[k]);
+  b->lm_work = {a[0], a[1], a[2], a[3], a[4], a[5], a[6], a[7], reinterpret_cast<int*>(p + off[8])};
+  b->lm_work_mem = mem;
+  return TWB_OK;
+}
+
+// Captures the solve graph of `c`:
+//   init -> WHILE { eval(G|JAC at x) -> trial -> eval(G at x_trial) -> accept -> count + condition } -> eval(G|JAC at x) ->
+//   trial with cg_iters = 0 -> count into the caller's outputs
+// The start and the tail are captured into the graph around the WHILE node, the body into the node's body graph.  The
+// evaluations are captured as kernels, as twb_batch_eval_device enqueues them without its graph cache (three streams joined by
+// events, RomNodeOut with programmatic dependent launch: both instantiate inside the conditional body on the B200).
+static cudaError_t CaptureSolveGraph(twb_batch* b, const LmSolveCall& c, cudaGraph_t* out) {
+  const twb::Formulation& f = b->prob->f;
+  const twb_batch::LmWork& w = b->lm_work;
+  const int B = b->B;
+  const twb_lm_solve_options& o = c.opt;
+  cudaStream_t s = b->stream;
+  const bool own = c.xl != nullptr, own_g = c.gl != nullptr;
+  const double *xl = own ? c.xl : b->d_xl, *xu = own ? c.xu : b->d_xu;
+  const double *gl = own_g ? c.gl : b->lm_pat.g_lower, *gu = own_g ? c.gu : b->lm_pat.g_upper;
+  const size_t xs = own ? (size_t)f.n : 0, gs = own_g ? (size_t)f.m : 0;
+  const twb::LmTrialArgs trial{c.mu, o.tol, c.status, w.x_trial, w.row_scale, w.merit, w.predicted};
+  auto eval = [&](const double* x, double* g, double* jac, unsigned flags) {
+    return EnqueueEval(b, x, g, jac, nullptr, nullptr, nullptr, flags, s, nullptr);
+  };
+  auto trial_step = [&](int cg_iters) {
+    return twb::LaunchLmStep(b->lm_pat, f.n, f.m, f.nnz, c.x, w.g, w.jac, xl, xu, xs, gl, gu, gs, 0.0, o.cap, cg_iters, c.violation, &trial, B, s);
+  };
+  cudaGraph_t graph = nullptr;
+  cudaGraphConditionalHandle cond = 0;
+  cudaGraphNodeParams loop{};
+  cudaError_t e = cudaGraphCreate(&graph, 0);
+  if (e == cudaSuccess) e = cudaGraphConditionalHandleCreate(&cond, graph, 0, 0);
+  if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(s, graph, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
+  if (e == cudaSuccess) {   // the start, the WHILE node after it, the tail after that
+    int rc = twb::LaunchLmSolveInit(B, o.mu0, c.mu, w.nu, c.status, c.iterations, w.loop, o.max_iters, cond, s);
+    cudaStreamCaptureStatus cs;
+    const cudaGraphNode_t* deps = nullptr;
+    size_t n_deps = 0;
+    cudaGraphNode_t node = nullptr;
+    if (rc == 0) rc = cudaStreamGetCaptureInfo(s, &cs, nullptr, nullptr, &deps, &n_deps);
+    if (rc == 0) {
+      loop.type = cudaGraphNodeTypeConditional;
+      loop.conditional.handle = cond;
+      loop.conditional.type = cudaGraphCondTypeWhile;
+      loop.conditional.size = 1;
+      rc = cudaGraphAddNode(&node, graph, deps, n_deps, &loop);
+    }
+    if (rc == 0) rc = cudaStreamUpdateCaptureDependencies(s, &node, 1, cudaStreamSetCaptureDependencies);
+    if (rc == 0) rc = eval(c.x, w.g, w.jac, TWB_EVAL_G | TWB_EVAL_JAC);
+    if (rc == 0) rc = trial_step(0);
+    if (rc == 0) rc = twb::LaunchLmCount(B, c.status, w.loop, o.max_iters, cond, false, c.counts, c.loop_count, s);
+    cudaGraph_t captured = nullptr;
+    e = cudaStreamEndCapture(s, &captured);
+    if (rc != 0) e = static_cast<cudaError_t>(rc);
+  }
+  if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(s, loop.conditional.phGraph_out[0], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
+  if (e == cudaSuccess) {   // the body
+    int rc = eval(c.x, w.g, w.jac, TWB_EVAL_G | TWB_EVAL_JAC);
+    if (rc == 0) rc = trial_step(o.cg_iters);
+    if (rc == 0) rc = eval(w.x_trial, w.g_trial, nullptr, TWB_EVAL_G);
+    if (rc == 0)
+      rc = twb::LaunchLmAccept(f.n, f.m, c.x, w.x_trial, w.g_trial, gl, gu, gs, w.row_scale, w.merit, w.predicted, c.mu, w.nu, c.status,
+                               c.iterations, o.eta, o.mu_min, o.mu_max, B, s);
+    if (rc == 0) rc = twb::LaunchLmCount(B, c.status, w.loop, o.max_iters, cond, true, nullptr, nullptr, s);
+    cudaGraph_t captured = nullptr;
+    e = cudaStreamEndCapture(s, &captured);
+    if (rc != 0) e = static_cast<cudaError_t>(rc);
+  }
+  if (e != cudaSuccess) {
+    if (graph) cudaGraphDestroy(graph);
+    cudaGetLastError();
+    return e;
+  }
+  *out = graph;
+  return cudaSuccess;
+}
+
+// the instantiated graph of `c`: from the cache, or captured and instantiated
+static int SolveGraph(twb_batch* b, const LmSolveCall& c, cudaGraphExec_t* exec) {
+  const void* key[11];
+  c.Key(key);
+  for (auto& gr : b->solve_graphs)
+    if (std::equal(key, key + 11, gr.ptr) && std::memcmp(&gr.opt, &c.opt, sizeof c.opt) == 0) {
+      gr.used = ++b->graph_clock; *exec = gr.exec; return TWB_OK;
+    }
+  cudaGraph_t graph = nullptr;
+  cudaError_t e = CaptureSolveGraph(b, c, &graph);
+  if (e == cudaSuccess) {
+    e = cudaGraphInstantiate(exec, graph, 0);
+    cudaGraphDestroy(graph);
+  }
+  if (e != cudaSuccess) { cudaGetLastError(); return CudaFail(e, "solve graph"); }
+  ++b->solve_instantiations;
+  if (b->solve_graphs.size() >= 16) {   // replace the least recently used
+    size_t lru = 0;
+    for (size_t i = 1; i < b->solve_graphs.size(); ++i) if (b->solve_graphs[i].used < b->solve_graphs[lru].used) lru = i;
+    cudaGraphExecDestroy(b->solve_graphs[lru].exec);
+    b->solve_graphs.erase(b->solve_graphs.begin() + lru);
+  }
+  b->solve_graphs.push_back({{}, c.opt, *exec, ++b->graph_clock});
+  std::copy(key, key + 11, b->solve_graphs.back().ptr);
+  return TWB_OK;
+}
+
+static int LmSolveCore(twb_batch* b, const LmSolveCall& c, cudaStream_t stream) {
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+  if ((e = cudaStreamIsCapturing(stream, &cs)) != cudaSuccess) { cudaGetLastError(); return CudaFail(e, "cudaStreamIsCapturing"); }
+  if (cs != cudaStreamCaptureStatusNone) return Fail(TWB_ERR_UNSUPPORTED, "the stream is being captured: a solve cannot be captured into a graph");
+  int rc = LmPatternReady(b);
+  if (rc == TWB_OK) rc = LmWorkReady(b);
+  cudaGraphExec_t exec = nullptr;
+  if (rc == TWB_OK) rc = SolveGraph(b, c, &exec);
+  if (rc != TWB_OK) return rc;
+  if ((e = cudaGraphLaunch(exec, stream)) != cudaSuccess) return CudaFail(e, "cudaGraphLaunch");
+  return TWB_OK;
+}
+
+int twb_batch_lm_solve_device(twb_batch* b, double* x, const double* x_lower, const double* x_upper, const double* g_lower,
+                              const double* g_upper, const twb_lm_solve_options* opt, int* solve_status, int* iterations,
+                              double* violation, double* mu, int* status_counts, int* loop_count, void* stream) {
+  if (!opt) return Fail(TWB_ERR_INVALID, "null argument");
+  const LmSolveCall c{x, x_lower, x_upper, g_lower, g_upper, solve_status, iterations, violation, mu, status_counts, loop_count, *opt};
+  const int rc = LmSolveArgs(b, c);
+  return rc != TWB_OK ? rc : LmSolveCore(b, c, static_cast<cudaStream_t>(stream));
+}
+
+int twb_batch_lm_solve_host(twb_batch* b, double* x, const double* x_lower, const double* x_upper, const double* g_lower,
+                            const double* g_upper, const twb_lm_solve_options* opt, int* solve_status, int* iterations,
+                            double* violation, double* mu, int* status_counts, int* loop_count) {
+  if (!opt) return Fail(TWB_ERR_INVALID, "null argument");
+  const LmSolveCall h{x, x_lower, x_upper, g_lower, g_upper, solve_status, iterations, violation, mu, status_counts, loop_count, *opt};
+  int rc = LmSolveArgs(b, h);
+  if (rc != TWB_OK) return rc;
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e != cudaSuccess) return CudaFail(e, "cudaSetDevice");
+  const twb::Formulation& f = b->prob->f;
+  const size_t B = b->B, xb = sizeof(double) * B * f.n, gb = sizeof(double) * B * f.m;
+  if (!b->lm_stage_mem) {   // x, x bounds, g bounds, violation, mu, status, iterations, counts, loop count: one allocation
+    auto up = [](size_t bytes) { return (bytes + 255) & ~(size_t)255; };
+    const size_t sizes[11] = {xb, xb, xb, gb, gb, sizeof(double) * B, sizeof(double) * B, sizeof(int) * B, sizeof(int) * B, sizeof(int) * 4, sizeof(int)};
+    size_t off[12] = {0};
+    for (int k = 0; k < 11; ++k) off[k + 1] = off[k] + up(sizes[k]);
+    void* mem = nullptr;
+    if ((e = cudaMalloc(&mem, off[11])) != cudaSuccess) return CudaFail(e, "cudaMalloc");
+    char* p = static_cast<char*>(mem);
+    auto d = [&](int k) { return reinterpret_cast<double*>(p + off[k]); };
+    auto i = [&](int k) { return reinterpret_cast<int*>(p + off[k]); };
+    b->lm_stage = {d(0), d(1), d(2), d(3), d(4), d(5), d(6), i(7), i(8), i(9), i(10)};
+    b->lm_stage_mem = mem;
+  }
+  const twb_batch::LmStage& st = b->lm_stage;
+  cudaStream_t s = b->stream;
+  cudaMemcpyAsync(st.x, x, xb, cudaMemcpyHostToDevice, s);
+  if (x_lower) { cudaMemcpyAsync(st.xl, x_lower, xb, cudaMemcpyHostToDevice, s); cudaMemcpyAsync(st.xu, x_upper, xb, cudaMemcpyHostToDevice, s); }
+  if (g_lower) { cudaMemcpyAsync(st.gl, g_lower, gb, cudaMemcpyHostToDevice, s); cudaMemcpyAsync(st.gu, g_upper, gb, cudaMemcpyHostToDevice, s); }
+  const LmSolveCall c{st.x, x_lower ? st.xl : nullptr, x_lower ? st.xu : nullptr, g_lower ? st.gl : nullptr, g_lower ? st.gu : nullptr, st.status,
+                      st.iterations, st.violation, st.mu, status_counts ? st.counts : nullptr, loop_count ? st.loop_count : nullptr, *opt};
+  rc = LmSolveCore(b, c, s);
+  if (rc == TWB_OK) {
+    cudaMemcpyAsync(x, st.x, xb, cudaMemcpyDeviceToHost, s);
+    cudaMemcpyAsync(solve_status, st.status, sizeof(int) * B, cudaMemcpyDeviceToHost, s);
+    cudaMemcpyAsync(iterations, st.iterations, sizeof(int) * B, cudaMemcpyDeviceToHost, s);
+    cudaMemcpyAsync(violation, st.violation, sizeof(double) * B, cudaMemcpyDeviceToHost, s);
+    cudaMemcpyAsync(mu, st.mu, sizeof(double) * B, cudaMemcpyDeviceToHost, s);
+    if (status_counts) cudaMemcpyAsync(status_counts, st.counts, sizeof(int) * 4, cudaMemcpyDeviceToHost, s);
+    if (loop_count) cudaMemcpyAsync(loop_count, st.loop_count, sizeof(int), cudaMemcpyDeviceToHost, s);
+  }
+  e = cudaStreamSynchronize(s);
+  if (rc != TWB_OK) return rc;
+  if (e != cudaSuccess) return CudaFail(e, "solve");
+  return TWB_OK;
+}
+
+int twb_batch_lm_solve_graph_stats(const twb_batch* b, int* instantiations) {
+  if (!b || !instantiations) return Fail(TWB_ERR_INVALID, "null argument");
+  *instantiations = b->solve_instantiations;
   return TWB_OK;
 }
 

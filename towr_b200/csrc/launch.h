@@ -83,6 +83,16 @@ int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const d
 int LaunchLmAccept(int n, int m, double* x, const double* x_trial, const double* g_trial, const double* g_lower, const double* g_upper,
                    size_t g_bound_stride, const double* row_scale, const double* merit, const double* predicted, double* mu, double* nu,
                    int* status, int* iterations, double eta, double mu_min, double mu_max, int nb, cudaStream_t s);
+// the device-side solve loop (twb_batch_lm_solve_device).  loop: kLoopInts device ints of loop state (iterations run, the
+// counts being added up); cond: the WHILE node's handle in the graph these kernels are captured into.
+constexpr int kLoopInts = 6;
+// per instance mu = mu0, nu = 2, status RUNNING, iterations 0; the loop state cleared; the condition = max_iters > 0
+int LaunchLmSolveInit(int nb, double mu0, double* mu, double* nu, int* status, int* iterations, int* loop, int max_iters,
+                      cudaGraphConditionalHandle cond, cudaStream_t s);
+// instances per status.  loop_step: iterations run += 1, condition = (RUNNING > 0 && iterations run < max_iters); else
+// status_counts[4] / loop_count[1] (each may be null) receive the counts and the iterations run, the condition is not touched
+int LaunchLmCount(int nb, const int* status, int* loop, int max_iters, cudaGraphConditionalHandle cond, bool loop_step, int* status_counts,
+                  int* loop_count, cudaStream_t s);
 // number of output kernels one evaluation launches for this plan
 int OutKernelsPerEval(const Plan& P, unsigned flags);
 // One batched evaluation of `nb` instances.  XT is [tiles][n+1][32] (zero-initialised once; row n stays 0; tile = 32

@@ -23,9 +23,13 @@
 // the instance would jump to its bounds and report a finite violation (a NaN bound would silently mean "unbounded").
 // +-Inf constraint bounds mean unbounded, like the 1e20 convention.  With lower > upper the lower bound wins (g < lo is
 // tested first).
+// The solve loop on the device (twb_batch_lm_solve_device) adds two small kernels: LmSolveInitKernel starts a solve (mu, nu,
+// status, iterations per instance; the loop counter; the WHILE condition of the solve graph) and LmCountKernel counts the
+// instances per status — at the end of every loop iteration it sets the condition, after the loop it reports the counts.
 #include <cuda_runtime.h>
 #include <math_constants.h>
 
+#include <algorithm>
 #include <cstdint>
 
 #include "launch.h"
@@ -282,6 +286,70 @@ __global__ void __launch_bounds__(256) LmAcceptKernel(int n, int m, double* __re
   }
 }
 
+// ---- the device-side solve loop (twb_batch_lm_solve_device): the start of a solve and the loop's exit test
+// loop[kLoopIter] = iterations the loop has run, loop[kLoopCount + s] = instances with status s (accumulated over the CTAs of
+// one count), loop[kLoopTicket] = CTAs of the current count that have added theirs
+constexpr int kLoopIter = 0, kLoopCount = 1, kLoopTicket = 5;
+constexpr int kCountThreads = 256, kCountPerThread = 4;
+
+__global__ void __launch_bounds__(256) LmSolveInitKernel(int nb, double mu0, double* __restrict__ mu, double* __restrict__ nu,
+                                                         int* __restrict__ status, int* __restrict__ iterations, int* __restrict__ loop,
+                                                         int max_iters, cudaGraphConditionalHandle cond) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b < nb) { mu[b] = mu0; nu[b] = 2.0; status[b] = kLmRunning; iterations[b] = 0; }
+  if (b == 0) {
+    for (int k = 0; k < kLoopInts; ++k) loop[k] = 0;
+    cudaGraphSetConditional(cond, max_iters > 0 ? 1u : 0u);
+  }
+}
+
+// Instances per status, one CTA per chunk of kCountThreads * kCountPerThread instances: integer counts per CTA, added up with
+// integer atomics (exact, so the result does not depend on the order of the CTAs); the last CTA to finish reads the totals.
+// loop_step: the last kernel of the loop body — loop[kLoopIter] += 1 and the WHILE condition becomes "an instance is RUNNING
+// and the budget is not spent".  Otherwise (after the tail): the counts and the loop's iterations go to the caller's
+// status_counts[4] / loop_count[1] when given.
+__global__ void __launch_bounds__(kCountThreads) LmCountKernel(int nb, const int* __restrict__ status, int* __restrict__ loop, int max_iters,
+                                                               cudaGraphConditionalHandle cond, bool loop_step, int* __restrict__ status_counts,
+                                                               int* __restrict__ loop_count) {
+  __shared__ int part[kCountThreads / 32][4];
+  __shared__ bool last;
+  int c[4] = {0, 0, 0, 0};
+  const int b0 = blockIdx.x * kCountThreads * kCountPerThread;
+  for (int k = 0; k < kCountPerThread; ++k) {
+    const int b = b0 + k * kCountThreads + threadIdx.x;
+    if (b < nb) {
+      const int s = status[b];
+      for (int q = 0; q < 4; ++q) c[q] += s == q;
+    }
+  }
+  for (int q = 0; q < 4; ++q) c[q] = __reduce_add_sync(0xffffffffu, c[q]);
+  if ((threadIdx.x & 31) == 0) for (int q = 0; q < 4; ++q) part[threadIdx.x >> 5][q] = c[q];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int q = 0; q < 4; ++q) {
+      int t = 0;
+      for (int w = 0; w < kCountThreads / 32; ++w) t += part[w][q];
+      if (t) atomicAdd(loop + kLoopCount + q, t);
+    }
+    __threadfence();
+    last = atomicAdd(loop + kLoopTicket, 1) == (int)gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!last || threadIdx.x != 0) return;
+  __threadfence();
+  int total[4];
+  for (int q = 0; q < 4; ++q) { total[q] = atomicExch(loop + kLoopCount + q, 0); }
+  loop[kLoopTicket] = 0;
+  if (loop_step) {
+    const int it = loop[kLoopIter] + 1;
+    loop[kLoopIter] = it;
+    cudaGraphSetConditional(cond, (total[kLmRunning] > 0 && it < max_iters) ? 1u : 0u);
+  } else {
+    if (status_counts) for (int q = 0; q < 4; ++q) status_counts[q] = total[q];
+    if (loop_count) *loop_count = loop[kLoopIter];
+  }
+}
+
 }  // namespace
 
 size_t LmSharedBytes(int n, int m) { return sizeof(double) * ((size_t)2 * m + 4 * (size_t)n + 32); }
@@ -308,6 +376,20 @@ int LaunchLmAccept(int n, int m, double* x, const double* x_trial, const double*
   if (nb <= 0) return 0;
   LmAcceptKernel<<<nb, 256, 0, s>>>(n, m, x, x_trial, g_trial, g_lower, g_upper, g_bound_stride, row_scale, merit, predicted, mu, nu, status,
                                     iterations, eta, mu_min, mu_max);
+  return (int)cudaGetLastError();
+}
+
+int LaunchLmSolveInit(int nb, double mu0, double* mu, double* nu, int* status, int* iterations, int* loop, int max_iters,
+                      cudaGraphConditionalHandle cond, cudaStream_t s) {
+  LmSolveInitKernel<<<(std::max(nb, 1) + 255) / 256, 256, 0, s>>>(nb, mu0, mu, nu, status, iterations, loop, max_iters, cond);
+  return (int)cudaGetLastError();
+}
+
+int LaunchLmCount(int nb, const int* status, int* loop, int max_iters, cudaGraphConditionalHandle cond, bool loop_step, int* status_counts,
+                  int* loop_count, cudaStream_t s) {
+  const int per_cta = kCountThreads * kCountPerThread;
+  LmCountKernel<<<(std::max(nb, 1) + per_cta - 1) / per_cta, kCountThreads, 0, s>>>(nb, status, loop, max_iters, cond, loop_step,
+                                                                                    status_counts, loop_count);
   return (int)cudaGetLastError();
 }
 

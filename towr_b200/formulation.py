@@ -699,6 +699,41 @@ class Batch:
                                              ptr(merit), ptr(predicted), ptr(mu), ptr(nu), ptr(solve_status), ptr(iterations),
                                              float(eta), float(mu_min), float(mu_max), C.c_void_p(stream.cuda_stream)))
 
+    def lm_solve_device(self, x, x_lower=None, x_upper=None, g_lower=None, g_upper=None, max_iters=60, tol=1e-6, mu0=1e-2, cap=0.1,
+                        cg_iters=25, eta=1e-4, mu_min=1e-12, mu_max=1e10, out=None, stream=None):
+        """twb_batch_lm_solve_device: a whole solve in one call that only enqueues — the loop of BatchedLevenbergMarquardt.solve
+        run on the device, stopping at the iteration after which no instance is RUNNING.  x (B, n) is updated in place;
+        x_lower / x_upper (B, n) and g_lower / g_upper (B, m): per-instance bounds or None (the problem's own).  Returns
+        (status, iterations, violation, mu, counts, loop_count): (B,) int32, (B,) int32, (B,) float64, (B,) float64, (4,) int32
+        instances per LM_* status and (1,) int32 loop iterations run, all CUDA tensors.  `out`: those six tensors from an
+        earlier call to write into instead; with the same tensors and arguments the call replays the batch's cached graph."""
+        import torch
+        f64, i32 = torch.float64, torch.int32
+        self._check_lm_tensors(x, ((x, f64, "n"), (x_lower, f64, "n"), (x_upper, f64, "n")), g_lower, g_upper)
+        if out is None:
+            dev = x.device
+            out = (torch.empty(self.B, dtype=i32, device=dev), torch.empty(self.B, dtype=i32, device=dev),
+                   torch.empty(self.B, dtype=f64, device=dev), torch.empty(self.B, dtype=f64, device=dev),
+                   torch.empty(4, dtype=i32, device=dev), torch.empty(1, dtype=i32, device=dev))
+        status, iterations, violation, mu, counts, loop_count = out
+        self._check_lm_tensors(x, ((status, i32, "1"), (iterations, i32, "1"), (violation, f64, "1"), (mu, f64, "1")), None, None)
+        assert counts.is_cuda and counts.dtype == i32 and counts.numel() == 4 and loop_count.is_cuda and loop_count.dtype == i32 \
+            and loop_count.numel() == 1, "bad counts / loop_count"
+        opt = capi.LmSolveOptions(float(mu0), float(cap), float(tol), float(eta), float(mu_min), float(mu_max), int(cg_iters), int(max_iters))
+        if stream is None:
+            stream = torch.cuda.current_stream(x.device)
+        ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        check(lib.twb_batch_lm_solve_device(self._h, ptr(x), ptr(x_lower), ptr(x_upper), ptr(g_lower), ptr(g_upper), C.byref(opt),
+                                            ptr(status), ptr(iterations), ptr(violation), ptr(mu), ptr(counts), ptr(loop_count),
+                                            C.c_void_p(stream.cuda_stream)))
+        return out
+
+    def lm_solve_graphs_instantiated(self):
+        """The solve graphs this batch has instantiated so far (twb_batch_lm_solve_graph_stats)."""
+        n = C.c_int()
+        check(lib.twb_batch_lm_solve_graph_stats(self._h, C.byref(n)))
+        return n.value
+
     def eval_device(self, x, g=None, jac=None, cost=None, grad=None, status=None,
                     flags=capi.EVAL_G | capi.EVAL_JAC, stream=None):
         """Device-pointer variant. Arguments are torch CUDA float64 tensors (or None);
