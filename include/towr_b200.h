@@ -361,22 +361,44 @@ int twb_batch_lm_accept_device(twb_batch* b, double* x, const double* x_trial, c
  * another stream must be ordered after the first by the caller.
  * Errors, with nothing enqueued and no output touched: NULL b / x / opt / solve_status / iterations / violation / mu, one of
  * x_lower / x_upper or of g_lower / g_upper NULL, max_iters < 0, tol < 0 or NaN, eta outside [0, 1), not
- * 0 < mu_min <= mu_max, mu0 <= 0 or NaN, cap <= 0 or NaN, cg_iters outside [0, 10000]: TWB_ERR_INVALID; a stream that is
- * being captured (a solve cannot be captured into the caller's graph), TWB_PROFILE set, or solver vectors over 200 KiB of
- * shared memory (as for twb_batch_lm_step_device): TWB_ERR_UNSUPPORTED. */
+ * 0 < mu_min <= mu_max, mu0 <= 0 or NaN, cap <= 0 or NaN, cg_iters outside [0, 10000], a step_rule other than the two
+ * below, and with TWB_LM_STEP_TRUST radius_max < cap or NaN: TWB_ERR_INVALID; a stream that is being captured (a solve
+ * cannot be captured into the caller's graph), TWB_PROFILE set, or solver vectors over 200 KiB of shared memory (as for
+ * twb_batch_lm_step_device): TWB_ERR_UNSUPPORTED.
+ *
+ * Step rules (twb_lm_solve_options.step_rule):
+ *   TWB_LM_STEP_CAP (the default): the trial step of twb_batch_lm_trial_device — the CG step scaled to max |dx| <= cap, then
+ *     projected onto the variable bounds.  radius_max is ignored.
+ *   TWB_LM_STEP_TRUST: a trust region of radius Delta[b] per instance, Delta = cap at the start.  Per trial:
+ *     free set: with gamma = Js^T s r, variable j is frozen if x_lower[j] == x_upper[j], or x_j <= x_lower[j] and
+ *       gamma_j > 0, or x_j >= x_upper[j] and gamma_j < 0 (the descent direction leaves the box); every other is free.  CG runs
+ *       on the free set only (a frozen j keeps dx_j = 0);
+ *     dx scaled to max |dx| <= Delta, then projected onto the bounds; predicted is computed from d = x_trial - x as for the cap
+ *       rule, and step_norm = max |d|.
+ *   Acceptance, rho and the mu update are those of twb_batch_lm_accept_device; after them
+ *     rho < 0.25 or rejected:                   Delta <- 0.25 step_norm
+ *     rho > 0.75 and step_norm >= 0.99 Delta:   Delta <- min(2 Delta, radius_max)
+ *     otherwise Delta is kept, and an instance whose Delta < 1e-12 max(1, max |x|) becomes TWB_LM_STALLED.
+ *   (0.25, 0.75, 2 and 0.99 are the textbook constants; they are not options.)  The batch allocates Delta and step_norm on its
+ *   first trust-region solve and frees them in twb_batch_destroy.  Each rule gets its own cached graph. */
+#define TWB_LM_STEP_CAP 0
+#define TWB_LM_STEP_TRUST 1
 typedef struct twb_lm_solve_options {
-  double mu0;      /* initial damping (> 0)                                      */
-  double cap;      /* largest step entry, as for twb_batch_lm_step_device         */
-  double tol;      /* CONVERGED when max |s r| <= tol                             */
-  double eta;      /* accept when the gain ratio rho > eta, eta in [0, 1)         */
-  double mu_min;   /* damping floor after an accepted trial                       */
-  double mu_max;   /* STALLED once a rejected trial raises mu past mu_max         */
-  int cg_iters;    /* conjugate-gradient iterations per trial                     */
-  int max_iters;   /* iteration budget (>= 0)                                     */
+  double mu0;        /* initial damping (> 0)                                      */
+  double cap;        /* largest step entry, as for twb_batch_lm_step_device; the    */
+                     /* first trust radius with TWB_LM_STEP_TRUST                   */
+  double tol;        /* CONVERGED when max |s r| <= tol                             */
+  double eta;        /* accept when the gain ratio rho > eta, eta in [0, 1)         */
+  double mu_min;     /* damping floor after an accepted trial                       */
+  double mu_max;     /* STALLED once a rejected trial raises mu past mu_max         */
+  int cg_iters;      /* conjugate-gradient iterations per trial                     */
+  int max_iters;     /* iteration budget (>= 0)                                     */
+  int step_rule;     /* TWB_LM_STEP_CAP or TWB_LM_STEP_TRUST                        */
+  double radius_max; /* largest trust radius (>= cap; TWB_LM_STEP_TRUST only)       */
 } twb_lm_solve_options;
 
 /* the defaults of BatchedLevenbergMarquardt.solve: mu0 1e-2, cap 0.1, tol 1e-6, eta 1e-4, mu_min 1e-12, mu_max 1e10,
- * cg_iters 25, max_iters 60 */
+ * cg_iters 25, max_iters 60; step_rule TWB_LM_STEP_CAP, radius_max 1e3 */
 void twb_lm_solve_options_default(twb_lm_solve_options* o);
 
 int twb_batch_lm_solve_device(twb_batch* b, double* x, const double* x_lower, const double* x_upper, const double* g_lower,
@@ -392,6 +414,11 @@ int twb_batch_lm_solve_host(twb_batch* b, double* x, const double* x_lower, cons
 
 /* For tests: the solve graphs this batch has instantiated so far (a call that reuses a cached graph adds none). */
 int twb_batch_lm_solve_graph_stats(const twb_batch* b, int* instantiations);
+
+/* For tests and diagnostics: the trust radius Delta [B] and step_norm [B] of the last trial an instance took in the loop
+ * (0 if it took none) (host arrays) of the batch's last TWB_LM_STEP_TRUST solve, copied after that solve's stream has been synchronised by the caller (the batch's own stream is
+ * synchronised here).  TWB_ERR_INVALID with NULL arguments or before the batch's first trust-region solve. */
+int twb_batch_lm_solve_radius(const twb_batch* b, double* radius, double* step_norm);
 
 /* Host-pointer variant: copies x up, evaluates, copies the requested outputs
  * back and synchronises. Pinned host memory makes the copies asynchronous. */

@@ -15,7 +15,7 @@ from ._spec import Spec
 class LmSolveOptions(C.Structure):
     """twb_lm_solve_options (include/towr_b200.h): the parameters of twb_batch_lm_solve_device."""
     _fields_ = [("mu0", C.c_double), ("cap", C.c_double), ("tol", C.c_double), ("eta", C.c_double), ("mu_min", C.c_double),
-                ("mu_max", C.c_double), ("cg_iters", C.c_int), ("max_iters", C.c_int)]
+                ("mu_max", C.c_double), ("cg_iters", C.c_int), ("max_iters", C.c_int), ("step_rule", C.c_int), ("radius_max", C.c_double)]
 
 
 LIB_PATH = os.environ.get("TWB_LIB") or os.path.join(os.path.dirname(os.path.abspath(__file__)), "libtowr_b200.so")
@@ -66,6 +66,7 @@ def _load():
         "twb_batch_lm_solve_device": (C.c_int, [P, P, P, P, P, P, C.POINTER(LmSolveOptions), P, P, P, P, P, P, P]),
         "twb_batch_lm_solve_host": (C.c_int, [P, D, D, D, D, D, C.POINTER(LmSolveOptions), I, I, D, D, I, I]),
         "twb_batch_lm_solve_graph_stats": (C.c_int, [P, I]),
+        "twb_batch_lm_solve_radius": (C.c_int, [P, D, D]),
         "twb_problem_trajectory_dims": (C.c_int, [P, C.c_double, I, I]),
         "twb_batch_sample_trajectory_host": (C.c_int, [P, P, C.c_double, P]),
         "twb_batch_initial_guess_host": (C.c_int, [P, P, P, C.c_int, P]),

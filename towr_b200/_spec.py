@@ -9,6 +9,7 @@ OK, ERR_INVALID, ERR_UNSUPPORTED, ERR_CUDA, ERR_NO_DEVICE = 0, 1, 2, 3, 4
 EVAL_G, EVAL_JAC, EVAL_COST, EVAL_ALL = 1, 2, 4, 7
 # solve status of an instance (twb_batch_lm_trial_device / twb_batch_lm_accept_device)
 LM_RUNNING, LM_CONVERGED, LM_STALLED, LM_NONFINITE = 0, 1, 2, 3
+LM_STEP_CAP, LM_STEP_TRUST = 0, 1
 
 # towr::RobotModel::Robot (robot_model.h:70-75)
 MONOPED, BIPED, HYQ, ANYMAL, GO1 = range(5)

@@ -124,6 +124,7 @@ struct twb_batch {
   struct LmWork { double *g, *jac, *x_trial, *g_trial, *row_scale, *merit, *predicted, *nu; int* loop; };
   void* lm_work_mem = nullptr;
   LmWork lm_work{};
+  double* lm_radius = nullptr;   // [2][B]: the trust radius and the last trial's max |d| (first trust-region solve)
   struct LmStage { double *x, *xl, *xu, *gl, *gu, *violation, *mu; int *status, *iterations, *counts, *loop_count; };
   void* lm_stage_mem = nullptr;
   LmStage lm_stage{};
@@ -466,7 +467,7 @@ void twb_batch_destroy(twb_batch* b) {
   for (void* p : b->owned) cudaFree(p);
   for (auto& sc : b->scratch) cudaFree(sc.first);
   for (auto& t : b->post_tables) cudaFree(t.mem);
-  cudaFree(b->lm_work_mem); cudaFree(b->lm_stage_mem);
+  cudaFree(b->lm_work_mem); cudaFree(b->lm_stage_mem); cudaFree(b->lm_radius);
   cudaFree(b->d_terrain); cudaFree(b->d_grid); cudaFree(b->d_gmap_pool); cudaFree(b->d_gmaps); cudaFree(b->d_XT); cudaFree(b->d_FS);
   for (auto ev : b->ev) if (ev) cudaEventDestroy(ev);
   if (b->aux0) cudaStreamDestroy(b->aux0);
@@ -968,14 +969,20 @@ int twb_batch_lm_accept_device(twb_batch* b, double* x, const double* x_trial, c
   if (rc != TWB_OK) return rc;
   const bool own_g = g_lower != nullptr;
   rc = twb::LaunchLmAccept(f.n, f.m, x, x_trial, g_trial, own_g ? g_lower : b->lm_pat.g_lower, own_g ? g_upper : b->lm_pat.g_upper,
-                           own_g ? (size_t)f.m : 0, row_scale, merit, predicted, mu, nu, solve_status, iterations, eta, mu_min, mu_max, b->B,
-                           static_cast<cudaStream_t>(stream));
+                           own_g ? (size_t)f.m : 0, row_scale, merit, predicted, mu, nu, solve_status, iterations, eta, mu_min, mu_max,
+                           nullptr, nullptr, 0.0, b->B, static_cast<cudaStream_t>(stream));
   if (rc != 0) return CudaFail(static_cast<cudaError_t>(rc), "solver accept launch");
   return TWB_OK;
 }
 
 void twb_lm_solve_options_default(twb_lm_solve_options* o) {
-  if (o) *o = twb_lm_solve_options{1e-2, 0.1, 1e-6, 1e-4, 1e-12, 1e10, 25, 60};
+  if (o) *o = twb_lm_solve_options{1e-2, 0.1, 1e-6, 1e-4, 1e-12, 1e10, 25, 60, TWB_LM_STEP_CAP, 1e3};
+}
+
+// the options as a graph-cache key, field by field (the struct has padding after step_rule)
+static bool SameOptions(const twb_lm_solve_options& a, const twb_lm_solve_options& b) {
+  return a.mu0 == b.mu0 && a.cap == b.cap && a.tol == b.tol && a.eta == b.eta && a.mu_min == b.mu_min && a.mu_max == b.mu_max &&
+         a.cg_iters == b.cg_iters && a.max_iters == b.max_iters && a.step_rule == b.step_rule && a.radius_max == b.radius_max;
 }
 
 // ---- twb_batch_lm_solve_device: the solve loop as one CUDA graph with a WHILE node --------------------------------------
@@ -1001,6 +1008,8 @@ static int LmSolveArgs(const twb_batch* b, const LmSolveCall& c) {
   if (!(o.eta >= 0.0 && o.eta < 1.0) || !(o.mu_min > 0.0 && o.mu_min <= o.mu_max) || !(o.mu0 > 0.0) || !(o.cap > 0.0) || o.cg_iters < 0 ||
       o.cg_iters > 10000)
     return Fail(TWB_ERR_INVALID, "bad solver parameter");
+  if (o.step_rule != TWB_LM_STEP_CAP && o.step_rule != TWB_LM_STEP_TRUST) return Fail(TWB_ERR_INVALID, "unknown step_rule");
+  if (o.step_rule == TWB_LM_STEP_TRUST && !(o.radius_max >= o.cap)) return Fail(TWB_ERR_INVALID, "radius_max < cap or NaN");
   if (g_prof_on) return Fail(TWB_ERR_UNSUPPORTED, "TWB_PROFILE records events around every kernel, which a device-side loop cannot hold");
   const twb::Formulation& f = b->prob->f;
   if (twb::LmSharedBytes(f.n, f.m) > 200 * 1024) return Fail(TWB_ERR_UNSUPPORTED, "problem too large for the shared-memory solver step");
@@ -1027,6 +1036,14 @@ static int LmWorkReady(twb_batch* b) {
   return TWB_OK;
 }
 
+// the trust-region rule's radius and step_norm [B] each, made on the first trust-region solve
+static int LmRadiusReady(twb_batch* b) {
+  if (b->lm_radius) return TWB_OK;
+  cudaError_t e = cudaMalloc(&b->lm_radius, sizeof(double) * 2 * (size_t)b->B);
+  if (e != cudaSuccess) { b->lm_radius = nullptr; return CudaFail(e, "cudaMalloc"); }
+  return TWB_OK;
+}
+
 // Captures the solve graph of `c`:
 //   init -> WHILE { eval(G|JAC at x) -> trial -> eval(G at x_trial) -> accept -> count + condition } -> eval(G|JAC at x) ->
 //   trial with cg_iters = 0 -> count into the caller's outputs
@@ -1043,12 +1060,18 @@ static cudaError_t CaptureSolveGraph(twb_batch* b, const LmSolveCall& c, cudaGra
   const double *xl = own ? c.xl : b->d_xl, *xu = own ? c.xu : b->d_xu;
   const double *gl = own_g ? c.gl : b->lm_pat.g_lower, *gu = own_g ? c.gu : b->lm_pat.g_upper;
   const size_t xs = own ? (size_t)f.n : 0, gs = own_g ? (size_t)f.m : 0;
-  const twb::LmTrialArgs trial{c.mu, o.tol, c.status, w.x_trial, w.row_scale, w.merit, w.predicted};
+  const bool trust = o.step_rule == TWB_LM_STEP_TRUST;
+  double* radius = trust ? b->lm_radius : nullptr;
+  double* step_norm = trust ? b->lm_radius + B : nullptr;
+  const twb::LmTrialArgs trial{c.mu, o.tol, c.status, w.x_trial, w.row_scale, w.merit, w.predicted, radius, step_norm};
+  // the tail only measures (cg_iters = 0: no step under either rule); the cap rule's trial there leaves step_norm as the
+  // last loop trial wrote it
+  const twb::LmTrialArgs tail{c.mu, o.tol, c.status, w.x_trial, w.row_scale, w.merit, w.predicted, nullptr, nullptr};
   auto eval = [&](const double* x, double* g, double* jac, unsigned flags) {
     return EnqueueEval(b, x, g, jac, nullptr, nullptr, nullptr, flags, s, nullptr);
   };
-  auto trial_step = [&](int cg_iters) {
-    return twb::LaunchLmStep(b->lm_pat, f.n, f.m, f.nnz, c.x, w.g, w.jac, xl, xu, xs, gl, gu, gs, 0.0, o.cap, cg_iters, c.violation, &trial, B, s);
+  auto trial_step = [&](int cg_iters, const twb::LmTrialArgs* args) {
+    return twb::LaunchLmStep(b->lm_pat, f.n, f.m, f.nnz, c.x, w.g, w.jac, xl, xu, xs, gl, gu, gs, 0.0, o.cap, cg_iters, c.violation, args, B, s);
   };
   cudaGraph_t graph = nullptr;
   cudaGraphConditionalHandle cond = 0;
@@ -1057,7 +1080,7 @@ static cudaError_t CaptureSolveGraph(twb_batch* b, const LmSolveCall& c, cudaGra
   if (e == cudaSuccess) e = cudaGraphConditionalHandleCreate(&cond, graph, 0, 0);
   if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(s, graph, nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
   if (e == cudaSuccess) {   // the start, the WHILE node after it, the tail after that
-    int rc = twb::LaunchLmSolveInit(B, o.mu0, c.mu, w.nu, c.status, c.iterations, w.loop, o.max_iters, cond, s);
+    int rc = twb::LaunchLmSolveInit(B, o.mu0, c.mu, w.nu, c.status, c.iterations, o.cap, radius, step_norm, w.loop, o.max_iters, cond, s);
     cudaStreamCaptureStatus cs;
     const cudaGraphNode_t* deps = nullptr;
     size_t n_deps = 0;
@@ -1072,7 +1095,7 @@ static cudaError_t CaptureSolveGraph(twb_batch* b, const LmSolveCall& c, cudaGra
     }
     if (rc == 0) rc = cudaStreamUpdateCaptureDependencies(s, &node, 1, cudaStreamSetCaptureDependencies);
     if (rc == 0) rc = eval(c.x, w.g, w.jac, TWB_EVAL_G | TWB_EVAL_JAC);
-    if (rc == 0) rc = trial_step(0);
+    if (rc == 0) rc = trial_step(0, &tail);
     if (rc == 0) rc = twb::LaunchLmCount(B, c.status, w.loop, o.max_iters, cond, false, c.counts, c.loop_count, s);
     cudaGraph_t captured = nullptr;
     e = cudaStreamEndCapture(s, &captured);
@@ -1081,11 +1104,11 @@ static cudaError_t CaptureSolveGraph(twb_batch* b, const LmSolveCall& c, cudaGra
   if (e == cudaSuccess) e = cudaStreamBeginCaptureToGraph(s, loop.conditional.phGraph_out[0], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
   if (e == cudaSuccess) {   // the body
     int rc = eval(c.x, w.g, w.jac, TWB_EVAL_G | TWB_EVAL_JAC);
-    if (rc == 0) rc = trial_step(o.cg_iters);
+    if (rc == 0) rc = trial_step(o.cg_iters, &trial);
     if (rc == 0) rc = eval(w.x_trial, w.g_trial, nullptr, TWB_EVAL_G);
     if (rc == 0)
       rc = twb::LaunchLmAccept(f.n, f.m, c.x, w.x_trial, w.g_trial, gl, gu, gs, w.row_scale, w.merit, w.predicted, c.mu, w.nu, c.status,
-                               c.iterations, o.eta, o.mu_min, o.mu_max, B, s);
+                               c.iterations, o.eta, o.mu_min, o.mu_max, radius, step_norm, o.radius_max, B, s);
     if (rc == 0) rc = twb::LaunchLmCount(B, c.status, w.loop, o.max_iters, cond, true, nullptr, nullptr, s);
     cudaGraph_t captured = nullptr;
     e = cudaStreamEndCapture(s, &captured);
@@ -1105,7 +1128,7 @@ static int SolveGraph(twb_batch* b, const LmSolveCall& c, cudaGraphExec_t* exec)
   const void* key[11];
   c.Key(key);
   for (auto& gr : b->solve_graphs)
-    if (std::equal(key, key + 11, gr.ptr) && std::memcmp(&gr.opt, &c.opt, sizeof c.opt) == 0) {
+    if (std::equal(key, key + 11, gr.ptr) && SameOptions(gr.opt, c.opt)) {
       gr.used = ++b->graph_clock; *exec = gr.exec; return TWB_OK;
     }
   cudaGraph_t graph = nullptr;
@@ -1135,6 +1158,7 @@ static int LmSolveCore(twb_batch* b, const LmSolveCall& c, cudaStream_t stream) 
   if (cs != cudaStreamCaptureStatusNone) return Fail(TWB_ERR_UNSUPPORTED, "the stream is being captured: a solve cannot be captured into a graph");
   int rc = LmPatternReady(b);
   if (rc == TWB_OK) rc = LmWorkReady(b);
+  if (rc == TWB_OK && c.opt.step_rule == TWB_LM_STEP_TRUST) rc = LmRadiusReady(b);
   cudaGraphExec_t exec = nullptr;
   if (rc == TWB_OK) rc = SolveGraph(b, c, &exec);
   if (rc != TWB_OK) return rc;
@@ -1201,6 +1225,17 @@ int twb_batch_lm_solve_host(twb_batch* b, double* x, const double* x_lower, cons
 int twb_batch_lm_solve_graph_stats(const twb_batch* b, int* instantiations) {
   if (!b || !instantiations) return Fail(TWB_ERR_INVALID, "null argument");
   *instantiations = b->solve_instantiations;
+  return TWB_OK;
+}
+
+int twb_batch_lm_solve_radius(const twb_batch* b, double* radius, double* step_norm) {
+  if (!b || !radius || !step_norm) return Fail(TWB_ERR_INVALID, "null argument");
+  if (!b->lm_radius) return Fail(TWB_ERR_INVALID, "no trust-region solve has run on this batch");
+  cudaError_t e = cudaSetDevice(b->device);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(b->stream);
+  if (e == cudaSuccess) e = cudaMemcpy(radius, b->lm_radius, sizeof(double) * b->B, cudaMemcpyDeviceToHost);
+  if (e == cudaSuccess) e = cudaMemcpy(step_norm, b->lm_radius + b->B, sizeof(double) * b->B, cudaMemcpyDeviceToHost);
+  if (e != cudaSuccess) return CudaFail(e, "radius copy");
   return TWB_OK;
 }
 

@@ -71,6 +71,8 @@ struct LmTrialArgs {
   double* row_scale;    // [nb][m] s at x
   double* merit;        // [nb] 1/2 ||s r(g)||^2
   double* predicted;    // [nb] merit - 1/2 ||s r(g + J d)||^2, d = x_trial - x
+  double* radius;       // [nb] trust-region rule: max |dx| <= radius[b] instead of cap, CG on the free set; null: the cap rule
+  double* step_norm;    // [nb] max |d| (trust-region rule only)
 };
 // one Levenberg-Marquardt feasibility step for nb instances (CTA = instance): x[b][n] in / out, g[b][m], jac[b][nnz] in,
 // variable bounds x_lower / x_upper at b * bound_stride and constraint bounds g_lower / g_upper at b * g_bound_stride (0: the
@@ -79,16 +81,19 @@ int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const d
                  const double* x_upper, size_t bound_stride, const double* g_lower, const double* g_upper, size_t g_bound_stride, double mu,
                  double cap, int cg_iters, double* violation, const LmTrialArgs* trial, int nb, cudaStream_t s);
 // the gain-ratio decision after a trial step for nb instances (CTA = instance, kLmRunning ones only): accept x <- x_trial and
-// lower mu, or keep x and raise mu (kLmStalled past mu_max); g_trial[b][m] is g at x_trial
+// lower mu, or keep x and raise mu (kLmStalled past mu_max); g_trial[b][m] is g at x_trial.  radius non-null: the
+// trust-region update of radius[b] from rho and step_norm[b] (clamped to radius_max; kLmStalled once it collapses)
 int LaunchLmAccept(int n, int m, double* x, const double* x_trial, const double* g_trial, const double* g_lower, const double* g_upper,
                    size_t g_bound_stride, const double* row_scale, const double* merit, const double* predicted, double* mu, double* nu,
-                   int* status, int* iterations, double eta, double mu_min, double mu_max, int nb, cudaStream_t s);
+                   int* status, int* iterations, double eta, double mu_min, double mu_max, double* radius, const double* step_norm,
+                   double radius_max, int nb, cudaStream_t s);
 // the device-side solve loop (twb_batch_lm_solve_device).  loop: kLoopInts device ints of loop state (iterations run, the
 // counts being added up); cond: the WHILE node's handle in the graph these kernels are captured into.
 constexpr int kLoopInts = 6;
-// per instance mu = mu0, nu = 2, status RUNNING, iterations 0; the loop state cleared; the condition = max_iters > 0
-int LaunchLmSolveInit(int nb, double mu0, double* mu, double* nu, int* status, int* iterations, int* loop, int max_iters,
-                      cudaGraphConditionalHandle cond, cudaStream_t s);
+// per instance mu = mu0, nu = 2, status RUNNING, iterations 0 (and radius = radius0, step_norm = 0 when radius is non-null);
+// the loop state cleared; the condition = max_iters > 0
+int LaunchLmSolveInit(int nb, double mu0, double* mu, double* nu, int* status, int* iterations, double radius0, double* radius,
+                      double* step_norm, int* loop, int max_iters, cudaGraphConditionalHandle cond, cudaStream_t s);
 // instances per status.  loop_step: iterations run += 1, condition = (RUNNING > 0 && iterations run < max_iters); else
 // status_counts[4] / loop_count[1] (each may be null) receive the counts and the iterations run, the condition is not touched
 int LaunchLmCount(int nb, const int* status, int* loop, int max_iters, cudaGraphConditionalHandle cond, bool loop_step, int* status_counts,

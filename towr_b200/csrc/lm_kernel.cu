@@ -23,6 +23,13 @@
 // the instance would jump to its bounds and report a finite violation (a NaN bound would silently mean "unbounded").
 // +-Inf constraint bounds mean unbounded, like the 1e20 convention.  With lower > upper the lower bound wins (g < lo is
 // tested first).
+// The trust-region rule (LmTrialArgs::radius non-null; the one-call solve with TWB_LM_STEP_TRUST) changes the trial step in
+// two places.  Free set: gamma = Js^T rs (the column pass that forms -b); variable j is frozen when x_lower[j] == x_upper[j],
+// or x_j <= x_lower[j] with gamma_j > 0, or x_j >= x_upper[j] with gamma_j < 0 — a frozen j starts CG with res_j = pd_j = 0
+// and its column product is skipped (ap_j = 0), so dx_j stays 0 and CG runs on the free variables only.  The frozen flags of
+// a thread's columns sit in one 32-bit register (bit k: its k-th column in col_order; n <= 32 x threads, which the 200 KiB
+// vector limit implies).  Radius: the cap becomes radius[b]; the trial also writes step_norm[b] = max |x_trial - x|.
+// LmAcceptKernel then updates the radius from the gain ratio (kTr* below) and stalls an instance whose radius collapsed.
 // The solve loop on the device (twb_batch_lm_solve_device) adds two small kernels: LmSolveInitKernel starts a solve (mu, nu,
 // status, iterations per instance; the loop counter; the WHILE condition of the solve graph) and LmCountKernel counts the
 // instances per status — at the end of every loop iteration it sets the condition, after the loop it reports the counts.
@@ -36,6 +43,11 @@
 
 namespace twb {
 namespace {
+
+// the trust-region update (textbook constants): shrink to kTrShrink x step_norm when rho < kTrLow or the trial is rejected;
+// grow to min(kTrGrow x radius, radius_max) when rho > kTrHigh and step_norm >= kTrEdge x radius; stalled once
+// radius < kTrCollapse x max(1, max |x|)
+constexpr double kTrShrink = 0.25, kTrLow = 0.25, kTrHigh = 0.75, kTrGrow = 2.0, kTrEdge = 0.99, kTrCollapse = 1e-12;
 
 // sum / max over the CTA, result broadcast to every thread (fixed tree: deterministic)
 __device__ __forceinline__ double BlockSum(double v, double* scratch) {
@@ -59,12 +71,15 @@ __device__ __forceinline__ double BlockMax(double v, double* scratch) {
   return t;
 }
 
+// kTrust (with kTrial; LmTrialArgs::radius non-null): the trust-region rule, a separate instantiation so that the cap
+// rule's kernels stay as they were.  Its minimum of one CTA per SM lets ptxas use 95-115 registers: without it ptxas held
+// these kernels to 40-64 registers and spilled (the cap rule's kernels keep their unchanged launch bound).
 // kSmemJ: the scaled values Js live in shared memory (after the vectors); else they are formed on the fly from global memory.
 // Idx: the pattern's index arrays as 16-bit (n, m, nnz < 65 536: 90 KB instead of 180 KB, so that they stay in the L1 beside
 // one CTA's shared memory — with 32-bit indices every index load was an L2 round trip: 14.6 instead of 10.5 ms per step) or 32-bit.
 // thread = row (Js p) / thread = column (Js^T u): measured faster than 16 lanes per row with shuffle trees (25.4 vs 14.6 ms).
-template <bool kSmemJ, class Idx, bool kTrial>
-__global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __restrict__ col_idx, const Idx* __restrict__ slot_t,
+template <bool kSmemJ, class Idx, bool kTrial, bool kTrust>
+__global__ void __launch_bounds__(512, kTrust ? 1 : 0) LmStepKernel(LmPattern pat, const Idx* __restrict__ col_idx, const Idx* __restrict__ slot_t,
                                                     const Idx* __restrict__ row_t, int n, int m, int nnz, double* __restrict__ X,
                                                     const double* __restrict__ G, const double* __restrict__ JAC, const double* __restrict__ x_lower,
                                                     const double* __restrict__ x_upper, size_t bound_stride,
@@ -90,6 +105,7 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
       return;
     }
     mu = tr.mu[b];
+    if constexpr (kTrust) cap = tr.radius[b];
   }
   // row scales, the scaled values and the scaled violation
   double vmax = 0.0, phi = 0.0;               // phi: sum of (s r)^2 (kTrial)
@@ -146,11 +162,16 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
     }
     return acc;
   };
-  // b = -Js^T rs
+  // b = -Js^T rs; the trust-region rule freezes j (bit k of `frozen` for this thread's k-th column) and zeroes its b_j
+  uint32_t frozen = 0;
   double rr = 0.0;
-  for (int q = tid; q < n; q += nt) {
+  for (int q = tid, k = 0; q < n; q += nt, ++k) {
     const int j = __ldg(pat.col_order + q);
-    const double bj = -col_dot(j);
+    double bj = -col_dot(j);
+    if constexpr (kTrust) {
+      const double xj = X[(size_t)b * n + j], lj = x_lower[(size_t)b * bound_stride + j], uj = x_upper[(size_t)b * bound_stride + j];
+      if (lj == uj || (xj <= lj && bj < 0.0) || (xj >= uj && bj > 0.0)) { frozen |= 1u << k; bj = 0.0; }
+    }
     dx[j] = 0.0; res[j] = bj; pd[j] = bj;
     rr += bj * bj;
   }
@@ -159,9 +180,9 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
     for (int q = tid; q < m; q += nt) { const int i = __ldg(pat.row_order + q); u[i] = row_dot(i); }
     __syncthreads();
     double pap = 0.0;
-    for (int q = tid; q < n; q += nt) {   // ap = Js^T (Js p) + mu p
+    for (int q = tid, k = 0; q < n; q += nt, ++k) {   // ap = Js^T (Js p) + mu p (0 for a frozen j)
       const int j = __ldg(pat.col_order + q);
-      const double a = col_dot(j) + mu * pd[j];
+      const double a = kTrust && ((frozen >> k) & 1u) ? 0.0 : col_dot(j) + mu * pd[j];
       ap[j] = a;
       pap += pd[j] * a;
     }
@@ -190,12 +211,19 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
   const double* up = x_upper + (size_t)b * bound_stride;
   if constexpr (kTrial) {
     double* xt = tr.x_trial + (size_t)b * n;
+    double dmax = 0.0;
     for (int j = tid; j < n; j += nt) {
       const double xj = x[j], v = fmin(fmax(xj + dx[j] * scale, lo[j]), up[j]);
       xt[j] = v;
       pd[j] = v - xj;                    // d: the step after cap and projection
+      if constexpr (kTrust) dmax = fmax(dmax, fabs(pd[j]));
     }
-    __syncthreads();
+    if constexpr (kTrust) {              // (also orders the writes of pd)
+      dmax = BlockMax(dmax, scratch);
+      if (tid == 0) tr.step_norm[b] = dmax;
+    } else {
+      __syncthreads();
+    }
     double phi_lin = 0.0;                // sum of (s r(g + J d))^2, J d = (Js d) / s
     for (int q = tid; q < m; q += nt) {
       const int i = __ldg(pat.row_order + q);
@@ -217,14 +245,14 @@ __global__ void __launch_bounds__(512) LmStepKernel(LmPattern pat, const Idx* __
   if (tid == 0 && violation) violation[b] = finite ? vmax : CUDART_NAN;
 }
 
-template <bool kSmemJ, class Idx, bool kTrial>
+template <bool kSmemJ, class Idx, bool kTrial, bool kTrust>
 int LaunchLmKernel(const LmPattern& pat, const Idx* col_idx, const Idx* slot_t, const Idx* row_t, int threads, size_t smem, int n, int m, int nnz,
                    double* x, const double* g, const double* jac, const double* xl, const double* xu, size_t bound_stride, const double* gl,
                    const double* gu, size_t g_bound_stride, double mu, double cap, int cg_iters, double* violation, const LmTrialArgs& tr, int nb,
                    cudaStream_t s) {
-  cudaError_t e = cudaFuncSetAttribute(LmStepKernel<kSmemJ, Idx, kTrial>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(LmStepKernel<kSmemJ, Idx, kTrial, kTrust>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  LmStepKernel<kSmemJ, Idx, kTrial><<<nb, threads, smem, s>>>(pat, col_idx, slot_t, row_t, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
+  LmStepKernel<kSmemJ, Idx, kTrial, kTrust><<<nb, threads, smem, s>>>(pat, col_idx, slot_t, row_t, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
                                                               g_bound_stride, mu, cap, cg_iters, violation, tr);
   return (int)cudaGetLastError();
 }
@@ -233,10 +261,13 @@ template <bool kSmemJ, class Idx>
 int LaunchLm(const LmPattern& pat, const Idx* col_idx, const Idx* slot_t, const Idx* row_t, int threads, size_t smem, int n, int m, int nnz, double* x,
              const double* g, const double* jac, const double* xl, const double* xu, size_t bound_stride, const double* gl, const double* gu,
              size_t g_bound_stride, double mu, double cap, int cg_iters, double* violation, const LmTrialArgs* trial, int nb, cudaStream_t s) {
+  if (trial && trial->radius)
+    return LaunchLmKernel<kSmemJ, Idx, true, true>(pat, col_idx, slot_t, row_t, threads, smem, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
+                                                   g_bound_stride, mu, cap, cg_iters, violation, *trial, nb, s);
   if (trial)
-    return LaunchLmKernel<kSmemJ, Idx, true>(pat, col_idx, slot_t, row_t, threads, smem, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
+    return LaunchLmKernel<kSmemJ, Idx, true, false>(pat, col_idx, slot_t, row_t, threads, smem, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
                                              g_bound_stride, mu, cap, cg_iters, violation, *trial, nb, s);
-  return LaunchLmKernel<kSmemJ, Idx, false>(pat, col_idx, slot_t, row_t, threads, smem, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
+  return LaunchLmKernel<kSmemJ, Idx, false, false>(pat, col_idx, slot_t, row_t, threads, smem, n, m, nnz, x, g, jac, xl, xu, bound_stride, gl, gu,
                                             g_bound_stride, mu, cap, cg_iters, violation, LmTrialArgs{}, nb, s);
 }
 
@@ -249,7 +280,8 @@ __global__ void __launch_bounds__(256) LmAcceptKernel(int n, int m, double* __re
                                                       const double* __restrict__ row_scale, const double* __restrict__ merit,
                                                       const double* __restrict__ predicted, double* __restrict__ mu, double* __restrict__ nu,
                                                       int* __restrict__ status, int* __restrict__ iterations, double eta, double mu_min,
-                                                      double mu_max) {
+                                                      double mu_max, double* __restrict__ radius, const double* __restrict__ step_norm,
+                                                      double radius_max) {
   __shared__ double scratch[32];
   const int b = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
   if (status[b] != kLmRunning) return;
@@ -271,6 +303,12 @@ __global__ void __launch_bounds__(256) LmAcceptKernel(int n, int m, double* __re
   const bool accept = pred > 0.0 && finite && rho > eta;
   if (accept)
     for (int j = tid; j < n; j += nt) X[(size_t)b * n + j] = x_trial[(size_t)b * n + j];
+  double xmax = 0.0;                     // max |x| after the decision (the trust-region rule's collapse test)
+  if (radius) {
+    const double* __restrict__ xn = (accept ? x_trial : X) + (size_t)b * n;
+    for (int j = tid; j < n; j += nt) xmax = fmax(xmax, fabs(xn[j]));
+    xmax = BlockMax(xmax, scratch);
+  }
   if (tid == 0) {
     if (accept) {                        // mu <- max(mu_min, mu max(1/3, 1 - (2 rho - 1)^3)), nu <- 2
       const double t = 2.0 * rho - 1.0;
@@ -281,6 +319,14 @@ __global__ void __launch_bounds__(256) LmAcceptKernel(int n, int m, double* __re
       mu[b] = mu_new;
       nu[b] = 2.0 * nu[b];
       if (mu_new > mu_max) status[b] = kLmStalled;
+    }
+    if (radius) {
+      const double sn = step_norm[b];
+      double r = radius[b];
+      if (!accept || rho < kTrLow) r = kTrShrink * sn;
+      else if (rho > kTrHigh && sn >= kTrEdge * r) r = fmin(kTrGrow * r, radius_max);
+      radius[b] = r;
+      if (r < kTrCollapse * fmax(1.0, xmax)) status[b] = kLmStalled;
     }
     iterations[b] += 1;
   }
@@ -293,10 +339,15 @@ constexpr int kLoopIter = 0, kLoopCount = 1, kLoopTicket = 5;
 constexpr int kCountThreads = 256, kCountPerThread = 4;
 
 __global__ void __launch_bounds__(256) LmSolveInitKernel(int nb, double mu0, double* __restrict__ mu, double* __restrict__ nu,
-                                                         int* __restrict__ status, int* __restrict__ iterations, int* __restrict__ loop,
-                                                         int max_iters, cudaGraphConditionalHandle cond) {
+                                                         int* __restrict__ status, int* __restrict__ iterations, double radius0,
+                                                         double* __restrict__ radius, double* __restrict__ step_norm,
+                                                         int* __restrict__ loop, int max_iters,
+                                                         cudaGraphConditionalHandle cond) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
-  if (b < nb) { mu[b] = mu0; nu[b] = 2.0; status[b] = kLmRunning; iterations[b] = 0; }
+  if (b < nb) {
+    mu[b] = mu0; nu[b] = 2.0; status[b] = kLmRunning; iterations[b] = 0;
+    if (radius) { radius[b] = radius0; step_norm[b] = 0.0; }
+  }
   if (b == 0) {
     for (int k = 0; k < kLoopInts; ++k) loop[k] = 0;
     cudaGraphSetConditional(cond, max_iters > 0 ? 1u : 0u);
@@ -361,6 +412,7 @@ int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const d
   const size_t vec = LmSharedBytes(n, m), with_j = vec + sizeof(double) * (size_t)nnz;
   const bool smem_j = with_j <= 220 * 1024;   // the scaled values fit beside the vectors: one CTA of 512 threads per SM
   const int threads = smem_j ? 512 : 256;
+  if (trial && trial->radius && n > 32 * threads) return (int)cudaErrorInvalidValue;   // one frozen bit per column and thread
   const size_t smem = smem_j ? with_j : vec;
   if (pat.col_idx16) {
     return smem_j ? LaunchLm<true>(pat, pat.col_idx16, pat.slot_t16, pat.row_t16, threads, smem, n, m, nnz, x, g, jac, x_lower, x_upper, bound_stride, g_lower, g_upper, g_bound_stride, mu, cap, cg_iters, violation, trial, nb, s)
@@ -372,16 +424,18 @@ int LaunchLmStep(const LmPattern& pat, int n, int m, int nnz, double* x, const d
 
 int LaunchLmAccept(int n, int m, double* x, const double* x_trial, const double* g_trial, const double* g_lower, const double* g_upper,
                    size_t g_bound_stride, const double* row_scale, const double* merit, const double* predicted, double* mu, double* nu,
-                   int* status, int* iterations, double eta, double mu_min, double mu_max, int nb, cudaStream_t s) {
+                   int* status, int* iterations, double eta, double mu_min, double mu_max, double* radius, const double* step_norm,
+                   double radius_max, int nb, cudaStream_t s) {
   if (nb <= 0) return 0;
   LmAcceptKernel<<<nb, 256, 0, s>>>(n, m, x, x_trial, g_trial, g_lower, g_upper, g_bound_stride, row_scale, merit, predicted, mu, nu, status,
-                                    iterations, eta, mu_min, mu_max);
+                                    iterations, eta, mu_min, mu_max, radius, step_norm, radius_max);
   return (int)cudaGetLastError();
 }
 
-int LaunchLmSolveInit(int nb, double mu0, double* mu, double* nu, int* status, int* iterations, int* loop, int max_iters,
-                      cudaGraphConditionalHandle cond, cudaStream_t s) {
-  LmSolveInitKernel<<<(std::max(nb, 1) + 255) / 256, 256, 0, s>>>(nb, mu0, mu, nu, status, iterations, loop, max_iters, cond);
+int LaunchLmSolveInit(int nb, double mu0, double* mu, double* nu, int* status, int* iterations, double radius0, double* radius,
+                      double* step_norm, int* loop, int max_iters, cudaGraphConditionalHandle cond, cudaStream_t s) {
+  LmSolveInitKernel<<<(std::max(nb, 1) + 255) / 256, 256, 0, s>>>(nb, mu0, mu, nu, status, iterations, radius0, radius, step_norm, loop,
+                                                                  max_iters, cond);
   return (int)cudaGetLastError();
 }
 

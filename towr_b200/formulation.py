@@ -700,13 +700,15 @@ class Batch:
                                              float(eta), float(mu_min), float(mu_max), C.c_void_p(stream.cuda_stream)))
 
     def lm_solve_device(self, x, x_lower=None, x_upper=None, g_lower=None, g_upper=None, max_iters=60, tol=1e-6, mu0=1e-2, cap=0.1,
-                        cg_iters=25, eta=1e-4, mu_min=1e-12, mu_max=1e10, out=None, stream=None):
+                        cg_iters=25, eta=1e-4, mu_min=1e-12, mu_max=1e10, step_rule="cap", radius_max=1e3, out=None, stream=None):
         """twb_batch_lm_solve_device: a whole solve in one call that only enqueues — the loop of BatchedLevenbergMarquardt.solve
         run on the device, stopping at the iteration after which no instance is RUNNING.  x (B, n) is updated in place;
         x_lower / x_upper (B, n) and g_lower / g_upper (B, m): per-instance bounds or None (the problem's own).  Returns
         (status, iterations, violation, mu, counts, loop_count): (B,) int32, (B,) int32, (B,) float64, (B,) float64, (4,) int32
         instances per LM_* status and (1,) int32 loop iterations run, all CUDA tensors.  `out`: those six tensors from an
-        earlier call to write into instead; with the same tensors and arguments the call replays the batch's cached graph."""
+        earlier call to write into instead; with the same tensors and arguments the call replays the batch's cached graph.
+        step_rule: "cap" (max |dx| <= cap, then clipped to the bounds) or "trust" (a trust radius per instance that starts at
+        cap, adapts to the gain ratio up to radius_max, with CG on the variables not held at a bound; include/towr_b200.h)."""
         import torch
         f64, i32 = torch.float64, torch.int32
         self._check_lm_tensors(x, ((x, f64, "n"), (x_lower, f64, "n"), (x_upper, f64, "n")), g_lower, g_upper)
@@ -719,7 +721,10 @@ class Batch:
         self._check_lm_tensors(x, ((status, i32, "1"), (iterations, i32, "1"), (violation, f64, "1"), (mu, f64, "1")), None, None)
         assert counts.is_cuda and counts.dtype == i32 and counts.numel() == 4 and loop_count.is_cuda and loop_count.dtype == i32 \
             and loop_count.numel() == 1, "bad counts / loop_count"
-        opt = capi.LmSolveOptions(float(mu0), float(cap), float(tol), float(eta), float(mu_min), float(mu_max), int(cg_iters), int(max_iters))
+        rules = {"cap": capi.LM_STEP_CAP, "trust": capi.LM_STEP_TRUST}
+        assert step_rule in rules, f"step_rule must be one of {sorted(rules)}"
+        opt = capi.LmSolveOptions(float(mu0), float(cap), float(tol), float(eta), float(mu_min), float(mu_max), int(cg_iters), int(max_iters),
+                                  rules[step_rule], float(radius_max))
         if stream is None:
             stream = torch.cuda.current_stream(x.device)
         ptr = lambda t: None if t is None else C.c_void_p(t.data_ptr())
@@ -727,6 +732,14 @@ class Batch:
                                             ptr(status), ptr(iterations), ptr(violation), ptr(mu), ptr(counts), ptr(loop_count),
                                             C.c_void_p(stream.cuda_stream)))
         return out
+
+    def lm_solve_radius(self):
+        """(radius, step_norm) as (B,) float64 numpy arrays after the batch's last trust-region solve, whose stream the caller
+        has synchronised (twb_batch_lm_solve_radius)."""
+        radius, step_norm = np.empty(self.B), np.empty(self.B)
+        check(lib.twb_batch_lm_solve_radius(self._h, radius.ctypes.data_as(C.POINTER(C.c_double)),
+                                            step_norm.ctypes.data_as(C.POINTER(C.c_double))))
+        return radius, step_norm
 
     def lm_solve_graphs_instantiated(self):
         """The solve graphs this batch has instantiated so far (twb_batch_lm_solve_graph_stats)."""
